@@ -48,6 +48,7 @@ sherlock_lines, host_corpus, device_corpus = C.sherlock_lines, C.host_corpus, C.
 # ncu --set full, scan_rev_fast<1> on 1 GiB of this corpus (profiles/): dram bytes read + written per haystack byte
 TRAFFIC_PER_BYTE = (1.779481e9 + 0.225388e9) / (1 << 30)  # profiles/r02_ncu_summaries.md section 1b
 METRIC = "haystack GB/s scanned (find_iter, bit-exact spans)"
+DUMP_SPANS = 1 << 21  # --dump-outputs: at most 2 Mi spans x (start, end, index) x 8 B = 48 MiB in all
 
 
 def parse_args():
@@ -65,7 +66,14 @@ def parse_args():
     ap.add_argument("--seg", type=int, default=0, help="scan segment bytes (0 = automatic)")
     ap.add_argument("--no-fuse", action="store_true")
     ap.add_argument("--no-tensor-tma", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed to DIR/<name>.npy (float64), to compare two "
+                         "builds on the same inputs: match_counts [this rank's matches, matches on earlier ranks, matches on all "
+                         "ranks]; the GPU search adds spans [k, 2] (all, or a fixed, seeded sample) and span_index [k]")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 # ------------------------------------------------------------------ clocks ----
@@ -158,7 +166,7 @@ def run_reference(args):
     else:
         host = torch.frombuffer(bytearray(host_corpus(n)), dtype=torch.uint8)
         how = "host generator (no GPU visible)"
-    steps = max(1, min(args.steps, 5))
+    steps = args.steps
     gbs, dt, count = cpu_reference_ptr(args.pattern, host.data_ptr(), n, threads, steps, min(args.warmup, 1))
     line = {
         "impl": "reference", "metric": METRIC, "value": round(gbs, 4),
@@ -172,6 +180,8 @@ def run_reference(args):
                                    f"(DfaSuffix where the reference selects it, exec.rs:1176-1210); matches={count}"},
         "e2e": {"value": round(gbs, 4), "unit": "GB/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
     }
+    if args.dump_outputs:  # one process scans the whole shard: it is rank 0 of a world of one
+        save_outputs(args.dump_outputs, {"match_counts": [count, 0, count]})
     print(json.dumps(line), flush=True)
 
 
@@ -283,6 +293,10 @@ def run_ours(args):
         wall = time.perf_counter() - t0
     launches = R.kernel_launches() - launches0
     assert got == n_local
+    if args.dump_outputs:  # what the last timed step returned; with N > 1 every rank adds _rank<r> to the names
+        idx, sample = span_sample(engine.spans, got, geom.buf_lo, world)
+        sfx = f"_rank{rank}" if world > 1 else ""
+        save_outputs(args.dump_outputs, {f"match_counts{sfx}": [got, offset, grand_total], f"spans{sfx}": sample, f"span_index{sfx}": idx})
     dev_s = e0.elapsed_time(e1) / 1e3
     t = torch.tensor([dev_s, wall], dtype=torch.float64, device=dev)
     if world > 1:
@@ -419,7 +433,7 @@ def run_ours(args):
         for _ in range(2):
             e2e_once()
         barrier()
-        k = max(1, min(args.steps, 3))
+        k = args.steps
         t0 = time.perf_counter()
         for _ in range(k):
             got_e2e = e2e_once()
@@ -458,6 +472,28 @@ def run_ours(args):
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
+
+
+def span_sample(spans, n_spans, pos_shift, world):
+    """The spans --dump-outputs writes: all of them, or when there are more than DUMP_SPANS / world a
+    fixed, seeded sample.  Returns their indices among this rank's spans and their [k, 2] start/end byte
+    offsets in the whole haystack."""
+    import numpy as np
+    import torch
+    k = DUMP_SPANS // world
+    if n_spans <= k:
+        idx = np.arange(n_spans, dtype=np.int64)
+    else:
+        idx = np.unique(np.random.Generator(np.random.PCG64(SEED)).integers(0, n_spans, size=k))
+    return idx, (spans[torch.from_numpy(idx).to(spans.device)] + pos_shift).cpu().numpy()
+
+
+def save_outputs(out_dir, arrays):
+    """--dump-outputs: DIR/<name>.npy for every array, float64 throughout (exact for offsets below 2**53)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.asarray(a, dtype=np.float64))
 
 
 def rg_leg(pattern, host, n, re_, text, geom):

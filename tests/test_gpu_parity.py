@@ -409,25 +409,50 @@ def test_sharded_search_matches_whole_haystack(world):
 
 
 # -------------------------------------------------- the reference's own C test ----
-def test_reference_ctest_binary():
-    """regex-capi/ctest/test.c, compiled unchanged against include/rure.h and linked to
-    librure_b200.so by __graft_entry__.build() (needs the reference tree, so the binary is
-    prebuilt).  All twelve tests must pass, the three that read capture groups included."""
+CTEST_CASES = {"test_is_match", "test_shortest_match", "test_find", "test_captures", "test_iter", "test_iter_capture_names", "test_flags",
+               "test_compile_error", "test_compile_error_size_limit", "test_regex_set_match", "test_regex_set_options",
+               "test_regex_set_match_start"}
+
+
+def _build_c_program(src, exe, flags):
     import subprocess
-    exe = os.path.join(os.path.dirname(os.path.abspath(__file__)), "_ref", "ctest")
-    if not os.path.exists(exe):
-        pytest.skip("tests/_ref/ctest not built (reference tree absent at build time)")
-    r = subprocess.run([exe], capture_output=True, text=True, timeout=300)
-    lines = [l for l in r.stderr.splitlines() if l.startswith(("PASSED", "FAILED"))]
-    failed = {l.split(": ")[1] for l in lines if l.startswith("FAILED")}
-    passed = {l.split(": ")[1] for l in lines if l.startswith("PASSED")}
-    assert not failed, (failed, r.stderr[-2000:])
-    assert passed >= {"test_is_match", "test_shortest_match", "test_find", "test_captures", "test_iter", "test_iter_capture_names",
-                      "test_flags", "test_compile_error", "test_compile_error_size_limit", "test_regex_set_match",
-                      "test_regex_set_options", "test_regex_set_match_start"}, (passed, r.stderr[-2000:])
-    # the iterator example (group 0 path) must run to completion over sherlock.txt
-    it = subprocess.run([os.path.join(os.path.dirname(exe), "iter_example")], capture_output=True, text=True, timeout=120, cwd=GOLDEN)
-    assert it.returncode == 0, it.stderr[-500:]
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    lib_dir = os.path.join(root, "regex_b200")
+    subprocess.check_call(["gcc", *flags, src, "-I" + os.path.join(root, "include"), "-L" + lib_dir, "-lrure_b200",
+                           "-Wl,-rpath," + lib_dir, "-o", exe])
+    return exe
+
+
+def test_reference_ctest_binary(tmp_path):
+    """The reference's C API test and iterator example (regex-capi/ctest/test.c and
+    examples/iter.c, restated in tests/capi/), compiled against include/rure.h as strict ANSI C
+    with warnings as errors and linked to librure_b200.so.  All twelve tests must pass,
+    the three that read capture groups included; the example must find what the oracle finds.
+    With REGEX_CAPI_DIR naming a checkout of the reference's regex-capi directory, its own two
+    files are compiled unchanged and run as well."""
+    import subprocess
+    here = os.path.dirname(os.path.abspath(__file__))
+    strict = ["-ansi", "-Wall", "-Werror"]
+    sources = [("restated", os.path.join(here, "capi", "ctest.c"), os.path.join(here, "capi", "iter.c"), ["-DDEBUG", *strict], strict)]
+    upstream = os.environ.get("REGEX_CAPI_DIR")
+    if upstream:
+        sources.append(("upstream", os.path.join(upstream, "ctest", "test.c"), os.path.join(upstream, "examples", "iter.c"), ["-DDEBUG"], []))
+    for kind, test_c, iter_c, test_flags, iter_flags in sources:
+        exe = _build_c_program(test_c, str(tmp_path / f"ctest_{kind}"), test_flags)
+        r = subprocess.run([exe], capture_output=True, text=True, timeout=300)
+        lines = [l for l in r.stderr.splitlines() if l.startswith(("PASSED", "FAILED"))]
+        failed = {l.split(": ")[1] for l in lines if l.startswith("FAILED")}
+        passed = {l.split(": ")[1] for l in lines if l.startswith("PASSED")}
+        assert not failed, (kind, failed, r.stderr[-2000:])
+        assert passed >= CTEST_CASES, (kind, passed, r.stderr[-2000:])
+        # the iterator example (captures iterator) must run to completion over sherlock.txt
+        exe = _build_c_program(iter_c, str(tmp_path / f"iter_{kind}"), iter_flags)
+        it = subprocess.run([exe], capture_output=True, text=True, timeout=120, cwd=GOLDEN)
+        assert it.returncode == 0, (kind, it.stderr[-500:])
+        if kind == "restated":
+            exp = O.OracleRegex(r"(?i)(\w+)\s+Holmes").find_iter(sherlock_text())
+            got = [tuple(int(v) for v in l.split(":")[0].split()[-1].split("..")) for l in it.stdout.splitlines() if l.startswith("match at")]
+            assert got == exp and it.stdout.splitlines()[-1] == f"{len(exp)} matches"
 
 
 @pytest.mark.gpu

@@ -11,8 +11,9 @@ without matches must hand on the restart point it RECEIVED, not the one it assum
 position); (2) is a "last chunk with matches" prefix propagation over runs of empty chunks and is
 what the remaining ~10 % are.  Patterns without look-arounds are unaffected
 (tests/test_stitch_trim_sim.py, shard fuzz)."""
-import sys, time
-sys.path.insert(0,'/root/repo'); sys.path.insert(0,'/root/repo/tests')
+import os, sys, time
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, 'tests'))
 import numpy as np
 import regex_b200 as R
 from dfa_sim import Sim

@@ -1,5 +1,6 @@
-import sys, numpy as np
-sys.path.insert(0,'/root/repo'); sys.path.insert(0,'/root/repo/tools')
+import os, sys, numpy as np
+ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
+sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, 'tools'))
 import regex_b200 as R, corpus as C
 SEG=3584; L=32
 text = np.frombuffer(bytes(C.host_corpus(SEG*L*4)), dtype=np.uint8)

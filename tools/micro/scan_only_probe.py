@@ -1,5 +1,6 @@
-import sys
-sys.path.insert(0,'/root/repo'); sys.path.insert(0,'/root/repo/tools')
+import os, sys
+ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
+sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, 'tools'))
 import torch, corpus as C, regex_b200 as R
 dev=torch.device("cuda",0)
 text=C.device_corpus(1<<30, C.SEED, dev)
