@@ -8,6 +8,8 @@
  *   rure_b200_is_match_batch  == rure_is_match(re, hay + off[i], off[i+1]-off[i], 0) per record
  *   rure_b200_find_batch      == rure_find(...)  per record (offsets relative to the record)
  *   rure_b200_set_matches_*   == rure_set_matches(...) packed into 64-bit masks
+ *   rure_b200_find_iter_batch == collecting rure_iter_next over each record (record-relative offsets)
+ *   rure_b200_captures_batch  == rure_find_captures(re, hay + off[i], off[i+1]-off[i], 0, ...) per record
  * Functions return true on success; on failure rure_b200_last_error() (thread
  * local) describes what went wrong.  A missing GPU is a failure, never a
  * silent CPU fallback.
@@ -102,6 +104,17 @@ bool rure_b200_find_batch(rure *re, const uint8_t *haystack, const uint64_t *off
                           size_t n_records, rure_match *out, uint8_t *found_bits);
 bool rure_b200_set_matches_batch(rure_set *set, const uint8_t *haystack, const uint64_t *offsets,
                                  size_t n_records, uint64_t *out_masks);
+/* Every match of every record.  match_offsets: n_records + 1 entries (always complete); the spans of
+ * record i are out[match_offsets[i] .. match_offsets[i+1]), record-relative; at most cap are stored,
+ * *n_total counts all.  out == NULL / cap == 0: counts and offsets only.  Str mode
+ * (rure_b200_compile_str) steps past an empty match by one UTF-8 scalar. */
+bool rure_b200_find_iter_batch(rure *re, const uint8_t *haystack, const uint64_t *offsets, size_t n_records,
+                               uint64_t *match_offsets, rure_match *out, size_t cap, size_t *n_total);
+/* The capture groups of the first match of every record.  slots: n_records * 2 * rure_b200_captures_len(re)
+ * entries, record-relative, SIZE_MAX where a group did not take part (every slot of a record without a
+ * match); found_bits as rure_b200_find_batch. */
+bool rure_b200_captures_batch(rure *re, const uint8_t *haystack, const uint64_t *offsets, size_t n_records,
+                              size_t *slots, uint8_t *found_bits);
 
 /* ---- device-resident inputs and outputs ----------------------------------- */
 bool rure_b200_find_all_device(rure *re, const uint8_t *d_haystack, size_t length, size_t start,
@@ -118,6 +131,13 @@ bool rure_b200_find_batch_device(rure *re, const uint8_t *d_haystack, const uint
 bool rure_b200_set_matches_batch_device(rure_set *set, const uint8_t *d_haystack,
                                         const uint64_t *d_offsets, size_t n_records,
                                         uint64_t *d_out_masks);
+/* as rure_b200_find_iter_batch; d_match_offsets and d_out in device memory, *n_total on the host */
+bool rure_b200_find_iter_batch_device(rure *re, const uint8_t *d_haystack, const uint64_t *d_offsets,
+                                      size_t n_records, uint64_t *d_match_offsets, rure_match *d_out,
+                                      size_t cap, size_t *n_total);
+/* as rure_b200_captures_batch; d_found_bits are 32-bit ballot words as rure_b200_find_batch_device */
+bool rure_b200_captures_batch_device(rure *re, const uint8_t *d_haystack, const uint64_t *d_offsets,
+                                     size_t n_records, size_t *d_slots, uint32_t *d_found_bits);
 
 /* ---- byte-range shards of one haystack (multi-GPU; one process per GPU) ------
  * Each rank holds [left context | owned bytes | right halo] of the haystack in its

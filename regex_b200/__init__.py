@@ -104,6 +104,8 @@ def _load():
         "rure_b200_is_match_batch": (c_bool, [vp, u8p, vp, sz, vp]),
         "rure_b200_find_batch": (c_bool, [vp, u8p, vp, sz, vp, vp]),
         "rure_b200_set_matches_batch": (c_bool, [vp, u8p, vp, sz, vp]),
+        "rure_b200_find_iter_batch": (c_bool, [vp, u8p, vp, sz, vp, vp, sz, POINTER(sz)]),
+        "rure_b200_captures_batch": (c_bool, [vp, u8p, vp, sz, vp, vp]),
         "rure_b200_find_all_device": (c_bool, [vp, vp, sz, sz, vp, sz, POINTER(sz)]),
         "rure_b200_find_all_shard_device": (c_bool, [vp, vp, sz, POINTER(_Shard), vp, sz]),
         "rure_b200_shortest_match_device": (c_bool, [vp, vp, sz, sz, POINTER(c_bool), POINTER(sz)]),
@@ -113,6 +115,8 @@ def _load():
         "rure_b200_is_match_batch_device": (c_bool, [vp, vp, vp, sz, vp]),
         "rure_b200_find_batch_device": (c_bool, [vp, vp, vp, sz, vp, vp]),
         "rure_b200_set_matches_batch_device": (c_bool, [vp, vp, vp, sz, vp]),
+        "rure_b200_find_iter_batch_device": (c_bool, [vp, vp, vp, sz, vp, vp, sz, POINTER(sz)]),
+        "rure_b200_captures_batch_device": (c_bool, [vp, vp, vp, sz, vp, vp]),
         "rure_b200_last_error": (c_char_p, []),
         "rure_b200_kernel_launches": (c_uint64, []),
         "rure_b200_last_stats": (None, [vp, POINTER(c_double)]),
@@ -401,6 +405,47 @@ class _Compiled:
             raise Error(_last_error())
         return np.unpackbits(bits, bitorder="little")[:n_rec].astype(bool), spans[:n_rec]
 
+    def find_iter_batch(self, text, offsets, cap=None):
+        """find_iter over every record: (match_offsets uint64[n+1], spans uint64[m, 2]); the spans of record i
+        are spans[match_offsets[i]:match_offsets[i+1]], relative to the record."""
+        p, n, keep = _buf(text)
+        off = np.ascontiguousarray(offsets, dtype=np.uint64)
+        n_rec = off.size - 1
+        moff = np.zeros(n_rec + 1, dtype=np.uint64)
+        total = c_size_t()
+        cap = max(4096, 2 * n_rec) if cap is None else cap
+        while True:
+            out = np.empty((max(cap, 1), 2), dtype=np.uint64)
+            if not _lib.rure_b200_find_iter_batch(self._h, p, off.ctypes.data, n_rec, moff.ctypes.data, out.ctypes.data, cap, byref(total)):
+                raise Error(_last_error())
+            if total.value <= cap:
+                return moff, out[: total.value]
+            cap = total.value
+
+    def count_batch(self, text, offsets):
+        """uint64[n]: the number of find_iter matches of every record (no spans are stored)."""
+        p, n, keep = _buf(text)
+        off = np.ascontiguousarray(offsets, dtype=np.uint64)
+        n_rec = off.size - 1
+        moff = np.zeros(n_rec + 1, dtype=np.uint64)
+        total = c_size_t()
+        if not _lib.rure_b200_find_iter_batch(self._h, p, off.ctypes.data, n_rec, moff.ctypes.data, None, 0, byref(total)):
+            raise Error(_last_error())
+        return np.diff(moff)
+
+    def captures_batch(self, text, offsets):
+        """`Regex::captures` on every record: (found bool[n], slots uint64[n, captures_len, 2]), record-relative,
+        2**64-1 where a group did not take part."""
+        p, n, keep = _buf(text)
+        off = np.ascontiguousarray(offsets, dtype=np.uint64)
+        n_rec = off.size - 1
+        g = self.captures_len()
+        bits = np.zeros((n_rec + 7) // 8 + 8, dtype=np.uint8)
+        slots = np.empty((max(n_rec, 1), g, 2), dtype=np.uint64)
+        if not _lib.rure_b200_captures_batch(self._h, p, off.ctypes.data, n_rec, slots.ctypes.data, bits.ctypes.data):
+            raise Error(_last_error())
+        return np.unpackbits(bits, bitorder="little")[:n_rec].astype(bool), slots[:n_rec]
+
     # ---- device-resident (torch CUDA tensors) --------------------------------
     def find_all_device(self, d_text, d_out=None, start=0):
         """d_text: uint8 CUDA tensor; d_out: optional (cap, 2) int64/uint64 CUDA tensor.
@@ -443,6 +488,25 @@ class _Compiled:
     def find_batch_device(self, d_text, d_offsets, d_spans, d_bits):
         n_rec = d_offsets.numel() - 1
         if not _lib.rure_b200_find_batch_device(self._h, d_text.data_ptr(), d_offsets.data_ptr(), n_rec, d_spans.data_ptr(), d_bits.data_ptr()):
+            raise Error(_last_error())
+
+    def find_iter_batch_device(self, d_text, d_offsets, d_match_offsets, d_out=None):
+        """find_iter over every record on the device.  d_match_offsets: (n_records + 1) int64/uint64 CUDA
+        tensor, always filled; d_out: optional (cap, 2) tensor for the spans (beyond cap they are counted,
+        not stored).  Returns the total number of matches."""
+        n_rec = d_offsets.numel() - 1
+        total = c_size_t()
+        cap = 0 if d_out is None else d_out.shape[0]
+        ptr = 0 if d_out is None else d_out.data_ptr()
+        if not _lib.rure_b200_find_iter_batch_device(self._h, d_text.data_ptr(), d_offsets.data_ptr(), n_rec, d_match_offsets.data_ptr(),
+                                                     ptr, cap, byref(total)):
+            raise Error(_last_error())
+        return total.value
+
+    def captures_batch_device(self, d_text, d_offsets, d_slots, d_bits):
+        """d_slots: n_records * 2 * captures_len() int64/uint64 CUDA tensor; d_bits: int32 ballot words."""
+        n_rec = d_offsets.numel() - 1
+        if not _lib.rure_b200_captures_batch_device(self._h, d_text.data_ptr(), d_offsets.data_ptr(), n_rec, d_slots.data_ptr(), d_bits.data_ptr()):
             raise Error(_last_error())
 
     # ---- diagnostics ------------------------------------------------------------

@@ -387,6 +387,27 @@ bool rure_b200_find_batch(rure* re, const uint8_t* haystack, const uint64_t* off
 bool rure_b200_set_matches_batch(rure_set* s, const uint8_t* haystack, const uint64_t* offsets, size_t n, uint64_t* out_masks) {
   return ok(s->re, s->re->set_matches_batch_host(haystack, offsets, n, out_masks));
 }
+bool rure_b200_find_iter_batch(rure* re, const uint8_t* haystack, const uint64_t* offsets, size_t n, uint64_t* match_offsets, rure_match* out,
+                               size_t cap, size_t* n_total) {
+  uint64_t total = 0;
+  const bool r = ok(re->re, re->re->find_iter_batch_host(haystack, offsets, n, match_offsets, (uint64_t*)out, out ? cap : 0, &total));
+  if (n_total) *n_total = total;
+  return r;
+}
+bool rure_b200_find_iter_batch_device(rure* re, const uint8_t* d_haystack, const uint64_t* d_offsets, size_t n, uint64_t* d_match_offsets,
+                                      rure_match* d_out, size_t cap, size_t* n_total) {
+  uint64_t total = 0;
+  const bool r = ok(re->re, re->re->find_iter_batch_device(d_haystack, d_offsets, n, d_match_offsets, (uint64_t*)d_out, d_out ? cap : 0, &total));
+  if (n_total) *n_total = total;
+  return r;
+}
+bool rure_b200_captures_batch(rure* re, const uint8_t* haystack, const uint64_t* offsets, size_t n, size_t* slots, uint8_t* found_bits) {
+  return ok(re->re, re->re->captures_batch_host(haystack, offsets, n, (uint64_t*)slots, found_bits));
+}
+bool rure_b200_captures_batch_device(rure* re, const uint8_t* d_haystack, const uint64_t* d_offsets, size_t n, size_t* d_slots,
+                                     uint32_t* d_found_bits) {
+  return ok(re->re, re->re->captures_batch_device(d_haystack, d_offsets, n, (uint64_t*)d_slots, d_found_bits));
+}
 bool rure_b200_find_all_device(rure* re, const uint8_t* d_haystack, size_t length, size_t start, rure_match* d_out, size_t cap, size_t* n_total) {
   uint64_t total = 0;
   bool r = ok(re->re, re->re->find_all_device(d_haystack, length, start, (uint64_t*)d_out, d_out ? cap : 0, &total));

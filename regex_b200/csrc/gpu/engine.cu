@@ -1458,6 +1458,96 @@ int Regex::find_batch_device(const uint8_t* d_text, const uint64_t* d_offsets, u
   return 0;
 }
 
+// find_iter per record into a CSR list: count pass, in-place exclusive scan of the counts (entry n_rec = the
+// total), write pass (kernels.cu batch_iter).
+int Regex::find_iter_batch_device(const uint8_t* d_text, const uint64_t* d_offsets, uint64_t n_rec, uint64_t* d_match_offsets,
+                                  uint64_t* d_out, uint64_t cap, uint64_t* total) {
+  std::lock_guard<std::recursive_mutex> lock(mu_);
+  *total = 0;
+  if (is_set_) return fail("find requires exactly one pattern");
+  DeviceDfa *fwd, *rev;
+  if (int rc = ensure(kFwdUnanchoredLF, &fwd)) return rc;
+  if (int rc = ensure(kRevAnchoredLongest, &rev)) return rc;
+  cudaStream_t st = (cudaStream_t)stream_;
+  if (n_rec == 0) {
+    RB_CUDA(cudaMemsetAsync(d_match_offsets, 0, 8, st));
+    RB_CUDA(cudaStreamSynchronize(st));
+    return 0;
+  }
+  BatchArgs a{};
+  a.fwd = fwd->view;
+  a.rev = rev->view;
+  a.text = d_text;
+  a.offsets = d_offsets;
+  a.n_rec = n_rec;
+  a.match_offsets = d_match_offsets;
+  a.out_spans = d_out;
+  a.cap = d_out ? cap : 0;
+  a.utf8 = only_utf8 ? 1 : 0;
+  const bool fast = fwd->hot.n && rev->hot.n && ((uintptr_t)d_text & 15) == 0 && !tuning.force_generic;
+  size_t fsm = 0;
+  uint32_t grid = (uint32_t)((n_rec + 255) / 256);
+  if (fast) {
+    a.fwd_hot = fwd->hot;
+    a.rev_hot = rev->hot;
+    a.fwd_g = (const DfaView*)fwd->view_dev;
+    a.rev_g = (const DfaView*)rev->view_dev;
+    fsm = hot_bytes(fwd->hot.n) + hot_bytes(rev->hot.n) + 256;
+    // __launch_bounds__(512, 2): two blocks per SM fit the registers of the iterator
+    const uint32_t per_sm = (uint32_t)std::max<size_t>(1, std::min<size_t>(2, (220 * 1024) / (fsm + 16384)));
+    grid = grid_for(n_rec, 512, per_sm);
+    RB_CUDA(allow_smem(batch_iter_fast<0>, fsm));
+    RB_CUDA(allow_smem(batch_iter_fast<1>, fsm));
+  }
+  // ---- count ----
+  a.fwd_only = !can_match_empty && !has_looks;
+  RB_CUDA(cudaMemsetAsync(d_match_offsets + n_rec, 0, 8, st));
+  if (fast) batch_iter_fast<0><<<grid, 512, fsm, st>>>(a);
+  else batch_iter<0><<<grid, 256, 0, st>>>(a);
+  RB_LAUNCH_CHECK("batch_iter<0>");
+  // ---- exclusive scan over n_rec + 1 entries ----
+  const uint64_t n_scan = n_rec + 1, n_blocks = (n_scan + 1023) / 1024;
+  uint64_t* block_sums = (uint64_t*)block_sums_.ensure((n_blocks + 1) * 8);
+  if (!block_sums) return fail("out of device memory (batch scan)");
+  unsigned long long* grand = (unsigned long long*)(block_sums + n_blocks);
+  scan_counts_local<<<(uint32_t)n_blocks, 1024, 0, st>>>(d_match_offsets, d_match_offsets, block_sums, n_scan);
+  RB_LAUNCH_CHECK("scan_counts_local");
+  scan_block_sums<<<1, 1024, 0, st>>>(block_sums, n_blocks, grand);
+  RB_LAUNCH_CHECK("scan_block_sums");
+  scan_add_block_offsets<<<(uint32_t)n_blocks, 1024, 0, st>>>(d_match_offsets, block_sums, n_scan);
+  RB_LAUNCH_CHECK("scan_add_block_offsets");
+  // ---- write ----
+  if (a.cap > 0) {
+    a.fwd_only = 0;
+    if (fast) batch_iter_fast<1><<<grid, 512, fsm, st>>>(a);
+    else batch_iter<1><<<grid, 256, 0, st>>>(a);
+    RB_LAUNCH_CHECK("batch_iter<1>");
+  }
+  uint64_t* h = (uint64_t*)pinned_;
+  RB_CUDA(cudaMemcpyAsync(h, grand, 8, cudaMemcpyDeviceToHost, st));
+  RB_CUDA(cudaStreamSynchronize(st));
+  *total = h[0];
+  return 0;
+}
+
+// Regex::captures per record: the first match of every record (find_batch), then the Pike VM over the
+// record-relative window of each (kernels.cu pike_captures with rec_offsets).
+int Regex::captures_batch_device(const uint8_t* d_text, const uint64_t* d_offsets, uint64_t n_rec, uint64_t* d_slots, uint32_t* d_bits) {
+  std::lock_guard<std::recursive_mutex> lock(mu_);
+  if (int rc = ensure_capture_program()) return rc;
+  if (n_rec == 0) return 0;
+  uint64_t* d_spans = (uint64_t*)cap_span_.ensure(n_rec * 16);
+  if (!d_spans) return fail("out of device memory (captures)");
+  if (int rc = find_batch_device(d_text, d_offsets, n_rec, d_spans, d_bits)) return rc;
+  if (int rc = launch_captures(d_text, 0, d_spans, n_rec, d_slots, d_offsets, d_bits)) return rc;
+  cudaStream_t st = (cudaStream_t)stream_;
+  // exec.rs:896-906: a record matches when the NFA found group 0 in its window
+  slot_found_bits<<<(uint32_t)((n_rec + 255) / 256), 256, 0, st>>>(d_slots, 2 * (uint32_t)n_groups_, n_rec, d_bits);
+  RB_LAUNCH_CHECK("slot_found_bits");
+  RB_CUDA(cudaStreamSynchronize(st));
+  return 0;
+}
+
 int Regex::set_matches_batch_device(const uint8_t* d_text, const uint64_t* d_offsets, uint64_t n_rec, uint64_t* d_masks) {
   std::lock_guard<std::recursive_mutex> lock(mu_);
   if (n_rec == 0) return 0;
@@ -1744,6 +1834,14 @@ int Regex::captures_device(const uint8_t* d_text, uint64_t n, const uint64_t* d_
   std::lock_guard<std::recursive_mutex> lock(mu_);
   if (int rc = ensure_capture_program()) return rc;
   if (m == 0) return 0;
+  if (int rc = launch_captures(d_text, n, d_spans, m, d_slots, nullptr, nullptr)) return rc;
+  RB_CUDA(cudaStreamSynchronize((cudaStream_t)stream_));
+  return 0;
+}
+
+// pike_captures over m spans (rec_offsets / rec_found: batched records, see launch.h CapArgs)
+int Regex::launch_captures(const uint8_t* d_text, uint64_t n, const uint64_t* d_spans, uint64_t m, uint64_t* d_slots,
+                           const uint64_t* rec_offsets, const uint32_t* rec_found) {
   CapArgs a{};
   a.insts = (const NfaInst*)cap_insts_.ptr;
   a.n_insts = cap_n_insts_;
@@ -1763,9 +1861,10 @@ int Regex::captures_device(const uint8_t* d_text, uint64_t n, const uint64_t* d_
   while (threads > 64 && threads * a.per_thread > (1ull << 30)) threads /= 2;
   a.scratch = (uint8_t*)cap_scratch_.ensure(threads * a.per_thread);
   if (!a.scratch) return fail("out of device memory (capture scratch)");
+  a.rec_offsets = rec_offsets;
+  a.rec_found = rec_found;
   pike_captures<<<(uint32_t)(threads / 64), 64, 0, (cudaStream_t)stream_>>>(a);
   RB_LAUNCH_CHECK("pike_captures");
-  RB_CUDA(cudaStreamSynchronize((cudaStream_t)stream_));
   return 0;
 }
 
@@ -2085,6 +2184,43 @@ int Regex::is_match_batch_host(const uint8_t* text, const uint64_t* offsets, uin
   RB_CUDA(cudaMemcpyAsync(d_off, offsets, (n_rec + 1) * 8, cudaMemcpyHostToDevice, (cudaStream_t)stream_));
   if ((rc = is_match_batch_device(d, d_off, n_rec, d_bits))) return rc;
   RB_CUDA(d2h(out_bits, d_bits, (n_rec + 7) / 8));
+  return 0;
+}
+int Regex::find_iter_batch_host(const uint8_t* text, const uint64_t* offsets, uint64_t n_rec, uint64_t* match_offsets, uint64_t* out,
+                                uint64_t cap, uint64_t* total) {
+  std::lock_guard<std::recursive_mutex> lock(mu_);
+  int rc;
+  const uint64_t n = n_rec ? offsets[n_rec] : 0;
+  const uint8_t* d = upload_text(text, n, &rc);
+  if (rc) return rc;
+  uint64_t* d_off = (uint64_t*)offsets_.ensure((n_rec + 1) * 8);
+  uint64_t* d_moff = (uint64_t*)count_.ensure((n_rec + 1) * 8);
+  if (!d_off || !d_moff) return fail("out of device memory (batch)");
+  RB_CUDA(cudaMemcpyAsync(d_off, offsets, (n_rec + 1) * 8, cudaMemcpyHostToDevice, (cudaStream_t)stream_));
+  if (!out) cap = 0;
+  uint64_t* d_spans = cap ? (uint64_t*)out_.ensure(cap * 16) : nullptr;
+  if (cap && !d_spans) return fail("out of device memory (batch spans)");
+  if ((rc = find_iter_batch_device(d, d_off, n_rec, d_moff, d_spans, cap, total))) return rc;
+  const uint64_t k = std::min(cap, *total);
+  if (k) RB_CUDA(d2h(out, d_spans, k * 16));
+  RB_CUDA(d2h(match_offsets, d_moff, (n_rec + 1) * 8));
+  return 0;
+}
+int Regex::captures_batch_host(const uint8_t* text, const uint64_t* offsets, uint64_t n_rec, uint64_t* slots, uint8_t* out_bits) {
+  std::lock_guard<std::recursive_mutex> lock(mu_);
+  int rc;
+  const uint64_t n = n_rec ? offsets[n_rec] : 0;
+  const uint8_t* d = upload_text(text, n, &rc);
+  if (rc) return rc;
+  const uint64_t ns = 2 * (uint64_t)n_groups_;
+  uint64_t* d_off = (uint64_t*)offsets_.ensure((n_rec + 1) * 8);
+  uint32_t* d_bits = (uint32_t*)bits_.ensure((n_rec + 31) / 32 * 4 + 4);
+  uint64_t* d_slots = (uint64_t*)cap_slots_.ensure(std::max<uint64_t>(n_rec, 1) * ns * 8);
+  if (!d_off || !d_bits || !d_slots) return fail("out of device memory (batch)");
+  RB_CUDA(cudaMemcpyAsync(d_off, offsets, (n_rec + 1) * 8, cudaMemcpyHostToDevice, (cudaStream_t)stream_));
+  if ((rc = captures_batch_device(d, d_off, n_rec, d_slots, d_bits))) return rc;
+  RB_CUDA(d2h(out_bits, d_bits, (n_rec + 7) / 8));
+  RB_CUDA(d2h(slots, d_slots, n_rec * ns * 8));
   return 0;
 }
 int Regex::find_batch_host(const uint8_t* text, const uint64_t* offsets, uint64_t n_rec, uint64_t* spans, uint8_t* out_bits) {

@@ -137,6 +137,14 @@ class Regex {
   int is_match_batch_device(const uint8_t* d_text, const uint64_t* d_offsets, uint64_t n_rec, uint32_t* d_bits);
   int find_batch_device(const uint8_t* d_text, const uint64_t* d_offsets, uint64_t n_rec, uint64_t* d_spans, uint32_t* d_bits);
   int set_matches_batch_device(const uint8_t* d_text, const uint64_t* d_offsets, uint64_t n_rec, uint64_t* d_masks);
+  // find_iter per record (re_trait.rs:197-220, the record as the whole text): d_match_offsets[n_rec + 1] = exclusive
+  // prefix sum of the per-record counts (always complete); record r's spans (record-relative) at
+  // d_out[d_match_offsets[r] ..), at most cap stored (d_out may be null to count only); *total = all matches (host).
+  int find_iter_batch_device(const uint8_t* d_text, const uint64_t* d_offsets, uint64_t n_rec, uint64_t* d_match_offsets,
+                             uint64_t* d_out, uint64_t cap, uint64_t* total);
+  // Regex::captures per record: d_slots[n_rec][2 * n_groups] record-relative (kNone = no group); d_bits = ballot
+  // words, bit r set when record r matches
+  int captures_batch_device(const uint8_t* d_text, const uint64_t* d_offsets, uint64_t n_rec, uint64_t* d_slots, uint32_t* d_bits);
 
   // ---- host-buffer wrappers (copies inside; the e2e path) ---------------------
   int find_all_host(const uint8_t* text, uint64_t n, uint64_t start, uint64_t* out, uint64_t cap, uint64_t* total);
@@ -146,6 +154,9 @@ class Regex {
   int is_match_batch_host(const uint8_t* text, const uint64_t* offsets, uint64_t n_rec, uint8_t* out_bits);
   int find_batch_host(const uint8_t* text, const uint64_t* offsets, uint64_t n_rec, uint64_t* spans, uint8_t* out_bits);
   int set_matches_batch_host(const uint8_t* text, const uint64_t* offsets, uint64_t n_rec, uint64_t* masks);
+  int find_iter_batch_host(const uint8_t* text, const uint64_t* offsets, uint64_t n_rec, uint64_t* match_offsets, uint64_t* out,
+                           uint64_t cap, uint64_t* total);
+  int captures_batch_host(const uint8_t* text, const uint64_t* offsets, uint64_t n_rec, uint64_t* slots, uint8_t* out_bits);
 
   // Run on a caller-owned CUDA stream (e.g. torch's current stream) instead of the private one.
   void set_stream(void* cuda_stream) { ext_stream_ = cuda_stream; use_ext_stream_ = true; }
@@ -173,6 +184,8 @@ class Regex {
   int resolve_long_run(const uint8_t* d_text, uint64_t n, uint64_t s, bool text_continues, uint64_t* e_out);
   int all_spans_device(const uint8_t* d_text, uint64_t n, uint64_t** d_spans, uint64_t* m);
   int ensure_capture_program();
+  int launch_captures(const uint8_t* d_text, uint64_t n, const uint64_t* d_spans, uint64_t m, uint64_t* d_slots,
+                      const uint64_t* rec_offsets, const uint32_t* rec_found);
   int replace_prepare(const uint8_t* d_text, uint64_t n, const uint8_t* rep, uint64_t rep_len, bool expand, uint64_t limit, uint64_t* out_len);
   int replace_emit(uint8_t* d_out, uint64_t out_cap);
   bool plan_prefilter();  // fills pf_words_ (launch.h PfArgs) when every match has one of <= 4 bytes at a fixed offset

@@ -2298,7 +2298,7 @@ struct PikeList {
   __device__ __forceinline__ void insert(uint32_t ip) { sparse[ip] = count; dense[count++] = ip; }
 };
 // pikevm.rs:274-352: follow the epsilon transitions from ip0 in priority order
-__device__ void pike_add(const CapArgs& a, PikeList& l, uint64_t* tc, uint32_t ip0, uint64_t n, uint64_t at, uint32_t* stk_tag, uint64_t* stk_pos) {
+__device__ void pike_add(const CapArgs& a, const uint8_t* text, PikeList& l, uint64_t* tc, uint32_t ip0, uint64_t n, uint64_t at, uint32_t* stk_tag, uint64_t* stk_pos) {
   uint32_t sp = 0;
   stk_tag[sp] = ip0; stk_pos[sp++] = 0;  // tag < 0x80000000: an instruction to visit; else: restore slot (tag & 0x7FFFFFFF) to pos
   while (sp) {
@@ -2312,7 +2312,7 @@ __device__ void pike_add(const CapArgs& a, PikeList& l, uint64_t* tc, uint32_t i
       const NfaInst in = a.insts[ip];
       const uint32_t op = in.op_look_lo_hi & 0xFF;
       if (op == 3) {         // EmptyLook
-        if (!look_holds((in.op_look_lo_hi >> 8) & 0xFF, a.text, n, at)) break;
+        if (!look_holds((in.op_look_lo_hi >> 8) & 0xFF, text, n, at)) break;
         ip = in.a;
       } else if (op == 1) {  // Save
         if (in.b < a.n_slots) {
@@ -2345,15 +2345,22 @@ __global__ void pike_captures(CapArgs a) {
   for (uint64_t m = tid; m < a.n_matches; m += n_threads) {
     const uint64_t s = a.spans[2 * m], e = a.spans[2 * m + 1];
     uint64_t* out = a.slots + m * ns;
+    for (uint32_t k = 0; k < ns; k++) { out[k] = kNone; tc[k] = kNone; }
+    const uint8_t* text = a.text;  // the text the match is relative to: the haystack, or record m
+    uint64_t tn = a.n;
+    if (a.rec_offsets) {
+      if (!((a.rec_found[m >> 5] >> (m & 31)) & 1u)) continue;
+      text = a.text + a.rec_offsets[m];
+      tn = a.rec_offsets[m + 1] - a.rec_offsets[m];
+    }
     // the window ends two characters past the match (look-ahead needs them; utf8.rs:24-40 next_utf8)
     uint64_t n = e;
     for (int r = 0; r < 2; r++) {
-      if (n >= a.n) { n = a.n; break; }
-      const uint32_t b = a.text[n];
+      if (n >= tn) { n = tn; break; }
+      const uint32_t b = text[n];
       n += b <= 0x7F ? 1 : b <= 0xDF ? 2 : b <= 0xEF ? 3 : 4;
     }
-    n = min(n, a.n);
-    for (uint32_t k = 0; k < ns; k++) { out[k] = kNone; tc[k] = kNone; }
+    n = min(n, tn);
     int cur = 0;
     L[0].count = L[1].count = 0;
     for (uint64_t i = 0; i < ni; i++) L[0].sparse[i] = L[1].sparse[i] = 0;
@@ -2366,7 +2373,7 @@ __global__ void pike_captures(CapArgs a) {
       // (pikevm.rs:172-175); its slots start out empty
       if (cl.count == 0 || (!a.anchored_start && !matched)) {
         for (uint32_t k = 0; k < ns; k++) tc[k] = kNone;
-        pike_add(a, cl, tc, a.start_ip, n, at, stk_tag, stk_pos);
+        pike_add(a, text, cl, tc, a.start_ip, n, at, stk_tag, stk_pos);
       }
       for (uint32_t i = 0; i < cl.count; i++) {
         const uint32_t ip = cl.dense[i];
@@ -2378,10 +2385,10 @@ __global__ void pike_captures(CapArgs a) {
           break;
         }
         if (op == 4 && at < n) {  // Bytes
-          const uint32_t b = a.text[at];
+          const uint32_t b = text[at];
           if (((in.op_look_lo_hi >> 16) & 0xFF) <= b && b <= (in.op_look_lo_hi >> 24)) {
             for (uint32_t k = 0; k < ns; k++) tc[k] = cl.caps[(uint64_t)ip * ns + k];
-            pike_add(a, nl, tc, in.a, n, at + 1, stk_tag, stk_pos);
+            pike_add(a, text, nl, tc, in.a, n, at + 1, stk_tag, stk_pos);
           }
         }
       }
@@ -2390,6 +2397,12 @@ __global__ void pike_captures(CapArgs a) {
       cur ^= 1;
     }
   }
+}
+
+__global__ void slot_found_bits(const uint64_t* slots, uint32_t n_slots, uint64_t n_rec, uint32_t* bits) {
+  const uint64_t r = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x;
+  const uint32_t b = __ballot_sync(0xffffffffu, r < n_rec && slots[r * n_slots] != kNone);
+  if ((threadIdx.x & 31) == 0 && r < n_rec) bits[r >> 5] = b;
 }
 
 // ---------------------------------------------------------------- batch mode --
@@ -2504,6 +2517,113 @@ __device__ __noinline__ bool slow_find_record(const DfaView* f, const DfaView* r
   return true;
 }
 
+// The forward loop of batch_fast: record bytes from q on, hot state e on entry (the start state for
+// position q), 16 bytes per window.  MODE 0: stops at the first match state, mx = highest state seen;
+// MODE 1: runs until the automaton dies, last = end of the leftmost-first match (kNone: none).
+// On return e == 1 (trap) means the record left the hot set: redo it on the full tables.
+template <int MODE>
+__device__ __forceinline__ void hot_forward(const BatchArgs& a, uint32_t fbase, const uint8_t* p, uint64_t len, uint64_t q,
+                                            const uint8_t* buf_hi, uint32_t& e, uint64_t& last, uint32_t& mx) {
+  const uint32_t fthr = a.fwd_hot.match_lo, flive = 2;
+  bool done = false;
+  while (!done) {
+    const uint64_t left = len - q;
+    if (left == 0) {  // EOF step
+      if (e >= flive && a.fwd_hot.eof[e] >= a.fwd.match_lo) { last = len; mx = 0xFFFFFFFFu; }
+      break;
+    }
+    const uint8_t* wp = p + q;
+    const uint8_t* al = reinterpret_cast<const uint8_t*>(reinterpret_cast<uintptr_t>(wp) & ~(uintptr_t)7);
+    if (al + 24 <= buf_hi) {
+      uint32_t v[4];
+      window16(wp, v);
+      const uint32_t nb = left >= 16 ? 16u : (uint32_t)left;
+      uint32_t lj = ~0u;
+      if (nb == 16) {
+#pragma unroll
+        for (int g = 0; g < 4; g++) {
+          e = hot_next<0>(fbase, v[g], e); if (MODE == 0) mx = max(mx, e); else if (e >= fthr) lj = 4 * g + 0;
+          e = hot_next<1>(fbase, v[g], e); if (MODE == 0) mx = max(mx, e); else if (e >= fthr) lj = 4 * g + 1;
+          e = hot_next<2>(fbase, v[g], e); if (MODE == 0) mx = max(mx, e); else if (e >= fthr) lj = 4 * g + 2;
+          e = hot_next<3>(fbase, v[g], e); if (MODE == 0) mx = max(mx, e); else if (e >= fthr) lj = 4 * g + 3;
+          if (e < flive || (MODE == 0 && mx >= fthr)) { done = true; break; }
+        }
+      } else {
+#pragma unroll
+        for (int i = 0; i < 15; i++) {
+          if ((uint32_t)i < nb) {
+            e = hot_next_b(fbase, window_byte(v, i), e);
+            if (MODE == 0) mx = max(mx, e);
+            else if (e >= fthr) lj = i;
+          }
+        }
+        if (e < flive || (MODE == 0 && mx >= fthr)) done = true;
+      }
+      if (MODE == 1 && lj != ~0u) last = q + lj;
+      q += nb;
+    } else {  // the last bytes of the whole buffer: byte loads
+      for (uint64_t i = 0; i < left && !done; i++) {
+        e = hot_next_b(fbase, p[q + i], e);
+        if (MODE == 0) mx = max(mx, e);
+        else if (e >= fthr) last = q + i;
+        if (e < flive || (MODE == 0 && mx >= fthr)) done = true;
+      }
+      q += left;
+    }
+  }
+}
+
+// The reverse loop of batch_fast: start of the match that ends at me > lo, found by the reverse longest
+// automaton over the slice p[lo..] (exec.rs:651-657; lo is that slice's beginning of text).  kNone: no
+// start.  rcold: the scan left the hot set and must be redone on the full tables (slice_start).
+__device__ __forceinline__ uint64_t hot_reverse(const BatchArgs& a, uint32_t rbase, const uint8_t* p, uint64_t len, uint64_t lo,
+                                                uint64_t me, const uint8_t* buf_hi, bool& rcold) {
+  const uint32_t rthr = a.rev_hot.match_lo, rlive = 2;
+  uint64_t start = kNone;
+  // flags at me of the slice p[lo..] are those of the record: me > lo
+  const uint32_t sf = a.rev.uniform_start ? a.rev.start[32] : a.rev.start[flags_reverse(p, len, me)];
+  const uint32_t hr = a.rev_hot.full2hot[sf];
+  if (sf == 0) {
+    start = kNone;
+  } else if (hr == 0xFFFFu) {
+    rcold = true;
+  } else {
+    uint32_t er = hr;
+    uint64_t at = me;
+    bool rdone = false;
+    while (at > lo && !rdone) {
+      const uint8_t* wp = p + at - 16;  // window = bytes [at-16, at); only the last min(16, at - lo) belong to the slice
+      const uint8_t* al = reinterpret_cast<const uint8_t*>(reinterpret_cast<uintptr_t>(wp) & ~(uintptr_t)7);
+      const uint32_t nb = at - lo >= 16 ? 16u : (uint32_t)(at - lo);
+      if (al >= a.text && al + 24 <= buf_hi) {
+        uint32_t v[4];
+        window16(wp, v);
+        uint32_t lj = ~0u;
+#pragma unroll
+        for (int i = 15; i >= 0; i--) {
+          if ((uint32_t)(15 - i) < nb && !rdone) {
+            er = hot_next_b(rbase, window_byte(v, i), er);
+            if (er >= rthr) lj = i;
+            if (er < rlive) rdone = true;
+          }
+        }
+        if (lj != ~0u) start = at - 16 + lj + 1;
+        at -= nb;
+      } else {
+        for (uint32_t i = 0; i < nb && !rdone; i++) {
+          at--;
+          er = hot_next_b(rbase, p[at], er);
+          if (er >= rthr) start = at + 1;
+          if (er < rlive) rdone = true;
+        }
+      }
+    }
+    if (er == 1u) rcold = true;
+    else if (!rdone && a.rev_hot.eof[er] >= a.rev.match_lo) start = lo;
+  }
+  return start;
+}
+
 // MODE 0: is_match (forward all-match automaton, stop at the first match state);
 // MODE 1: find (forward leftmost-first end, then the reverse longest automaton for the start).
 template <int MODE>
@@ -2513,8 +2633,7 @@ __global__ void __launch_bounds__(512) batch_fast(BatchArgs a) {
   hot_stage(a.fwd_hot, fbase);
   if (MODE == 1) hot_stage(a.rev_hot, rbase);
   __syncthreads();
-  const uint32_t fthr = a.fwd_hot.match_lo, flive = 2;
-  const uint32_t rthr = a.rev_hot.match_lo, rlive = 2;
+  const uint32_t fthr = a.fwd_hot.match_lo;
   const uint8_t* const buf_hi = a.text + a.offsets[a.n_rec];
   const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;  // multiple of 32: warps stay on one ballot word
   const uint32_t lane = threadIdx.x & 31;
@@ -2530,53 +2649,7 @@ __global__ void __launch_bounds__(512) batch_fast(BatchArgs a) {
       uint32_t e = h0 == 0xFFFFu ? 1u : h0;
       uint64_t last = kNone;
       uint32_t mx = 0;
-      uint64_t q = 0;
-      bool done = false;
-      while (!done) {
-        const uint64_t left = len - q;
-        if (left == 0) {  // EOF step
-          if (e >= flive && a.fwd_hot.eof[e] >= a.fwd.match_lo) { last = len; mx = 0xFFFFFFFFu; }
-          break;
-        }
-        const uint8_t* wp = p + q;
-        const uint8_t* al = reinterpret_cast<const uint8_t*>(reinterpret_cast<uintptr_t>(wp) & ~(uintptr_t)7);
-        if (al + 24 <= buf_hi) {
-          uint32_t v[4];
-          window16(wp, v);
-          const uint32_t nb = left >= 16 ? 16u : (uint32_t)left;
-          uint32_t lj = ~0u;
-          if (nb == 16) {
-#pragma unroll
-            for (int g = 0; g < 4; g++) {
-              e = hot_next<0>(fbase, v[g], e); if (MODE == 0) mx = max(mx, e); else if (e >= fthr) lj = 4 * g + 0;
-              e = hot_next<1>(fbase, v[g], e); if (MODE == 0) mx = max(mx, e); else if (e >= fthr) lj = 4 * g + 1;
-              e = hot_next<2>(fbase, v[g], e); if (MODE == 0) mx = max(mx, e); else if (e >= fthr) lj = 4 * g + 2;
-              e = hot_next<3>(fbase, v[g], e); if (MODE == 0) mx = max(mx, e); else if (e >= fthr) lj = 4 * g + 3;
-              if (e < flive || (MODE == 0 && mx >= fthr)) { done = true; break; }
-            }
-          } else {
-#pragma unroll
-            for (int i = 0; i < 15; i++) {
-              if ((uint32_t)i < nb) {
-                e = hot_next_b(fbase, window_byte(v, i), e);
-                if (MODE == 0) mx = max(mx, e);
-                else if (e >= fthr) lj = i;
-              }
-            }
-            if (e < flive || (MODE == 0 && mx >= fthr)) done = true;
-          }
-          if (MODE == 1 && lj != ~0u) last = q + lj;
-          q += nb;
-        } else {  // the last bytes of the whole buffer: byte loads
-          for (uint64_t i = 0; i < left && !done; i++) {
-            e = hot_next_b(fbase, p[q + i], e);
-            if (MODE == 0) mx = max(mx, e);
-            else if (e >= fthr) last = q + i;
-            if (e < flive || (MODE == 0 && mx >= fthr)) done = true;
-          }
-          q += left;
-        }
-      }
+      hot_forward<MODE>(a, fbase, p, len, 0, buf_hi, e, last, mx);
       if (e == 1u && !(MODE == 0 && mx >= fthr)) cold = true;  // trap row
       if (MODE == 0) {
         hit = cold ? slow_is_match_record(a.fwd_g, p, len) : mx >= fthr;
@@ -2585,52 +2658,8 @@ __global__ void __launch_bounds__(512) batch_fast(BatchArgs a) {
       } else if (last != kNone) {
         // ---- reverse from the match end (exec.rs:651-657; the record is its own slice) ----
         me = last;
-        uint64_t start = kNone;
         bool rcold = false;
-        if (me == 0) {
-          start = 0;
-        } else {
-          const uint32_t sf = a.rev.uniform_start ? a.rev.start[32] : a.rev.start[flags_reverse(p, len, me)];
-          const uint32_t hr = a.rev_hot.full2hot[sf];
-          if (sf == 0) {
-            start = kNone;
-          } else if (hr == 0xFFFFu) {
-            rcold = true;
-          } else {
-            uint32_t er = hr;
-            uint64_t at = me;
-            bool rdone = false;
-            while (at > 0 && !rdone) {
-              const uint8_t* wp = p + at - 16;  // window = bytes [at-16, at); only the last min(16, at) belong to the record
-              const uint8_t* al = reinterpret_cast<const uint8_t*>(reinterpret_cast<uintptr_t>(wp) & ~(uintptr_t)7);
-              const uint32_t nb = at >= 16 ? 16u : (uint32_t)at;
-              if (al >= a.text && al + 24 <= buf_hi) {
-                uint32_t v[4];
-                window16(wp, v);
-                uint32_t lj = ~0u;
-#pragma unroll
-                for (int i = 15; i >= 0; i--) {
-                  if ((uint32_t)(15 - i) < nb && !rdone) {
-                    er = hot_next_b(rbase, window_byte(v, i), er);
-                    if (er >= rthr) lj = i;
-                    if (er < rlive) rdone = true;
-                  }
-                }
-                if (lj != ~0u) start = at - 16 + lj + 1;
-                at -= nb;
-              } else {
-                for (uint32_t i = 0; i < nb && !rdone; i++) {
-                  at--;
-                  er = hot_next_b(rbase, p[at], er);
-                  if (er >= rthr) start = at + 1;
-                  if (er < rlive) rdone = true;
-                }
-              }
-            }
-            if (er == 1u) rcold = true;
-            else if (!rdone && a.rev_hot.eof[er] >= a.rev.match_lo) start = 0;
-          }
-        }
+        const uint64_t start = me == 0 ? 0 : hot_reverse(a, rbase, p, len, 0, me, buf_hi, rcold);
         if (rcold) {
           hit = slow_find_record(a.fwd_g, a.rev_g, p, len, &ms, &me);
         } else if (start != kNone) {
@@ -2649,6 +2678,108 @@ __global__ void __launch_bounds__(512) batch_fast(BatchArgs a) {
 }
 template __global__ void batch_fast<0>(BatchArgs);
 template __global__ void batch_fast<1>(BatchArgs);
+
+// ---- batch_iter: find_iter per record (re_trait.rs:197-220 with the record as the whole text) ----
+// From p: the end e of the leftmost-first match found from p (forward unanchored automaton, start state by
+// the flags at p), its start by the reverse scan over the slice [p..] (exec.rs:651-657, so p is judged as
+// beginning of text: SURVEY H1), then the empty-match rule (exec.rs:335-377).  Two launches of one kernel
+// build the CSR output: PASS 0 counts the matches of each record, an exclusive scan turns the counts into
+// offsets, PASS 1 runs the iterator again and stores.  Match counts per record are unbounded, so a single
+// pass would need per-record staging of unbounded size; the second pass costs a second read of the text.
+// fwd(q) -> match end or kNone; rev(q, e) -> match start (e > q) or kNone.
+template <int PASS, class Fwd, class Rev>
+__device__ __forceinline__ void iter_record(const BatchArgs& a, uint64_t r, const uint8_t* p, uint64_t len, Fwd fwd, Rev rev) {
+  const uint64_t base = PASS == 1 ? a.match_offsets[r] : 0;
+  uint64_t k = 0, q = 0, lm = kNone;
+  while (q <= len) {
+    const uint64_t e = fwd(q);
+    if (e == kNone) break;
+    if (PASS == 0 && a.fwd_only) {  // no empty match, no look-around: s < e and the reverse scan cannot fail
+      k++;
+      q = e;
+      continue;
+    }
+    const uint64_t s = e == q ? q : rev(q, e);
+    if (s == kNone) break;  // the reverse-on-slice scan failed: the reference's iteration ends here
+    if (s == e) {
+      q = a.utf8 ? next_utf8(p, len, e) : e + 1;
+      if (e == lm) continue;
+    } else {
+      q = e;
+    }
+    lm = e;
+    if (PASS == 1 && base + k < a.cap) {
+      a.out_spans[2 * (base + k)] = s;
+      a.out_spans[2 * (base + k) + 1] = e;
+    }
+    k++;
+  }
+  if (PASS == 0) a.match_offsets[r] = k;
+}
+
+// leftmost-first match end from q on the class-indexed tables (the generic kernel and cold records)
+__device__ __forceinline__ uint64_t table_forward_end(const DfaView& f, const uint8_t* p, uint64_t len, uint64_t q) {
+  uint32_t s = pick_start_fwd(f, p, len, q);
+  uint64_t e = kNone;
+  for (; s != 0; q++) {
+    s = q < len ? f.trans[s * f.stride + f.classes[p[q]]] : f.trans[s * f.stride + f.stride - 1];
+    if (s >= f.match_lo) e = q;
+    if (q >= len) break;
+  }
+  return e;
+}
+
+// One thread per record on the hot tables, as batch_fast<1> (persistent blocks, 16-byte windows).  A
+// record that leaves the hot set finishes its iteration on the full tables in global memory.
+template <int PASS>
+__global__ void __launch_bounds__(512, 2) batch_iter_fast(BatchArgs a) {
+  const uint32_t fbase = ((uint32_t)__cvta_generic_to_shared(g_smem) + 255u) & ~255u;
+  const uint32_t rbase = fbase + hot_table_bytes(a.fwd_hot.n);
+  hot_stage(a.fwd_hot, fbase);
+  hot_stage(a.rev_hot, rbase);
+  __syncthreads();
+  const uint8_t* const buf_hi = a.text + a.offsets[a.n_rec];
+  const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
+  for (uint64_t r = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x; r < a.n_rec; r += stride) {
+    const uint64_t lo = a.offsets[r], len = a.offsets[r + 1] - lo;
+    const uint8_t* p = a.text + lo;
+    bool cold = false;
+    auto fwd = [&](uint64_t q) -> uint64_t {
+      if (!cold) {
+        const uint32_t h0 = a.fwd.uniform_start ? a.fwd_hot.start : a.fwd_hot.full2hot[a.fwd.start[flags_forward(p, len, q)]];
+        uint32_t e = h0 == 0xFFFFu ? 1u : h0, mx = 0;
+        uint64_t last = kNone;
+        hot_forward<1>(a, fbase, p, len, q, buf_hi, e, last, mx);
+        if (e != 1u) return last;
+        cold = true;
+      }
+      return table_forward_end(*a.fwd_g, p, len, q);
+    };
+    auto rev = [&](uint64_t q, uint64_t e) -> uint64_t {
+      if (!cold) {
+        const uint64_t s = hot_reverse(a, rbase, p, len, q, e, buf_hi, cold);
+        if (!cold) return s;
+      }
+      return slice_start(*a.rev_g, p, len, q, e);
+    };
+    iter_record<PASS>(a, r, p, len, fwd, rev);
+  }
+}
+template __global__ void batch_iter_fast<0>(BatchArgs);
+template __global__ void batch_iter_fast<1>(BatchArgs);
+
+// Generic: one thread per record on the class-indexed tables (no hot set, unaligned haystacks, force_generic).
+template <int PASS>
+__global__ void batch_iter(BatchArgs a) {
+  const uint64_t r = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x;
+  if (r >= a.n_rec) return;
+  const uint64_t lo = a.offsets[r], len = a.offsets[r + 1] - lo;
+  const uint8_t* p = a.text + lo;
+  iter_record<PASS>(a, r, p, len, [&](uint64_t q) { return table_forward_end(a.fwd, p, len, q); },
+                    [&](uint64_t q, uint64_t e) { return slice_start(a.rev, p, len, q, e); });
+}
+template __global__ void batch_iter<0>(BatchArgs);
+template __global__ void batch_iter<1>(BatchArgs);
 
 // ---- batch_refill: batch_fast<0> with the lanes of a warp kept busy ----
 // batch_fast gives every lane one record and waits for the slowest of the 32: on log lines 70 % of the

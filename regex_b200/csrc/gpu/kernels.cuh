@@ -17,6 +17,8 @@
 //   compact_spans     chunk, validated against the left neighbour, ordered compaction
 //   batch_fast,       one thread per record: is_match / find / set matches, the
 //   *_batch           reference algorithm verbatim per record (exec.rs:632-662)
+//   batch_iter*       one thread per record: find_iter (re_trait.rs:197-220) per record,
+//                     count pass + prefix sum + write pass (CSR output)
 #pragma once
 #include <cstdint>
 #include <cuda_runtime.h>

@@ -138,8 +138,14 @@ struct CapArgs {
   uint64_t* slots;         // [n_matches][n_slots], kNone = the group did not take part
   uint8_t* scratch;        // per resident thread: two thread lists with their slot arrays, a stack (see kernels.cu)
   uint64_t per_thread;
+  // batched records (null otherwise): match m is the first match of record m, spans are record-relative and
+  // the record is the text; records whose bit in rec_found (ballot words) is clear are skipped
+  const uint64_t* rec_offsets;
+  const uint32_t* rec_found;
 };
 __global__ void pike_captures(CapArgs a);
+// ballot words: bit r = group 0 of record r took part (slots[r * n_slots] != kNone)
+__global__ void slot_found_bits(const uint64_t* slots, uint32_t n_slots, uint64_t n_rec, uint32_t* bits);
 
 struct BatchArgs {
   DfaView fwd;
@@ -156,10 +162,20 @@ struct BatchArgs {
   uint64_t* out_masks;  // mask_words per record
   unsigned long long* task_counter;  // batch_refill: next task to hand out (zeroed before the launch)
   uint32_t task_recs;                // batch_refill: records per task (multiple of 32, <= 2048)
+  // batch_iter*: per-record find_iter
+  uint64_t* match_offsets;  // count pass: matches of record r at [r]; write pass: exclusive prefix sum (first slot of record r)
+  uint64_t cap;             // write pass: spans stored at out_spans[0, cap)
+  int utf8;                 // empty matches advance by one UTF-8 scalar (Regex on str)
+  int fwd_only;             // count pass of a pattern that cannot match empty and has no look-around: no reverse scan
 };
 
 template <int MODE>
 __global__ void batch_fast(BatchArgs a);
+// PASS 0: count the matches of every record; PASS 1: write them.  _fast: hot tables in shared memory.
+template <int PASS>
+__global__ void batch_iter_fast(BatchArgs a);
+template <int PASS>
+__global__ void batch_iter(BatchArgs a);
 template <int MODE>
 __global__ void batch_refill(BatchArgs a);
 __global__ void scan_rev_bitmap(ScanArgs a);
