@@ -10,6 +10,9 @@
  *   rure_b200_set_matches_*   == rure_set_matches(...) packed into 64-bit masks
  *   rure_b200_find_iter_batch == collecting rure_iter_next over each record (record-relative offsets)
  *   rure_b200_captures_batch  == rure_find_captures(re, hay + off[i], off[i+1]-off[i], 0, ...) per record
+ *   rure_b200_replace_batch   == rure_b200_replace(re, hay + off[i], off[i+1]-off[i], rep, ..., limit, ...) per record
+ *   rure_b200_split_batch     == rure_b200_split(re, hay + off[i], off[i+1]-off[i], has_limit, limit, ...) per record
+ *   rure_b200_captures_iter_batch == rure_b200_captures_all(re, hay + off[i], off[i+1]-off[i], ...) per record
  * Functions return true on success; on failure rure_b200_last_error() (thread
  * local) describes what went wrong.  A missing GPU is a failure, never a
  * silent CPU fallback.
@@ -115,6 +118,25 @@ bool rure_b200_find_iter_batch(rure *re, const uint8_t *haystack, const uint64_t
  * match); found_bits as rure_b200_find_batch. */
 bool rure_b200_captures_batch(rure *re, const uint8_t *haystack, const uint64_t *offsets, size_t n_records,
                               size_t *slots, uint8_t *found_bits);
+/* replacen, split / splitn and captures_iter of every record, with the record as the whole haystack.  Each
+ * result is CSR-shaped: an offsets array of n_records + 1 entries (always complete, [0] = 0) and a payload of
+ * which at most the given capacity is stored, the total always being reported; a NULL payload or a capacity
+ * of 0 asks for sizes only.  Str mode steps past an empty match by one UTF-8 scalar.
+ * replace: record i's result is out[out_offsets[i] .. out_offsets[i+1]); rep / expand / limit as
+ * rure_b200_replace, limit applying to every record (0 = all matches); *out_len = all output bytes. */
+bool rure_b200_replace_batch(rure *re, const uint8_t *haystack, const uint64_t *offsets, size_t n_records,
+                             const uint8_t *rep, size_t rep_len, int expand, size_t limit,
+                             uint64_t *out_offsets, uint8_t *out, size_t out_cap, size_t *out_len);
+/* split: record i's pieces (record-relative start, end) are out[piece_offsets[i] .. piece_offsets[i+1]);
+ * has_limit / limit as rure_b200_split, per record (limit 0: no pieces; limit 1: the whole record, even an
+ * empty one; the last piece is the rest of the record, empty or not). */
+bool rure_b200_split_batch(rure *re, const uint8_t *haystack, const uint64_t *offsets, size_t n_records,
+                           int has_limit, size_t limit, uint64_t *piece_offsets, rure_match *out, size_t cap,
+                           size_t *n_total);
+/* captures_iter: record i's matches are rows match_offsets[i] .. match_offsets[i+1] of
+ * slots[min(cap, *n_total)][2 * rure_b200_captures_len(re)], record-relative, SIZE_MAX = group absent. */
+bool rure_b200_captures_iter_batch(rure *re, const uint8_t *haystack, const uint64_t *offsets, size_t n_records,
+                                   uint64_t *match_offsets, size_t *slots, size_t cap, size_t *n_total);
 
 /* ---- device-resident inputs and outputs ----------------------------------- */
 bool rure_b200_find_all_device(rure *re, const uint8_t *d_haystack, size_t length, size_t start,
@@ -138,6 +160,17 @@ bool rure_b200_find_iter_batch_device(rure *re, const uint8_t *d_haystack, const
 /* as rure_b200_captures_batch; d_found_bits are 32-bit ballot words as rure_b200_find_batch_device */
 bool rure_b200_captures_batch_device(rure *re, const uint8_t *d_haystack, const uint64_t *d_offsets,
                                      size_t n_records, size_t *d_slots, uint32_t *d_found_bits);
+/* as the three calls above; d_* in device memory (rep stays on the host), totals on the host */
+bool rure_b200_replace_batch_device(rure *re, const uint8_t *d_haystack, const uint64_t *d_offsets,
+                                    size_t n_records, const uint8_t *rep, size_t rep_len, int expand,
+                                    size_t limit, uint64_t *d_out_offsets, uint8_t *d_out, size_t out_cap,
+                                    size_t *out_len);
+bool rure_b200_split_batch_device(rure *re, const uint8_t *d_haystack, const uint64_t *d_offsets,
+                                  size_t n_records, int has_limit, size_t limit, uint64_t *d_piece_offsets,
+                                  rure_match *d_out, size_t cap, size_t *n_total);
+bool rure_b200_captures_iter_batch_device(rure *re, const uint8_t *d_haystack, const uint64_t *d_offsets,
+                                          size_t n_records, uint64_t *d_match_offsets, size_t *d_slots,
+                                          size_t cap, size_t *n_total);
 
 /* ---- byte-range shards of one haystack (multi-GPU; one process per GPU) ------
  * Each rank holds [left context | owned bytes | right halo] of the haystack in its

@@ -106,6 +106,9 @@ def _load():
         "rure_b200_set_matches_batch": (c_bool, [vp, u8p, vp, sz, vp]),
         "rure_b200_find_iter_batch": (c_bool, [vp, u8p, vp, sz, vp, vp, sz, POINTER(sz)]),
         "rure_b200_captures_batch": (c_bool, [vp, u8p, vp, sz, vp, vp]),
+        "rure_b200_replace_batch": (c_bool, [vp, u8p, vp, sz, c_char_p, sz, c_int, sz, vp, vp, sz, POINTER(sz)]),
+        "rure_b200_split_batch": (c_bool, [vp, u8p, vp, sz, c_int, sz, vp, vp, sz, POINTER(sz)]),
+        "rure_b200_captures_iter_batch": (c_bool, [vp, u8p, vp, sz, vp, vp, sz, POINTER(sz)]),
         "rure_b200_find_all_device": (c_bool, [vp, vp, sz, sz, vp, sz, POINTER(sz)]),
         "rure_b200_find_all_shard_device": (c_bool, [vp, vp, sz, POINTER(_Shard), vp, sz]),
         "rure_b200_shortest_match_device": (c_bool, [vp, vp, sz, sz, POINTER(c_bool), POINTER(sz)]),
@@ -117,6 +120,9 @@ def _load():
         "rure_b200_set_matches_batch_device": (c_bool, [vp, vp, vp, sz, vp]),
         "rure_b200_find_iter_batch_device": (c_bool, [vp, vp, vp, sz, vp, vp, sz, POINTER(sz)]),
         "rure_b200_captures_batch_device": (c_bool, [vp, vp, vp, sz, vp, vp]),
+        "rure_b200_replace_batch_device": (c_bool, [vp, vp, vp, sz, c_char_p, sz, c_int, sz, vp, vp, sz, POINTER(sz)]),
+        "rure_b200_split_batch_device": (c_bool, [vp, vp, vp, sz, c_int, sz, vp, vp, sz, POINTER(sz)]),
+        "rure_b200_captures_iter_batch_device": (c_bool, [vp, vp, vp, sz, vp, vp, sz, POINTER(sz)]),
         "rure_b200_last_error": (c_char_p, []),
         "rure_b200_kernel_launches": (c_uint64, []),
         "rure_b200_last_stats": (None, [vp, POINTER(c_double)]),
@@ -446,6 +452,76 @@ class _Compiled:
             raise Error(_last_error())
         return np.unpackbits(bits, bitorder="little")[:n_rec].astype(bool), slots[:n_rec]
 
+    def replacen_batch(self, text, offsets, limit, rep, expand=True):
+        """`replacen` on every record: (out_offsets uint64[n+1], out uint8[...]); record i's result is
+        out[out_offsets[i]:out_offsets[i+1]].  limit applies to every record (0 = all matches); rep / expand as
+        replacen."""
+        p, n, keep = _buf(text)
+        off = np.ascontiguousarray(offsets, dtype=np.uint64)
+        n_rec = off.size - 1
+        r = rep.encode("utf-8") if isinstance(rep, str) else bytes(rep)
+        ooff = np.zeros(n_rec + 1, dtype=np.uint64)
+        ol = c_size_t()
+        cap = n + 4096
+        while True:
+            out = np.empty(max(cap, 1), dtype=np.uint8)
+            if not _lib.rure_b200_replace_batch(self._h, p, off.ctypes.data, n_rec, r, len(r), int(expand), limit, ooff.ctypes.data,
+                                                out.ctypes.data, cap, byref(ol)):
+                raise Error(_last_error())
+            if ol.value <= cap:
+                return ooff, out[: ol.value]
+            cap = ol.value
+
+    def replace_batch(self, text, offsets, rep, expand=True):
+        return self.replacen_batch(text, offsets, 1, rep, expand)
+
+    def replace_all_batch(self, text, offsets, rep, expand=True):
+        return self.replacen_batch(text, offsets, 0, rep, expand)
+
+    def _split_batch(self, text, offsets, has_limit, limit):
+        p, n, keep = _buf(text)
+        off = np.ascontiguousarray(offsets, dtype=np.uint64)
+        n_rec = off.size - 1
+        poff = np.zeros(n_rec + 1, dtype=np.uint64)
+        total = c_size_t()
+        cap = max(4096, 2 * n_rec)
+        while True:
+            out = np.empty((max(cap, 1), 2), dtype=np.uint64)
+            if not _lib.rure_b200_split_batch(self._h, p, off.ctypes.data, n_rec, has_limit, limit, poff.ctypes.data, out.ctypes.data, cap,
+                                              byref(total)):
+                raise Error(_last_error())
+            if total.value <= cap:
+                return poff, out[: total.value]
+            cap = total.value
+
+    def split_batch(self, text, offsets):
+        """`split` on every record: (piece_offsets uint64[n+1], pieces uint64[m, 2]); the pieces of record i are
+        pieces[piece_offsets[i]:piece_offsets[i+1]], relative to the record."""
+        return self._split_batch(text, offsets, 0, 0)
+
+    def splitn_batch(self, text, offsets, limit):
+        """`splitn` on every record, as split_batch: at most `limit` pieces per record, the last one being the rest."""
+        return self._split_batch(text, offsets, 1, limit)
+
+    def captures_iter_batch(self, text, offsets):
+        """`captures_iter` on every record: (match_offsets uint64[n+1], slots uint64[m, captures_len, 2]); the
+        matches of record i are slots[match_offsets[i]:match_offsets[i+1]], relative to the record, 2**64-1 where
+        a group did not take part."""
+        p, n, keep = _buf(text)
+        off = np.ascontiguousarray(offsets, dtype=np.uint64)
+        n_rec = off.size - 1
+        g = self.captures_len()
+        moff = np.zeros(n_rec + 1, dtype=np.uint64)
+        total = c_size_t()
+        cap = max(4096, 2 * n_rec)
+        while True:
+            out = np.empty((max(cap, 1), g, 2), dtype=np.uint64)
+            if not _lib.rure_b200_captures_iter_batch(self._h, p, off.ctypes.data, n_rec, moff.ctypes.data, out.ctypes.data, cap, byref(total)):
+                raise Error(_last_error())
+            if total.value <= cap:
+                return moff, out[: total.value]
+            cap = total.value
+
     # ---- device-resident (torch CUDA tensors) --------------------------------
     def find_all_device(self, d_text, d_out=None, start=0):
         """d_text: uint8 CUDA tensor; d_out: optional (cap, 2) int64/uint64 CUDA tensor.
@@ -508,6 +584,43 @@ class _Compiled:
         n_rec = d_offsets.numel() - 1
         if not _lib.rure_b200_captures_batch_device(self._h, d_text.data_ptr(), d_offsets.data_ptr(), n_rec, d_slots.data_ptr(), d_bits.data_ptr()):
             raise Error(_last_error())
+
+    def replacen_batch_device(self, d_text, d_offsets, limit, rep, d_out_offsets, d_out=None, expand=True):
+        """replacen_batch on the device.  d_out_offsets: (n_records + 1) int64/uint64 CUDA tensor, always filled;
+        d_out: optional uint8 CUDA tensor (beyond its size the output is counted, not stored).  Returns the total
+        output length."""
+        n_rec = d_offsets.numel() - 1
+        r = rep.encode("utf-8") if isinstance(rep, str) else bytes(rep)
+        ol = c_size_t()
+        ptr, cap = (0, 0) if d_out is None else (d_out.data_ptr(), d_out.numel())
+        if not _lib.rure_b200_replace_batch_device(self._h, d_text.data_ptr(), d_offsets.data_ptr(), n_rec, r, len(r), int(expand), limit,
+                                                   d_out_offsets.data_ptr(), ptr, cap, byref(ol)):
+            raise Error(_last_error())
+        return ol.value
+
+    def split_batch_device(self, d_text, d_offsets, d_piece_offsets, d_out=None, limit=None):
+        """split_batch (splitn_batch when limit is given) on the device.  d_piece_offsets: (n_records + 1) CUDA
+        tensor, always filled; d_out: optional (cap, 2) tensor for the pieces.  Returns the total number of pieces."""
+        n_rec = d_offsets.numel() - 1
+        total = c_size_t()
+        cap = 0 if d_out is None else d_out.shape[0]
+        ptr = 0 if d_out is None else d_out.data_ptr()
+        if not _lib.rure_b200_split_batch_device(self._h, d_text.data_ptr(), d_offsets.data_ptr(), n_rec, int(limit is not None), limit or 0,
+                                                 d_piece_offsets.data_ptr(), ptr, cap, byref(total)):
+            raise Error(_last_error())
+        return total.value
+
+    def captures_iter_batch_device(self, d_text, d_offsets, d_match_offsets, d_slots=None):
+        """captures_iter_batch on the device.  d_match_offsets: (n_records + 1) CUDA tensor, always filled; d_slots:
+        optional (cap, captures_len(), 2) tensor.  Returns the total number of matches."""
+        n_rec = d_offsets.numel() - 1
+        total = c_size_t()
+        cap = 0 if d_slots is None else d_slots.shape[0]
+        ptr = 0 if d_slots is None else d_slots.data_ptr()
+        if not _lib.rure_b200_captures_iter_batch_device(self._h, d_text.data_ptr(), d_offsets.data_ptr(), n_rec, d_match_offsets.data_ptr(),
+                                                         ptr, cap, byref(total)):
+            raise Error(_last_error())
+        return total.value
 
     # ---- diagnostics ------------------------------------------------------------
     def last_stats(self):

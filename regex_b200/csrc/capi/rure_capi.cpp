@@ -408,6 +408,51 @@ bool rure_b200_captures_batch_device(rure* re, const uint8_t* d_haystack, const 
                                      uint32_t* d_found_bits) {
   return ok(re->re, re->re->captures_batch_device(d_haystack, d_offsets, n, (uint64_t*)d_slots, d_found_bits));
 }
+bool rure_b200_replace_batch(rure* re, const uint8_t* haystack, const uint64_t* offsets, size_t n, const uint8_t* rep, size_t rep_len, int expand,
+                             size_t limit, uint64_t* out_offsets, uint8_t* out, size_t out_cap, size_t* out_len) {
+  uint64_t ol = 0;
+  const bool r = ok(re->re, re->re->replace_batch_host(haystack, offsets, n, rep, rep_len, expand != 0, limit, out_offsets, out, out ? out_cap : 0, &ol));
+  if (out_len) *out_len = ol;
+  return r;
+}
+bool rure_b200_replace_batch_device(rure* re, const uint8_t* d_haystack, const uint64_t* d_offsets, size_t n, const uint8_t* rep, size_t rep_len,
+                                    int expand, size_t limit, uint64_t* d_out_offsets, uint8_t* d_out, size_t out_cap, size_t* out_len) {
+  uint64_t ol = 0;
+  const bool r = ok(re->re, re->re->replace_batch_device(d_haystack, d_offsets, n, rep, rep_len, expand != 0, limit, d_out_offsets, d_out,
+                                                         d_out ? out_cap : 0, &ol));
+  if (out_len) *out_len = ol;
+  return r;
+}
+bool rure_b200_split_batch(rure* re, const uint8_t* haystack, const uint64_t* offsets, size_t n, int has_limit, size_t limit, uint64_t* piece_offsets,
+                           rure_match* out, size_t cap, size_t* n_total) {
+  uint64_t total = 0;
+  const bool r = ok(re->re, re->re->split_batch_host(haystack, offsets, n, has_limit != 0, limit, piece_offsets, (uint64_t*)out, out ? cap : 0, &total));
+  if (n_total) *n_total = total;
+  return r;
+}
+bool rure_b200_split_batch_device(rure* re, const uint8_t* d_haystack, const uint64_t* d_offsets, size_t n, int has_limit, size_t limit,
+                                  uint64_t* d_piece_offsets, rure_match* d_out, size_t cap, size_t* n_total) {
+  uint64_t total = 0;
+  const bool r = ok(re->re, re->re->split_batch_device(d_haystack, d_offsets, n, has_limit != 0, limit, d_piece_offsets, (uint64_t*)d_out,
+                                                       d_out ? cap : 0, &total));
+  if (n_total) *n_total = total;
+  return r;
+}
+bool rure_b200_captures_iter_batch(rure* re, const uint8_t* haystack, const uint64_t* offsets, size_t n, uint64_t* match_offsets, size_t* slots,
+                                   size_t cap, size_t* n_total) {
+  uint64_t total = 0;
+  const bool r = ok(re->re, re->re->captures_iter_batch_host(haystack, offsets, n, match_offsets, (uint64_t*)slots, slots ? cap : 0, &total));
+  if (n_total) *n_total = total;
+  return r;
+}
+bool rure_b200_captures_iter_batch_device(rure* re, const uint8_t* d_haystack, const uint64_t* d_offsets, size_t n, uint64_t* d_match_offsets,
+                                          size_t* d_slots, size_t cap, size_t* n_total) {
+  uint64_t total = 0;
+  const bool r = ok(re->re, re->re->captures_iter_batch_device(d_haystack, d_offsets, n, d_match_offsets, (uint64_t*)d_slots, d_slots ? cap : 0,
+                                                               &total));
+  if (n_total) *n_total = total;
+  return r;
+}
 bool rure_b200_find_all_device(rure* re, const uint8_t* d_haystack, size_t length, size_t start, rure_match* d_out, size_t cap, size_t* n_total) {
   uint64_t total = 0;
   bool r = ok(re->re, re->re->find_all_device(d_haystack, length, start, (uint64_t*)d_out, d_out ? cap : 0, &total));

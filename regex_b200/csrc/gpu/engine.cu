@@ -1463,6 +1463,11 @@ int Regex::find_batch_device(const uint8_t* d_text, const uint64_t* d_offsets, u
 int Regex::find_iter_batch_device(const uint8_t* d_text, const uint64_t* d_offsets, uint64_t n_rec, uint64_t* d_match_offsets,
                                   uint64_t* d_out, uint64_t cap, uint64_t* total) {
   std::lock_guard<std::recursive_mutex> lock(mu_);
+  return iter_batch(d_text, d_offsets, n_rec, d_match_offsets, d_out, cap, total, nullptr);
+}
+
+int Regex::iter_batch(const uint8_t* d_text, const uint64_t* d_offsets, uint64_t n_rec, uint64_t* d_match_offsets, uint64_t* d_out,
+                      uint64_t cap, uint64_t* total, DeviceBuf* grow) {
   *total = 0;
   if (is_set_) return fail("find requires exactly one pattern");
   DeviceDfa *fwd, *rev;
@@ -1506,16 +1511,16 @@ int Regex::find_iter_batch_device(const uint8_t* d_text, const uint64_t* d_offse
   else batch_iter<0><<<grid, 256, 0, st>>>(a);
   RB_LAUNCH_CHECK("batch_iter<0>");
   // ---- exclusive scan over n_rec + 1 entries ----
-  const uint64_t n_scan = n_rec + 1, n_blocks = (n_scan + 1023) / 1024;
-  uint64_t* block_sums = (uint64_t*)block_sums_.ensure((n_blocks + 1) * 8);
-  if (!block_sums) return fail("out of device memory (batch scan)");
-  unsigned long long* grand = (unsigned long long*)(block_sums + n_blocks);
-  scan_counts_local<<<(uint32_t)n_blocks, 1024, 0, st>>>(d_match_offsets, d_match_offsets, block_sums, n_scan);
-  RB_LAUNCH_CHECK("scan_counts_local");
-  scan_block_sums<<<1, 1024, 0, st>>>(block_sums, n_blocks, grand);
-  RB_LAUNCH_CHECK("scan_block_sums");
-  scan_add_block_offsets<<<(uint32_t)n_blocks, 1024, 0, st>>>(d_match_offsets, block_sums, n_scan);
-  RB_LAUNCH_CHECK("scan_add_block_offsets");
+  unsigned long long* grand;
+  if (int rc = prefix_sum(d_match_offsets, d_match_offsets, n_rec + 1, &grand)) return rc;
+  uint64_t* h = (uint64_t*)pinned_;
+  if (grow) {  // every span, into a buffer sized by the count
+    RB_CUDA(cudaMemcpyAsync(h, grand, 8, cudaMemcpyDeviceToHost, st));
+    RB_CUDA(cudaStreamSynchronize(st));
+    a.out_spans = (uint64_t*)grow->ensure(std::max<uint64_t>(h[0], 1) * 16);
+    if (!a.out_spans) return fail("out of device memory (batch spans)");
+    a.cap = h[0];
+  }
   // ---- write ----
   if (a.cap > 0) {
     a.fwd_only = 0;
@@ -1523,7 +1528,6 @@ int Regex::find_iter_batch_device(const uint8_t* d_text, const uint64_t* d_offse
     else batch_iter<1><<<grid, 256, 0, st>>>(a);
     RB_LAUNCH_CHECK("batch_iter<1>");
   }
-  uint64_t* h = (uint64_t*)pinned_;
   RB_CUDA(cudaMemcpyAsync(h, grand, 8, cudaMemcpyDeviceToHost, st));
   RB_CUDA(cudaStreamSynchronize(st));
   *total = h[0];
@@ -1575,6 +1579,26 @@ int Regex::set_matches_batch_device(const uint8_t* d_text, const uint64_t* d_off
   return 0;
 }
 
+// exclusive prefix sum of in[0, n) into out (kernels.cu scan_counts_local / scan_block_sums / scan_add_block_offsets)
+int Regex::prefix_sum(const uint64_t* in, uint64_t* out, uint64_t n, unsigned long long** d_total) {
+  cudaStream_t st = (cudaStream_t)stream_;
+  const uint64_t n_blocks = (n + 1023) / 1024;
+  uint64_t* block_sums = (uint64_t*)block_sums_.ensure((n_blocks + 1) * 8);
+  if (!block_sums) return fail("out of device memory (scan)");
+  *d_total = (unsigned long long*)(block_sums + n_blocks);
+  if (n_blocks == 0) {
+    RB_CUDA(cudaMemsetAsync(*d_total, 0, 8, st));
+    return 0;
+  }
+  scan_counts_local<<<(uint32_t)n_blocks, 1024, 0, st>>>(in, out, block_sums, n);
+  RB_LAUNCH_CHECK("scan_counts_local");
+  scan_block_sums<<<1, 1024, 0, st>>>(block_sums, n_blocks, *d_total);
+  RB_LAUNCH_CHECK("scan_block_sums");
+  scan_add_block_offsets<<<(uint32_t)n_blocks, 1024, 0, st>>>(out, block_sums, n);
+  RB_LAUNCH_CHECK("scan_add_block_offsets");
+  return 0;
+}
+
 // ------------------------------------------------------- replace_all / split ----
 // All spans of the haystack in spans_all_ (device); *m = their number.
 int Regex::all_spans_device(const uint8_t* d_text, uint64_t n, uint64_t** d_spans, uint64_t* m) {
@@ -1604,7 +1628,23 @@ int Regex::replace_device(const uint8_t* d_text, uint64_t n, const uint8_t* rep,
 int Regex::replace_prepare(const uint8_t* d_text, uint64_t n, const uint8_t* rep, uint64_t rep_len, bool expand, uint64_t limit,
                            uint64_t* out_len) {
   if (is_set_) return fail("replace requires exactly one pattern");
-  // ---- the replacement template (src/expand.rs:50-90) ----
+  bool needs_groups = false;
+  if (int rc = replace_template(rep, rep_len, expand, &needs_groups)) return rc;
+  uint64_t* spans;
+  uint64_t m;
+  if (int rc = all_spans_device(d_text, n, &spans, &m)) return rc;
+  if (limit && m > limit) m = limit;
+  uint64_t* d_slots = nullptr;
+  if (needs_groups && m) {  // `$1`, `$name`: the groups of every match (capture pass on the narrowed windows)
+    d_slots = (uint64_t*)cap_slots_.ensure(m * 2 * (uint64_t)n_groups_ * 8);
+    if (!d_slots) return fail("out of device memory (captures)");
+    if (int rc = captures_device(d_text, n, spans, m, d_slots)) return rc;
+  }
+  return replace_sums(d_text, n, spans, m, d_slots, out_len);
+}
+
+// ---- the replacement template (src/expand.rs:50-90) ----
+int Regex::replace_template(const uint8_t* rep, uint64_t rep_len, bool expand, bool* needs_groups_out) {
   rep_args_.assign(sizeof(ReplaceArgs), 0);
   ReplaceArgs& a = *reinterpret_cast<ReplaceArgs*>(rep_args_.data());
   a = ReplaceArgs{};
@@ -1667,18 +1707,18 @@ int Regex::replace_prepare(const uint8_t* d_text, uint64_t n, const uint8_t* rep
     }
   }
   if (!fits) return fail("replacement template has too many parts");
-  uint64_t* spans;
-  uint64_t m;
-  if (int rc = all_spans_device(d_text, n, &spans, &m)) return rc;
-  if (limit && m > limit) m = limit;
+  *needs_groups_out = needs_groups;
+  return 0;
+}
+
+int Regex::replace_sums(const uint8_t* d_text, uint64_t n, const uint64_t* spans, uint64_t m, const uint64_t* slots, uint64_t* out_len) {
+  ReplaceArgs& a = *reinterpret_cast<ReplaceArgs*>(rep_args_.data());
+  const std::vector<uint8_t>& lits = rep_lits_;
   cudaStream_t st = (cudaStream_t)stream_;
   uint64_t* lens = (uint64_t*)lens_.ensure(std::max<uint64_t>(m, 1) * 8);
   uint64_t* before = (uint64_t*)offset_.ensure(std::max<uint64_t>(m, 1) * 8);
-  const uint64_t n_blocks = (m + 1023) / 1024;
-  uint64_t* block_sums = (uint64_t*)block_sums_.ensure(std::max<uint64_t>(n_blocks, 1) * 8);
-  uint32_t* counters = (uint32_t*)counters_.ensure(128);
   uint8_t* d_lits = (uint8_t*)lits_.ensure(std::max<size_t>(lits.size(), 16));
-  if (!lens || !before || !block_sums || !counters || !d_lits) return fail("out of device memory (replace scratch)");
+  if (!lens || !before || !d_lits) return fail("out of device memory (replace scratch)");
   uint64_t* reps_before = (uint64_t*)reps_before_.ensure(std::max<uint64_t>(m, 1) * 8);
   if (!reps_before) return fail("out of device memory (replace scratch)");
   a.text = d_text;
@@ -1688,23 +1728,13 @@ int Regex::replace_prepare(const uint8_t* d_text, uint64_t n, const uint8_t* rep
   a.lens_before = before;
   a.reps_before = reps_before;
   a.lits = d_lits;
-  if (needs_groups && m) {  // `$1`, `$name`: the groups of every match (capture pass on the narrowed windows)
-    a.n_slots = 2 * (uint32_t)n_groups_;
-    uint64_t* d_slots = (uint64_t*)cap_slots_.ensure(m * a.n_slots * 8);
-    if (!d_slots) return fail("out of device memory (captures)");
-    if (int rc = captures_device(d_text, n, spans, m, d_slots)) return rc;
-    a.slots = d_slots;
-  }
+  a.slots = slots;
+  a.n_slots = slots ? 2 * (uint32_t)n_groups_ : 0;
   uint64_t matched = 0, replaced = 0;
   if (m) {
-    unsigned long long* grand = (unsigned long long*)(counters + 4);
     auto prefix = [&](uint64_t* out, uint64_t* total) -> int {  // exclusive prefix sum of lens[] into out[]
-      scan_counts_local<<<(uint32_t)n_blocks, 1024, 0, st>>>(lens, out, block_sums, m);
-      RB_LAUNCH_CHECK("scan_counts_local");
-      scan_block_sums<<<1, 1024, 0, st>>>(block_sums, n_blocks, grand);
-      RB_LAUNCH_CHECK("scan_block_sums");
-      scan_add_block_offsets<<<(uint32_t)n_blocks, 1024, 0, st>>>(out, block_sums, m);
-      RB_LAUNCH_CHECK("scan_add_block_offsets");
+      unsigned long long* grand;
+      if (int rc = prefix_sum(lens, out, m, &grand)) return rc;
       RB_CUDA(d2h(total, grand, 8));
       return 0;
     };
@@ -1841,7 +1871,7 @@ int Regex::captures_device(const uint8_t* d_text, uint64_t n, const uint64_t* d_
 
 // pike_captures over m spans (rec_offsets / rec_found: batched records, see launch.h CapArgs)
 int Regex::launch_captures(const uint8_t* d_text, uint64_t n, const uint64_t* d_spans, uint64_t m, uint64_t* d_slots,
-                           const uint64_t* rec_offsets, const uint32_t* rec_found) {
+                           const uint64_t* rec_offsets, const uint32_t* rec_found, const uint64_t* rec_csr, uint64_t n_rec) {
   CapArgs a{};
   a.insts = (const NfaInst*)cap_insts_.ptr;
   a.n_insts = cap_n_insts_;
@@ -1863,6 +1893,8 @@ int Regex::launch_captures(const uint8_t* d_text, uint64_t n, const uint64_t* d_
   if (!a.scratch) return fail("out of device memory (capture scratch)");
   a.rec_offsets = rec_offsets;
   a.rec_found = rec_found;
+  a.rec_csr = rec_csr;
+  a.n_rec = n_rec;
   pike_captures<<<(uint32_t)(threads / 64), 64, 0, (cudaStream_t)stream_>>>(a);
   RB_LAUNCH_CHECK("pike_captures");
   return 0;
@@ -1943,6 +1975,189 @@ int Regex::captures_all_host(const uint8_t* text, uint64_t n, uint64_t* slots, u
     count++;
   }
   *m = count;
+  return 0;
+}
+
+// ------------------------------------------- batched records: replacen / splitn / captures_iter ----
+// Each record is its own haystack.  The spans come from the per-record find_iter (iter_batch: record-relative,
+// CSR-shaped, in bspans_ / bmoff_).  Replace makes them relative to offsets[0] and runs the whole-haystack
+// kernels unchanged on the concatenated records; split and captures find each item's record by a binary search.
+int Regex::replace_batch_device(const uint8_t* d_text, const uint64_t* d_offsets, uint64_t n_rec, const uint8_t* rep, uint64_t rep_len,
+                                bool expand, uint64_t limit, uint64_t* d_out_offsets, uint8_t* d_out, uint64_t out_cap, uint64_t* out_len) {
+  std::lock_guard<std::recursive_mutex> lock(mu_);
+  *out_len = 0;
+  if (is_set_) return fail("replace requires exactly one pattern");
+  bool needs_groups = false;
+  if (int rc = replace_template(rep, rep_len, expand, &needs_groups)) return rc;
+  if (needs_groups)
+    if (int rc = ensure_capture_program()) return rc;
+  uint64_t* moff = (uint64_t*)bmoff_.ensure((n_rec + 1) * 8);
+  if (!moff) return fail("out of device memory (batch)");
+  uint64_t m = 0;
+  if (int rc = iter_batch(d_text, d_offsets, n_rec, moff, nullptr, 0, &m, &bspans_)) return rc;
+  cudaStream_t st = (cudaStream_t)stream_;
+  if (n_rec == 0) {
+    RB_CUDA(cudaMemsetAsync(d_out_offsets, 0, 8, st));
+    RB_CUDA(cudaStreamSynchronize(st));
+    return 0;
+  }
+  uint64_t* spans = (uint64_t*)bspans_.ptr;
+  if (limit && m > limit) {  // replacen: the first `limit` matches of every record
+    uint64_t* koff = (uint64_t*)bkoff_.ensure((n_rec + 1) * 8);
+    if (!koff) return fail("out of device memory (batch)");
+    csr_counts<<<grid_for(n_rec + 1, 256, 8), 256, 0, st>>>(moff, n_rec, limit, koff);
+    RB_LAUNCH_CHECK("csr_counts");
+    unsigned long long* grand;
+    if (int rc = prefix_sum(koff, koff, n_rec + 1, &grand)) return rc;
+    uint64_t kept = 0;
+    RB_CUDA(d2h(&kept, grand, 8));
+    if (kept < m) {
+      uint64_t* ks = (uint64_t*)bkspans_.ensure(std::max<uint64_t>(kept, 1) * 16);
+      if (!ks) return fail("out of device memory (batch spans)");
+      batch_keep_spans<<<grid_for(m, 256, 8), 256, 0, st>>>(moff, koff, n_rec, spans, m, ks);
+      RB_LAUNCH_CHECK("batch_keep_spans");
+      spans = ks;
+      moff = koff;
+      m = kept;
+    }
+  }
+  uint64_t first = 0, last = 0;
+  RB_CUDA(d2h(&first, d_offsets, 8));
+  RB_CUDA(d2h(&last, d_offsets + n_rec, 8));
+  const uint32_t ns = 2 * (uint32_t)n_groups_;
+  uint64_t* slots = nullptr;
+  if (needs_groups && m) {  // record-relative groups of every kept match, the window cut at its record's end
+    slots = (uint64_t*)bslots_.ensure(m * ns * 8);
+    if (!slots) return fail("out of device memory (captures)");
+    if (int rc = launch_captures(d_text, 0, spans, m, slots, d_offsets, nullptr, moff, n_rec)) return rc;
+  }
+  if (m) {
+    batch_to_base<<<grid_for(m, 256, 8), 256, 0, st>>>(d_offsets, moff, n_rec, spans, m, slots, ns);
+    RB_LAUNCH_CHECK("batch_to_base");
+  }
+  if (int rc = replace_sums(d_text + first, last - first, spans, m, slots, out_len)) return rc;
+  batch_replace_offsets<<<grid_for(n_rec + 1, 256, 8), 256, 0, st>>>(d_offsets, moff, n_rec, (const uint64_t*)offset_.ptr,
+                                                                      (const uint64_t*)reps_before_.ptr, m, rep_totals_[0], rep_totals_[1],
+                                                                      d_out_offsets);
+  RB_LAUNCH_CHECK("batch_replace_offsets");
+  if (!d_out) {
+    RB_CUDA(cudaStreamSynchronize(st));
+    return 0;
+  }
+  return replace_emit(d_out, out_cap);
+}
+
+int Regex::split_batch_device(const uint8_t* d_text, const uint64_t* d_offsets, uint64_t n_rec, bool has_limit, uint64_t limit,
+                              uint64_t* d_piece_offsets, uint64_t* d_pieces, uint64_t cap, uint64_t* n_total) {
+  std::lock_guard<std::recursive_mutex> lock(mu_);
+  *n_total = 0;
+  if (is_set_) return fail("split requires exactly one pattern");
+  if (int rc = init_device()) return rc;
+  cudaStream_t st = (cudaStream_t)stream_;
+  if (n_rec == 0 || (has_limit && limit == 0)) {  // re_bytes.rs:738-740: splitn(0) yields nothing
+    RB_CUDA(cudaMemsetAsync(d_piece_offsets, 0, (n_rec + 1) * 8, st));
+    RB_CUDA(cudaStreamSynchronize(st));
+    return 0;
+  }
+  uint64_t* moff = (uint64_t*)bmoff_.ensure((n_rec + 1) * 8);
+  if (!moff) return fail("out of device memory (batch)");
+  uint64_t m = 0;
+  if (int rc = iter_batch(d_text, d_offsets, n_rec, moff, nullptr, 0, &m, &bspans_)) return rc;
+  const uint64_t* spans = (const uint64_t*)bspans_.ptr;
+  batch_split_counts<<<grid_for(n_rec + 1, 256, 8), 256, 0, st>>>(d_offsets, moff, spans, n_rec, has_limit ? 1 : 0, limit, d_piece_offsets);
+  RB_LAUNCH_CHECK("batch_split_counts");
+  unsigned long long* grand;
+  if (int rc = prefix_sum(d_piece_offsets, d_piece_offsets, n_rec + 1, &grand)) return rc;
+  RB_CUDA(d2h(n_total, grand, 8));
+  const uint64_t k = d_pieces ? std::min(cap, *n_total) : 0;
+  if (k) {
+    batch_split_pieces<<<grid_for(k, 256, 8), 256, 0, st>>>(d_offsets, moff, spans, d_piece_offsets, n_rec, has_limit ? 1 : 0, limit,
+                                                            d_pieces, k);
+    RB_LAUNCH_CHECK("batch_split_pieces");
+  }
+  RB_CUDA(cudaStreamSynchronize(st));
+  return 0;
+}
+
+int Regex::captures_iter_batch_device(const uint8_t* d_text, const uint64_t* d_offsets, uint64_t n_rec, uint64_t* d_match_offsets,
+                                      uint64_t* d_slots, uint64_t cap, uint64_t* n_total) {
+  std::lock_guard<std::recursive_mutex> lock(mu_);
+  *n_total = 0;
+  if (int rc = ensure_capture_program()) return rc;
+  if (!d_slots) cap = 0;
+  uint64_t* moff = (uint64_t*)bmoff_.ensure((n_rec + 1) * 8);
+  if (!moff) return fail("out of device memory (batch)");
+  uint64_t m = 0;
+  if (int rc = iter_batch(d_text, d_offsets, n_rec, moff, nullptr, 0, &m, &bspans_)) return rc;
+  cudaStream_t st = (cudaStream_t)stream_;
+  if (n_rec == 0) {
+    RB_CUDA(cudaMemsetAsync(d_match_offsets, 0, 8, st));
+    RB_CUDA(cudaStreamSynchronize(st));
+    return 0;
+  }
+  const uint32_t ns = 2 * (uint32_t)n_groups_;
+  const uint64_t* spans = (const uint64_t*)bspans_.ptr;
+  const uint64_t words = (n_rec + 31) / 32;
+  uint64_t* slots = (uint64_t*)bslots_.ensure(std::max<uint64_t>(m, 1) * ns * 8);
+  uint32_t* flags = (uint32_t*)bflags_.ensure((words + 1) * 4);
+  uint64_t* list = (uint64_t*)blist_.ensure(n_rec * 8);
+  if (!slots || !flags || !list) return fail("out of device memory (captures)");
+  unsigned int* n_list = (unsigned int*)(flags + words);
+  RB_CUDA(cudaMemsetAsync(flags, 0, (words + 1) * 4, st));
+  if (m) {
+    if (int rc = launch_captures(d_text, 0, spans, m, slots, d_offsets, nullptr, moff, n_rec)) return rc;
+    batch_diverged<<<(uint32_t)((m + 255) / 256), 256, 0, st>>>(moff, n_rec, spans, m, slots, ns, flags, list, n_list);
+    RB_LAUNCH_CHECK("batch_diverged");
+  }
+  unsigned int n_redo = 0;
+  RB_CUDA(d2h(&n_redo, n_list, 4));
+  if (n_redo == 0) {  // group 0 is the find_iter span everywhere (always so without look-around): the CSR stands
+    RB_CUDA(cudaMemcpyAsync(d_match_offsets, moff, (n_rec + 1) * 8, cudaMemcpyDeviceToDevice, st));
+    if (std::min(cap, m)) RB_CUDA(cudaMemcpyAsync(d_slots, slots, std::min(cap, m) * ns * 8, cudaMemcpyDeviceToDevice, st));
+    RB_CUDA(cudaStreamSynchronize(st));
+    *n_total = m;
+    return 0;
+  }
+  // CaptureMatches (re_trait.rs:236-263) iterates on the NFA's group 0.  Where that differs from the find_iter span
+  // (the reverse-on-slice rule, SURVEY H1), captures_all_host, which follows the reference from the first such
+  // match on, reruns the record alone.  Such records are rare, so this path is driven from the host.  Everything
+  // it needs of d_text and d_offsets is read first: captures_all_host reuses the whole-haystack scratch.
+  std::vector<uint64_t> recs(n_redo);
+  RB_CUDA(d2h(recs.data(), list, n_redo * 8));
+  std::vector<std::vector<uint8_t>> bytes(n_redo);
+  for (unsigned int i = 0; i < n_redo; i++) {
+    uint64_t lohi[2];
+    RB_CUDA(d2h(lohi, d_offsets + recs[i], 16));
+    bytes[i].resize(lohi[1] - lohi[0]);
+    if (!bytes[i].empty()) RB_CUDA(d2h(bytes[i].data(), d_text + lohi[0], bytes[i].size()));
+  }
+  std::vector<std::vector<uint64_t>> rows(n_redo);
+  std::vector<uint64_t> counts(n_redo);
+  for (unsigned int i = 0; i < n_redo; i++) {
+    const uint64_t len = bytes[i].size(), room = len + 2;  // a record of len bytes has at most len + 1 matches
+    rows[i].resize(room * ns);
+    if (int rc = captures_all_host(bytes[i].data(), len, rows[i].data(), room, &counts[i])) return rc;
+  }
+  // the new CSR: the old counts with the redone ones, scanned; old rows move, redone rows are uploaded
+  uint64_t* cnt = (uint64_t*)bkoff_.ensure((n_rec + 1) * 8);
+  if (!cnt) return fail("out of device memory (batch)");
+  csr_counts<<<grid_for(n_rec + 1, 256, 8), 256, 0, st>>>(moff, n_rec, kNone, cnt);
+  RB_LAUNCH_CHECK("csr_counts");
+  for (unsigned int i = 0; i < n_redo; i++) RB_CUDA(cudaMemcpyAsync(cnt + recs[i], &counts[i], 8, cudaMemcpyHostToDevice, st));
+  unsigned long long* grand;
+  if (int rc = prefix_sum(cnt, d_match_offsets, n_rec + 1, &grand)) return rc;
+  RB_CUDA(d2h(n_total, grand, 8));
+  if (cap) {
+    batch_move_rows<<<grid_for(m, 256, 8), 256, 0, st>>>(moff, d_match_offsets, n_rec, flags, slots, m, ns, d_slots, cap);
+    RB_LAUNCH_CHECK("batch_move_rows");
+    for (unsigned int i = 0; i < n_redo; i++) {
+      uint64_t at = 0;
+      RB_CUDA(d2h(&at, d_match_offsets + recs[i], 8));
+      const uint64_t k = at < cap ? std::min(counts[i], cap - at) : 0;
+      if (k) RB_CUDA(cudaMemcpyAsync(d_slots + at * ns, rows[i].data(), k * ns * 8, cudaMemcpyHostToDevice, st));
+    }
+  }
+  RB_CUDA(cudaStreamSynchronize(st));
   return 0;
 }
 
@@ -2221,6 +2436,71 @@ int Regex::captures_batch_host(const uint8_t* text, const uint64_t* offsets, uin
   if ((rc = captures_batch_device(d, d_off, n_rec, d_slots, d_bits))) return rc;
   RB_CUDA(d2h(out_bits, d_bits, (n_rec + 7) / 8));
   RB_CUDA(d2h(slots, d_slots, n_rec * ns * 8));
+  return 0;
+}
+int Regex::upload_batch(const uint8_t* text, const uint64_t* offsets, uint64_t n_rec, const uint8_t** d_text, uint64_t** d_offsets) {
+  int rc;
+  *d_text = upload_text(text, n_rec ? offsets[n_rec] : 0, &rc);
+  if (rc) return rc;
+  *d_offsets = (uint64_t*)boffsets_.ensure((n_rec + 1) * 8);
+  if (!*d_offsets) return fail("out of device memory (batch)");
+  RB_CUDA(cudaMemcpyAsync(*d_offsets, offsets, (n_rec + 1) * 8, cudaMemcpyHostToDevice, (cudaStream_t)stream_));
+  return 0;
+}
+int Regex::replace_batch_host(const uint8_t* text, const uint64_t* offsets, uint64_t n_rec, const uint8_t* rep, uint64_t rep_len, bool expand,
+                              uint64_t limit, uint64_t* out_offsets, uint8_t* out, uint64_t out_cap, uint64_t* out_len) {
+  std::lock_guard<std::recursive_mutex> lock(mu_);
+  *out_len = 0;
+  const uint8_t* d;
+  uint64_t* d_off;
+  if (int rc = upload_batch(text, offsets, n_rec, &d, &d_off)) return rc;
+  uint64_t* d_oo = (uint64_t*)bres_off_.ensure((n_rec + 1) * 8);
+  if (!d_oo) return fail("out of device memory (batch)");
+  if (int rc = replace_batch_device(d, d_off, n_rec, rep, rep_len, expand, limit, d_oo, nullptr, 0, out_len)) return rc;
+  const uint64_t k = out ? std::min(out_cap, *out_len) : 0;
+  if (k) {
+    uint8_t* d_out = (uint8_t*)bres_.ensure(*out_len);
+    if (!d_out) return fail("out of device memory (replace output)");
+    if (int rc = replace_emit(d_out, *out_len)) return rc;
+    RB_CUDA(d2h(out, d_out, k));
+  }
+  RB_CUDA(d2h(out_offsets, d_oo, (n_rec + 1) * 8));
+  return 0;
+}
+int Regex::split_batch_host(const uint8_t* text, const uint64_t* offsets, uint64_t n_rec, bool has_limit, uint64_t limit, uint64_t* piece_offsets,
+                            uint64_t* pieces, uint64_t cap, uint64_t* n_total) {
+  std::lock_guard<std::recursive_mutex> lock(mu_);
+  *n_total = 0;
+  const uint8_t* d;
+  uint64_t* d_off;
+  if (int rc = upload_batch(text, offsets, n_rec, &d, &d_off)) return rc;
+  if (!pieces) cap = 0;
+  uint64_t* d_po = (uint64_t*)bres_off_.ensure((n_rec + 1) * 8);
+  uint64_t* d_p = cap ? (uint64_t*)bres_.ensure(cap * 16) : nullptr;
+  if (!d_po || (cap && !d_p)) return fail("out of device memory (batch pieces)");
+  if (int rc = split_batch_device(d, d_off, n_rec, has_limit, limit, d_po, d_p, cap, n_total)) return rc;
+  const uint64_t k = std::min(cap, *n_total);
+  if (k) RB_CUDA(d2h(pieces, d_p, k * 16));
+  RB_CUDA(d2h(piece_offsets, d_po, (n_rec + 1) * 8));
+  return 0;
+}
+int Regex::captures_iter_batch_host(const uint8_t* text, const uint64_t* offsets, uint64_t n_rec, uint64_t* match_offsets, uint64_t* slots,
+                                    uint64_t cap, uint64_t* n_total) {
+  std::lock_guard<std::recursive_mutex> lock(mu_);
+  *n_total = 0;
+  if (int rc = ensure_capture_program()) return rc;
+  const uint8_t* d;
+  uint64_t* d_off;
+  if (int rc = upload_batch(text, offsets, n_rec, &d, &d_off)) return rc;
+  if (!slots) cap = 0;
+  const uint64_t ns = 2 * (uint64_t)n_groups_;
+  uint64_t* d_mo = (uint64_t*)bres_off_.ensure((n_rec + 1) * 8);
+  uint64_t* d_s = cap ? (uint64_t*)bres_.ensure(cap * ns * 8) : nullptr;
+  if (!d_mo || (cap && !d_s)) return fail("out of device memory (batch captures)");
+  if (int rc = captures_iter_batch_device(d, d_off, n_rec, d_mo, d_s, cap, n_total)) return rc;
+  const uint64_t k = std::min(cap, *n_total);
+  if (k) RB_CUDA(d2h(slots, d_s, k * ns * 8));
+  RB_CUDA(d2h(match_offsets, d_mo, (n_rec + 1) * 8));
   return 0;
 }
 int Regex::find_batch_host(const uint8_t* text, const uint64_t* offsets, uint64_t n_rec, uint64_t* spans, uint8_t* out_bits) {

@@ -145,6 +145,18 @@ class Regex {
   // Regex::captures per record: d_slots[n_rec][2 * n_groups] record-relative (kNone = no group); d_bits = ballot
   // words, bit r set when record r matches
   int captures_batch_device(const uint8_t* d_text, const uint64_t* d_offsets, uint64_t n_rec, uint64_t* d_slots, uint32_t* d_bits);
+  // replace_device per record (limit per record, 0 = all): record r's output is d_out[d_out_offsets[r] ..
+  // d_out_offsets[r + 1]) (n_rec + 1 entries, always complete); at most out_cap bytes stored (d_out may be null to
+  // size); *out_len = all output bytes (host)
+  int replace_batch_device(const uint8_t* d_text, const uint64_t* d_offsets, uint64_t n_rec, const uint8_t* rep, uint64_t rep_len, bool expand,
+                           uint64_t limit, uint64_t* d_out_offsets, uint8_t* d_out, uint64_t out_cap, uint64_t* out_len);
+  // split_device per record: record r's pieces (record-relative) at d_pieces[d_piece_offsets[r] ..), at most cap stored
+  int split_batch_device(const uint8_t* d_text, const uint64_t* d_offsets, uint64_t n_rec, bool has_limit, uint64_t limit, uint64_t* d_piece_offsets,
+                         uint64_t* d_pieces, uint64_t cap, uint64_t* n_total);
+  // captures_all_host per record: record r's matches at d_slots[d_match_offsets[r] ..][2 * n_groups], record-relative,
+  // at most cap rows stored
+  int captures_iter_batch_device(const uint8_t* d_text, const uint64_t* d_offsets, uint64_t n_rec, uint64_t* d_match_offsets, uint64_t* d_slots,
+                                 uint64_t cap, uint64_t* n_total);
 
   // ---- host-buffer wrappers (copies inside; the e2e path) ---------------------
   int find_all_host(const uint8_t* text, uint64_t n, uint64_t start, uint64_t* out, uint64_t cap, uint64_t* total);
@@ -157,6 +169,12 @@ class Regex {
   int find_iter_batch_host(const uint8_t* text, const uint64_t* offsets, uint64_t n_rec, uint64_t* match_offsets, uint64_t* out,
                            uint64_t cap, uint64_t* total);
   int captures_batch_host(const uint8_t* text, const uint64_t* offsets, uint64_t n_rec, uint64_t* slots, uint8_t* out_bits);
+  int replace_batch_host(const uint8_t* text, const uint64_t* offsets, uint64_t n_rec, const uint8_t* rep, uint64_t rep_len, bool expand,
+                         uint64_t limit, uint64_t* out_offsets, uint8_t* out, uint64_t out_cap, uint64_t* out_len);
+  int split_batch_host(const uint8_t* text, const uint64_t* offsets, uint64_t n_rec, bool has_limit, uint64_t limit, uint64_t* piece_offsets,
+                       uint64_t* pieces, uint64_t cap, uint64_t* n_total);
+  int captures_iter_batch_host(const uint8_t* text, const uint64_t* offsets, uint64_t n_rec, uint64_t* match_offsets, uint64_t* slots,
+                               uint64_t cap, uint64_t* n_total);
 
   // Run on a caller-owned CUDA stream (e.g. torch's current stream) instead of the private one.
   void set_stream(void* cuda_stream) { ext_stream_ = cuda_stream; use_ext_stream_ = true; }
@@ -185,8 +203,19 @@ class Regex {
   int all_spans_device(const uint8_t* d_text, uint64_t n, uint64_t** d_spans, uint64_t* m);
   int ensure_capture_program();
   int launch_captures(const uint8_t* d_text, uint64_t n, const uint64_t* d_spans, uint64_t m, uint64_t* d_slots,
-                      const uint64_t* rec_offsets, const uint32_t* rec_found);
+                      const uint64_t* rec_offsets, const uint32_t* rec_found, const uint64_t* rec_csr = nullptr, uint64_t n_rec = 0);
+  // find_iter_batch_device; with grow (and d_out null) every span is stored in *grow, sized after the count pass
+  int iter_batch(const uint8_t* d_text, const uint64_t* d_offsets, uint64_t n_rec, uint64_t* d_match_offsets, uint64_t* d_out, uint64_t cap,
+                 uint64_t* total, DeviceBuf* grow);
+  // exclusive prefix sum of in[0, n) into out (in == out allowed); *d_total = device address of the sum
+  int prefix_sum(const uint64_t* in, uint64_t* out, uint64_t n, unsigned long long** d_total);
+  // text of every record of a host batch on the device (text_, boffsets_)
+  int upload_batch(const uint8_t* text, const uint64_t* offsets, uint64_t n_rec, const uint8_t** d_text, uint64_t** d_offsets);
   int replace_prepare(const uint8_t* d_text, uint64_t n, const uint8_t* rep, uint64_t rep_len, bool expand, uint64_t limit, uint64_t* out_len);
+  // the replacement template into rep_args_ / rep_lits_; *needs_groups = it refers to a group other than 0
+  int replace_template(const uint8_t* rep, uint64_t rep_len, bool expand, bool* needs_groups);
+  // prefix sums of the match and replacement lengths over m ordered spans of d_text[0, n) (slots: their groups, or null)
+  int replace_sums(const uint8_t* d_text, uint64_t n, const uint64_t* spans, uint64_t m, const uint64_t* slots, uint64_t* out_len);
   int replace_emit(uint8_t* d_out, uint64_t out_cap);
   bool plan_prefilter();  // fills pf_words_ (launch.h PfArgs) when every match has one of <= 4 bytes at a fixed offset
   int forward_reduce(const uint8_t* d_text, uint64_t n, uint64_t start, bool want_masks, uint64_t* result_host, uint64_t end = ~0ull,
@@ -228,6 +257,10 @@ class Regex {
   DeviceBuf cap_insts_, cap_scratch_, cap_slots_, cap_span_;
   uint32_t cap_n_insts_ = 0, cap_start_ = 0;  // capture program on the device (0 = not uploaded yet)
   bool cap_anchored_ = false;
+  // batched replace / split / captures_iter (never shared with the whole-haystack calls, which the per-record
+  // captures_iter redo runs in between): match CSR and spans, kept CSR and spans, slots, divergence flags and list,
+  // and the host wrappers' offsets and results
+  DeviceBuf bmoff_, bspans_, bkoff_, bkspans_, bslots_, bflags_, blist_, boffsets_, bres_off_, bres_;
   DeviceBuf in_p_, in_lm_, out_p_, out_lm_, count_, offset_, dirty_, first_cand_, skip_, meta_, excl_, btot_, present_, kidx_, kstates_, maps_, comp_, bentry_, exact_, stage_, block_sums_, out_, bits_, masks_;
   void* pinned_ = nullptr;  // small pinned staging area for counters / scalars
   void* timing_events_[3] = {nullptr, nullptr, nullptr};

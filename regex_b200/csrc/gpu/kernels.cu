@@ -2257,12 +2257,112 @@ __global__ void replace_matches(ReplaceArgs a) {
 }
 // Split (re_bytes.rs:699-721): piece i is the text between match i-1 and match i; the text after
 // the last match is a piece only when it is not empty; SplitN (:734-749): the n-th piece is the rest.
+__device__ __forceinline__ void split_piece(const uint64_t* spans, uint64_t n_matches, uint64_t n, uint64_t n_pieces, int last_is_rest, uint64_t i,
+                                            uint64_t* piece) {
+  piece[0] = i == 0 ? 0 : (i - 1 < n_matches ? spans[2 * (i - 1) + 1] : n);
+  piece[1] = (i < n_matches && !(last_is_rest && i + 1 == n_pieces)) ? spans[2 * i] : n;
+}
 __global__ void split_pieces(const uint64_t* spans, uint64_t n_matches, uint64_t n, uint64_t n_pieces, int last_is_rest, uint64_t* pieces, uint64_t cap) {
-  for (uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x; i < n_pieces && i < cap; i += (uint64_t)gridDim.x * blockDim.x) {
-    const uint64_t from = i == 0 ? 0 : (i - 1 < n_matches ? spans[2 * (i - 1) + 1] : n);
-    const uint64_t to = (i < n_matches && !(last_is_rest && i + 1 == n_pieces)) ? spans[2 * i] : n;
-    pieces[2 * i] = from;
-    pieces[2 * i + 1] = to;
+  for (uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x; i < n_pieces && i < cap; i += (uint64_t)gridDim.x * blockDim.x)
+    split_piece(spans, n_matches, n, n_pieces, last_is_rest, i, pieces + 2 * i);
+}
+
+// ------------------------------------ batched records: replacen / splitn / captures_iter ----
+// Per-record forms of the loops above.  Every item (match, piece) finds its record by a binary search in a CSR
+// list rather than one thread walking each record, so a record with a million matches does not serialise.
+// The record of item i: the last r with csr[r] <= i (csr[0] = 0 <= i < csr[n_rec]; empty records are passed over).
+__device__ __forceinline__ uint64_t csr_row(const uint64_t* csr, uint64_t n_rec, uint64_t i) {
+  uint64_t lo = 0, hi = n_rec;
+  while (hi - lo > 1) {
+    const uint64_t mid = (lo + hi) >> 1;
+    if (csr[mid] <= i) lo = mid; else hi = mid;
+  }
+  return lo;
+}
+__global__ void csr_counts(const uint64_t* csr, uint64_t n_rec, uint64_t limit, uint64_t* counts) {
+  for (uint64_t r = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x; r <= n_rec; r += (uint64_t)gridDim.x * blockDim.x)
+    counts[r] = r < n_rec ? min(csr[r + 1] - csr[r], limit) : 0;
+}
+__global__ void batch_keep_spans(const uint64_t* csr, const uint64_t* kcsr, uint64_t n_rec, const uint64_t* spans, uint64_t m, uint64_t* kept) {
+  for (uint64_t j = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x; j < m; j += (uint64_t)gridDim.x * blockDim.x) {
+    const uint64_t r = csr_row(csr, n_rec, j), i = j - csr[r];
+    if (i < kcsr[r + 1] - kcsr[r]) {
+      kept[2 * (kcsr[r] + i)] = spans[2 * j];
+      kept[2 * (kcsr[r] + i) + 1] = spans[2 * j + 1];
+    }
+  }
+}
+__global__ void batch_to_base(const uint64_t* offsets, const uint64_t* csr, uint64_t n_rec, uint64_t* spans, uint64_t m, uint64_t* slots,
+                              uint32_t n_slots) {
+  for (uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x; i < m; i += (uint64_t)gridDim.x * blockDim.x) {
+    const uint64_t b = offsets[csr_row(csr, n_rec, i)] - offsets[0];
+    spans[2 * i] += b;
+    spans[2 * i + 1] += b;
+    if (slots)
+      for (uint32_t k = 0; k < n_slots; k++)
+        if (slots[i * n_slots + k] != kNone) slots[i * n_slots + k] += b;
+  }
+}
+// With the spans of all records in one ordered list relative to offsets[0], the records' outputs are the pieces of
+// the concatenated output: record r's output begins where its first kept match K would have landed had it been
+// its first byte, i.e. at (offsets[r] - offsets[0]) - L[K] + P[K] (replace_gaps' shift).
+__global__ void batch_replace_offsets(const uint64_t* offsets, const uint64_t* csr, uint64_t n_rec, const uint64_t* lens_before,
+                                      const uint64_t* reps_before, uint64_t m, uint64_t matched_total, uint64_t replaced_total,
+                                      uint64_t* out_offsets) {
+  for (uint64_t r = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x; r <= n_rec; r += (uint64_t)gridDim.x * blockDim.x) {
+    const uint64_t k = csr[r];
+    const uint64_t l = k < m ? lens_before[k] : matched_total, p = k < m ? reps_before[k] : replaced_total;
+    out_offsets[r] = offsets[r] - offsets[0] - l + p;
+  }
+}
+// split_device per record: one piece per match, the rest when it is not empty; SplitN clamps to `limit`, and the
+// limit-th piece is the rest (so limit 0 gives none and limit 1 the whole record, even an empty one)
+__global__ void batch_split_counts(const uint64_t* offsets, const uint64_t* csr, const uint64_t* spans, uint64_t n_rec, int has_limit,
+                                   uint64_t limit, uint64_t* counts) {
+  for (uint64_t r = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x; r <= n_rec; r += (uint64_t)gridDim.x * blockDim.x) {
+    if (r == n_rec) { counts[r] = 0; continue; }
+    const uint64_t c = csr[r + 1] - csr[r], len = offsets[r + 1] - offsets[r];
+    const uint64_t last_end = c ? spans[2 * (csr[r + 1] - 1) + 1] : 0;
+    uint64_t p = c + (last_end < len ? 1 : 0);
+    if (has_limit && p + 1 >= limit) p = limit;
+    counts[r] = p;
+  }
+}
+__global__ void batch_split_pieces(const uint64_t* offsets, const uint64_t* csr, const uint64_t* spans, const uint64_t* pcsr, uint64_t n_rec,
+                                   int has_limit, uint64_t limit, uint64_t* pieces, uint64_t n_out) {
+  for (uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x; i < n_out; i += (uint64_t)gridDim.x * blockDim.x) {
+    const uint64_t r = csr_row(pcsr, n_rec, i), np = pcsr[r + 1] - pcsr[r];
+    // a record has `limit` pieces only when the SplitN clamp applied (otherwise it has fewer than limit - 1)
+    split_piece(spans + 2 * csr[r], csr[r + 1] - csr[r], offsets[r + 1] - offsets[r], np, has_limit && np == limit, i - pcsr[r], pieces + 2 * i);
+  }
+}
+__global__ void batch_diverged(const uint64_t* csr, uint64_t n_rec, const uint64_t* spans, uint64_t m, const uint64_t* slots, uint32_t n_slots,
+                               uint32_t* flags, uint64_t* list, unsigned int* n_list) {
+  const uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x;
+  const uint32_t lane = threadIdx.x & 31;
+  uint64_t r = 0;
+  bool first = false;
+  if (i < m && (slots[i * n_slots] != spans[2 * i] || slots[i * n_slots + 1] != spans[2 * i + 1])) {
+    r = csr_row(csr, n_rec, i);
+    const uint32_t bit = 1u << (r & 31);
+    first = !(atomicOr(&flags[r >> 5], bit) & bit);
+  }
+  const uint32_t b = __ballot_sync(0xffffffffu, first);
+  if (!b) return;
+  const int leader = __ffs(b) - 1;
+  unsigned int base = 0;
+  if ((int)lane == leader) base = atomicAdd(n_list, (unsigned int)__popc(b));
+  base = __shfl_sync(0xffffffffu, base, leader);
+  if (first) list[base + __popc(b & ((1u << lane) - 1))] = r;
+}
+__global__ void batch_move_rows(const uint64_t* csr, const uint64_t* new_csr, uint64_t n_rec, const uint32_t* skip, const uint64_t* src, uint64_t m,
+                                uint32_t width, uint64_t* dst, uint64_t cap) {
+  for (uint64_t j = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x; j < m; j += (uint64_t)gridDim.x * blockDim.x) {
+    const uint64_t r = csr_row(csr, n_rec, j);
+    if ((skip[r >> 5] >> (r & 31)) & 1u) continue;
+    const uint64_t d = new_csr[r] + (j - csr[r]);
+    if (d >= cap) continue;
+    for (uint32_t k = 0; k < width; k++) dst[d * width + k] = src[j * width + k];
   }
 }
 
@@ -2349,9 +2449,11 @@ __global__ void pike_captures(CapArgs a) {
     const uint8_t* text = a.text;  // the text the match is relative to: the haystack, or record m
     uint64_t tn = a.n;
     if (a.rec_offsets) {
-      if (!((a.rec_found[m >> 5] >> (m & 31)) & 1u)) continue;
-      text = a.text + a.rec_offsets[m];
-      tn = a.rec_offsets[m + 1] - a.rec_offsets[m];
+      uint64_t r = m;
+      if (a.rec_csr) r = csr_row(a.rec_csr, a.n_rec, m);
+      else if (!((a.rec_found[m >> 5] >> (m & 31)) & 1u)) continue;
+      text = a.text + a.rec_offsets[r];
+      tn = a.rec_offsets[r + 1] - a.rec_offsets[r];
     }
     // the window ends two characters past the match (look-ahead needs them; utf8.rs:24-40 next_utf8)
     uint64_t n = e;

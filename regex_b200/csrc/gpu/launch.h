@@ -125,6 +125,34 @@ __global__ void replace_matches(ReplaceArgs a);
 // pieces[i] = text between match i-1 and match i; limit as splitn (0 = none)
 __global__ void split_pieces(const uint64_t* spans, uint64_t n_matches, uint64_t n, uint64_t n_pieces, int last_is_rest, uint64_t* pieces, uint64_t cap);
 
+// ---- batched records: replacen / splitn / captures_iter per record (engine.cu *_batch_device) ----
+// A CSR list (csr[n_rec + 1], csr[0] = 0) gives the items of record r at [csr[r], csr[r + 1]); spans are record-relative.
+// counts[r] = min(csr[r + 1] - csr[r], limit), counts[n_rec] = 0 (ready for an exclusive scan into a new CSR)
+__global__ void csr_counts(const uint64_t* csr, uint64_t n_rec, uint64_t limit, uint64_t* counts);
+// the first kcsr[r + 1] - kcsr[r] spans of every record, compacted to kept[kcsr[r] ..)
+__global__ void batch_keep_spans(const uint64_t* csr, const uint64_t* kcsr, uint64_t n_rec, const uint64_t* spans, uint64_t m, uint64_t* kept);
+// record-relative -> relative to offsets[0]: spans and, when slots is not null, every group slot that took part
+__global__ void batch_to_base(const uint64_t* offsets, const uint64_t* csr, uint64_t n_rec, uint64_t* spans, uint64_t m, uint64_t* slots,
+                              uint32_t n_slots);
+// out_offsets[r] = (offsets[r] - offsets[0]) - L[csr[r]] + P[csr[r]]; L / P = lens_before / reps_before extended by the totals
+__global__ void batch_replace_offsets(const uint64_t* offsets, const uint64_t* csr, uint64_t n_rec, const uint64_t* lens_before,
+                                      const uint64_t* reps_before, uint64_t m, uint64_t matched_total, uint64_t replaced_total,
+                                      uint64_t* out_offsets);
+// pieces of every record as split_device counts them (counts[n_rec] = 0); has_limit / limit as splitn
+__global__ void batch_split_counts(const uint64_t* offsets, const uint64_t* csr, const uint64_t* spans, uint64_t n_rec, int has_limit,
+                                   uint64_t limit, uint64_t* counts);
+// piece i < n_out of the piece CSR pcsr, record-relative (split_pieces of its record)
+__global__ void batch_split_pieces(const uint64_t* offsets, const uint64_t* csr, const uint64_t* spans, const uint64_t* pcsr, uint64_t n_rec,
+                                   int has_limit, uint64_t limit, uint64_t* pieces, uint64_t n_out);
+// records where the NFA's group 0 of some match differs from its find_iter span: bit r of flags (zeroed before) set
+// once, r appended to list[*n_list]
+__global__ void batch_diverged(const uint64_t* csr, uint64_t n_rec, const uint64_t* spans, uint64_t m, const uint64_t* slots, uint32_t n_slots,
+                               uint32_t* flags, uint64_t* list, unsigned int* n_list);
+// rows (width words) of the records whose bit in skip is clear, from their place in csr to their place in new_csr
+// (rows at or beyond cap are dropped)
+__global__ void batch_move_rows(const uint64_t* csr, const uint64_t* new_csr, uint64_t n_rec, const uint32_t* skip, const uint64_t* src, uint64_t m,
+                                uint32_t width, uint64_t* dst, uint64_t cap);
+
 // ---- capture groups on the narrowed window (src/exec.rs:861-875, src/pikevm.rs:130-352) ----
 struct NfaInst { uint32_t op_look_lo_hi; uint32_t a, b; };  // op | look << 8 | lo << 16 | hi << 24; a, b as rb::Inst
 struct CapArgs {
@@ -142,6 +170,10 @@ struct CapArgs {
   // the record is the text; records whose bit in rec_found (ballot words) is clear are skipped
   const uint64_t* rec_offsets;
   const uint32_t* rec_found;
+  // batched records with any number of matches each (null otherwise; rec_found is then unused): match m belongs
+  // to the record r with rec_csr[r] <= m < rec_csr[r + 1] (n_rec + 1 entries)
+  const uint64_t* rec_csr;
+  uint64_t n_rec;
 };
 __global__ void pike_captures(CapArgs a);
 // ballot words: bit r = group 0 of record r took part (slots[r * n_slots] != kNone)
