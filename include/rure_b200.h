@@ -245,14 +245,17 @@ uint64_t rure_b200_kernel_launches(void);
 void rure_b200_last_stats(rure *re, double *out8);
 /* The same plus out[8..11] = sequential stitch passes, state-map passes (segments run from
  * every boundary state), waves of the last forward search, path of the last find_all
- * (0 generic scan, 1 fast scan, 2 fused scan+walk, 3 literal prefilter), out[12] = matches longer
+ * (0 generic scan, 1 fast scan, 2 fused scan+walk, 3 literal prefilter, 4 candidate starts: a pattern whose
+ * unanchored automata exceed the DFA budget, searched with the anchored one), out[12] = matches longer
  * than 256 KiB that were measured by the parallel long-run pass.  n = doubles to write. */
 void rure_b200_last_stats_ex(rure *re, double *out, size_t n);
 void rure_b200_set_last_stats_ex(rure_set *set, double *out, size_t n);
 /* Named knobs (tests, tuning): "wave0" bytes of the first wave of is_match / shortest_match /
  * set matches (x16 per wave, 0 = one wave), "narrow_sets" 0/1, "max_stitch_rounds",
  * "max_redo_rounds", "batch_refill" 0/1 (batched is_match: lanes refill from a task of records), "prefilter" (0 never, 1 automatic: only for a single rare byte, 2 whenever the
- * pattern qualifies).  Returns false for an unknown name. */
+ * pattern qualifies), "candidate_starts" 0/1 (tests: search from candidate starts with the anchored
+ * automaton, as patterns over the DFA budget do, even when the unanchored automata fit).
+ * Returns false for an unknown name. */
 bool rure_b200_set_option(rure *re, const char *name, uint64_t value);
 bool rure_b200_set_set_option(rure_set *set, const char *name, uint64_t value);
 /* seg/chunk are positions per scan segment / walk chunk (multiples of 64);
@@ -271,7 +274,8 @@ void rure_b200_set_fuse(rure *re, int yes);
 void rure_b200_set_tensor_tma(rure *re, int yes);
 /* Dense tables, for tests and tooling.  kind: 0 forward anchored leftmost-first,
  * 1 reverse unanchored all-match, 2 forward unanchored all-match, 3 reverse
- * anchored longest, 4 forward unanchored leftmost-first.
+ * anchored longest, 4 forward unanchored leftmost-first.  A pattern searched from candidate
+ * starts has kinds 0 and 3 only: kinds 1, 2 and 4 return false with a message.
  * info[0..5] = n_states, n_classes (last = EOF), match_lo, mask_words, uniform_start, raw_states.
  * Buffers may be NULL to query sizes: trans n_states*n_classes u16, classes 256 u8,
  * start 128 u16, masks n_states*mask_words u64. */

@@ -574,6 +574,7 @@ static bool set_option(Regex* r, const char* name, uint64_t value) {
   else if (k == "max_stitch_rounds") t.max_stitch_rounds = (uint32_t)value;
   else if (k == "max_redo_rounds") t.max_redo_rounds = (uint32_t)value;
   else if (k == "prefilter") t.prefilter = (int)value;
+  else if (k == "candidate_starts") t.candidate_starts = value != 0;
   else { g_last_error = "unknown option: " + k; return false; }
   return true;
 }

@@ -133,10 +133,29 @@ Regex* Regex::compile(const std::vector<std::string>& patterns, const CompileOpt
     return nullptr;
   }
   // Determinize the tables every object needs so budget errors surface at compile time.
-  if (!re->host_dfa(kFwdUnanchoredAll, err)) return nullptr;
-  if (!re->is_set_) {
-    if (!re->host_dfa(kFwdAnchoredLF, err)) return nullptr;
-    if (!re->host_dfa(kRevUnanchoredAll, err)) return nullptr;
+  if (re->is_set_) {  // set semantics need the all-match product automaton
+    if (!re->host_dfa(kFwdUnanchoredAll, err)) return nullptr;
+    return re.release();
+  }
+  // A single pattern: the anchored automaton first (cheap).  When it fits but an unanchored one does not (it tracks
+  // every earlier start that may still begin a match: `error.{0,100}timeout` has 2^100 such subsets), the object
+  // searches from candidate starts with kinds 0 and 3 (DESIGN.md §2).  Only one over-budget unanchored
+  // determinization is paid for.  When kind 0 or kind 3 is over budget as well, the error is the one an eager
+  // kind 2, 0, 1 sequence reports.
+  if (!re->host_dfa(kFwdAnchoredLF, err)) {
+    rb::Error e2;
+    if (!re->host_dfa(kFwdUnanchoredAll, &e2)) *err = e2;
+    return nullptr;
+  }
+  for (DfaKind k : {kFwdUnanchoredAll, kRevUnanchoredAll}) {
+    if (re->host_dfa(k, err)) continue;
+    if (err->kind != rb::Error::DfaTooBig) return nullptr;
+    rb::Error e3;
+    if (!re->host_dfa(kRevAnchoredLongest, &e3)) return nullptr;  // *err: the unanchored automaton's error
+    re->unanchored_too_big_ = true;
+    for (DfaKind u : {kRevUnanchoredAll, kFwdUnanchoredAll, kFwdUnanchoredLF}) re->host_[u].reset();
+    *err = rb::Error();
+    break;
   }
   return re.release();
 }
@@ -157,6 +176,12 @@ const rb::Dfa* Regex::host_dfa(DfaKind k, rb::Error* err) {
   if (patterns_.empty()) {  // an empty RegexSet matches nothing and has no automaton
     err->kind = rb::Error::Syntax;
     err->msg = "an empty pattern set has no automaton";
+    return nullptr;
+  }
+  if (unanchored_too_big_ && k != kFwdAnchoredLF && k != kRevAnchoredLongest) {
+    err->kind = rb::Error::DfaTooBig;
+    err->msg = "the unanchored automata of this pattern exceed the DFA table budget: it is searched from candidate starts "
+               "with the anchored automata (kinds 0 and 3) only";
     return nullptr;
   }
   rb::CompileOptions co;
@@ -376,7 +401,30 @@ static const uint16_t kByteFreq[256] = {
 // 1.33 TB/s here and at 2.93 TB/s on the fused DFA path, so the automatic choice is conservative:
 static constexpr uint32_t kPrefilterMaxFreq = 600;   // structural limit (tuning.prefilter == 2): ~0.9 % of the bytes
 static constexpr uint32_t kPrefilterAutoFreq = 80;   // automatic (tuning.prefilter == 1): ~0.12 %, i.e. one rare byte
-static constexpr uint32_t kPrefilterState = 0xFFFEu; // what a prefilter shard reports as its boundary states
+static constexpr uint32_t kPrefilterState = 0xFFFEu; // what a prefilter or candidate-start shard reports as its boundary states
+
+// allowed[d][b] = 1 when some start state of the anchored automaton d survives d + 1 steps with byte b as the last one
+// (every match of at least `depth` bytes has such a byte at offset d).  Start states: all of them unless uniform.
+static std::vector<std::vector<uint8_t>> start_byte_sets(const rb::Dfa& d, uint32_t depth) {
+  std::vector<std::vector<uint8_t>> allowed(depth, std::vector<uint8_t>(256, 0));
+  std::vector<uint8_t> reach(d.n_states, 0), next(d.n_states, 0);
+  if (d.uniform_start) reach[d.start[32]] = 1;
+  else for (uint16_t s : d.start) reach[s] = 1;
+  reach[0] = 0;
+  for (uint32_t dep = 0; dep < depth; dep++) {
+    std::fill(next.begin(), next.end(), 0);
+    for (uint32_t st = 1; st < d.n_states; st++) {
+      if (!reach[st]) continue;
+      for (int b = 0; b < 256; b++) {
+        const uint16_t t = d.next((uint16_t)st, (uint8_t)b);
+        if (t) { allowed[dep][b] = 1; next[t] = 1; }
+      }
+    }
+    reach.swap(next);
+  }
+  return allowed;
+}
+
 bool Regex::plan_prefilter() {
   if (pf_state_) return pf_state_ > 0;
   pf_state_ = -1;
@@ -385,20 +433,7 @@ bool Regex::plan_prefilter() {
   const rb::Dfa* d = host_dfa(kFwdAnchoredLF, &err);
   if (!d || !d->uniform_start) return false;
   const uint32_t depth = (uint32_t)std::min<uint64_t>(min_len, 8);
-  std::vector<std::vector<uint8_t>> allowed(depth, std::vector<uint8_t>(256, 0));
-  std::vector<uint8_t> reach(d->n_states, 0), next(d->n_states, 0);
-  reach[d->start[32]] = 1;
-  for (uint32_t dep = 0; dep < depth; dep++) {
-    std::fill(next.begin(), next.end(), 0);
-    for (uint32_t st = 1; st < d->n_states; st++) {
-      if (!reach[st]) continue;
-      for (int b = 0; b < 256; b++) {
-        const uint16_t t = d->next((uint16_t)st, (uint8_t)b);
-        if (t) { allowed[dep][b] = 1; next[t] = 1; }
-      }
-    }
-    reach.swap(next);
-  }
+  const std::vector<std::vector<uint8_t>> allowed = start_byte_sets(*d, depth);
   uint32_t best_o = 0, best_f = ~0u;
   for (uint32_t o = 0; o < depth; o++) {
     uint32_t cnt = 0, f = 0;
@@ -417,6 +452,138 @@ bool Regex::plan_prefilter() {
   pf_freq_ = best_f;
   pf_state_ = 1;
   return true;
+}
+
+// ---------------------------------------------------------- candidate starts --
+// Candidate-start mode (DESIGN.md §2).  find_at(p) = (s*, A(s*)) with s* the first position >= p at which the
+// anchored automaton A finds a match; that holds for any superset of the match starts, so kind 0 (and kind 3 for
+// the reverse-on-slice rule) answers every single-pattern call.  The candidates: positions whose first
+// D = min(min_len, 4) bytes lie in the byte sets of start_byte_sets; every position when min_len == 0.
+int Regex::cand_args(void* out) {
+  if (cand_image_.empty()) {
+    rb::Error err;
+    const rb::Dfa* d = host_dfa(kFwdAnchoredLF, &err);
+    if (!d) return fail(err.msg);
+    CandArgs c{};
+    c.depth = (uint32_t)std::min<uint64_t>(min_len, 4);
+    const std::vector<std::vector<uint8_t>> allowed = start_byte_sets(*d, c.depth);
+    for (uint32_t dep = 0; dep < c.depth; dep++)
+      for (int b = 0; b < 256; b++) if (allowed[dep][b]) c.mask[b] |= (uint8_t)(1u << dep);
+    c.utf8_boundaries = only_utf8 && can_match_empty;  // as scan_starts: the reverse scan drops those starts too
+    c.slice_rule = has_looks;
+    cand_image_.resize(sizeof c);
+    std::memcpy(cand_image_.data(), &c, sizeof c);
+  }
+  std::memcpy(out, cand_image_.data(), sizeof(CandArgs));
+  return 0;
+}
+
+int Regex::cand_starts(const uint8_t* d_text, uint64_t n, uint64_t base, uint64_t limit, bool text_continues) {
+  CandArgs c;
+  if (int rc = cand_args(&c)) return rc;
+  uint64_t* bm = (uint64_t*)bitmap_.ensure(((n >> 6) + 2) * 8);
+  uint32_t* counters = (uint32_t*)counters_.ensure(128);
+  if (!bm || !counters) return fail("out of device memory (bitmap)");
+  const uint64_t words = std::max<uint64_t>(1, ((limit + 63) >> 6) - (base >> 6));
+  cand_bitmap<<<grid_for(words, 256, 8), 256, 0, (cudaStream_t)stream_>>>(d_text, n, base, limit, text_continues ? 1 : 0, c, bm,
+                                                                        (uint8_t*)(counters + 24));
+  RB_LAUNCH_CHECK("cand_bitmap");
+  return 0;
+}
+
+// shortest_match / is_match: min over the candidates s >= start of the first match state the anchored automaton
+// enters from s, in the waves of forward_reduce (64 MiB, x16 each); a wave is the last one once the best end lies
+// at or before the next wave's first candidate.
+int Regex::cand_shortest(const uint8_t* d_text, uint64_t n, uint64_t start, bool* found, uint64_t* end) {
+  DeviceDfa* fwd;
+  if (int rc = ensure(kFwdAnchoredLF, &fwd)) return rc;
+  CandArgs c;
+  if (int rc = cand_args(&c)) return rc;
+  c.utf8_boundaries = 0;  // the earliest end: an empty match inside a UTF-8 sequence never ends before one at `start`
+  cudaStream_t st = (cudaStream_t)stream_;
+  if (lazy_ && lazy_->done < lazy_->n) {  // host haystack: an anchored run may read to its end
+    RB_CUDA(cudaMemcpyAsync(lazy_->dst + lazy_->done, lazy_->src + lazy_->done, lazy_->n - lazy_->done, cudaMemcpyHostToDevice, st));
+    lazy_->done = lazy_->n;
+  }
+  uint32_t* counters = (uint32_t*)counters_.ensure(128);
+  if (!counters) return fail("out of device memory (counters)");
+  unsigned long long* best = (unsigned long long*)(counters + 20);
+  RB_CUDA(cudaMemsetAsync(best, 0xFF, 8, st));
+  const size_t smem = smem_for(fwd->view);
+  RB_CUDA(allow_smem(rbgpu::cand_shortest, smem));  // (the kernel, not this member)
+  const uint32_t seg = 1024;
+  uint64_t wave = tuning.wave0 ? (tuning.wave0 + 4095) / 4096 * 4096 : 0;
+  uint64_t lo = start, b = kNone;
+  const uint64_t hi = n + 1;  // candidate positions [start, n]
+  stats.scan_redo_rounds = stats.scan_redo_segments = stats.map_passes = stats.waves = 0;
+  for (;;) {
+    uint64_t limit = hi;
+    if (wave && hi - lo > 2 * wave) limit = lo + wave;
+    const uint64_t n_seg = (limit - lo + seg - 1) / seg;
+    rbgpu::cand_shortest<<<grid_for(n_seg, 256, tuning.blocks_per_sm), 256, smem, st>>>(fwd->view, smem != 0, c, d_text, n, lo, limit, seg, best);
+    RB_LAUNCH_CHECK("cand_shortest");
+    stats.waves++;
+    RB_CUDA(d2h(&b, best, 8));
+    if (limit == hi || (b != kNone && b <= limit)) break;
+    lo = limit;
+    wave *= 16;
+  }
+  if (b != kNone) { *found = true; *end = b; }
+  return 0;
+}
+
+// Batched find / find_iter run the unanchored leftmost-first automaton (kind 4), built on first use.  When it is
+// over the budget the object switches to candidate starts instead of failing (kind 3 must fit).
+int Regex::batch_route(bool* cand) {
+  *cand = candidate_mode();
+  if (*cand) return 0;
+  rb::Error err;
+  if (host_dfa(kFwdUnanchoredLF, &err)) return 0;
+  if (err.kind != rb::Error::DfaTooBig) return fail(err.msg);
+  rb::Error e3;
+  if (!host_dfa(kRevAnchoredLongest, &e3)) return fail(err.msg);
+  unanchored_too_big_ = true;
+  *cand = true;
+  return 0;
+}
+
+int Regex::cand_batch(int mode, const uint8_t* d_text, const uint64_t* d_offsets, uint64_t n_rec, uint32_t* d_bits, uint64_t* d_spans,
+                      uint64_t* d_match_offsets, uint64_t cap) {
+  DeviceDfa *fwd, *rev = nullptr;
+  if (int rc = ensure(kFwdAnchoredLF, &fwd)) return rc;
+  if (mode != 0 && has_looks) if (int rc = ensure(kRevAnchoredLongest, &rev)) return rc;
+  CandArgs c;
+  if (int rc = cand_args(&c)) return rc;
+  BatchArgs a{};
+  a.fwd = fwd->view;
+  if (rev) a.rev = rev->view;
+  const size_t smem = smem_for(fwd->view);
+  a.use_smem = smem != 0;
+  a.text = d_text;
+  a.offsets = d_offsets;
+  a.n_rec = n_rec;
+  a.out_bits = d_bits;
+  a.out_spans = d_spans;
+  a.match_offsets = d_match_offsets;
+  a.cap = cap;
+  a.utf8 = only_utf8 ? 1 : 0;
+  cudaStream_t st = (cudaStream_t)stream_;
+  const uint32_t grid = grid_for(n_rec, 256, tuning.blocks_per_sm);
+#define RB_CAND(M)                                              \
+  {                                                             \
+    RB_CUDA(allow_smem(batch_cand<M>, smem));                   \
+    batch_cand<M><<<grid, 256, smem, st>>>(a, c);               \
+    RB_LAUNCH_CHECK("batch_cand<" #M ">");                      \
+  }
+  switch (mode) {
+    case 0: RB_CAND(0) break;
+    case 1: RB_CAND(1) break;
+    case 2: RB_CAND(2) break;
+    default: RB_CAND(3) break;
+  }
+#undef RB_CAND
+  if (mode <= 1) RB_CUDA(cudaStreamSynchronize(st));
+  return 0;
 }
 
 // ------------------------------------------------------------ long matches ----
@@ -782,16 +949,18 @@ int Regex::find_all_shard_device(const uint8_t* d_text, uint64_t n, ShardIO* io,
   if (int rc = ensure(kFwdAnchoredLF, &fwd)) return rc;
   const bool emulate = has_looks;
   if (emulate) if (int rc = ensure(kRevAnchoredLongest, &rev)) return rc;
-  DeviceDfa* revall;
-  if (int rc = ensure(kRevUnanchoredAll, &revall)) return rc;
+  // candidate-start mode: the start bitmap is a superset of the match starts (cand_bitmap), not the reverse scan's
+  const bool cand = candidate_mode();
+  DeviceDfa* revall = nullptr;
+  if (!cand) if (int rc = ensure(kRevUnanchoredAll, &revall)) return rc;
   cudaStream_t st = (cudaStream_t)stream_;
   cudaEvent_t ev[3] = {(cudaEvent_t)timing_events_[0], (cudaEvent_t)timing_events_[1], (cudaEvent_t)timing_events_[2]};
   RB_CUDA(cudaEventRecord(ev[0], st));
   const ScanPlan plan = plan_scan(d_text, io->own_lo, io->own_hi,
-                                   hot_signed_ok(revall->hot) && fast_scan_smem(hot_bytes_signed(revall->hot)) <= 227 * 1024);
-  // runner: 2 = fixed-length (no haystack access), 1 = byte-indexed shared-memory table
-  // (uniform start state, 8-byte aligned text), 0 = generic
-  const bool wfixed = min_len == max_len && min_len > 0 && !emulate && !tuning.force_generic;
+                                   !cand && hot_signed_ok(revall->hot) && fast_scan_smem(hot_bytes_signed(revall->hot)) <= 227 * 1024);
+  // runner: 2 = fixed-length (no haystack access: every candidate must be a match start, so not with candidate
+  // starts), 1 = byte-indexed shared-memory table (uniform start state, 8-byte aligned text), 0 = generic
+  const bool wfixed = min_len == max_len && min_len > 0 && !emulate && !tuning.force_generic && !cand;
   const bool wfast = !wfixed && fwd->hot.n != 0 && fwd->view.uniform_start && ((uintptr_t)d_text & 15) == 0 && !tuning.force_generic;
   const int wkind = wfixed ? 2 : wfast ? 1 : 0;
   // literal prefilter: no start bitmap at all -- literal_scan finds, verifies and chains the candidates
@@ -801,7 +970,7 @@ int Regex::find_all_shard_device(const uint8_t* d_text, uint64_t n, ShardIO* io,
   if (use_pf) std::memcpy(&pf, pf_words_.data(), sizeof pf);
   const bool pf_fast = use_pf && fwd->hot.n != 0 && fwd->view.uniform_start;
   // fused: every lane of the fast scan kernel also walks its own segment (chunk == segment)
-  const bool fused = !use_pf && plan.fast && wkind != 0 && tuning.fuse && !io->reuse_scan &&
+  const bool fused = !use_pf && !cand && plan.fast && wkind != 0 && tuning.fuse && !io->reuse_scan &&
                      fast_scan_smem(hot_bytes_signed(revall->hot) + (wkind == 1 ? hot_bytes(fwd->hot.n) : 0)) <= 227 * 1024;
 
   WalkArgs w{};
@@ -903,13 +1072,21 @@ int Regex::find_all_shard_device(const uint8_t* d_text, uint64_t n, ShardIO* io,
     else if (wkind == 1) walk_chunks<1><<<g, 256, wsmem, st>>>(args);
     else walk_chunks<0><<<g, 256, wsmem, st>>>(args);
   };
-  if (use_pf) {
-    RB_CUDA(launch_pf(w, nc, 0));
-    RB_LAUNCH_CHECK("literal_scan");
+  if (use_pf || cand) {
+    if (use_pf) {
+      RB_CUDA(launch_pf(w, nc, 0));
+      RB_LAUNCH_CHECK("literal_scan");
+    } else {
+      if (int rc = cand_starts(d_text, n, io->own_lo, io->own_hi, !io->is_last)) return rc;
+    }
     io->rev_guess = io->rev_entry != kNoState ? io->rev_entry : kPrefilterState;  // no reverse scan, nothing to guess
     io->rev_left = kPrefilterState;
     stats.scan_redo_rounds = stats.scan_redo_segments = stats.map_passes = 0;
     RB_CUDA(cudaEventRecord(ev[1], st));
+    if (!use_pf) {
+      launch_walk(w, nc);
+      RB_LAUNCH_CHECK("walk_chunks");
+    }
   } else {
     if (int rc = scan_starts(d_text, n, io->own_lo, io->own_hi, io, plan, fused ? &w : nullptr)) return rc;
     RB_CUDA(cudaEventRecord(ev[1], st));
@@ -1038,7 +1215,7 @@ int Regex::find_all_shard_device(const uint8_t* d_text, uint64_t n, ShardIO* io,
   io->halo_overflow = ((uint32_t*)(h + 3))[0] != 0;
   io->left_ctx_short = ((uint32_t*)(h + 3))[1] != 0;
   stats.fused = fused;
-  stats.path = use_pf ? 3 : fused ? 2 : plan.fast ? 1 : 0;
+  stats.path = use_pf ? 3 : cand ? 4 : fused ? 2 : plan.fast ? 1 : 0;
   cudaEventElapsedTime(&stats.scan_ms, ev[0], ev[1]);
   cudaEventElapsedTime(&stats.walk_ms, ev[1], ev[2]);
   cudaEventElapsedTime(&stats.total_ms, ev[0], ev[2]);
@@ -1298,6 +1475,7 @@ int Regex::shortest_match_device(const uint8_t* d_text, uint64_t n, uint64_t sta
   std::lock_guard<std::recursive_mutex> lock(mu_);
   *found = false;
   if (patterns_.empty() || start > n) return 0;
+  if (candidate_mode()) return cand_shortest(d_text, n, start, found, end);
   uint64_t res[1 + kMaxMaskWords];
   if (int rc = forward_reduce(d_text, n, start, false, res)) return rc;
   if (res[0] != kNone) { *found = true; *end = res[0]; }
@@ -1333,6 +1511,9 @@ int Regex::forward_shard_device(const uint8_t* d_text, uint64_t n, uint64_t own_
   *entry_used = *exit_state = entry;
   if (patterns_.empty()) return 0;
   if (own_lo > own_hi || own_hi > n) return fail("bad shard geometry");
+  if (candidate_mode())
+    return fail("sharded shortest_match / is_match is not available for a pattern searched from candidate starts (its unanchored "
+                "automaton exceeds the DFA table budget); use shortest_match on the whole haystack");
   DeviceDfa* fwd;
   if (int rc = ensure(kFwdUnanchoredAll, &fwd)) return rc;
   if (entry == kNoEntry && own_lo > 0) {
@@ -1370,6 +1551,7 @@ int Regex::is_match_batch_device(const uint8_t* d_text, const uint64_t* d_offset
     RB_CUDA(cudaStreamSynchronize((cudaStream_t)stream_));
     return 0;
   }
+  if (candidate_mode()) return cand_batch(0, d_text, d_offsets, n_rec, d_bits, nullptr, nullptr, 0);
   DeviceDfa* fwd;
   if (int rc = ensure(kFwdUnanchoredAll, &fwd)) return rc;
   BatchArgs a{};
@@ -1417,6 +1599,9 @@ int Regex::find_batch_device(const uint8_t* d_text, const uint64_t* d_offsets, u
   std::lock_guard<std::recursive_mutex> lock(mu_);
   if (n_rec == 0) return 0;
   if (is_set_) return fail("find requires exactly one pattern");
+  bool cand;
+  if (int rc = batch_route(&cand)) return rc;
+  if (cand) return cand_batch(1, d_text, d_offsets, n_rec, d_bits, d_spans, nullptr, 0);
   DeviceDfa *fwd, *rev;
   if (int rc = ensure(kFwdUnanchoredLF, &fwd)) return rc;
   if (int rc = ensure(kRevAnchoredLongest, &rev)) return rc;
@@ -1470,8 +1655,10 @@ int Regex::iter_batch(const uint8_t* d_text, const uint64_t* d_offsets, uint64_t
                       uint64_t cap, uint64_t* total, DeviceBuf* grow) {
   *total = 0;
   if (is_set_) return fail("find requires exactly one pattern");
+  bool cand;
+  if (int rc = batch_route(&cand)) return rc;
   DeviceDfa *fwd, *rev;
-  if (int rc = ensure(kFwdUnanchoredLF, &fwd)) return rc;
+  if (int rc = ensure(cand ? kFwdAnchoredLF : kFwdUnanchoredLF, &fwd)) return rc;
   if (int rc = ensure(kRevAnchoredLongest, &rev)) return rc;
   cudaStream_t st = (cudaStream_t)stream_;
   if (n_rec == 0) {
@@ -1489,7 +1676,7 @@ int Regex::iter_batch(const uint8_t* d_text, const uint64_t* d_offsets, uint64_t
   a.out_spans = d_out;
   a.cap = d_out ? cap : 0;
   a.utf8 = only_utf8 ? 1 : 0;
-  const bool fast = fwd->hot.n && rev->hot.n && ((uintptr_t)d_text & 15) == 0 && !tuning.force_generic;
+  const bool fast = !cand && fwd->hot.n && rev->hot.n && ((uintptr_t)d_text & 15) == 0 && !tuning.force_generic;
   size_t fsm = 0;
   uint32_t grid = (uint32_t)((n_rec + 255) / 256);
   if (fast) {
@@ -1505,11 +1692,15 @@ int Regex::iter_batch(const uint8_t* d_text, const uint64_t* d_offsets, uint64_t
     RB_CUDA(allow_smem(batch_iter_fast<1>, fsm));
   }
   // ---- count ----
-  a.fwd_only = !can_match_empty && !has_looks;
+  a.fwd_only = !can_match_empty && !has_looks && !cand;  // (the forward-only count needs kind 4)
   RB_CUDA(cudaMemsetAsync(d_match_offsets + n_rec, 0, 8, st));
-  if (fast) batch_iter_fast<0><<<grid, 512, fsm, st>>>(a);
-  else batch_iter<0><<<grid, 256, 0, st>>>(a);
-  RB_LAUNCH_CHECK("batch_iter<0>");
+  if (cand) {
+    if (int rc = cand_batch(2, d_text, d_offsets, n_rec, nullptr, nullptr, d_match_offsets, 0)) return rc;
+  } else {
+    if (fast) batch_iter_fast<0><<<grid, 512, fsm, st>>>(a);
+    else batch_iter<0><<<grid, 256, 0, st>>>(a);
+    RB_LAUNCH_CHECK("batch_iter<0>");
+  }
   // ---- exclusive scan over n_rec + 1 entries ----
   unsigned long long* grand;
   if (int rc = prefix_sum(d_match_offsets, d_match_offsets, n_rec + 1, &grand)) return rc;
@@ -1522,7 +1713,9 @@ int Regex::iter_batch(const uint8_t* d_text, const uint64_t* d_offsets, uint64_t
     a.cap = h[0];
   }
   // ---- write ----
-  if (a.cap > 0) {
+  if (a.cap > 0 && cand) {
+    if (int rc = cand_batch(3, d_text, d_offsets, n_rec, nullptr, a.out_spans, d_match_offsets, a.cap)) return rc;
+  } else if (a.cap > 0) {
     a.fwd_only = 0;
     if (fast) batch_iter_fast<1><<<grid, 512, fsm, st>>>(a);
     else batch_iter<1><<<grid, 256, 0, st>>>(a);

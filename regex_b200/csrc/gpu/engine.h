@@ -41,6 +41,7 @@ struct Tuning {
                                  // to win (one byte, <= ~0.12 % of the haystack), 2 whenever the pattern qualifies structurally       // RegexSet::matches: continue with the automaton of the still-unmatched patterns
   uint32_t max_stitch_rounds = 16;  // re-walk rounds before the stitch falls back to one sequential pass
   uint32_t max_redo_rounds = 3;     // scan redo rounds before segment entry states are solved by state-map composition
+  bool candidate_starts = false;    // tests: search from candidate starts (as over-budget patterns do) even when the unanchored automata fit
 };
 
 struct Stats {  // filled by the last single-haystack call (diagnostics, bench roofline)
@@ -48,7 +49,7 @@ struct Stats {  // filled by the last single-haystack call (diagnostics, bench r
   uint64_t stitch_rounds = 0, stitch_dirty_chunks = 0, sequential_passes = 0, map_passes = 0, waves = 0, long_runs = 0;
   float scan_ms = 0, walk_ms = 0, total_ms = 0;
   bool fused = false;  // the scan kernel also walked the chains (scan_ms covers both)
-  int path = 0;        // last find_all: 0 generic scan, 1 fast scan, 2 fused scan + walk, 3 literal prefilter
+  int path = 0;        // last find_all: 0 generic scan, 1 fast scan, 2 fused scan + walk, 3 literal prefilter, 4 candidate starts
 };
 
 constexpr uint32_t kNoState = 0xFFFFFFFFu;
@@ -185,6 +186,9 @@ class Regex {
   bool can_match_empty = false;
   bool has_looks = false;
   bool only_utf8 = false;
+  // Candidate-start mode (DESIGN.md §2): a single pattern whose unanchored automata exceed the table budget is
+  // searched from candidate starts with the anchored automaton (kinds 0 and 3); kinds 1, 2 and 4 are never built.
+  bool candidate_mode() const { return !is_set_ && (unanchored_too_big_ || tuning.candidate_starts); }
 
  private:
   Regex() = default;
@@ -218,6 +222,15 @@ class Regex {
   int replace_sums(const uint8_t* d_text, uint64_t n, const uint64_t* spans, uint64_t m, const uint64_t* slots, uint64_t* out_len);
   int replace_emit(uint8_t* d_out, uint64_t out_cap);
   bool plan_prefilter();  // fills pf_words_ (launch.h PfArgs) when every match has one of <= 4 bytes at a fixed offset
+  // ---- candidate-start mode ----
+  int cand_args(void* out);  // launch.h CandArgs: byte sets of the first min(min_len, 4) offsets of a match
+  // start bitmap (scan_rev format) of the candidates at positions (base, limit], plus position 0 when base == 0
+  int cand_starts(const uint8_t* d_text, uint64_t n, uint64_t base, uint64_t limit, bool text_continues);
+  int cand_shortest(const uint8_t* d_text, uint64_t n, uint64_t start, bool* found, uint64_t* end);
+  // batched records from candidate starts: mode 0 is_match, 1 find, 2 / 3 find_iter count / write pass
+  int cand_batch(int mode, const uint8_t* d_text, const uint64_t* d_offsets, uint64_t n_rec, uint32_t* d_bits, uint64_t* d_spans,
+                 uint64_t* d_match_offsets, uint64_t cap);
+  int batch_route(bool* cand);  // batched find / find_iter: candidate starts, or kind 4 (switches to the mode when it is over budget)
   int forward_reduce(const uint8_t* d_text, uint64_t n, uint64_t start, bool want_masks, uint64_t* result_host, uint64_t end = ~0ull,
                      uint32_t entry = 0xFFFFFFFFu, uint32_t* exit_out = nullptr);
   int forward_range(const uint8_t* d_text, uint64_t n, uint64_t start, uint64_t limit, uint32_t entry, bool want_masks,
@@ -235,6 +248,8 @@ class Regex {
   CompileOptions opt_;
   std::vector<rb::Expr> exprs_;
   std::unique_ptr<rb::Dfa> host_[kNumDfaKinds];
+  bool unanchored_too_big_ = false;  // an unanchored automaton failed with DfaTooBig: candidate-start mode
+  std::vector<uint8_t> cand_image_;  // launch.h CandArgs image (built on first use)
   DeviceDfa* dev_[kNumDfaKinds] = {nullptr, nullptr, nullptr, nullptr, nullptr};
   std::string error_;
   std::recursive_mutex mu_;

@@ -684,14 +684,15 @@ __device__ __forceinline__ uint64_t chunk_walk(const WalkArgs& a, const Runner& 
     return wi + (uint64_t)(__ffsll((long long)ahead) - 1);
   };
   bool at_zero = c.p == 0 && cb == 0 && *a.flag0;  // position 0 has no bitmap bit
+  uint64_t q = 0;  // candidates below q were no match start (candidate-start bitmaps are a superset)
   while (c.p != kNone) {
     uint64_t s;
     if (at_zero) {
       s = 0;
       at_zero = false;
     } else {
-      // next candidate position >= max(p, cb + 1): bit index = position - 1
-      uint64_t bit = max(c.p, cb + 1) - 1;
+      // next candidate position >= max(p, q, cb + 1): bit index = position - 1
+      uint64_t bit = max(max(c.p, q), cb + 1) - 1;
       uint64_t m = 0;
       while (bit < ce) {
         uint64_t wi = bit >> 6;
@@ -713,7 +714,11 @@ __device__ __forceinline__ uint64_t chunk_walk(const WalkArgs& a, const Runner& 
     if (fc == kNone) fc = s;
     const uint64_t e = run_end(a, T, s, exact);
     if (e == kTooLong) { *first_cand = kTooLong; return 0; }  // deferred: see kSpecRunCap
-    if (e == kNone) { c.p = s + 1; c.chain = false; continue; }  // unreachable for consistent tables
+    if (e == kNone) {  // no match starts at s (a candidate start): the iterator state stays, the walk moves on
+      if (fc == s) fc = kNone;
+      q = s + 1;
+      continue;
+    }
     uint64_t ms = s;
     if (a.emulate_slice && c.chain && e != c.p) {
       // exec.rs:647-657: an empty match at the restart point short-circuits; otherwise
@@ -782,7 +787,7 @@ __device__ __forceinline__ uint64_t chunk_walk_simple(const WalkArgs& a, const R
     fc = 0;
     const uint64_t e = run_end(a, T, 0, exact);
     if (e == kTooLong) too_long = true;
-    else if (e == kNone) { c.p = 1; c.chain = false; }
+    else if (e == kNone) fc = kNone;  // a candidate that is no match start: as if its bit were clear
     else { emit(0, e); c.p = c.lm = e; c.chain = true; }
   }
   // bit r of the chunk <-> position cb + r + 1
@@ -808,10 +813,9 @@ __device__ __forceinline__ uint64_t chunk_walk_simple(const WalkArgs& a, const R
     pending = e == kPending;
     if (pending) return false;  // the same candidate again, without the trip cap, once the warp is through its short runs
     if (e == kTooLong) { too_long = true; return false; }
-    if (e == kNone) {  // unreachable for consistent tables
+    if (e == kNone) {  // a candidate that is no match start: as if its bit were clear
       cur &= cur - 1;
-      c.p = s + 1;
-      c.chain = false;
+      if (fc == s) fc = kNone;
       return true;
     }
     emit(s, e);
@@ -867,7 +871,7 @@ __device__ __forceinline__ uint64_t chunk_walk_lean(const WalkArgs& a, const Fas
   const bool exact = c.chain;
   uint32_t total = 0, fc_rel = ~0u;
   uint64_t held_s = 0, held_e = 0, last_e = kNone;
-  bool too_long = false, lost = false;
+  bool too_long = false;
   auto emit = [&](uint64_t ms, uint64_t e) {  // spans leave two at a time as whole 32-byte sectors
     if (!(total & 1u)) { held_s = ms; held_e = e; }
     else if (total < room) st_sector(reinterpret_cast<uint64_t*>(o + (total - 1)), held_s, held_e, ms, e);
@@ -879,7 +883,7 @@ __device__ __forceinline__ uint64_t chunk_walk_lean(const WalkArgs& a, const Fas
     fc0 = 0;
     const uint64_t e = run_end(a, T, 0, exact);
     if (e == kTooLong) too_long = true;
-    else if (e == kNone) { c.p = 1; c.chain = false; }
+    else if (e == kNone) fc0 = kNone;  // a candidate that is no match start: as if its bit were clear
     else { emit(0, e); c.p = last_e = e; c.chain = true; }
   }
   uint32_t r = c.p > cb + 1 ? (uint32_t)min(c.p - cb - 1, (uint64_t)nbits) : 0u;
@@ -947,16 +951,14 @@ __device__ __forceinline__ uint64_t chunk_walk_lean(const WalkArgs& a, const Fas
       pending = e_abs == kPending;
       if (pending) return false;  // the same candidate again, without the trip cap, once the warp is through its short runs
       if (e_abs == kTooLong) { too_long = true; return false; }
-      if (e_abs == kNone) {  // unreachable for consistent tables
+      if (e_abs == kNone) {  // a candidate that is no match start: as if its bit were clear
         cur &= cur - 1;
-        c.p = cb + s_rel + 1;
-        lost = true;
+        if (fc_rel == s_rel) fc_rel = ~0u;
         return true;
       }
     }
     emit(cb + s_rel, e_abs);
     last_e = e_abs;
-    lost = false;
     const uint64_t er = e_abs - 1 - cb;  // next candidate bit >= er
     if (er >= nbits) return false;
     r = (uint32_t)er;
@@ -983,8 +985,7 @@ __device__ __forceinline__ uint64_t chunk_walk_lean(const WalkArgs& a, const Fas
   }
   if (too_long) { *first_cand = kTooLong; return 0; }
   if ((total & 1u) && total - 1 < room) o[total - 1] = make_ulonglong2(held_s, held_e);
-  if (lost) c.chain = false;
-  else if (last_e != kNone) { c.p = c.lm = last_e; c.chain = true; }
+  if (last_e != kNone) { c.p = c.lm = last_e; c.chain = true; }
   *first_cand = fc0 != kNone ? fc0 : fc_rel != ~0u ? cb + fc_rel : kNone;
   return total;
 }
@@ -3148,5 +3149,165 @@ __global__ void set_matches_batch(BatchArgs a) {
   for (uint32_t w = 0; w < kMaxMaskWords; w++)
     if (w < mw) a.out_masks[r * mw + w] = acc[w];
 }
+
+
+// ---------------------------------------------------------- candidate starts --
+// Candidate-start mode (DESIGN.md §2): patterns whose unanchored automata exceed the table budget.  Every
+// position whose first min(min_len, 4) bytes lie in the byte sets of the anchored automaton is a candidate
+// start; the anchored automaton (kind 0) decides each, so the candidates only need to be a superset of the
+// match starts.
+
+// s is a candidate of a text of n bytes (cm: shared-memory byte masks, bit d = in the set of offset d)
+__device__ __forceinline__ bool cand_at(const uint8_t* cm, uint32_t depth, const uint8_t* t, uint64_t n, uint64_t s) {
+  for (uint32_t d = 0; d < depth; d++)
+    if (s + d >= n || !((cm[t[s + d]] >> d) & 1u)) return false;
+  return true;
+}
+
+// The start bitmap in scan_rev's format.  One thread per bitmap word (64 positions): the 80 bytes
+// [64w, 64w + 80) come in as five 16-byte loads where they lie inside the haystack, the masks are looked up in
+// shared memory, and the 32 words of a warp are 256 consecutive bytes, so the stores leave as whole sectors.
+__global__ void cand_bitmap(const uint8_t* text, uint64_t n, uint64_t base, uint64_t limit, int text_continues, CandArgs c,
+                            uint64_t* bitmap, uint8_t* flag0) {
+  __shared__ uint8_t cm[256];
+  for (uint32_t i = threadIdx.x; i < 256; i += blockDim.x) cm[i] = c.mask[i];
+  __syncthreads();
+  const uint32_t depth = c.depth;
+  const bool vec = (reinterpret_cast<uintptr_t>(text) & 15) == 0;
+  const uint32_t past_end = text_continues ? 0xFu : 0u;  // a shard's halo ends at n: the text goes on
+  const uint64_t w_lo = base >> 6, w_hi = max((limit + 63) >> 6, w_lo + (base == 0 ? 1 : 0));  // word 0 also sets *flag0
+  for (uint64_t w = w_lo + blockIdx.x * (uint64_t)blockDim.x + threadIdx.x; w < w_hi; w += (uint64_t)gridDim.x * blockDim.x) {
+    const uint64_t at = w << 6;  // bit k of word w <-> position at + 1 + k
+    uint64_t m0 = 0, m1 = 0, m2 = 0, m3 = 0, cont = 0;
+    // byte at + j (j = 1..67) in the set of offset d marks position at + j - d
+    auto take = [&](int j, uint32_t raw, bool inside) {
+      const uint32_t t = inside ? (uint32_t)cm[raw] : past_end;
+      if (j <= 64) { m0 |= (uint64_t)(t & 1u) << (j - 1); if (inside && (raw & 0xC0u) == 0x80u) cont |= 1ull << (j - 1); }
+      if (j >= 2 && j <= 65) m1 |= (uint64_t)((t >> 1) & 1u) << (j - 2);
+      if (j >= 3 && j <= 66) m2 |= (uint64_t)((t >> 2) & 1u) << (j - 3);
+      if (j >= 4) m3 |= (uint64_t)((t >> 3) & 1u) << (j - 4);
+    };
+    if (vec && at + 80 <= n) {
+      uint4 v[5];
+#pragma unroll
+      for (int i = 0; i < 5; i++) v[i] = ldg128(text + at + 16 * i);
+#pragma unroll
+      for (int j = 1; j < 68; j++) take(j, word_byte(v[j >> 4], j & 15), true);
+    } else {
+#pragma unroll 1
+      for (int j = 1; j < 68; j++) take(j, at + j < n ? text[at + j] : 0u, at + j < n);
+    }
+    uint64_t word = ~0ull;
+    if (depth > 0) word &= m0;
+    if (depth > 1) word &= m1;
+    if (depth > 2) word &= m2;
+    if (depth > 3) word &= m3;
+    if (c.utf8_boundaries) word &= ~cont;
+    if (at + 64 > limit) word &= limit > at ? ~0ull >> (64 - (limit - at)) : 0ull;  // positions up to limit
+    bitmap[w] = word;
+    if (at == 0) {  // position 0 has no bit
+      bool hit = true;
+      for (uint32_t d = 0; d < depth; d++)
+        if (d < n ? !((cm[text[d]] >> d) & 1u) : !text_continues) hit = false;
+      if (c.utf8_boundaries && n > 0 && (text[0] & 0xC0u) == 0x80u) hit = false;
+      *flag0 = hit;
+    }
+  }
+}
+
+// shortest_match from candidate starts: one lane per segment of seg positions runs the anchored automaton from
+// each of its candidates s below the best end known so far and stops at the first match state (before the
+// first Match nothing is cut, so that is the earliest end of any match from s).
+__global__ void cand_shortest(DfaView fwd, int use_smem, CandArgs c, const uint8_t* text, uint64_t n, uint64_t lo, uint64_t hi,
+                              uint32_t seg, unsigned long long* best) {
+  __shared__ uint8_t cm[256];
+  for (uint32_t i = threadIdx.x; i < 256; i += blockDim.x) cm[i] = c.mask[i];
+  __syncthreads();
+  const Table T = stage_table(fwd, g_smem, use_smem);
+  const uint64_t n_seg = (hi - lo + seg - 1) / seg;
+  for (uint64_t t = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x; t < n_seg; t += (uint64_t)gridDim.x * blockDim.x) {
+    uint64_t b = *(volatile unsigned long long*)best;
+    const uint64_t s_lo = lo + t * seg, s_hi = min(s_lo + seg, hi);
+    for (uint64_t s = s_lo; s < s_hi && s < b; s++) {
+      if ((s & 255) == 0) b = min(b, (uint64_t)*(volatile unsigned long long*)best);
+      if (!cand_at(cm, c.depth, text, n, s)) continue;
+      uint32_t st = pick_start_fwd(fwd, text, n, s);
+      for (uint64_t q = s; st != 0 && q < b; q++) {
+        st = q < n ? T.step(st, __ldg(text + q)) : T.step_eof(st);
+        if (st >= fwd.match_lo) {
+          b = q;
+          atomicMin(best, (unsigned long long)q);
+          break;
+        }
+        if (q >= n) break;
+      }
+    }
+  }
+}
+
+// Batched records from candidate starts, one thread per record (class-indexed tables, the anchored one in shared
+// memory when it fits).  find_at(q) = (s*, A(s*)) with s* the first candidate >= q at which the anchored automaton
+// finds a match A(s*); with look-arounds the start comes from the reverse-on-slice rule (SURVEY H1) instead.
+template <int MODE>
+__global__ void batch_cand(BatchArgs a, CandArgs c) {
+  __shared__ uint8_t cm[256];
+  for (uint32_t i = threadIdx.x; i < 256; i += blockDim.x) cm[i] = c.mask[i];
+  __syncthreads();
+  const Table T = stage_table(a.fwd, g_smem, a.use_smem);
+  const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;  // multiple of 32: warps stay on one ballot word
+  const uint32_t lane = threadIdx.x & 31;
+  for (uint64_t r = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x; r - lane < a.n_rec; r += stride) {
+    bool hit = false;
+    uint64_t ms = 0, me = 0;
+    if (r < a.n_rec) {
+      const uint64_t lo = a.offsets[r], len = a.offsets[r + 1] - lo;
+      const uint8_t* p = a.text + lo;
+      auto is_cand = [&](uint64_t s) {
+        return cand_at(cm, c.depth, p, len, s) && !(c.utf8_boundaries && s < len && (p[s] & 0xC0u) == 0x80u);
+      };
+      if (MODE == 0) {
+        for (uint64_t s = 0; s <= len && !hit; s++) {
+          if (!is_cand(s)) continue;
+          uint32_t st = pick_start_fwd(a.fwd, p, len, s);
+          for (uint64_t q = s; st != 0; q++) {
+            st = q < len ? T.step(st, p[q]) : T.step_eof(st);
+            if (st >= a.fwd.match_lo) { hit = true; break; }
+            if (q >= len) break;
+          }
+        }
+      } else {
+        uint64_t s_star = 0;
+        auto fwd = [&](uint64_t q) -> uint64_t {  // end of the match at the first candidate >= q that starts one
+          for (uint64_t s = q; s <= len; s++) {
+            if (!is_cand(s)) continue;
+            const uint64_t e = anchored_end(a.fwd, T, p, len, s);
+            if (e != kNone) { s_star = s; return e; }
+          }
+          return kNone;
+        };
+        auto rev = [&](uint64_t q, uint64_t e) -> uint64_t { return c.slice_rule ? slice_start(a.rev, p, len, q, e) : s_star; };
+        if (MODE == 1) {
+          me = fwd(0);
+          if (me != kNone) {
+            ms = me == 0 ? 0 : rev(0, me);
+            hit = ms != kNone;
+          }
+          a.out_spans[2 * r] = hit ? ms : 0;
+          a.out_spans[2 * r + 1] = hit ? me : 0;
+        } else {
+          iter_record<MODE - 2>(a, r, p, len, fwd, rev);
+        }
+      }
+    }
+    if (MODE <= 1) {
+      const uint32_t bits = __ballot_sync(0xffffffffu, hit);
+      if (lane == 0) a.out_bits[r >> 5] = bits;
+    }
+  }
+}
+template __global__ void batch_cand<0>(BatchArgs, CandArgs);
+template __global__ void batch_cand<1>(BatchArgs, CandArgs);
+template __global__ void batch_cand<2>(BatchArgs, CandArgs);
+template __global__ void batch_cand<3>(BatchArgs, CandArgs);
 
 }  // namespace rbgpu

@@ -96,6 +96,24 @@ template <int FAST, int NB>  // NB = PfArgs::n_bytes
 __global__ void literal_scan(const __grid_constant__ WalkArgs a, const __grid_constant__ PfArgs pf, int mode);
 __global__ void compact_staged(WalkArgs a);
 
+// Candidate-start mode (DESIGN.md §2): position s is a candidate when text[s + d] is in the byte set of offset d for
+// every d < depth (the bytes with which some start state of the anchored automaton survives d + 1 steps).
+// Candidates are a superset of the match starts; the anchored automaton decides each.
+struct CandArgs {
+  uint32_t depth;        // min(min_len, 4); 0 = every position is a candidate, n included
+  int utf8_boundaries;   // as ScanArgs: drop positions inside a UTF-8 sequence (Regex on str, empty matches)
+  int slice_rule;        // batched find: the start of a match comes from the reverse-on-slice scan (look-arounds)
+  uint8_t mask[256];     // bit d set when the byte is in the set of offset d
+};
+// bitmap bits [base, limit) (bit i <-> position i + 1) and, when base == 0, *flag0 (position 0); base is 64-aligned.
+// text_continues: a shard's halo ends at n, positions whose sets reach past it stay candidates
+__global__ void cand_bitmap(const uint8_t* text, uint64_t n, uint64_t base, uint64_t limit, int text_continues, CandArgs c,
+                            uint64_t* bitmap, uint8_t* flag0);
+// *best = min(*best, the first position where the anchored automaton, started at a candidate s in [lo, hi), enters a
+// match state); one lane per seg positions
+__global__ void cand_shortest(DfaView fwd, int use_smem, CandArgs c, const uint8_t* text, uint64_t n, uint64_t lo, uint64_t hi,
+                              uint32_t seg, unsigned long long* best);
+
 // ---- bulk operations over the span list (src/re_bytes.rs:316-360 split, :476-535 replacen) ----
 // The replacement of one match is a sequence of parts: literal bytes, or the text of a capture
 // group of that match (`$0`, `$2`, `$name`; src/expand.rs:50-90).
@@ -208,6 +226,10 @@ template <int PASS>
 __global__ void batch_iter_fast(BatchArgs a);
 template <int PASS>
 __global__ void batch_iter(BatchArgs a);
+// batched records from candidate starts (fwd = anchored leftmost-first, rev = reverse anchored longest):
+// MODE 0 is_match, 1 find, 2 find_iter count pass, 3 find_iter write pass
+template <int MODE>
+__global__ void batch_cand(BatchArgs a, CandArgs c);
 template <int MODE>
 __global__ void batch_refill(BatchArgs a);
 __global__ void scan_rev_bitmap(ScanArgs a);
