@@ -209,7 +209,9 @@ bool rure_b200_find_all_shard_device(rure *re, const uint8_t *d_buffer, size_t n
  * guess it from the left context; regex_b200/sharded.py (forward_sharded) compares entry_used
  * with the neighbour's exit_state and searches again on a mismatch.  Results: first_end = end of
  * the first match that ends in this shard (buffer-relative; shortest_match = min over ranks),
- * masks = patterns that match inside it (RegexSet::matches = OR over ranks; 4 words = 256 patterns). */
+ * masks = patterns that match inside it (RegexSet::matches = OR over ranks; 4 words = 256 patterns).
+ * rure_b200_set_matches_shard_device returns false with a message for a set searched in pattern
+ * groups (see rure_b200_set_groups): one entry state and 256 mask bits cannot describe it. */
 typedef struct rure_b200_fwd_shard {
   /* in */
   uint64_t own_lo, own_hi;
@@ -249,15 +251,30 @@ void rure_b200_last_stats(rure *re, double *out8);
  * unanchored automata exceed the DFA budget, searched with the anchored one), out[12] = matches longer
  * than 256 KiB that were measured by the parallel long-run pass.  n = doubles to write. */
 void rure_b200_last_stats_ex(rure *re, double *out, size_t n);
+/* rure_b200_set_last_stats_ex also has out[13] = pattern groups searched in the first wave of the last
+ * set call (1 = the product automaton; see rure_b200_set_groups). */
 void rure_b200_set_last_stats_ex(rure_set *set, double *out, size_t n);
 /* Named knobs (tests, tuning): "wave0" bytes of the first wave of is_match / shortest_match /
  * set matches (x16 per wave, 0 = one wave), "narrow_sets" 0/1, "max_stitch_rounds",
  * "max_redo_rounds", "batch_refill" 0/1 (batched is_match: lanes refill from a task of records), "prefilter" (0 never, 1 automatic: only for a single rare byte, 2 whenever the
  * pattern qualifies), "candidate_starts" 0/1 (tests: search from candidate starts with the anchored
  * automaton, as patterns over the DFA budget do, even when the unanchored automata fit).
- * Returns false for an unknown name. */
+ * Returns false for an unknown name.
+ * Sets also take "set_group_patterns" k (tests): search in groups of at most k patterns even when
+ * the product automaton fits, each group split further while its automaton is over the budget;
+ * 0 (the default) = automatic.  The new plan is compiled at once; false when a group fails to compile
+ * (the plan is then unchanged). */
 bool rure_b200_set_option(rure *re, const char *name, uint64_t value);
 bool rure_b200_set_set_option(rure_set *set, const char *name, uint64_t value);
+/* RegexSets of any size.  A set of at most 256 patterns whose forward all-match automaton fits the DFA
+ * budget is searched with that one product automaton.  Larger sets, and sets whose product automaton is
+ * over the budget, are searched in pattern groups: contiguous pattern ranges of at most 256 patterns, each
+ * with its own automaton within the budget (chunks of 256, halved while over the budget, on multiples of
+ * 64 above 64 patterns).  A single pattern over the budget is still a compile error.  Every set call
+ * answers the same either way; rure_set_matches takes any set size.  Returns the number of groups (1 for
+ * the product automaton, 0 for an empty set) and writes the first pattern index of up to cap of them to first_pattern
+ * (may be NULL). */
+size_t rure_b200_set_groups(rure_set *set, size_t *first_pattern, size_t cap);
 /* seg/chunk are positions per scan segment / walk chunk (multiples of 64);
  * warm = warm-up bytes (0 = automatic); 0 keeps the current value elsewhere. */
 void rure_b200_set_tuning(rure *re, uint32_t seg, uint32_t chunk, uint32_t warm, uint32_t block,
@@ -275,7 +292,8 @@ void rure_b200_set_tensor_tma(rure *re, int yes);
 /* Dense tables, for tests and tooling.  kind: 0 forward anchored leftmost-first,
  * 1 reverse unanchored all-match, 2 forward unanchored all-match, 3 reverse
  * anchored longest, 4 forward unanchored leftmost-first.  A pattern searched from candidate
- * starts has kinds 0 and 3 only: kinds 1, 2 and 4 return false with a message.
+ * starts has kinds 0 and 3 only: kinds 1, 2 and 4 return false with a message.  Kind 2 of a set
+ * searched in pattern groups returns false with a message that lists the groups.
  * info[0..5] = n_states, n_classes (last = EOF), match_lo, mask_words, uniform_start, raw_states.
  * Buffers may be NULL to query sizes: trans n_states*n_classes u16, classes 256 u8,
  * start 128 u16, masks n_states*mask_words u64. */

@@ -24,6 +24,7 @@ DFA_FWD_ANCHORED_LF, DFA_REV_UNANCHORED_ALL, DFA_FWD_UNANCHORED_ALL, DFA_REV_ANC
 
 _STAT_KEYS = ["scan_ms", "walk_ms", "total_ms", "scan_redo_rounds", "scan_redo_segments", "stitch_rounds", "stitch_dirty_chunks",
               "fused", "sequential_passes", "map_passes", "waves", "path", "long_runs"]
+_SET_STAT_KEYS = _STAT_KEYS + ["groups"]
 
 
 class Error(Exception):
@@ -130,6 +131,7 @@ def _load():
         "rure_b200_set_last_stats_ex": (None, [vp, POINTER(c_double), sz]),
         "rure_b200_set_option": (c_bool, [vp, c_char_p, c_uint64]),
         "rure_b200_set_set_option": (c_bool, [vp, c_char_p, c_uint64]),
+        "rure_b200_set_groups": (sz, [vp, POINTER(sz), sz]),
         "rure_b200_set_tuning": (None, [vp, c_uint32, c_uint32, c_uint32, c_uint32, c_uint32]),
         "rure_b200_force_generic": (None, [vp, c_int]),
         "rure_b200_set_stream": (None, [vp, vp]),
@@ -683,13 +685,23 @@ class _SetBase:
     _only_utf8 = False
 
     def last_stats(self):
-        out = (c_double * 13)()
-        _lib.rure_b200_set_last_stats_ex(self._h, out, 13)
-        return dict(zip(_STAT_KEYS, list(out)))
+        out = (c_double * len(_SET_STAT_KEYS))()
+        _lib.rure_b200_set_last_stats_ex(self._h, out, len(_SET_STAT_KEYS))
+        return dict(zip(_SET_STAT_KEYS, list(out)))
 
     def set_option(self, name, value):
+        """Named engine knobs (include/rure_b200.h: rure_b200_set_set_option), including "set_group_patterns"."""
         if not _lib.rure_b200_set_set_option(self._h, name.encode(), int(value)):
             raise Error(_last_error())
+
+    def groups(self):
+        """Pattern groups the set is searched in, as (lo, hi) index ranges: [(0, len(self))] for one product
+        automaton (include/rure_b200.h: rure_b200_set_groups)."""
+        n = int(_lib.rure_b200_set_groups(self._h, None, 0))
+        first = (c_size_t * n)()
+        _lib.rure_b200_set_groups(self._h, first, n)
+        bounds = list(first) + [len(self)]
+        return [(bounds[i], bounds[i + 1]) for i in range(n)]
 
     def __init__(self, patterns, flags=FLAG_UNICODE, size_limit=10 << 20, dfa_size_limit=2 << 20):
         pats = [p.encode("utf-8") if isinstance(p, str) else bytes(p) for p in patterns]

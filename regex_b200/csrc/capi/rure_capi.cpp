@@ -2,6 +2,7 @@
 // Thin: argument checks, object lifetime, and calls into rbgpu::Regex.
 #include <cstdio>
 #include <cstdlib>
+#include <algorithm>
 #include <cstring>
 #include <mutex>
 #include <string>
@@ -44,7 +45,7 @@ struct Lease {
     for (Regex* c : h->clones)
       if (c->try_acquire()) { r = c; return; }
     rb::Error err;
-    Regex* c = Regex::compile(h->pats, h->opts, &err);
+    Regex* c = h->re->clone(&err);  // a grouped set compiles its planned groups, not the failed product automaton
     if (!c) {  // cannot happen for a source that compiled once; wait for the primary then
       h->re->acquire();
       r = h->re;
@@ -323,10 +324,10 @@ bool rure_set_is_match(rure_set* s, const uint8_t* haystack, size_t length, size
 bool rure_set_matches(rure_set* s, const uint8_t* haystack, size_t length, size_t start, bool* matches) {
   const size_t n = s->re->n_patterns();
   for (size_t i = 0; i < n; i++) matches[i] = false;
-  uint64_t masks[4] = {0, 0, 0, 0};
+  std::vector<uint64_t> masks(std::max<size_t>(1, (n + 63) / 64), 0);
   bool any = false;
   Lease l(s);
-  if (!ok(l.r, l->set_matches_host(haystack, length, start, &any, masks))) die("rure_set_matches");
+  if (!ok(l.r, l->set_matches_host(haystack, length, start, &any, masks.data()))) die("rure_set_matches");
   for (size_t i = 0; i < n; i++) matches[i] = (masks[i / 64] >> (i % 64)) & 1;
   return any;
 }
@@ -557,11 +558,11 @@ void rure_b200_last_stats(rure* re, double* out8) {
 }
 static void stats_ex(Regex* r, double* out, size_t n) {
   const rbgpu::Stats& s = r->stats;
-  const double v[13] = {s.scan_ms, s.walk_ms, s.total_ms, (double)s.scan_redo_rounds, (double)s.scan_redo_segments,
+  const double v[14] = {s.scan_ms, s.walk_ms, s.total_ms, (double)s.scan_redo_rounds, (double)s.scan_redo_segments,
                         (double)s.stitch_rounds, (double)s.stitch_dirty_chunks, s.fused ? 1.0 : 0.0,
                         (double)s.sequential_passes, (double)s.map_passes, (double)s.waves, (double)s.path,
-                        (double)s.long_runs};
-  for (size_t i = 0; i < n && i < 13; i++) out[i] = v[i];
+                        (double)s.long_runs, (double)s.groups};
+  for (size_t i = 0; i < n && i < 14; i++) out[i] = v[i];
 }
 void rure_b200_last_stats_ex(rure* re, double* out, size_t n) { stats_ex(re->re, out, n); }
 void rure_b200_set_last_stats_ex(rure_set* set, double* out, size_t n) { stats_ex(set->re, out, n); }
@@ -579,7 +580,26 @@ static bool set_option(Regex* r, const char* name, uint64_t value) {
   return true;
 }
 bool rure_b200_set_option(rure* re, const char* name, uint64_t value) { return set_option(re->re, name, value); }
-bool rure_b200_set_set_option(rure_set* set, const char* name, uint64_t value) { return set_option(set->re, name, value); }
+bool rure_b200_set_set_option(rure_set* set, const char* name, uint64_t value) {
+  if (name && std::string(name) == "set_group_patterns") {
+    if (value > 0xFFFFFFFFull) { g_last_error = "set_group_patterns: value out of range"; return false; }
+    std::lock_guard<std::mutex> g(set->mu);
+    if (!ok(set->re, set->re->set_group_patterns((uint32_t)value))) return false;
+    for (Regex* c : set->clones) {  // clones take the new plan the next time they are needed
+      c->acquire();
+      c->release();
+      delete c;
+    }
+    set->clones.clear();
+    return true;
+  }
+  return set_option(set->re, name, value);
+}
+size_t rure_b200_set_groups(rure_set* set, size_t* first_pattern, size_t cap) {
+  const std::vector<uint32_t> f = set->re->group_firsts();
+  for (size_t i = 0; i < f.size() && i < cap && first_pattern; i++) first_pattern[i] = f[i];
+  return f.size();
+}
 void rure_b200_set_tuning(rure* re, uint32_t seg, uint32_t chunk, uint32_t warm, uint32_t block, uint32_t blocks_per_sm) {
   rbgpu::Tuning& t = re->re->tuning;
   if (seg) t.seg = (seg + 63) / 64 * 64;

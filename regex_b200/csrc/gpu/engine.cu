@@ -81,6 +81,19 @@ struct Regex::DeviceDfa {
 
 // ------------------------------------------------------------------ compile --
 Regex* Regex::compile(const std::vector<std::string>& patterns, const CompileOptions& opt, rb::Error* err) {
+  return compile_impl(patterns, opt, err, nullptr, 0);
+}
+
+Regex* Regex::clone(rb::Error* err) const {
+  const std::vector<uint32_t> one{0};
+  return compile_impl(patterns_, opt_, err, groups_.empty() ? &one : &group_first_, 0);
+}
+
+// plan: null = automatic (the product automaton of a set of <= 256 patterns when it fits, else pattern groups);
+// {0} = one product automaton or its error; more entries = exactly these groups.  chunk: groups of at most this many
+// patterns before the budget splits them (set_group_patterns), 0 = automatic.
+Regex* Regex::compile_impl(const std::vector<std::string>& patterns, const CompileOptions& opt, rb::Error* err,
+                           const std::vector<uint32_t>* plan, uint32_t chunk) {
   std::unique_ptr<Regex> re(new Regex());
   re->patterns_ = patterns;
   re->opt_ = opt;
@@ -127,15 +140,21 @@ Regex* Regex::compile(const std::vector<std::string>& patterns, const CompileOpt
     err->msg = "Unicode word boundaries (\\b, \\B) are not supported by the B200 DFA backend; use (?-u:\\b).";
     return nullptr;
   }
-  if (patterns.size() > 64 * kMaxMaskWords) {
-    err->kind = rb::Error::DfaTooBig;
-    err->msg = "regex sets larger than 256 patterns exceed the per-state mask budget";
-    return nullptr;
-  }
   // Determinize the tables every object needs so budget errors surface at compile time.
-  if (re->is_set_) {  // set semantics need the all-match product automaton
-    if (!re->host_dfa(kFwdUnanchoredAll, err)) return nullptr;
-    return re.release();
+  if (re->is_set_) {
+    // Set semantics need the all-match automaton of every pattern, or (DESIGN.md §2, RegexSets in groups) the
+    // automata of contiguous pattern ranges: matches[i] only says that pattern i matches somewhere, so the OR of
+    // the groups' masks is the same answer.  A group holds at most 64 * kMaxMaskWords patterns.
+    if (plan && plan->size() > 1) return re->build_groups(plan, 0, false, err) ? re.release() : nullptr;
+    const bool one_table = plan != nullptr;
+    if (one_table || (chunk == 0 && patterns.size() <= 64 * kMaxMaskWords)) {
+      if (re->host_dfa(kFwdUnanchoredAll, err)) { re->product_fits_ = true; return re.release(); }
+      if (one_table || err->kind != rb::Error::DfaTooBig || patterns.size() == 1) return nullptr;
+    }
+    *err = rb::Error();
+    // a set of <= 256 patterns lands here after its product automaton failed: that range is split at once
+    return re->build_groups(nullptr, chunk ? chunk : 64 * kMaxMaskWords, patterns.size() <= 64 * kMaxMaskWords && chunk == 0, err)
+               ? re.release() : nullptr;
   }
   // A single pattern: the anchored automaton first (cheap).  When it fits but an unanchored one does not (it tracks
   // every earlier start that may still begin a match: `error.{0,100}timeout` has 2^100 such subsets), the object
@@ -176,6 +195,16 @@ const rb::Dfa* Regex::host_dfa(DfaKind k, rb::Error* err) {
   if (patterns_.empty()) {  // an empty RegexSet matches nothing and has no automaton
     err->kind = rb::Error::Syntax;
     err->msg = "an empty pattern set has no automaton";
+    return nullptr;
+  }
+  if (k == kFwdUnanchoredAll && !groups_.empty()) {
+    std::string ranges;
+    for (size_t g = 0; g < groups_.size(); g++)
+      ranges += (g ? ", [" : "[") + std::to_string(group_first_[g]) + ", " +
+                std::to_string(g + 1 < groups_.size() ? group_first_[g + 1] : patterns_.size()) + ")";
+    err->kind = rb::Error::DfaTooBig;
+    err->msg = "this RegexSet is searched in " + std::to_string(groups_.size()) + " pattern groups (" + ranges +
+               "), each with its own automaton; there is no product automaton of the whole set";
     return nullptr;
   }
   if (unanchored_too_big_ && k != kFwdAnchoredLF && k != kRevAnchoredLongest) {
@@ -1389,20 +1418,40 @@ int Regex::forward_range(const uint8_t* d_text, uint64_t n, uint64_t start, uint
 // state after the last position (what the right-hand shard must be entered with).
 int Regex::forward_reduce(const uint8_t* d_text, uint64_t n, uint64_t start, bool want_masks, uint64_t* result_host, uint64_t end,
                           uint32_t entry, uint32_t* exit_out) {
-  result_host[0] = kNone;
-  for (uint32_t w = 0; w < kMaxMaskWords; w++) result_host[1 + w] = 0;
   const uint32_t n_pat = (uint32_t)patterns_.size();
+  const uint32_t rw = result_words() - 1;
+  result_host[0] = kNone;
+  for (uint32_t w = 0; w < rw; w++) result_host[1 + w] = 0;
+  if (int rc = init_device()) return rc;
+  // The automata of this search: the product automaton, or one per pattern group.  Every wave runs each group that
+  // is still open over the same positions; each group carries its own state into the next wave.
+  std::vector<Regex*> tabs{this};
+  std::vector<uint32_t> firsts{0};
+  if (!groups_.empty()) {
+    if (entry != kNoEntry || end != ~0ull) return fail("a RegexSet searched in pattern groups cannot be searched in shards");
+    tabs.clear();
+    for (auto& g : groups_) {
+      g->tuning = tuning;
+      g->sparse_set_ = sparse_set_;
+      g->set_stream(stream_);
+      tabs.push_back(g.get());
+    }
+    firsts = group_first_;
+  }
+  const uint32_t n_tab = (uint32_t)tabs.size();
+  std::vector<uint32_t> entries(n_tab, entry);
+  std::vector<char> done(n_tab, 0);
   uint64_t wave = tuning.wave0 ? (tuning.wave0 + 4095) / 4096 * 4096 : 0;
   uint64_t lo = start;
   end = std::min(end, n + 1);
   const bool whole = end == n + 1 && entry == kNoEntry;  // narrowing restarts the search at `start` with a fresh automaton
   if (exit_out) *exit_out = entry == kNoEntry ? kNoState : entry;
   stats.scan_redo_rounds = stats.scan_redo_segments = stats.map_passes = stats.waves = 0;
+  stats.groups = n_tab;
+  std::vector<uint64_t> before(rw);
   for (uint32_t wi = 0;; wi++) {
     uint64_t limit = end;
     if (wave && end - lo > 2 * wave) limit = (lo + wave) / 4096 * 4096;
-    uint64_t r[1 + kMaxMaskWords];
-    uint32_t exit_state = 0;
     if (lazy_) {  // host haystack: bring in what this wave reads (plus a little for the flags at its end)
       const uint64_t want = std::min(lazy_->n, limit + 64);
       if (want > lazy_->done) {
@@ -1410,18 +1459,32 @@ int Regex::forward_reduce(const uint8_t* d_text, uint64_t n, uint64_t start, boo
         lazy_->done = want;
       }
     }
-    if (int rc = forward_range(d_text, n, lo, limit, entry, want_masks, r, &exit_state)) return rc;
-    stats.waves++;
-    result_host[0] = std::min(result_host[0], r[0]);
-    bool fresh = false;
-    for (uint32_t w = 0; w < kMaxMaskWords; w++) {
-      fresh = fresh || (r[1 + w] & ~result_host[1 + w]);
-      result_host[1 + w] |= r[1 + w];
+    std::copy(result_host + 1, result_host + 1 + rw, before.begin());
+    bool live = false;
+    for (uint32_t g = 0; g < n_tab; g++) {
+      if (done[g]) continue;
+      uint64_t r[1 + kMaxMaskWords];
+      uint32_t exit_state = 0;
+      if (int rc = tabs[g]->forward_range(d_text, n, lo, limit, entries[g], want_masks, r, &exit_state))
+        return tabs[g] == this ? rc : fail(tabs[g]->last_error());
+      result_host[0] = std::min(result_host[0], r[0]);
+      // group-local mask bit j is pattern firsts[g] + j
+      const uint32_t w0 = firsts[g] / 64, sh = firsts[g] % 64;
+      for (uint32_t w = 0; w < kMaxMaskWords && w0 + w < rw; w++) {
+        result_host[1 + w0 + w] |= r[1 + w] << sh;
+        if (sh && w0 + w + 1 < rw) result_host[2 + w0 + w] |= r[1 + w] >> (64 - sh);
+      }
+      entries[g] = exit_state;
+      if (exit_out) *exit_out = exit_state;
+      if (exit_state == 0) done[g] = 1;  // dead state: an anchored search that can no longer match
+      live = live || !done[g];
     }
-    if (exit_out) *exit_out = exit_state;
+    stats.waves++;
+    bool fresh = false;
+    for (uint32_t w = 0; w < rw; w++) fresh = fresh || (result_host[1 + w] & ~before[w]);
     if (limit == end) break;
     if (!want_masks && result_host[0] != kNone) break;
-    if (exit_state == 0) break;  // dead state: an anchored search that can no longer match
+    if (!live) break;
     if (want_masks) {
       std::vector<uint32_t> open;
       for (uint32_t i = 0; i < n_pat; i++)
@@ -1430,12 +1493,12 @@ int Regex::forward_reduce(const uint8_t* d_text, uint64_t n, uint64_t start, boo
       if (tuning.narrow_sets && whole && wi < 2 && fresh && open.size() < n_pat) {
         Regex* sub = nullptr;
         if (int rc = subset(open, &sub)) return rc;
-        uint64_t sr[1 + kMaxMaskWords];
+        std::vector<uint64_t> sr(sub->result_words());
         sub->tuning.wave0 = tuning.wave0;
         sub->set_stream(stream_);
         sub->lazy_ = lazy_;
         std::lock_guard<std::recursive_mutex> lock(sub->mu_);
-        const int src = sub->forward_reduce(d_text, n, start, true, sr);
+        const int src = sub->forward_reduce(d_text, n, start, true, sr.data());
         sub->lazy_ = nullptr;
         if (src) return fail(sub->last_error());
         stats.waves += sub->stats.waves;
@@ -1443,11 +1506,99 @@ int Regex::forward_reduce(const uint8_t* d_text, uint64_t n, uint64_t start, boo
           if ((sr[1 + j / 64] >> (j % 64)) & 1) result_host[1 + open[j] / 64] |= 1ull << (open[j] % 64);
         break;
       }
+      // a group whose patterns have all matched needs no further waves
+      for (uint32_t g = 0; g < n_tab && n_tab > 1; g++) {
+        const uint32_t hi = g + 1 < n_tab ? firsts[g + 1] : n_pat;
+        bool all = true;
+        for (uint32_t i = firsts[g]; i < hi && all; i++) all = (result_host[1 + i / 64] >> (i % 64)) & 1;
+        if (all) done[g] = 1;
+      }
     }
     lo = limit;
-    entry = exit_state;
     wave *= 16;
   }
+  return 0;
+}
+
+// ------------------------------------------------------------ pattern groups --
+// One group: the set-mode Regex of patterns [lo, hi) with one product automaton (or the error of its determinization).
+Regex* Regex::compile_group(const std::vector<std::string>& all, uint32_t lo, uint32_t hi, const CompileOptions& opt, rb::Error* err) {
+  const std::vector<std::string> pats(all.begin() + lo, all.begin() + hi);
+  CompileOptions o = opt;
+  o.as_set = true;
+  const std::vector<uint32_t> one{0};
+  return compile_impl(pats, o, err, &one, 0);
+}
+
+// Groups for [lo, hi): the range itself when its automaton fits (and it is not known not to), else its two halves.
+// Ranges of more than 64 patterns split on a multiple of 64 so that large groups own whole mask words.  A single
+// pattern over budget fails with its determinization's error.
+bool Regex::plan_range(uint32_t lo, uint32_t hi, bool known_too_big, std::vector<std::unique_ptr<Regex>>* out,
+                       std::vector<uint32_t>* firsts, rb::Error* err) {
+  if (!known_too_big) {
+    rb::Error e;
+    if (Regex* g = compile_group(patterns_, lo, hi, opt_, &e)) {
+      out->emplace_back(g);
+      firsts->push_back(lo);
+      return true;
+    }
+    if (e.kind != rb::Error::DfaTooBig || hi - lo == 1) { *err = e; return false; }
+  }
+  const uint32_t n = hi - lo;
+  uint32_t mid = lo + n / 2;
+  if (n > 64) {
+    mid = (lo + n / 2 + 32) / 64 * 64;
+    if (mid <= lo) mid += 64;
+    if (mid >= hi) mid -= 64;
+  }
+  return plan_range(lo, mid, false, out, firsts, err) && plan_range(mid, hi, false, out, firsts, err);
+}
+
+// Replaces the group plan: `plan` = the first pattern of each group, compiled as given; else chunks of `chunk`
+// patterns split by the budget (the first chunk is known to be over budget when `first_too_big`).  One resulting
+// group is the product automaton.  On failure the object is unchanged.
+bool Regex::build_groups(const std::vector<uint32_t>* plan, uint32_t chunk, bool first_too_big, rb::Error* err) {
+  const uint32_t n = (uint32_t)patterns_.size();
+  std::vector<std::unique_ptr<Regex>> gs;
+  std::vector<uint32_t> firsts;
+  if (plan) {
+    for (size_t i = 0; i < plan->size(); i++) {
+      const uint32_t lo = (*plan)[i], hi = i + 1 < plan->size() ? (*plan)[i + 1] : n;
+      Regex* g = compile_group(patterns_, lo, hi, opt_, err);
+      if (!g) return false;
+      gs.emplace_back(g);
+      firsts.push_back(lo);
+    }
+  } else {
+    for (uint32_t lo = 0; lo < n; lo += chunk)
+      if (!plan_range(lo, std::min(n, lo + chunk), lo == 0 && first_too_big, &gs, &firsts, err)) return false;
+  }
+  subsets_.clear();
+  if (gs.size() == 1) {
+    host_[kFwdUnanchoredAll] = std::move(gs[0]->host_[kFwdUnanchoredAll]);
+    product_fits_ = true;
+    groups_.clear();
+    group_first_.clear();
+    return true;
+  }
+  groups_ = std::move(gs);
+  group_first_ = std::move(firsts);
+  return true;
+}
+
+int Regex::set_group_patterns(uint32_t k) {
+  std::lock_guard<std::recursive_mutex> lock(mu_);
+  if (!is_set_) return fail("set_group_patterns applies to a RegexSet");
+  if (patterns_.empty()) return 0;  // an empty set has no automaton and nothing to group
+  if (k == 0 && product_fits_) {
+    groups_.clear();
+    group_first_.clear();
+    subsets_.clear();
+    return 0;
+  }
+  rb::Error err;
+  const uint32_t cap = 64 * kMaxMaskWords;
+  if (!build_groups(nullptr, k ? std::min(k, cap) : cap, k == 0 && patterns_.size() <= cap, &err)) return fail("set_group_patterns: " + err.msg);
   return 0;
 }
 
@@ -1476,8 +1627,8 @@ int Regex::shortest_match_device(const uint8_t* d_text, uint64_t n, uint64_t sta
   *found = false;
   if (patterns_.empty() || start > n) return 0;
   if (candidate_mode()) return cand_shortest(d_text, n, start, found, end);
-  uint64_t res[1 + kMaxMaskWords];
-  if (int rc = forward_reduce(d_text, n, start, false, res)) return rc;
+  std::vector<uint64_t> res(result_words());
+  if (int rc = forward_reduce(d_text, n, start, false, res.data())) return rc;
   if (res[0] != kNone) { *found = true; *end = res[0]; }
   return 0;
 }
@@ -1488,8 +1639,8 @@ int Regex::set_matches_device(const uint8_t* d_text, uint64_t n, uint64_t start,
   const uint32_t mw = (uint32_t)((patterns_.size() + 63) / 64);
   for (uint32_t w = 0; w < mw; w++) masks[w] = 0;
   if (patterns_.empty() || start > n) return 0;
-  uint64_t res[1 + kMaxMaskWords];
-  if (int rc = forward_reduce(d_text, n, start, true, res)) return rc;
+  std::vector<uint64_t> res(result_words());
+  if (int rc = forward_reduce(d_text, n, start, true, res.data())) return rc;
   for (uint32_t w = 0; w < mw; w++) { masks[w] = res[1 + w]; if (res[1 + w]) *any = true; }
   return 0;
 }
@@ -1514,6 +1665,10 @@ int Regex::forward_shard_device(const uint8_t* d_text, uint64_t n, uint64_t own_
   if (candidate_mode())
     return fail("sharded shortest_match / is_match is not available for a pattern searched from candidate starts (its unanchored "
                 "automaton exceeds the DFA table budget); use shortest_match on the whole haystack");
+  if (!groups_.empty())
+    return fail("sharded RegexSet searches are not available for a set searched in " + std::to_string(groups_.size()) +
+                " pattern groups (the shard protocol carries one automaton state and at most 256 pattern bits); use "
+                "set_matches on the whole haystack");
   DeviceDfa* fwd;
   if (int rc = ensure(kFwdUnanchoredAll, &fwd)) return rc;
   if (entry == kNoEntry && own_lo > 0) {
@@ -1533,9 +1688,9 @@ int Regex::forward_shard_device(const uint8_t* d_text, uint64_t n, uint64_t own_
     entry = st;
   }
   *entry_used = entry;
-  uint64_t res[1 + kMaxMaskWords];
+  std::vector<uint64_t> res(result_words());
   const uint64_t end = is_last ? n + 1 : own_hi;
-  if (int rc = forward_reduce(d_text, n, own_lo, want_masks, res, end, entry, exit_state)) return rc;
+  if (int rc = forward_reduce(d_text, n, own_lo, want_masks, res.data(), end, entry, exit_state)) return rc;
   if (res[0] != kNone) { *found = true; *first_end = res[0]; }
   for (uint32_t w = 0; w < mw; w++) { masks[w] = res[1 + w]; if (want_masks && res[1 + w]) *found = true; }
   return 0;
@@ -1755,6 +1910,8 @@ int Regex::set_matches_batch_device(const uint8_t* d_text, const uint64_t* d_off
     RB_CUDA(cudaStreamSynchronize((cudaStream_t)stream_));
     return 0;
   }
+  if (!groups_.empty()) return set_matches_batch_grouped(d_text, d_offsets, n_rec, d_masks);
+  stats.groups = 1;
   DeviceDfa* fwd;
   if (int rc = ensure(kFwdUnanchoredAll, &fwd)) return rc;
   BatchArgs a{};
@@ -1769,6 +1926,46 @@ int Regex::set_matches_batch_device(const uint8_t* d_text, const uint64_t* d_off
   set_matches_batch<<<(uint32_t)((n_rec + 255) / 256), 256, smem, (cudaStream_t)stream_>>>(a);
   RB_LAUNCH_CHECK("set_matches_batch");
   RB_CUDA(cudaStreamSynchronize((cudaStream_t)stream_));
+  return 0;
+}
+
+// One launch for every group of a grouped set (gridDim.y = groups): each CTA stages its group's table when it fits.
+int Regex::set_matches_batch_grouped(const uint8_t* d_text, const uint64_t* d_offsets, uint64_t n_rec, uint64_t* d_masks) {
+  if (int rc = init_device()) return rc;
+  const uint32_t n_pat = (uint32_t)patterns_.size(), n_g = (uint32_t)groups_.size(), rw = (n_pat + 63) / 64;
+  cudaStream_t st = (cudaStream_t)stream_;
+  std::vector<GroupDesc> descs(n_g);
+  size_t smem = 0;
+  for (uint32_t g = 0; g < n_g; g++) {
+    Regex* gr = groups_[g].get();
+    gr->tuning = tuning;
+    gr->set_stream(stream_);
+    DeviceDfa* fwd;
+    if (gr->ensure(kFwdUnanchoredAll, &fwd)) return fail(gr->last_error());
+    const size_t s = smem_for(fwd->view);
+    descs[g].view = fwd->view;
+    descs[g].lo = group_first_[g];
+    descs[g].hi = g + 1 < n_g ? group_first_[g + 1] : n_pat;
+    descs[g].use_smem = s != 0;
+    smem = std::max(smem, s);
+  }
+  GroupDesc* d_descs = (GroupDesc*)group_descs_.ensure(n_g * sizeof(GroupDesc));
+  if (!d_descs) return fail("out of device memory (group tables)");
+  RB_CUDA(cudaMemcpyAsync(d_descs, descs.data(), n_g * sizeof(GroupDesc), cudaMemcpyHostToDevice, st));
+  RB_CUDA(cudaMemsetAsync(d_masks, 0, n_rec * 8 * rw, st));
+  GroupBatchArgs a{};
+  a.groups = d_descs;
+  a.text = d_text;
+  a.offsets = d_offsets;
+  a.n_rec = n_rec;
+  a.out_masks = d_masks;
+  a.row_words = rw;
+  a.n_patterns = n_pat;
+  RB_CUDA(allow_smem(set_matches_batch_groups, smem));
+  set_matches_batch_groups<<<dim3((uint32_t)((n_rec + 255) / 256), n_g), 256, smem, st>>>(a);
+  RB_LAUNCH_CHECK("set_matches_batch_groups");
+  RB_CUDA(cudaStreamSynchronize(st));
+  stats.groups = n_g;
   return 0;
 }
 

@@ -4,6 +4,7 @@
 // search runs on the GPU -- there is no CPU matching path in this library.
 #pragma once
 #include <cstdint>
+#include <algorithm>
 #include <map>
 #include <memory>
 #include <mutex>
@@ -50,6 +51,7 @@ struct Stats {  // filled by the last single-haystack call (diagnostics, bench r
   float scan_ms = 0, walk_ms = 0, total_ms = 0;
   bool fused = false;  // the scan kernel also walked the chains (scan_ms covers both)
   int path = 0;        // last find_all: 0 generic scan, 1 fast scan, 2 fused scan + walk, 3 literal prefilter, 4 candidate starts
+  uint32_t groups = 0; // RegexSet calls: pattern groups (automata) searched in the first wave
 };
 
 constexpr uint32_t kNoState = 0xFFFFFFFFu;
@@ -85,10 +87,23 @@ class DeviceBuf {
 class Regex {
  public:
   static Regex* compile(const std::vector<std::string>& patterns, const CompileOptions& opt, rb::Error* err);
+  // The same patterns, options and pattern groups, compiled again (a second engine for another thread): a grouped
+  // set compiles its planned groups directly and never repeats the determinization that failed.
+  Regex* clone(rb::Error* err) const;
   ~Regex();
 
   size_t n_patterns() const { return patterns_.size(); }
   bool is_set() const { return is_set_; }
+  // RegexSets in groups (DESIGN.md §2): first pattern index of each group; one entry (0) when one product
+  // automaton covers the whole set, none for an empty set.
+  std::vector<uint32_t> group_firsts() const {
+    if (patterns_.empty()) return {};
+    return groups_.empty() ? std::vector<uint32_t>{0} : group_first_;
+  }
+  bool grouped() const { return !groups_.empty(); }
+  // Re-plan the groups with at most k patterns each (then split further by the table budget); 0 = automatic
+  // (the product automaton when it fits).  Fails when a group does not compile; the plan is then unchanged.
+  int set_group_patterns(uint32_t k);
   // Exclusive use of this object's device scratch for one call (the entry points lock mu_ themselves; the C ABI
   // uses these to find an idle engine when several threads share one rure*).
   bool try_acquire() { return mu_.try_lock(); }
@@ -231,11 +246,22 @@ class Regex {
   int cand_batch(int mode, const uint8_t* d_text, const uint64_t* d_offsets, uint64_t n_rec, uint32_t* d_bits, uint64_t* d_spans,
                  uint64_t* d_match_offsets, uint64_t cap);
   int batch_route(bool* cand);  // batched find / find_iter: candidate starts, or kind 4 (switches to the mode when it is over budget)
+  // words of forward_reduce's result: first match end + the pattern mask (at least kMaxMaskWords words)
+  uint32_t result_words() const { return 1 + std::max<uint32_t>(4, (uint32_t)((patterns_.size() + 63) / 64)); }
   int forward_reduce(const uint8_t* d_text, uint64_t n, uint64_t start, bool want_masks, uint64_t* result_host, uint64_t end = ~0ull,
                      uint32_t entry = 0xFFFFFFFFu, uint32_t* exit_out = nullptr);
   int forward_range(const uint8_t* d_text, uint64_t n, uint64_t start, uint64_t limit, uint32_t entry, bool want_masks,
                     uint64_t* result_host, uint32_t* exit_state);
   int subset(const std::vector<uint32_t>& members, Regex** out);
+  // Pattern groups: plan contiguous ranges of at most `chunk` patterns whose kind-2 automata fit the budget
+  // (ranges over budget are halved); `plan` non-null compiles those ranges as given.
+  static Regex* compile_impl(const std::vector<std::string>& patterns, const CompileOptions& opt, rb::Error* err,
+                             const std::vector<uint32_t>* plan, uint32_t chunk);
+  bool build_groups(const std::vector<uint32_t>* plan, uint32_t chunk, bool first_too_big, rb::Error* err);
+  static Regex* compile_group(const std::vector<std::string>& all, uint32_t lo, uint32_t hi, const CompileOptions& opt, rb::Error* err);
+  bool plan_range(uint32_t lo, uint32_t hi, bool known_too_big, std::vector<std::unique_ptr<Regex>>* out, std::vector<uint32_t>* firsts,
+                  rb::Error* err);
+  int set_matches_batch_grouped(const uint8_t* d_text, const uint64_t* d_offsets, uint64_t n_rec, uint64_t* d_masks);
   const uint8_t* upload_text(const uint8_t* text, uint64_t n, int* rc);
   int find_all_host_pipelined(const uint8_t* text, uint64_t n, uint8_t* d, uint64_t* d_out, uint64_t* out, uint64_t cap, uint64_t* total);
 
@@ -245,6 +271,10 @@ class Regex {
   bool is_set_ = false;
   bool sparse_set_ = false;  // a narrowed RegexSet: none of its patterns matched in the first waves
   std::map<std::vector<uint32_t>, std::unique_ptr<Regex>> subsets_;
+  std::vector<uint32_t> group_first_;                // grouped set: first pattern of each group
+  std::vector<std::unique_ptr<Regex>> groups_;       // grouped set: one set-mode Regex per group (empty: one product automaton)
+  bool product_fits_ = false;                        // the whole set's kind-2 automaton was determinized within budget
+  DeviceBuf group_descs_;                            // launch.h GroupDesc per group (batched records)
   CompileOptions opt_;
   std::vector<rb::Expr> exprs_;
   std::unique_ptr<rb::Dfa> host_[kNumDfaKinds];

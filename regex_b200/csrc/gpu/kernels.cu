@@ -3104,29 +3104,26 @@ __global__ void __launch_bounds__(512) batch_refill(BatchArgs a) {
 template __global__ void batch_refill<0>(BatchArgs);
 template __global__ void batch_refill<1>(BatchArgs);
 
-// dfa.rs:525-570 per record: OR of the per-state pattern masks along the scan.
-__global__ void set_matches_batch(BatchArgs a) {
-  const Table T = stage_table(a.fwd, g_smem, a.use_smem);
-  const uint64_t r = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x;
-  if (r >= a.n_rec) return;
-  const uint64_t lo = a.offsets[r], len = a.offsets[r + 1] - lo;
-  const uint8_t* p = a.text + lo;
-  const uint32_t mw = a.fwd.mask_words;
-  uint64_t acc[kMaxMaskWords] = {0, 0, 0, 0};
-  uint32_t s = pick_start_fwd(a.fwd, p, len, 0);
+// dfa.rs:525-570 per record: OR of the per-state pattern masks of automaton d along the scan of record r.
+__device__ __forceinline__ void set_record_masks(const Table& T, const DfaView& d, const uint8_t* text, const uint64_t* offsets,
+                                                 uint64_t n_rec, uint64_t r, uint64_t (&acc)[kMaxMaskWords]) {
+  const uint64_t lo = offsets[r], len = offsets[r + 1] - lo;
+  const uint8_t* p = text + lo;
+  const uint32_t mw = d.mask_words;
+  uint32_t s = pick_start_fwd(d, p, len, 0);
   uint32_t last_match = 0;  // masks of this state are already in acc
   auto consume = [&](uint32_t ns) {
     s = ns;
-    if (s >= a.fwd.match_lo && s != last_match) {
+    if (s >= d.match_lo && s != last_match) {
       last_match = s;
 #pragma unroll
       for (uint32_t w = 0; w < kMaxMaskWords; w++)
-        if (w < mw) acc[w] |= a.fwd.masks[(uint64_t)s * mw + w];
+        if (w < mw) acc[w] |= d.masks[(uint64_t)s * mw + w];
     }
   };
   // the record 16 bytes at a time (three aligned 8-byte loads) while that stays inside the buffer
-  const bool aligned = (reinterpret_cast<uintptr_t>(a.text) & 7) == 0;
-  const uint8_t* const buf_hi = a.text + a.offsets[a.n_rec];
+  const bool aligned = (reinterpret_cast<uintptr_t>(text) & 7) == 0;
+  const uint8_t* const buf_hi = text + offsets[n_rec];
   uint64_t q = 0;
   while (q < len && s != 0) {
     const uint8_t* wp = p + q;
@@ -3145,9 +3142,41 @@ __global__ void set_matches_batch(BatchArgs a) {
     }
   }
   if (s != 0) consume(T.step_eof(s));
+}
+
+__global__ void set_matches_batch(BatchArgs a) {
+  const Table T = stage_table(a.fwd, g_smem, a.use_smem);
+  const uint64_t r = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x;
+  if (r >= a.n_rec) return;
+  uint64_t acc[kMaxMaskWords] = {0, 0, 0, 0};
+  set_record_masks(T, a.fwd, a.text, a.offsets, a.n_rec, r, acc);
+  const uint32_t mw = a.fwd.mask_words;
 #pragma unroll
   for (uint32_t w = 0; w < kMaxMaskWords; w++)
     if (w < mw) a.out_masks[r * mw + w] = acc[w];
+}
+
+// A RegexSet in pattern groups: blockIdx.y is the group.  Its bit j is bit lo + j of the record's row; a word that
+// two groups share takes an atomic OR, a word the group owns alone a plain store (the rows are zeroed before).
+__global__ void set_matches_batch_groups(GroupBatchArgs a) {
+  const GroupDesc& g = a.groups[blockIdx.y];
+  const Table T = stage_table(g.view, g_smem, g.use_smem);
+  const uint64_t r = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x;
+  if (r >= a.n_rec) return;
+  uint64_t acc[kMaxMaskWords] = {0, 0, 0, 0};
+  set_record_masks(T, g.view, a.text, a.offsets, a.n_rec, r, acc);
+  const uint32_t w0 = g.lo / 64, sh = g.lo % 64, w_last = (g.hi - 1) / 64;
+  uint64_t* row = a.out_masks + r * a.row_words;
+#pragma unroll
+  for (uint32_t i = 0; i <= kMaxMaskWords; i++) {
+    const uint32_t k = w0 + i;
+    if (k > w_last) break;
+    uint64_t v = i < kMaxMaskWords ? acc[i % kMaxMaskWords] << sh : 0;
+    if (sh && i > 0) v |= acc[i - 1] >> (64 - sh);
+    const bool owned = g.lo <= 64 * k && g.hi >= min(64 * k + 64, a.n_patterns);
+    if (owned) row[k] = v;
+    else if (v) atomicOr(reinterpret_cast<unsigned long long*>(row + k), (unsigned long long)v);
+  }
 }
 
 

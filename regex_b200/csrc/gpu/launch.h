@@ -286,5 +286,21 @@ __global__ void scan_add_block_offsets(uint64_t* out, const uint64_t* block_sums
 __global__ void is_match_batch(BatchArgs a);
 __global__ void find_batch(BatchArgs a);
 __global__ void set_matches_batch(BatchArgs a);
+// A RegexSet in pattern groups (engine.cu set_matches_batch_groups): group g owns patterns [lo, hi)
+struct GroupDesc {
+  DfaView view;
+  uint32_t lo, hi;
+  int use_smem;  // the group's table is staged in shared memory
+};
+struct GroupBatchArgs {
+  const GroupDesc* groups;  // gridDim.y entries, in global memory
+  const uint8_t* text;
+  const uint64_t* offsets;  // n_rec + 1
+  uint64_t n_rec;
+  uint64_t* out_masks;      // row_words per record, zeroed before the launch
+  uint32_t row_words;       // (n_patterns + 63) / 64
+  uint32_t n_patterns;
+};
+__global__ void set_matches_batch_groups(GroupBatchArgs a);
 
 }  // namespace rbgpu
