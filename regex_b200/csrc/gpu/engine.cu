@@ -584,18 +584,13 @@ int Regex::cand_batch(int mode, const uint8_t* d_text, const uint64_t* d_offsets
   CandArgs c;
   if (int rc = cand_args(&c)) return rc;
   BatchArgs a{};
-  a.fwd = fwd->view;
-  if (rev) a.rev = rev->view;
-  const size_t smem = smem_for(fwd->view);
-  a.use_smem = smem != 0;
-  a.text = d_text;
-  a.offsets = d_offsets;
-  a.n_rec = n_rec;
+  size_t smem;
+  uint32_t per_sm;
+  batch_args(&a, d_text, d_offsets, n_rec, fwd, rev, 0, 0, &smem, &per_sm);
   a.out_bits = d_bits;
   a.out_spans = d_spans;
   a.match_offsets = d_match_offsets;
   a.cap = cap;
-  a.utf8 = only_utf8 ? 1 : 0;
   cudaStream_t st = (cudaStream_t)stream_;
   const uint32_t grid = grid_for(n_rec, 256, tuning.blocks_per_sm);
 #define RB_CAND(M)                                              \
@@ -1697,6 +1692,30 @@ int Regex::forward_shard_device(const uint8_t* d_text, uint64_t n, uint64_t own_
 }
 
 // -------------------------------------------------------------------- batch ----
+bool Regex::batch_args(BatchArgs* a, const uint8_t* d_text, const uint64_t* d_offsets, uint64_t n_rec, DeviceDfa* fwd, DeviceDfa* rev,
+                       size_t reserve, uint32_t max_per_sm, size_t* smem, uint32_t* per_sm) {
+  a->fwd = fwd->view;
+  if (rev) a->rev = rev->view;
+  *smem = smem_for(fwd->view);
+  a->use_smem = *smem != 0;
+  a->text = d_text;
+  a->offsets = d_offsets;
+  a->n_rec = n_rec;
+  a->utf8 = only_utf8 ? 1 : 0;
+  *per_sm = 0;
+  if (!max_per_sm || !fwd->hot.n || (rev && !rev->hot.n) || ((uintptr_t)d_text & 15) != 0 || tuning.force_generic) return false;
+  a->fwd_hot = fwd->hot;
+  a->fwd_g = (const DfaView*)fwd->view_dev;
+  *smem = hot_bytes(fwd->hot.n) + 256;
+  if (rev) {
+    a->rev_hot = rev->hot;
+    a->rev_g = (const DfaView*)rev->view_dev;
+    *smem += hot_bytes(rev->hot.n);
+  }
+  *per_sm = (uint32_t)std::max<size_t>(1, std::min<size_t>(max_per_sm, (220 * 1024) / (*smem + reserve)));
+  return true;
+}
+
 int Regex::is_match_batch_device(const uint8_t* d_text, const uint64_t* d_offsets, uint64_t n_rec, uint32_t* d_bits) {
   std::lock_guard<std::recursive_mutex> lock(mu_);
   if (n_rec == 0) return 0;
@@ -1710,18 +1729,11 @@ int Regex::is_match_batch_device(const uint8_t* d_text, const uint64_t* d_offset
   DeviceDfa* fwd;
   if (int rc = ensure(kFwdUnanchoredAll, &fwd)) return rc;
   BatchArgs a{};
-  a.fwd = fwd->view;
-  const size_t smem = smem_for(fwd->view);
-  a.use_smem = smem != 0;
-  a.text = d_text;
-  a.offsets = d_offsets;
-  a.n_rec = n_rec;
+  size_t smem;
+  uint32_t per_sm;
+  const bool hot = batch_args(&a, d_text, d_offsets, n_rec, fwd, nullptr, 8192, 4, &smem, &per_sm);
   a.out_bits = d_bits;
-  if (fwd->hot.n && ((uintptr_t)d_text & 15) == 0 && !tuning.force_generic) {
-    a.fwd_hot = fwd->hot;
-    a.fwd_g = (const DfaView*)fwd->view_dev;
-    const size_t fsm = hot_bytes(fwd->hot.n) + 256;
-    const uint32_t per_sm = (uint32_t)std::max<size_t>(1, std::min<size_t>(4, (220 * 1024) / (fsm + 8192)));
+  if (hot) {
     // tasks of 96..2048 records, at least four per warp of the grid; smaller batches keep one record per lane
     const uint32_t grid0 = grid_for(n_rec, 512, per_sm);
     const uint64_t per_task = n_rec / ((uint64_t)grid0 * 16 * 4);
@@ -1733,12 +1745,12 @@ int Regex::is_match_batch_device(const uint8_t* d_text, const uint64_t* d_offset
       a.task_counter = (unsigned long long*)(counters + 16);
       RB_CUDA(cudaMemsetAsync(a.task_counter, 0, 8, (cudaStream_t)stream_));
       // (8 KB of static shared memory for the result words on top of the table: opt in whenever the sum may pass 48 KB)
-      RB_CUDA(allow_smem(batch_refill<0>, fsm, 48 * 1024));
-      batch_refill<0><<<grid_for(n_rec, 512, per_sm), 512, fsm, (cudaStream_t)stream_>>>(a);
-      RB_LAUNCH_CHECK("batch_refill<0>");
+      RB_CUDA(allow_smem(batch_refill, smem, 48 * 1024));
+      batch_refill<<<grid_for(n_rec, 512, per_sm), 512, smem, (cudaStream_t)stream_>>>(a);
+      RB_LAUNCH_CHECK("batch_refill");
     } else {
-      RB_CUDA(allow_smem(batch_fast<0>, fsm));
-      batch_fast<0><<<grid_for(n_rec, 512, per_sm), 512, fsm, (cudaStream_t)stream_>>>(a);
+      RB_CUDA(allow_smem(batch_fast<0>, smem));
+      batch_fast<0><<<grid_for(n_rec, 512, per_sm), 512, smem, (cudaStream_t)stream_>>>(a);
       RB_LAUNCH_CHECK("batch_fast<0>");
     }
   } else {
@@ -1761,35 +1773,15 @@ int Regex::find_batch_device(const uint8_t* d_text, const uint64_t* d_offsets, u
   if (int rc = ensure(kFwdUnanchoredLF, &fwd)) return rc;
   if (int rc = ensure(kRevAnchoredLongest, &rev)) return rc;
   BatchArgs a{};
-  a.fwd = fwd->view;
-  a.rev = rev->view;
-  a.text = d_text;
-  a.offsets = d_offsets;
-  a.n_rec = n_rec;
+  size_t smem;
+  uint32_t per_sm;
+  const bool hot = batch_args(&a, d_text, d_offsets, n_rec, fwd, rev, 16384, 4, &smem, &per_sm);
   a.out_bits = d_bits;
   a.out_spans = d_spans;
-  if (fwd->hot.n && rev->hot.n && ((uintptr_t)d_text & 15) == 0 && !tuning.force_generic) {
-    a.fwd_hot = fwd->hot;
-    a.rev_hot = rev->hot;
-    a.fwd_g = (const DfaView*)fwd->view_dev;
-    a.rev_g = (const DfaView*)rev->view_dev;
-    const size_t fsm = hot_bytes(fwd->hot.n) + hot_bytes(rev->hot.n) + 256;
-    const uint32_t per_sm = (uint32_t)std::max<size_t>(1, std::min<size_t>(4, (220 * 1024) / (fsm + 16384)));
-    const uint64_t per_task = n_rec / ((uint64_t)grid_for(n_rec, 512, per_sm) * 16 * 4);
-    a.task_recs = (uint32_t)std::max<uint64_t>(32, std::min<uint64_t>(2048, per_task / 32 * 32));
-    if (tuning.batch_refill > 1) {  // find: measured slower than batch_fast<1> on log lines, off unless asked for
-      uint32_t* counters = (uint32_t*)counters_.ensure(128);
-      if (!counters) return fail("out of device memory (batch scratch)");
-      a.task_counter = (unsigned long long*)(counters + 16);
-      RB_CUDA(cudaMemsetAsync(a.task_counter, 0, 8, (cudaStream_t)stream_));
-      RB_CUDA(allow_smem(batch_refill<1>, fsm, 48 * 1024));
-      batch_refill<1><<<grid_for(n_rec, 512, per_sm), 512, fsm, (cudaStream_t)stream_>>>(a);
-      RB_LAUNCH_CHECK("batch_refill<1>");
-    } else {
-      RB_CUDA(allow_smem(batch_fast<1>, fsm));
-      batch_fast<1><<<grid_for(n_rec, 512, per_sm), 512, fsm, (cudaStream_t)stream_>>>(a);
-      RB_LAUNCH_CHECK("batch_fast<1>");
-    }
+  if (hot) {
+    RB_CUDA(allow_smem(batch_fast<1>, smem));
+    batch_fast<1><<<grid_for(n_rec, 512, per_sm), 512, smem, (cudaStream_t)stream_>>>(a);
+    RB_LAUNCH_CHECK("batch_fast<1>");
   } else {
     find_batch<<<(uint32_t)((n_rec + 255) / 256), 256, 0, (cudaStream_t)stream_>>>(a);
     RB_LAUNCH_CHECK("find_batch");
@@ -1822,26 +1814,15 @@ int Regex::iter_batch(const uint8_t* d_text, const uint64_t* d_offsets, uint64_t
     return 0;
   }
   BatchArgs a{};
-  a.fwd = fwd->view;
-  a.rev = rev->view;
-  a.text = d_text;
-  a.offsets = d_offsets;
-  a.n_rec = n_rec;
+  size_t fsm;
+  uint32_t per_sm;
+  // __launch_bounds__(512, 2): two blocks per SM fit the registers of the iterator
+  const bool fast = batch_args(&a, d_text, d_offsets, n_rec, fwd, rev, 16384, cand ? 0 : 2, &fsm, &per_sm);
   a.match_offsets = d_match_offsets;
   a.out_spans = d_out;
   a.cap = d_out ? cap : 0;
-  a.utf8 = only_utf8 ? 1 : 0;
-  const bool fast = !cand && fwd->hot.n && rev->hot.n && ((uintptr_t)d_text & 15) == 0 && !tuning.force_generic;
-  size_t fsm = 0;
   uint32_t grid = (uint32_t)((n_rec + 255) / 256);
   if (fast) {
-    a.fwd_hot = fwd->hot;
-    a.rev_hot = rev->hot;
-    a.fwd_g = (const DfaView*)fwd->view_dev;
-    a.rev_g = (const DfaView*)rev->view_dev;
-    fsm = hot_bytes(fwd->hot.n) + hot_bytes(rev->hot.n) + 256;
-    // __launch_bounds__(512, 2): two blocks per SM fit the registers of the iterator
-    const uint32_t per_sm = (uint32_t)std::max<size_t>(1, std::min<size_t>(2, (220 * 1024) / (fsm + 16384)));
     grid = grid_for(n_rec, 512, per_sm);
     RB_CUDA(allow_smem(batch_iter_fast<0>, fsm));
     RB_CUDA(allow_smem(batch_iter_fast<1>, fsm));
@@ -1915,12 +1896,9 @@ int Regex::set_matches_batch_device(const uint8_t* d_text, const uint64_t* d_off
   DeviceDfa* fwd;
   if (int rc = ensure(kFwdUnanchoredAll, &fwd)) return rc;
   BatchArgs a{};
-  a.fwd = fwd->view;
-  const size_t smem = smem_for(fwd->view);
-  a.use_smem = smem != 0;
-  a.text = d_text;
-  a.offsets = d_offsets;
-  a.n_rec = n_rec;
+  size_t smem;
+  uint32_t per_sm;
+  batch_args(&a, d_text, d_offsets, n_rec, fwd, nullptr, 0, 0, &smem, &per_sm);
   a.out_masks = d_masks;
   RB_CUDA(allow_smem(set_matches_batch, smem));
   set_matches_batch<<<(uint32_t)((n_rec + 255) / 256), 256, smem, (cudaStream_t)stream_>>>(a);
@@ -2779,14 +2757,12 @@ int Regex::set_matches_host(const uint8_t* text, uint64_t n, uint64_t start, boo
 }
 int Regex::is_match_batch_host(const uint8_t* text, const uint64_t* offsets, uint64_t n_rec, uint8_t* out_bits) {
   std::lock_guard<std::recursive_mutex> lock(mu_);
-  int rc;
-  const uint64_t n = n_rec ? offsets[n_rec] : 0;
-  const uint8_t* d = upload_text(text, n, &rc);
+  const uint8_t* d;
+  uint64_t* d_off;
+  int rc = upload_batch(text, offsets, n_rec, &d, &d_off);
   if (rc) return rc;
-  uint64_t* d_off = (uint64_t*)offsets_.ensure((n_rec + 1) * 8);
   uint32_t* d_bits = (uint32_t*)bits_.ensure((n_rec + 31) / 32 * 4 + 4);
-  if (!d_off || !d_bits) return fail("out of device memory (batch)");
-  RB_CUDA(cudaMemcpyAsync(d_off, offsets, (n_rec + 1) * 8, cudaMemcpyHostToDevice, (cudaStream_t)stream_));
+  if (!d_bits) return fail("out of device memory (batch)");
   if ((rc = is_match_batch_device(d, d_off, n_rec, d_bits))) return rc;
   RB_CUDA(d2h(out_bits, d_bits, (n_rec + 7) / 8));
   return 0;
@@ -2794,14 +2770,12 @@ int Regex::is_match_batch_host(const uint8_t* text, const uint64_t* offsets, uin
 int Regex::find_iter_batch_host(const uint8_t* text, const uint64_t* offsets, uint64_t n_rec, uint64_t* match_offsets, uint64_t* out,
                                 uint64_t cap, uint64_t* total) {
   std::lock_guard<std::recursive_mutex> lock(mu_);
-  int rc;
-  const uint64_t n = n_rec ? offsets[n_rec] : 0;
-  const uint8_t* d = upload_text(text, n, &rc);
+  const uint8_t* d;
+  uint64_t* d_off;
+  int rc = upload_batch(text, offsets, n_rec, &d, &d_off);
   if (rc) return rc;
-  uint64_t* d_off = (uint64_t*)offsets_.ensure((n_rec + 1) * 8);
   uint64_t* d_moff = (uint64_t*)count_.ensure((n_rec + 1) * 8);
-  if (!d_off || !d_moff) return fail("out of device memory (batch)");
-  RB_CUDA(cudaMemcpyAsync(d_off, offsets, (n_rec + 1) * 8, cudaMemcpyHostToDevice, (cudaStream_t)stream_));
+  if (!d_moff) return fail("out of device memory (batch)");
   if (!out) cap = 0;
   uint64_t* d_spans = cap ? (uint64_t*)out_.ensure(cap * 16) : nullptr;
   if (cap && !d_spans) return fail("out of device memory (batch spans)");
@@ -2813,16 +2787,14 @@ int Regex::find_iter_batch_host(const uint8_t* text, const uint64_t* offsets, ui
 }
 int Regex::captures_batch_host(const uint8_t* text, const uint64_t* offsets, uint64_t n_rec, uint64_t* slots, uint8_t* out_bits) {
   std::lock_guard<std::recursive_mutex> lock(mu_);
-  int rc;
-  const uint64_t n = n_rec ? offsets[n_rec] : 0;
-  const uint8_t* d = upload_text(text, n, &rc);
+  const uint8_t* d;
+  uint64_t* d_off;
+  int rc = upload_batch(text, offsets, n_rec, &d, &d_off);
   if (rc) return rc;
   const uint64_t ns = 2 * (uint64_t)n_groups_;
-  uint64_t* d_off = (uint64_t*)offsets_.ensure((n_rec + 1) * 8);
   uint32_t* d_bits = (uint32_t*)bits_.ensure((n_rec + 31) / 32 * 4 + 4);
   uint64_t* d_slots = (uint64_t*)cap_slots_.ensure(std::max<uint64_t>(n_rec, 1) * ns * 8);
-  if (!d_off || !d_bits || !d_slots) return fail("out of device memory (batch)");
-  RB_CUDA(cudaMemcpyAsync(d_off, offsets, (n_rec + 1) * 8, cudaMemcpyHostToDevice, (cudaStream_t)stream_));
+  if (!d_bits || !d_slots) return fail("out of device memory (batch)");
   if ((rc = captures_batch_device(d, d_off, n_rec, d_slots, d_bits))) return rc;
   RB_CUDA(d2h(out_bits, d_bits, (n_rec + 7) / 8));
   RB_CUDA(d2h(slots, d_slots, n_rec * ns * 8));
@@ -2895,15 +2867,13 @@ int Regex::captures_iter_batch_host(const uint8_t* text, const uint64_t* offsets
 }
 int Regex::find_batch_host(const uint8_t* text, const uint64_t* offsets, uint64_t n_rec, uint64_t* spans, uint8_t* out_bits) {
   std::lock_guard<std::recursive_mutex> lock(mu_);
-  int rc;
-  const uint64_t n = n_rec ? offsets[n_rec] : 0;
-  const uint8_t* d = upload_text(text, n, &rc);
+  const uint8_t* d;
+  uint64_t* d_off;
+  int rc = upload_batch(text, offsets, n_rec, &d, &d_off);
   if (rc) return rc;
-  uint64_t* d_off = (uint64_t*)offsets_.ensure((n_rec + 1) * 8);
   uint32_t* d_bits = (uint32_t*)bits_.ensure((n_rec + 31) / 32 * 4 + 4);
   uint64_t* d_spans = (uint64_t*)out_.ensure(std::max<uint64_t>(n_rec, 1) * 16);
-  if (!d_off || !d_bits || !d_spans) return fail("out of device memory (batch)");
-  RB_CUDA(cudaMemcpyAsync(d_off, offsets, (n_rec + 1) * 8, cudaMemcpyHostToDevice, (cudaStream_t)stream_));
+  if (!d_bits || !d_spans) return fail("out of device memory (batch)");
   if ((rc = find_batch_device(d, d_off, n_rec, d_spans, d_bits))) return rc;
   RB_CUDA(d2h(out_bits, d_bits, (n_rec + 7) / 8));
   RB_CUDA(d2h(spans, d_spans, n_rec * 16));
@@ -2911,15 +2881,13 @@ int Regex::find_batch_host(const uint8_t* text, const uint64_t* offsets, uint64_
 }
 int Regex::set_matches_batch_host(const uint8_t* text, const uint64_t* offsets, uint64_t n_rec, uint64_t* masks) {
   std::lock_guard<std::recursive_mutex> lock(mu_);
-  int rc;
-  const uint64_t n = n_rec ? offsets[n_rec] : 0;
-  const uint8_t* d = upload_text(text, n, &rc);
+  const uint8_t* d;
+  uint64_t* d_off;
+  int rc = upload_batch(text, offsets, n_rec, &d, &d_off);
   if (rc) return rc;
   const uint32_t mw = (uint32_t)std::max<size_t>(1, (patterns_.size() + 63) / 64);
-  uint64_t* d_off = (uint64_t*)offsets_.ensure((n_rec + 1) * 8);
   uint64_t* d_masks = (uint64_t*)masks_.ensure(std::max<uint64_t>(n_rec, 1) * 8 * mw);
-  if (!d_off || !d_masks) return fail("out of device memory (batch)");
-  RB_CUDA(cudaMemcpyAsync(d_off, offsets, (n_rec + 1) * 8, cudaMemcpyHostToDevice, (cudaStream_t)stream_));
+  if (!d_masks) return fail("out of device memory (batch)");
   if ((rc = set_matches_batch_device(d, d_off, n_rec, d_masks))) return rc;
   RB_CUDA(d2h(masks, d_masks, n_rec * 8 * mw));
   return 0;

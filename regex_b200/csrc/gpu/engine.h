@@ -16,6 +16,8 @@
 
 namespace rbgpu {
 
+struct BatchArgs;  // launch.h
+
 struct CompileOptions {
   uint32_t flags = 32;               // RURE_FLAG_* bits (rure.h:56-68); default = UNICODE
   size_t size_limit = 10u << 20;     // program size limit (re_builder.rs:29)
@@ -37,7 +39,8 @@ struct Tuning {
   uint32_t blocks_per_sm = 8;
   uint64_t wave0 = 64ull << 20;  // first wave of a forward search in bytes (x16 per wave); 0 = one wave
   bool narrow_sets = true;
-  int batch_refill = 1;          // 0 off, 1 is_match on large batches, 2 always and also find: batched is_match: lanes take the next record as soon as theirs is decided (batch_refill) instead of one record per lane per round
+  int batch_refill = 1;          // batched is_match: lanes take the next record as soon as theirs is decided (kernels.cu batch_refill) instead of
+                                 // one record per lane per round; 0 off, 1 batches large enough for tasks of >= 96 records, 2 any size (tests)
   int prefilter = 1;             // literal_scan instead of the DFA scan: 0 never, 1 when the scanned byte is estimated rare enough
                                  // to win (one byte, <= ~0.12 % of the haystack), 2 whenever the pattern qualifies structurally       // RegexSet::matches: continue with the automaton of the still-unmatched patterns
   uint32_t max_stitch_rounds = 16;  // re-walk rounds before the stitch falls back to one sequential pass
@@ -228,6 +231,14 @@ class Regex {
                  uint64_t* total, DeviceBuf* grow);
   // exclusive prefix sum of in[0, n) into out (in == out allowed); *d_total = device address of the sum
   int prefix_sum(const uint64_t* in, uint64_t* out, uint64_t n, unsigned long long** d_total);
+  // The fields every batched kernel takes (launch.h BatchArgs): views, text, offsets, n_rec, utf8; with the hot path
+  // also the hot tables and the views' device copies.  Returns whether the hot path applies: hot tables for fwd and
+  // rev (when given), 16-byte-aligned text, no force_generic, and max_per_sm > 0 (0: the caller has no hot kernel).
+  // *smem: dynamic shared memory, the hot tables on the hot path, else fwd's class-indexed table (0: not staged).
+  // *per_sm (hot path): blocks per SM, min(max_per_sm, 220 KiB / (*smem + reserve)), reserve = what a block is
+  // budgeted beyond its tables.
+  bool batch_args(BatchArgs* a, const uint8_t* d_text, const uint64_t* d_offsets, uint64_t n_rec, DeviceDfa* fwd, DeviceDfa* rev,
+                  size_t reserve, uint32_t max_per_sm, size_t* smem, uint32_t* per_sm);
   // text of every record of a host batch on the device (text_, boffsets_)
   int upload_batch(const uint8_t* text, const uint64_t* offsets, uint64_t n_rec, const uint8_t** d_text, uint64_t** d_offsets);
   int replace_prepare(const uint8_t* d_text, uint64_t n, const uint8_t* rep, uint64_t rep_len, bool expand, uint64_t limit, uint64_t* out_len);
@@ -290,7 +301,7 @@ class Regex {
   void* ext_stream_ = nullptr;
   bool use_ext_stream_ = false;
   // scratch (grow-only)
-  DeviceBuf text_, offsets_, bitmap_, guess_, fin_, redo_, counters_, seg_first_, seg_mask_;
+  DeviceBuf text_, bitmap_, guess_, fin_, redo_, counters_, seg_first_, seg_mask_;
   DeviceBuf long_tab_;
   static constexpr uint32_t kMaxLongRuns = 256;
   DeviceBuf spans_all_, lens_, lits_, rep_out_, pieces_, reps_before_;
@@ -304,7 +315,7 @@ class Regex {
   bool cap_anchored_ = false;
   // batched replace / split / captures_iter (never shared with the whole-haystack calls, which the per-record
   // captures_iter redo runs in between): match CSR and spans, kept CSR and spans, slots, divergence flags and list,
-  // and the host wrappers' offsets and results
+  // and the host wrappers' results; the record offsets of every batched host wrapper (boffsets_)
   DeviceBuf bmoff_, bspans_, bkoff_, bkspans_, bslots_, bflags_, blist_, boffsets_, bres_off_, bres_;
   DeviceBuf in_p_, in_lm_, out_p_, out_lm_, count_, offset_, dirty_, first_cand_, skip_, meta_, excl_, btot_, present_, kidx_, kstates_, maps_, comp_, bentry_, exact_, stage_, block_sums_, out_, bits_, masks_;
   void* pinned_ = nullptr;  // small pinned staging area for counters / scalars

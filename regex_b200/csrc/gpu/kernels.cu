@@ -469,7 +469,8 @@ __device__ __forceinline__ uint64_t next_bit(const uint64_t* bm, const uint8_t* 
 
 // End of the leftmost-first match anchored at s (src/dfa.rs:576-764 run on the
 // anchored program): last position at which a match state was entered, with the
-// one-byte delay and the EOF flush.
+// one-byte delay and the EOF flush.  On an unanchored leftmost-first automaton: the
+// end of the leftmost-first match found from s (the batched find_iter).
 // halo_err: non-null when the buffer is a shard whose text continues past n (running
 // into n then means the halo was too short, not end-of-text).
 __device__ __forceinline__ uint64_t anchored_end(const DfaView& d, const Table& T, const uint8_t* text, uint64_t n, uint64_t s,
@@ -484,6 +485,19 @@ __device__ __forceinline__ uint64_t anchored_end(const DfaView& d, const Table& 
     if (st == 0 || q >= n) break;
   }
   return last;
+}
+
+// First position at which the automaton, started at s with the flags there, enters a match state (the
+// shortest_match_at end, exec.rs:382-468); kNone when it dies first or reaches `bound`.
+__device__ __forceinline__ uint64_t earliest_end(const DfaView& d, const Table& T, const uint8_t* text, uint64_t n, uint64_t s,
+                                                 uint64_t bound = kNone) {
+  uint32_t st = pick_start_fwd(d, text, n, s);
+  for (uint64_t q = s; st != 0 && q < bound; q++) {
+    st = q < n ? T.step(st, __ldg(text + q)) : T.step_eof(st);
+    if (st >= d.match_lo) return q;
+    if (q >= n) break;
+  }
+  return kNone;
 }
 
 // Start of the match ending at e, found the way the reference does it: the
@@ -2516,39 +2530,43 @@ __global__ void is_match_batch(BatchArgs a) {
   bool matched = false;
   if (r < a.n_rec) {
     const uint64_t lo = a.offsets[r], len = a.offsets[r + 1] - lo;
-    const uint8_t* p = a.text + lo;
-    uint32_t s = pick_start_fwd(a.fwd, p, len, 0);
-    for (uint64_t q = 0; s != 0; q++) {
-      s = q < len ? T.step(s, p[q]) : T.step_eof(s);
-      if (s >= a.fwd.match_lo) { matched = true; break; }
-      if (q >= len) break;
-    }
+    matched = earliest_end(a.fwd, T, a.text + lo, len, 0) != kNone;
   }
   const uint32_t bits = __ballot_sync(0xffffffffu, matched);
   if ((threadIdx.x & 31) == 0 && r < a.n_rec) a.out_bits[r >> 5] = bits;
 }
 
-// exec.rs:632-662 per record: forward leftmost-first end, then reverse longest start.
+// exec.rs:632-662 per record on the class-indexed tables in global memory: forward leftmost-first end e, then
+// the start ms by the reverse longest automaton over the record.  false: no match (ms, me left as they are).
+// The forward loop is anchored_end's with plain loads instead of __ldg: through slow_find_record, __ldg here
+// changes the code of batch_fast<1> and costs it 0.4 % on C3 find (B200, 1000 W).
+__device__ __forceinline__ bool find_in_record(const DfaView& f, const DfaView& rv, const uint8_t* p, uint64_t len, uint64_t& ms,
+                                               uint64_t& me) {
+  uint32_t st = pick_start_fwd(f, p, len, 0);
+  uint64_t e = kNone;
+  for (uint64_t q = 0; st != 0; q++) {
+    st = q < len ? f.trans[st * f.stride + f.classes[p[q]]] : f.trans[st * f.stride + f.stride - 1];
+    if (st >= f.match_lo) e = q;
+    if (q >= len) break;
+  }
+  if (e == kNone) return false;
+  const uint64_t s = e == 0 ? 0 : slice_start(rv, p, len, 0, e);
+  if (s == kNone) return false;
+  ms = s;
+  me = e;
+  return true;
+}
+
 __global__ void find_batch(BatchArgs a) {
   const uint64_t r = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x;
   bool found = false;
   if (r < a.n_rec) {
     const uint64_t lo = a.offsets[r], len = a.offsets[r + 1] - lo;
-    const uint8_t* p = a.text + lo;
-    const DfaView& f = a.fwd;
-    uint32_t s = pick_start_fwd(f, p, len, 0);
-    uint64_t e = kNone;
-    for (uint64_t q = 0; s != 0; q++) {
-      s = q < len ? f.trans[s * f.stride + f.classes[p[q]]] : f.trans[s * f.stride + f.stride - 1];
-      if (s >= f.match_lo) e = q;
-      if (q >= len) break;
-    }
-    uint64_t ms = kNone;
-    if (e != kNone) ms = e == 0 ? 0 : slice_start(a.rev, p, len, 0, e);
-    if (ms != kNone) {
+    uint64_t ms, me;
+    if (find_in_record(a.fwd, a.rev, a.text + lo, len, ms, me)) {
       found = true;
       a.out_spans[2 * r] = ms;
-      a.out_spans[2 * r + 1] = e;
+      a.out_spans[2 * r + 1] = me;
     } else {
       a.out_spans[2 * r] = 0;
       a.out_spans[2 * r + 1] = 0;
@@ -2595,29 +2613,13 @@ __device__ __forceinline__ void window16q(const uint8_t* p, uint32_t (&v)[4]) {
 __device__ __forceinline__ uint32_t window_byte(const uint32_t (&v)[4], int i) {  // byte i, i compile-time
   return (v[i >> 2] >> (8 * (i & 3))) & 0xFFu;
 }
+// A record that left the hot set, again on the full tables (pointer arguments for the reason given at
+// slow_anchored_end).
 __device__ __noinline__ bool slow_is_match_record(const DfaView* f, const uint8_t* p, uint64_t len) {
-  uint32_t s = f->uniform_start ? f->start[32] : f->start[flags_forward(p, len, 0)];
-  for (uint64_t q = 0; s != 0; q++) {
-    s = q < len ? f->trans[s * f->stride + f->classes[p[q]]] : f->trans[s * f->stride + f->stride - 1];
-    if (s >= f->match_lo) return true;
-    if (q >= len) break;
-  }
-  return false;
+  return earliest_end(*f, global_table(*f), p, len, 0) != kNone;
 }
 __device__ __noinline__ bool slow_find_record(const DfaView* f, const DfaView* rv, const uint8_t* p, uint64_t len, uint64_t* ms_out, uint64_t* e_out) {
-  uint32_t s = f->uniform_start ? f->start[32] : f->start[flags_forward(p, len, 0)];
-  uint64_t e = kNone;
-  for (uint64_t q = 0; s != 0; q++) {
-    s = q < len ? f->trans[s * f->stride + f->classes[p[q]]] : f->trans[s * f->stride + f->stride - 1];
-    if (s >= f->match_lo) e = q;
-    if (q >= len) break;
-  }
-  if (e == kNone) return false;
-  const uint64_t ms = e == 0 ? 0 : slice_start(*rv, p, len, 0, e);
-  if (ms == kNone) return false;
-  *ms_out = ms;
-  *e_out = e;
-  return true;
+  return find_in_record(*f, *rv, p, len, *ms_out, *e_out);
 }
 
 // The forward loop of batch_fast: record bytes from q on, hot state e on entry (the start state for
@@ -2820,18 +2822,6 @@ __device__ __forceinline__ void iter_record(const BatchArgs& a, uint64_t r, cons
   if (PASS == 0) a.match_offsets[r] = k;
 }
 
-// leftmost-first match end from q on the class-indexed tables (the generic kernel and cold records)
-__device__ __forceinline__ uint64_t table_forward_end(const DfaView& f, const uint8_t* p, uint64_t len, uint64_t q) {
-  uint32_t s = pick_start_fwd(f, p, len, q);
-  uint64_t e = kNone;
-  for (; s != 0; q++) {
-    s = q < len ? f.trans[s * f.stride + f.classes[p[q]]] : f.trans[s * f.stride + f.stride - 1];
-    if (s >= f.match_lo) e = q;
-    if (q >= len) break;
-  }
-  return e;
-}
-
 // One thread per record on the hot tables, as batch_fast<1> (persistent blocks, 16-byte windows).  A
 // record that leaves the hot set finishes its iteration on the full tables in global memory.
 template <int PASS>
@@ -2856,7 +2846,7 @@ __global__ void __launch_bounds__(512, 2) batch_iter_fast(BatchArgs a) {
         if (e != 1u) return last;
         cold = true;
       }
-      return table_forward_end(*a.fwd_g, p, len, q);
+      return anchored_end(*a.fwd_g, global_table(*a.fwd_g), p, len, q);
     };
     auto rev = [&](uint64_t q, uint64_t e) -> uint64_t {
       if (!cold) {
@@ -2878,7 +2868,7 @@ __global__ void batch_iter(BatchArgs a) {
   if (r >= a.n_rec) return;
   const uint64_t lo = a.offsets[r], len = a.offsets[r + 1] - lo;
   const uint8_t* p = a.text + lo;
-  iter_record<PASS>(a, r, p, len, [&](uint64_t q) { return table_forward_end(a.fwd, p, len, q); },
+  iter_record<PASS>(a, r, p, len, [&](uint64_t q) { return anchored_end(a.fwd, global_table(a.fwd), p, len, q); },
                     [&](uint64_t q, uint64_t e) { return slice_start(a.rev, p, len, q, e); });
 }
 template __global__ void batch_iter<0>(BatchArgs);
@@ -2891,28 +2881,20 @@ template __global__ void batch_iter<1>(BatchArgs);
 // records; a lane that has decided its record takes the next one of the task as soon as kBatchRefill lanes
 // are free (the refill code runs for all of them together), so a step of the loop is one 16-byte window for
 // (nearly) every lane.  Result bits are collected in shared memory and leave as whole words.
+// is_match only: the same scheme for find (a forward loop, then a reverse loop for the starts) measured
+// slower than batch_fast<1> on log lines (profiles/r02_ncu_summaries.md §3b).
 constexpr uint32_t kBatchTask = 2048, kBatchRefill = 8;
-// MODE 0: is_match.  MODE 1: find -- two such loops per task: the forward one leaves the leftmost-first end of
-// every record that matches (and a bit in `todo`), the reverse one takes those records again for their start
-// (exec.rs:651-657 with the record as its own slice).  One loop with both phases mixed ran both code paths in
-// every step and was slower than batch_fast<1>.
-template <int MODE>
 __global__ void __launch_bounds__(512) batch_refill(BatchArgs a) {
-  __shared__ uint32_t task_bits[16][kBatchTask / 32];                   // blockDim.x == 512
-  __shared__ uint32_t task_todo[MODE == 1 ? 16 : 1][kBatchTask / 32];  // MODE 1: records that wait for the reverse loop
+  __shared__ uint32_t task_bits[16][kBatchTask / 32];  // blockDim.x == 512
   const uint32_t fbase = ((uint32_t)__cvta_generic_to_shared(g_smem) + 255u) & ~255u;
-  const uint32_t rbase = fbase + hot_table_bytes(a.fwd_hot.n);
   hot_stage(a.fwd_hot, fbase);
-  if (MODE == 1) hot_stage(a.rev_hot, rbase);
   __syncthreads();
   const uint32_t fthr = a.fwd_hot.match_lo, flive = 2;
-  const uint32_t rthr = a.rev_hot.match_lo, rlive = 2;
   const uint8_t* const buf_hi = a.text + a.offsets[a.n_rec];
   const uint32_t lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
   const uint32_t task_recs = a.task_recs;  // multiple of 32, at most kBatchTask (the host sizes it so that every warp gets several)
   const uint64_t n_tasks = (a.n_rec + task_recs - 1) / task_recs;
   uint32_t* bits = task_bits[wid];
-  uint32_t* todo = task_todo[MODE == 1 ? wid : 0];
   for (;;) {
     // tasks are handed out through a global counter: with a fixed assignment the warps that get one task
     // more than the others decide the kernel's time
@@ -2921,32 +2903,17 @@ __global__ void __launch_bounds__(512) batch_refill(BatchArgs a) {
     task = __shfl_sync(0xffffffffu, task, 0);
     if (task >= n_tasks) break;
     const uint64_t r_lo = task * task_recs, r_hi = min(r_lo + task_recs, a.n_rec);
-    for (uint32_t i = lane; i < task_recs / 32; i += 32) { bits[i] = 0; if (MODE == 1) todo[i] = 0; }
+    for (uint32_t i = lane; i < task_recs / 32; i += 32) bits[i] = 0;
     __syncwarp();
     uint64_t next = r_lo;  // warp-uniform: first record of the task not handed out yet
     bool idle = true;
     uint64_t r = 0, len = 0, q = 0;
     const uint8_t* p = a.text;
     uint32_t e = 0, mx = 0;
-    uint64_t last = kNone;  // MODE 1: match end
-    auto finish = [&](bool hit, uint64_t ms, uint64_t me) {
+    auto finish = [&](bool hit) {
       if (hit) atomicOr(&bits[(uint32_t)(r - r_lo) >> 5], 1u << ((uint32_t)(r - r_lo) & 31u));
-      if (MODE == 1) {
-        a.out_spans[2 * r] = hit ? ms : 0;
-        a.out_spans[2 * r + 1] = hit ? me : 0;
-      }
       idle = true;
     };
-    auto finish_slow = [&]() {  // the record left the hot set: again on the full tables
-      if (MODE == 0) {
-        finish(slow_is_match_record(a.fwd_g, p, len), 0, 0);
-      } else {
-        uint64_t ms = 0, me = 0;
-        const bool hit = slow_find_record(a.fwd_g, a.rev_g, p, len, &ms, &me);
-        finish(hit, ms, me);
-      }
-    };
-    // ---- forward loop ----
     for (;;) {
       const uint32_t idle_m = __ballot_sync(0xffffffffu, idle);
       if (idle_m == 0xffffffffu && next >= r_hi) break;
@@ -2959,7 +2926,6 @@ __global__ void __launch_bounds__(512) batch_refill(BatchArgs a) {
           p = a.text + lo;
           q = 0;
           mx = 0;
-          last = kNone;
           const uint32_t h0 = a.fwd.uniform_start ? a.fwd_hot.start : a.fwd_hot.full2hot[a.fwd.start[flags_forward(p, len, 0)]];
           e = h0 == 0xFFFFu ? 1u : h0;
           idle = false;
@@ -2970,7 +2936,7 @@ __global__ void __launch_bounds__(512) batch_refill(BatchArgs a) {
       bool done = false;
       const uint64_t left = len - q;
       if (left == 0) {  // EOF step
-        if (e >= flive && a.fwd_hot.eof[e] >= a.fwd.match_lo) { mx = 0xFFFFFFFFu; last = len; }
+        if (e >= flive && a.fwd_hot.eof[e] >= a.fwd.match_lo) mx = 0xFFFFFFFFu;
         done = true;
       } else if (e < flive) {
         done = true;  // dead or trap from the start state
@@ -2981,118 +2947,35 @@ __global__ void __launch_bounds__(512) batch_refill(BatchArgs a) {
           uint32_t v[4];
           window16q(wp, v);
           const uint32_t nb = left >= 16 ? 16u : (uint32_t)left;
-          uint32_t lj = ~0u;
           if (nb == 16) {
 #pragma unroll
             for (int g = 0; g < 4; g++) {
-              e = hot_next<0>(fbase, v[g], e); if (MODE == 0) mx = max(mx, e); else if (e >= fthr) lj = 4 * g + 0;
-              e = hot_next<1>(fbase, v[g], e); if (MODE == 0) mx = max(mx, e); else if (e >= fthr) lj = 4 * g + 1;
-              e = hot_next<2>(fbase, v[g], e); if (MODE == 0) mx = max(mx, e); else if (e >= fthr) lj = 4 * g + 2;
-              e = hot_next<3>(fbase, v[g], e); if (MODE == 0) mx = max(mx, e); else if (e >= fthr) lj = 4 * g + 3;
+              e = hot_next<0>(fbase, v[g], e); mx = max(mx, e);
+              e = hot_next<1>(fbase, v[g], e); mx = max(mx, e);
+              e = hot_next<2>(fbase, v[g], e); mx = max(mx, e);
+              e = hot_next<3>(fbase, v[g], e); mx = max(mx, e);
             }
           } else {
 #pragma unroll
             for (int i = 0; i < 15; i++)
               if ((uint32_t)i < nb) {
                 e = hot_next_b(fbase, window_byte(v, i), e);
-                if (MODE == 0) mx = max(mx, e); else if (e >= fthr) lj = i;
+                mx = max(mx, e);
               }
           }
-          if (MODE == 1 && lj != ~0u && e != 1u) last = q + lj;
           q += nb;
         } else {  // the last bytes of the whole buffer: byte loads
-          for (uint64_t i = 0; i < left && e >= flive && (MODE == 1 || mx < fthr); i++) {
+          for (uint64_t i = 0; i < left && e >= flive && mx < fthr; i++) {
             e = hot_next_b(fbase, p[q + i], e);
-            if (MODE == 0) mx = max(mx, e); else if (e >= fthr) last = q + i;
+            mx = max(mx, e);
           }
           q += left;
         }
-        if (e < flive || (MODE == 0 && mx >= fthr)) done = true;
+        if (e < flive || mx >= fthr) done = true;
       }
       if (done) {
-        if (e == 1u && !(MODE == 0 && mx >= fthr)) {
-          finish_slow();
-        } else if (MODE == 0) {
-          finish(mx >= fthr, 0, 0);
-        } else if (last == kNone) {
-          finish(false, 0, 0);
-        } else if (last == 0) {
-          finish(true, 0, 0);
-        } else {  // the reverse loop finds the start
-          a.out_spans[2 * r + 1] = last;
-          atomicOr(&todo[(uint32_t)(r - r_lo) >> 5], 1u << ((uint32_t)(r - r_lo) & 31u));
-          idle = true;
-        }
-      }
-    }
-    if (MODE == 1) {
-      // ---- reverse loop over the records marked in `todo` ----
-      __syncwarp();
-      uint32_t w = 0, m = todo[0];  // warp-uniform cursor: word index and its bits not handed out yet
-      uint64_t start = kNone;
-      idle = true;
-      for (;;) {
-        while (m == 0 && w + 1 < task_recs / 32) m = todo[++w];
-        const uint32_t idle_m = __ballot_sync(0xffffffffu, idle);
-        if (idle_m == 0xffffffffu && m == 0) break;
-        if (m != 0 && ((uint32_t)__popc(idle_m) >= kBatchRefill || idle_m == 0xffffffffu)) {
-          const uint32_t rank = (uint32_t)__popc(idle_m & ((1u << lane) - 1u));
-          const uint32_t take = min((uint32_t)__popc(idle_m), (uint32_t)__popc(m));
-          if (idle && rank < take) {
-            const uint32_t bit = __fns(m, 0, rank + 1);
-            r = r_lo + w * 32u + bit;
-            const uint64_t lo = a.offsets[r];
-            len = a.offsets[r + 1] - lo;
-            p = a.text + lo;
-            last = a.out_spans[2 * r + 1];
-            q = last;
-            start = kNone;
-            idle = false;
-            const uint32_t sf = a.rev.uniform_start ? a.rev.start[32] : a.rev.start[flags_reverse(p, len, last)];
-            const uint32_t hr = a.rev_hot.full2hot[sf];
-            if (sf == 0) finish(false, 0, 0);
-            else if (hr == 0xFFFFu) finish_slow();
-            else e = hr;
-          }
-          const uint32_t cut = take == (uint32_t)__popc(m) ? 32u : __fns(m, 0, take + 1);  // position of the first bit left
-          m = cut >= 32u ? 0u : m & ~((1u << cut) - 1u);
-        }
-        if (idle) continue;
-        // one window, bytes [q-16, q): only the last min(16, q) belong to the record
-        bool rdone = false;
-        const uint8_t* wp = p + q - 16;
-        const uint8_t* al = reinterpret_cast<const uint8_t*>(reinterpret_cast<uintptr_t>(wp) & ~(uintptr_t)15);
-        const uint32_t nb = q >= 16 ? 16u : (uint32_t)q;
-        if (al >= a.text && al + 32 <= buf_hi) {
-          uint32_t v[4];
-          window16q(wp, v);
-          uint32_t lj = ~0u;
-#pragma unroll
-          for (int i = 15; i >= 0; i--) {
-            if ((uint32_t)(15 - i) < nb && !rdone) {
-              e = hot_next_b(rbase, window_byte(v, i), e);
-              if (e >= rthr) lj = i;
-              if (e < rlive) rdone = true;
-            }
-          }
-          if (lj != ~0u) start = q - 16 + lj + 1;
-          q -= nb;
-        } else {
-          for (uint32_t i = 0; i < nb && !rdone; i++) {
-            q--;
-            e = hot_next_b(rbase, p[q], e);
-            if (e >= rthr) start = q + 1;
-            if (e < rlive) rdone = true;
-          }
-        }
-        if (rdone || q == 0) {
-          if (e == 1u) {
-            finish_slow();
-          } else {
-            if (!rdone && a.rev_hot.eof[e] >= a.rev.match_lo) start = 0;
-            finish(start != kNone, start, last);
-          }
-        }
+        if (e == 1u && !(mx >= fthr)) finish(slow_is_match_record(a.fwd_g, p, len));  // left the hot set: again on the full tables
+        else finish(mx >= fthr);
       }
     }
     __syncwarp();
@@ -3101,8 +2984,6 @@ __global__ void __launch_bounds__(512) batch_refill(BatchArgs a) {
     __syncwarp();
   }
 }
-template __global__ void batch_refill<0>(BatchArgs);
-template __global__ void batch_refill<1>(BatchArgs);
 
 // dfa.rs:525-570 per record: OR of the per-state pattern masks of automaton d along the scan of record r.
 __device__ __forceinline__ void set_record_masks(const Table& T, const DfaView& d, const uint8_t* text, const uint64_t* offsets,
@@ -3260,15 +3141,10 @@ __global__ void cand_shortest(DfaView fwd, int use_smem, CandArgs c, const uint8
     for (uint64_t s = s_lo; s < s_hi && s < b; s++) {
       if ((s & 255) == 0) b = min(b, (uint64_t)*(volatile unsigned long long*)best);
       if (!cand_at(cm, c.depth, text, n, s)) continue;
-      uint32_t st = pick_start_fwd(fwd, text, n, s);
-      for (uint64_t q = s; st != 0 && q < b; q++) {
-        st = q < n ? T.step(st, __ldg(text + q)) : T.step_eof(st);
-        if (st >= fwd.match_lo) {
-          b = q;
-          atomicMin(best, (unsigned long long)q);
-          break;
-        }
-        if (q >= n) break;
+      const uint64_t e = earliest_end(fwd, T, text, n, s, b);
+      if (e != kNone) {
+        b = e;
+        atomicMin(best, (unsigned long long)e);
       }
     }
   }
@@ -3295,15 +3171,8 @@ __global__ void batch_cand(BatchArgs a, CandArgs c) {
         return cand_at(cm, c.depth, p, len, s) && !(c.utf8_boundaries && s < len && (p[s] & 0xC0u) == 0x80u);
       };
       if (MODE == 0) {
-        for (uint64_t s = 0; s <= len && !hit; s++) {
-          if (!is_cand(s)) continue;
-          uint32_t st = pick_start_fwd(a.fwd, p, len, s);
-          for (uint64_t q = s; st != 0; q++) {
-            st = q < len ? T.step(st, p[q]) : T.step_eof(st);
-            if (st >= a.fwd.match_lo) { hit = true; break; }
-            if (q >= len) break;
-          }
-        }
+        for (uint64_t s = 0; s <= len && !hit; s++)
+          hit = is_cand(s) && earliest_end(a.fwd, T, p, len, s) != kNone;
       } else {
         uint64_t s_star = 0;
         auto fwd = [&](uint64_t q) -> uint64_t {  // end of the match at the first candidate >= q that starts one

@@ -17,8 +17,10 @@
 //   compact_spans     chunk, validated against the left neighbour, ordered compaction
 //   batch_fast,       one thread per record: is_match / find / set matches, the
 //   *_batch           reference algorithm verbatim per record (exec.rs:632-662)
+//   batch_refill      batched is_match with a warp's lanes refilled from a task of records
 //   batch_iter*       one thread per record: find_iter (re_trait.rs:197-220) per record,
 //                     count pass + prefix sum + write pass (CSR output)
+//   batch_cand        batched records from candidate starts (over-budget patterns)
 #pragma once
 #include <cstdint>
 #include <cuda_runtime.h>
@@ -132,5 +134,7 @@ __device__ __forceinline__ Table stage_table(const DfaView& d, unsigned char* sm
   }
   return t;
 }
+// The table and class map where the view keeps them (global memory).
+__device__ __forceinline__ Table global_table(const DfaView& d) { return Table{d.trans, d.classes, d.stride}; }
 
 }  // namespace rbgpu

@@ -230,7 +230,7 @@ __global__ void batch_iter(BatchArgs a);
 // MODE 0 is_match, 1 find, 2 find_iter count pass, 3 find_iter write pass
 template <int MODE>
 __global__ void batch_cand(BatchArgs a, CandArgs c);
-template <int MODE>
+// batched is_match, the lanes of a warp refilled from a task of task_recs records
 __global__ void batch_refill(BatchArgs a);
 __global__ void scan_rev_bitmap(ScanArgs a);
 template <int FUSED>

@@ -297,7 +297,7 @@ def test_batched_lines_match_scalar_api():
     for pat in [r"(\d{4})-(\d{2})-(\d{2})", r"(?-u)(\d{4})-(\d{2})-(\d{2})", r"^\d+ host", r"svc\[\d+\]:$", r"(?i)holmes", r"\n$",
                 r"\w+\s\w+$", r"(?-u:\b)\d{2}(?-u:\b)", r"^$", r"[a-z]+ing"]:
         o = O.OracleRegex(pat)
-        # batch_fast (one record per lane per round), batch_refill for is_match (the default) and for find, generic
+        # batch_fast (one record per lane per round), batch_refill for is_match (1 the default, 2 whatever the batch size), generic
         for generic, refill in ((False, 1), (False, 0), (False, 2), (True, 1)):
             r = R.BytesRegex(pat)
             r.force_generic(generic)

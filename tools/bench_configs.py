@@ -89,7 +89,7 @@ def c3(dev, n_lines, check_lines=20000):
     res = {}
     for pat in (r"(\d{4})-(\d{2})-(\d{2})", r"(?-u)(\d{4})-(\d{2})-(\d{2})"):
         r = use_torch_stream(R.BytesRegex(pat))
-        if os.environ.get("RB_BATCH_REFILL"):  # experiments: 0 batch_fast, 1 refill for is_match, 2 also for find
+        if os.environ.get("RB_BATCH_REFILL"):  # experiments: 0 batch_fast, 1 refill for is_match on large batches, 2 on any
             r.set_option("batch_refill", int(os.environ["RB_BATCH_REFILL"]))
         bits = torch.zeros((n_lines + 31) // 32, dtype=torch.int32, device=dev)
         spans = torch.empty((n_lines, 2), dtype=torch.int64, device=dev)
