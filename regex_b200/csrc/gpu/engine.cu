@@ -26,7 +26,17 @@ static EncodeTiledFn encode_tiled() {
   }();
   return fn;
 }
-
+// 2-D view of `rows` consecutive segments of `seg` bytes from `base` for the fast scan kernels' tiled TMA loads
+// (rows = segments, cols = bytes); one box = the 64-byte group of all 32 lanes' segments.
+static bool encode_segments(CUtensorMap* tmap, const uint8_t* base, uint32_t seg, uint64_t rows) {
+  if (!encode_tiled()) return false;
+  cuuint64_t dims[2] = {seg, rows};
+  cuuint64_t strides[1] = {seg};
+  cuuint32_t box[2] = {64, 32};
+  cuuint32_t estr[2] = {1, 1};
+  return encode_tiled()(tmap, CU_TENSOR_MAP_DATA_TYPE_UINT8, 2, (void*)base, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                        CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
+}
 
 static std::atomic<uint64_t> g_launches{0};
 uint64_t kernel_launches() { return g_launches.load(); }
@@ -592,20 +602,11 @@ int Regex::cand_batch(int mode, const uint8_t* d_text, const uint64_t* d_offsets
   a.match_offsets = d_match_offsets;
   a.cap = cap;
   cudaStream_t st = (cudaStream_t)stream_;
-  const uint32_t grid = grid_for(n_rec, 256, tuning.blocks_per_sm);
-#define RB_CAND(M)                                              \
-  {                                                             \
-    RB_CUDA(allow_smem(batch_cand<M>, smem));                   \
-    batch_cand<M><<<grid, 256, smem, st>>>(a, c);               \
-    RB_LAUNCH_CHECK("batch_cand<" #M ">");                      \
-  }
-  switch (mode) {
-    case 0: RB_CAND(0) break;
-    case 1: RB_CAND(1) break;
-    case 2: RB_CAND(2) break;
-    default: RB_CAND(3) break;
-  }
-#undef RB_CAND
+  static void (*const kBatchCand[4])(BatchArgs, CandArgs) = {batch_cand<0>, batch_cand<1>, batch_cand<2>, batch_cand<3>};
+  const auto kernel = kBatchCand[mode];
+  RB_CUDA(allow_smem(kernel, smem));
+  kernel<<<grid_for(n_rec, 256, tuning.blocks_per_sm), 256, smem, st>>>(a, c);
+  RB_LAUNCH_CHECK("batch_cand");
   if (mode <= 1) RB_CUDA(cudaStreamSynchronize(st));
   return 0;
 }
@@ -620,7 +621,6 @@ int Regex::resolve_long_run(const uint8_t* d_text, uint64_t n, uint64_t s, bool 
   DeviceDfa* fwd;
   if (int rc = ensure(kFwdAnchoredLF, &fwd)) return rc;
   cudaStream_t st = (cudaStream_t)stream_;
-  const uint32_t k_max = fwd->view.n_states;
   const uint32_t seg = 4096;
   ScanArgs g{};
   g.dfa = fwd->view;
@@ -631,9 +631,6 @@ int Regex::resolve_long_run(const uint8_t* d_text, uint64_t n, uint64_t s, bool 
   g.base = s;
   g.seg = seg;
   uint32_t* counters = (uint32_t*)counters_.ptr;
-  uint16_t* d_states = (uint16_t*)kstates_.ensure(k_max * 2);
-  uint16_t* d_kidx = (uint16_t*)kidx_.ensure(65536 * 2);
-  if (!d_states || !d_kidx) return fail("out of device memory (long run)");
   // the start state at s: the look-behind flags come from the bytes next to s (pick_start_fwd)
   uint16_t start_state = fwd->view.start[32];
   if (!fwd->view.uniform_start) {
@@ -652,9 +649,8 @@ int Regex::resolve_long_run(const uint8_t* d_text, uint64_t n, uint64_t s, bool 
     if (last) f |= 64;
     start_state = fwd->view.start[f];
   }
-  // K: the states the run is in at segment boundaries, closed under the per-segment maps, found as in
-  // solve_entries: start from the run's start state, run the segments from the states known so far, add
-  // the states their maps lead to, repeat (`(?s)foo.*bar`: 6 of 25 states)
+  // K: the states the run is in at segment boundaries, found as in solve_entries from the run's start state
+  // (`(?s)foo.*bar`: 6 of 25 states); it only grows from one window to the next
   uint8_t* present = (uint8_t*)present_.ensure(65536);
   uint16_t* d_first = (uint16_t*)(counters + 11);
   if (!present) return fail("out of device memory (long run)");
@@ -665,53 +661,17 @@ int Regex::resolve_long_run(const uint8_t* d_text, uint64_t n, uint64_t s, bool 
     RB_CUDA(cudaMemcpyAsync(d_first, &start_state, 2, cudaMemcpyHostToDevice, st));
     RB_CUDA(cudaStreamSynchronize(st));
   }
-  std::vector<uint8_t> h_present(65536);
-  std::vector<uint16_t> K, kidx;
-  RB_CUDA(allow_smem(scan_map, smem));
   RB_CUDA(allow_smem(scan_last_match, smem));
   // growing windows from s: a long match is rarely the whole rest of the haystack
   for (uint64_t window = 8ull << 20;; window *= 8) {
     const uint64_t end = window >= n - s ? n : s + window;
-    const uint64_t n_seg = std::max<uint64_t>(1, (end - s + seg - 1) / seg);
-    const uint64_t n_blocks = (n_seg + kMapBlock - 1) / kMapBlock;
     g.limit = end;
-    g.n_seg = n_seg;
-    uint32_t k = 0;
-    uint16_t* maps = nullptr;
-    for (;;) {
-      RB_CUDA(d2h(h_present.data(), present, 65536));
-      K.clear();
-      kidx.assign(65536, 0xFFFF);
-      for (uint32_t v = 0; v < k_max; v++)
-        if (h_present[v]) { kidx[v] = (uint16_t)K.size(); K.push_back((uint16_t)v); }
-      k = (uint32_t)K.size();
-      maps = (uint16_t*)maps_.ensure(n_seg * k * 2);
-      if (!maps) return fail("out of device memory (long run)");
-      RB_CUDA(cudaMemcpyAsync(d_states, K.data(), k * 2, cudaMemcpyHostToDevice, st));
-      RB_CUDA(cudaMemcpyAsync(d_kidx, kidx.data(), 65536 * 2, cudaMemcpyHostToDevice, st));
-      scan_map<<<grid_for(n_seg * k, 256, tuning.blocks_per_sm), 256, smem, st>>>(g, 0, d_states, k, maps);
-      RB_LAUNCH_CHECK("scan_map");
-      stats.map_passes += k;
-      RB_CUDA(cudaMemsetAsync(counters + 8, 0, 4, st));
-      closure_check<<<grid_for(n_seg * k, 256, 8), 256, 0, st>>>(maps, n_seg * k, d_kidx, present, counters + 8);
-      RB_LAUNCH_CHECK("closure_check");
-      uint32_t n_new = 0;
-      RB_CUDA(d2h(&n_new, counters + 8, 4));
-      if (n_new == 0) break;
-    }
-    uint16_t* comp = (uint16_t*)comp_.ensure(n_blocks * k * 2);
-    uint16_t* bentry = (uint16_t*)bentry_.ensure(n_blocks * 2);
-    uint16_t* exact = (uint16_t*)exact_.ensure(n_seg * 2);
-    if (!comp || !bentry || !exact) return fail("out of device memory (long run)");
-    compose_blocks<<<(uint32_t)((n_blocks * k + 255) / 256), 256, 0, st>>>(maps, d_kidx, d_states, k, n_seg, 0, comp);
-    RB_LAUNCH_CHECK("compose_blocks");
-    compose_top<<<1, 32, 0, st>>>(comp, d_kidx, k, n_blocks, 0, d_first, bentry);
-    RB_LAUNCH_CHECK("compose_top");
-    compose_fill<<<(uint32_t)((n_blocks + 255) / 256), 256, 0, st>>>(maps, d_kidx, k, n_seg, 0, bentry, exact);
-    RB_LAUNCH_CHECK("compose_fill");
+    g.n_seg = std::max<uint64_t>(1, (end - s + seg - 1) / seg);
+    if (int rc = compose_entries(g, false, d_first)) return rc;
+    const uint16_t* exact = (const uint16_t*)exact_.ptr;
     unsigned long long* best = (unsigned long long*)(counters + 8);
     RB_CUDA(cudaMemsetAsync(best, 0, 12, st));  // best, then the alive flag at counters[10]
-    scan_last_match<<<grid_for(n_seg, 256, tuning.blocks_per_sm), 256, smem, st>>>(g, exact, best, counters + 10);
+    scan_last_match<<<grid_for(g.n_seg, 256, tuning.blocks_per_sm), 256, smem, st>>>(g, exact, best, counters + 10);
     RB_LAUNCH_CHECK("scan_last_match");
     uint32_t h[4] = {0, 0, 0, 0};
     RB_CUDA(d2h(h, best, 12));
@@ -734,27 +694,64 @@ int Regex::resolve_long_run(const uint8_t* d_text, uint64_t n, uint64_t s, bool 
 }
 
 // ------------------------------------------------- bounded fix-up of entry states --
+int Regex::settle_segments(const ScanArgs& a, bool reverse, const std::function<int(uint32_t)>& redo) {
+  cudaStream_t st = (cudaStream_t)stream_;
+  uint32_t* counters = (uint32_t*)counters_.ptr;
+  for (uint32_t round = 0;; round++) {
+    RB_CUDA(cudaMemsetAsync(counters, 0, 4, st));
+    verify_segments<<<grid_for(a.n_seg, 256, 8), 256, 0, st>>>(a.guess, a.fin, a.n_seg, reverse ? 1 : 0, (uint32_t*)redo_.ptr, counters);
+    RB_LAUNCH_CHECK("verify_segments");
+    RB_CUDA(cudaMemcpyAsync(pinned_, counters, 4, cudaMemcpyDeviceToHost, st));
+    RB_CUDA(cudaStreamSynchronize(st));
+    const uint32_t n_redo = *(uint32_t*)pinned_;
+    if (n_redo == 0) return 0;
+    if (round == tuning.max_redo_rounds) {
+      // wrong guesses keep cascading: solve every entry state at once, then one more redo round
+      if (int rc = solve_entries(a, reverse)) return rc;
+      continue;
+    }
+    stats.scan_redo_rounds++;
+    stats.scan_redo_segments += n_redo;
+    if (int rc = redo(n_redo)) return rc;
+  }
+}
+
 // Exact entry state of every segment by state-map composition (kernels.cu, "exact entry states"):
-// K = the states seen at segment boundaries, closed under the per-segment maps; on return
-// fin[] holds, next to every segment, the exact state it is entered with, so that one
-// verify + redo round completes the scan.  Used when the plain redo rounds do not converge.
-int Regex::solve_entries(const void* scan_args, bool reverse) {
-  ScanArgs g = *(const ScanArgs*)scan_args;
+// K = the states seen at segment boundaries (guesses and exits); on return fin[] holds, next to
+// every segment, the exact state it is entered with, so that one verify + redo round completes
+// the scan.  Used when the plain redo rounds do not converge.
+int Regex::solve_entries(const ScanArgs& g, bool reverse) {
+  cudaStream_t st = (cudaStream_t)stream_;
+  const uint64_t n_seg = g.n_seg;
+  uint8_t* present = (uint8_t*)present_.ensure(65536);
+  if (!present) return fail("out of device memory (state maps)");
+  RB_CUDA(cudaMemsetAsync(present, 0, 65536, st));
+  mark_states<<<grid_for(n_seg, 256, 8), 256, 0, st>>>(g.guess, n_seg, present);
+  RB_LAUNCH_CHECK("mark_states");
+  mark_states<<<grid_for(n_seg, 256, 8), 256, 0, st>>>(g.fin, n_seg, present);
+  RB_LAUNCH_CHECK("mark_states");
+  if (int rc = compose_entries(g, reverse, reverse ? g.guess + (n_seg - 1) : g.guess)) return rc;
+  publish_exact<<<grid_for(n_seg, 256, 8), 256, 0, st>>>((const uint16_t*)exact_.ptr, n_seg, reverse ? 1 : 0, g.fin);
+  RB_LAUNCH_CHECK("publish_exact");
+  return 0;
+}
+
+// Run every segment from every state of K (scan_map), add the states the maps lead to, repeat until K is closed;
+// then compose the maps along the scan direction: per block of kMapBlock segments, over the blocks from the first
+// entry state, and back into every segment.  (|K| + 2) passes over the segments.
+int Regex::compose_entries(const ScanArgs& scan_args, bool reverse, const uint16_t* d_entry) {
+  ScanArgs g = scan_args;
   cudaStream_t st = (cudaStream_t)stream_;
   const size_t smem = smem_for(g.dfa);
   g.use_smem = smem != 0;
   g.redo_list = nullptr;
   RB_CUDA(allow_smem(scan_map, smem));
   const uint64_t n_seg = g.n_seg;
-  uint8_t* present = (uint8_t*)present_.ensure(65536);
+  const int dir = reverse ? 1 : 0;
+  uint8_t* present = (uint8_t*)present_.ptr;
   uint16_t* d_kidx = (uint16_t*)kidx_.ensure(65536 * 2);
   uint32_t* counters = (uint32_t*)counters_.ptr;
-  if (!present || !d_kidx) return fail("out of device memory (state maps)");
-  RB_CUDA(cudaMemsetAsync(present, 0, 65536, st));
-  mark_states<<<grid_for(n_seg, 256, 8), 256, 0, st>>>(g.guess, n_seg, present);
-  RB_LAUNCH_CHECK("mark_states");
-  mark_states<<<grid_for(n_seg, 256, 8), 256, 0, st>>>(g.fin, n_seg, present);
-  RB_LAUNCH_CHECK("mark_states");
+  if (!d_kidx) return fail("out of device memory (state maps)");
   std::vector<uint8_t> h_present(65536);
   std::vector<uint16_t> K, kidx;
   uint16_t *d_states = nullptr, *maps = nullptr;
@@ -762,8 +759,8 @@ int Regex::solve_entries(const void* scan_args, bool reverse) {
     RB_CUDA(d2h(h_present.data(), present, 65536));
     K.clear();
     kidx.assign(65536, 0xFFFF);
-    for (uint32_t v = 0; v < 65536; v++)
-      if (h_present[v] && v < g.dfa.n_states) { kidx[v] = (uint16_t)K.size(); K.push_back((uint16_t)v); }
+    for (uint32_t v = 0; v < g.dfa.n_states; v++)
+      if (h_present[v]) { kidx[v] = (uint16_t)K.size(); K.push_back((uint16_t)v); }
     const uint32_t k = (uint32_t)K.size();
     if (k > 512) return fail("the automaton reaches more than 512 distinct states at segment boundaries; state-map composition refused");
     d_states = (uint16_t*)kstates_.ensure(k * 2);
@@ -771,7 +768,7 @@ int Regex::solve_entries(const void* scan_args, bool reverse) {
     if (!d_states || !maps) return fail("out of device memory (state maps)");
     RB_CUDA(cudaMemcpyAsync(d_states, K.data(), k * 2, cudaMemcpyHostToDevice, st));
     RB_CUDA(cudaMemcpyAsync(d_kidx, kidx.data(), 65536 * 2, cudaMemcpyHostToDevice, st));
-    scan_map<<<grid_for(n_seg * k, 256, tuning.blocks_per_sm), 256, smem, st>>>(g, reverse ? 1 : 0, d_states, k, maps);
+    scan_map<<<grid_for(n_seg * k, 256, tuning.blocks_per_sm), 256, smem, st>>>(g, dir, d_states, k, maps);
     RB_LAUNCH_CHECK("scan_map");
     stats.map_passes += k;
     RB_CUDA(cudaMemsetAsync(counters + 8, 0, 4, st));
@@ -787,14 +784,12 @@ int Regex::solve_entries(const void* scan_args, bool reverse) {
   uint16_t* bentry = (uint16_t*)bentry_.ensure(n_blocks * 2);
   uint16_t* exact = (uint16_t*)exact_.ensure(n_seg * 2);
   if (!comp || !bentry || !exact) return fail("out of device memory (state maps)");
-  compose_blocks<<<(uint32_t)((n_blocks * k + 255) / 256), 256, 0, st>>>(maps, d_kidx, d_states, k, n_seg, reverse ? 1 : 0, comp);
+  compose_blocks<<<(uint32_t)((n_blocks * k + 255) / 256), 256, 0, st>>>(maps, d_kidx, d_states, k, n_seg, dir, comp);
   RB_LAUNCH_CHECK("compose_blocks");
-  compose_top<<<1, 32, 0, st>>>(comp, d_kidx, k, n_blocks, reverse ? 1 : 0, reverse ? g.guess + (n_seg - 1) : g.guess, bentry);
+  compose_top<<<1, 32, 0, st>>>(comp, d_kidx, k, n_blocks, dir, d_entry, bentry);
   RB_LAUNCH_CHECK("compose_top");
-  compose_fill<<<(uint32_t)((n_blocks + 255) / 256), 256, 0, st>>>(maps, d_kidx, k, n_seg, reverse ? 1 : 0, bentry, exact);
+  compose_fill<<<(uint32_t)((n_blocks + 255) / 256), 256, 0, st>>>(maps, d_kidx, k, n_seg, dir, bentry, exact);
   RB_LAUNCH_CHECK("compose_fill");
-  publish_exact<<<grid_for(n_seg, 256, 8), 256, 0, st>>>(exact, n_seg, reverse ? 1 : 0, g.fin);
-  RB_LAUNCH_CHECK("publish_exact");
   return 0;
 }
 
@@ -849,6 +844,9 @@ int Regex::scan_starts(const uint8_t* d_text, uint64_t n, uint64_t base, uint64_
   uint32_t block;
   const WalkArgs* fw = (const WalkArgs*)fused_walk;
   WalkArgs no_walk{};
+  // scan_rev_fast<FUSED>: 0 no walk, 1 the fused walk with the table runner, 2 with the fixed-length runner
+  static void (*const kScanRevFast[3])(ScanArgs, WalkArgs, CUtensorMap) = {scan_rev_fast<0>, scan_rev_fast<1>, scan_rev_fast<2>};
+  const auto rev_fast = kScanRevFast[!fw ? 0 : fw->fixed_len ? 2 : 1];
   if (fast) {
     block = 1024;
     const bool fw_fixed = fw && fw->fixed_len != 0;
@@ -858,35 +856,20 @@ int Regex::scan_starts(const uint8_t* d_text, uint64_t n, uint64_t base, uint64_
       a.tbase_off = after_rings + (uint32_t)hot_bytes(rev->hot.n - rev->hot.match_lo);
       a.fbase_off = after_rings + (uint32_t)hot_bytes_signed(rev->hot);
     }
-    if (fw_fixed) RB_CUDA(allow_smem(scan_rev_fast<2>, smem));
-    else if (fw) RB_CUDA(allow_smem(scan_rev_fast<1>, smem));
-    else RB_CUDA(allow_smem(scan_rev_fast<0>, smem));
+    RB_CUDA(allow_smem(rev_fast, smem));
   } else {
     smem = smem_for(rev->view);
     a.use_smem = smem != 0;
     block = tuning.block;
     RB_CUDA(allow_smem(scan_rev_bitmap, smem));
   }
-  // 2-D view of the haystack for the tiled TMA loads: rows = full segments, cols = bytes
-  CUtensorMap tmap;
-  std::memset(&tmap, 0, sizeof tmap);
-  if (fast && tuning.tensor_tma && encode_tiled() && seg >= 64 && seg % 16 == 0 && a.warm <= seg) {
+  CUtensorMap tmap{};
+  if (fast && tuning.tensor_tma && seg >= 64 && seg % 16 == 0 && a.warm <= seg) {
     const uint64_t rows = (n - base) / seg;  // only rows that lie entirely inside the buffer
-    if (rows >= 34) {
-      cuuint64_t dims[2] = {seg, rows};
-      cuuint64_t strides[1] = {seg};
-      cuuint32_t box[2] = {64, 32};  // one box = the 64-byte group of all 32 lanes' segments
-      cuuint32_t estr[2] = {1, 1};
-      CUresult r = encode_tiled()(&tmap, CU_TENSOR_MAP_DATA_TYPE_UINT8, 2, (void*)(d_text + base), dims, strides, box, estr,
-                                  CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                                  CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-      if (r == CUDA_SUCCESS) a.tmap_rows = rows;
-    }
+    if (rows >= 34 && encode_segments(&tmap, d_text + base, seg, rows)) a.tmap_rows = rows;
   }
   auto launch = [&](const ScanArgs& args, uint64_t work) {
-    if (fast && fw && fw->fixed_len) scan_rev_fast<2><<<grid_for(work, block, 1), block, smem, st>>>(args, *fw, tmap);
-    else if (fast && fw) scan_rev_fast<1><<<grid_for(work, block, 1), block, smem, st>>>(args, *fw, tmap);
-    else if (fast) scan_rev_fast<0><<<grid_for(work, block, 1), block, smem, st>>>(args, no_walk, tmap);
+    if (fast) rev_fast<<<grid_for(work, block, 1), block, smem, st>>>(args, fw ? *fw : no_walk, tmap);
     else scan_rev_bitmap<<<grid_for(work, block, tuning.blocks_per_sm), block, smem, st>>>(args);
   };
   const bool reuse = io && io->reuse_scan;
@@ -895,12 +878,10 @@ int Regex::scan_starts(const uint8_t* d_text, uint64_t n, uint64_t base, uint64_
     RB_LAUNCH_CHECK("scan_rev");
   }
   stats.scan_redo_rounds = stats.scan_redo_segments = stats.map_passes = 0;
-  auto redo_round = [&](uint32_t n_redo) -> int {
-    stats.scan_redo_rounds++;
-    stats.scan_redo_segments += n_redo;
-    ScanArgs r = a;
-    r.redo_list = redo;
-    r.n_redo = counters;
+  ScanArgs r = a;  // a redo round: only the listed segments, each entered with its neighbour's exit
+  r.redo_list = redo;
+  r.n_redo = counters;
+  auto redo_launch = [&](uint32_t n_redo) -> int {
     launch(r, n_redo);
     RB_LAUNCH_CHECK("scan_rev(redo)");
     return 0;
@@ -920,25 +901,13 @@ int Regex::scan_starts(const uint8_t* d_text, uint64_t n, uint64_t base, uint64_
       RB_CUDA(cudaMemcpyAsync(a.fin + n_seg, h16 + 1, 2, cudaMemcpyHostToDevice, st));
       RB_CUDA(cudaMemcpyAsync(redo, h32, 4, cudaMemcpyHostToDevice, st));
       RB_CUDA(cudaMemcpyAsync(counters, h32 + 1, 4, cudaMemcpyHostToDevice, st));
-      if (int rc = redo_round(1)) return rc;
+      stats.scan_redo_rounds++;
+      stats.scan_redo_segments++;
+      if (int rc = redo_launch(1)) return rc;
       io->rev_guess = io->rev_entry;
     }
   }
-  for (uint32_t round = 0;; round++) {
-    RB_CUDA(cudaMemsetAsync(counters, 0, 4, st));
-    verify_segments<<<grid_for(n_seg, 256, 8), 256, 0, st>>>(a.guess, a.fin, n_seg, 1, redo, counters);
-    RB_LAUNCH_CHECK("verify_segments");
-    RB_CUDA(cudaMemcpyAsync(pinned_, counters, 4, cudaMemcpyDeviceToHost, st));
-    RB_CUDA(cudaStreamSynchronize(st));
-    const uint32_t n_redo = *(uint32_t*)pinned_;
-    if (n_redo == 0) break;
-    if (round == tuning.max_redo_rounds) {
-      // wrong guesses keep cascading: solve every entry state at once, then one more redo round
-      if (int rc = solve_entries(&a, true)) return rc;
-      continue;
-    }
-    if (int rc = redo_round(n_redo)) return rc;
-  }
+  if (int rc = settle_segments(a, true, redo_launch)) return rc;
   if (shard) {
     RB_CUDA(cudaMemcpyAsync(h16, a.fin, 2, cudaMemcpyDeviceToHost, st));
     RB_CUDA(cudaStreamSynchronize(st));
@@ -960,6 +929,16 @@ int Regex::find_all_device(const uint8_t* d_text, uint64_t n, uint64_t start, ui
   *total = io.n_matches;
   return rc;
 }
+
+// Chain-walk kernels by runner kind (find_all_shard_device: 0 generic, 1 byte-indexed shared-memory table, 2 fixed
+// length), and the literal prefilter by [table runner][number of scanned bytes - 1].
+using WalkKernel = void (*)(WalkArgs);
+using PfKernel = void (*)(WalkArgs, PfArgs, int);
+static const WalkKernel kWalkChunks[3] = {walk_chunks<0>, walk_chunks<1>, walk_chunks<2>};
+static const WalkKernel kCompactSpans[3] = {compact_spans<0>, compact_spans<1>, compact_spans<2>};
+static const WalkKernel kWalkSequential[3] = {walk_sequential<0>, walk_sequential<1>, walk_sequential<2>};
+static const PfKernel kLiteralScan[2][4] = {{literal_scan<0, 1>, literal_scan<0, 2>, literal_scan<0, 3>, literal_scan<0, 4>},
+                                            {literal_scan<1, 1>, literal_scan<1, 2>, literal_scan<1, 3>, literal_scan<1, 4>}};
 
 int Regex::find_all_shard_device(const uint8_t* d_text, uint64_t n, ShardIO* io, uint64_t* d_out, uint64_t cap) {
   std::lock_guard<std::recursive_mutex> lock(mu_);
@@ -1024,9 +1003,8 @@ int Regex::find_all_shard_device(const uint8_t* d_text, uint64_t n, ShardIO* io,
   w.meta = (uint32_t*)meta_.ensure(nc * 4);
   w.stage = (uint64_t*)stage_.ensure(nc * (uint64_t)w.stage_cap * 16);
   const uint64_t n_blocks = (nc + 1023) / 1024;
-  uint64_t* block_sums = (uint64_t*)block_sums_.ensure(n_blocks * 8);
   uint32_t* counters = (uint32_t*)counters_.ensure(128);
-  if (!w.in_p || !w.in_lm || !w.out_p || !w.out_lm || !w.count || !offset || !dirty_list || !w.first_cand || !w.skip || !w.meta || !w.stage || !block_sums || !counters)
+  if (!w.in_p || !w.in_lm || !w.out_p || !w.out_lm || !w.count || !offset || !dirty_list || !w.first_cand || !w.skip || !w.meta || !w.stage || !counters)
     return fail("out of device memory (walk scratch)");
   w.offset = offset;
   w.out = d_out;
@@ -1057,13 +1035,9 @@ int Regex::find_all_shard_device(const uint8_t* d_text, uint64_t n, ShardIO* io,
   } else if (wfast) {
     wsmem = hot_bytes(fwd->hot.n) + 256;
     w.fwd_hot = fwd->hot;
-    RB_CUDA(allow_smem(walk_chunks<1>, wsmem));
-    RB_CUDA(allow_smem(compact_spans<1>, wsmem));
   } else {
     wsmem = smem_for(fwd->view);
     w.use_smem = wsmem != 0;
-    RB_CUDA(allow_smem(walk_chunks<0>, wsmem));
-    RB_CUDA(allow_smem(compact_spans<0>, wsmem));
   }
   if (use_pf) {  // the prefilter's verifier: table runner (shared-memory hot table) or generic
     w.fixed_len = 0;
@@ -1075,30 +1049,27 @@ int Regex::find_all_shard_device(const uint8_t* d_text, uint64_t n, ShardIO* io,
       w.use_smem = wsmem != 0;
     }
   }
-  auto launch_pf = [&](const WalkArgs& args, uint64_t chunks, int mode) -> cudaError_t {
+  const WalkKernel walk = kWalkChunks[wkind], compact = kCompactSpans[wkind], sequential = kWalkSequential[wkind];
+  const PfKernel pf_scan = use_pf ? kLiteralScan[pf_fast][pf.n_bytes - 1] : nullptr;
+  if (use_pf) {
+    // the kernel also has ~9 KB of static shared memory: opt in whenever the sum could pass 48 KB
+    RB_CUDA(allow_smem(pf_scan, wsmem, 48 * 1024));
+  } else {
+    RB_CUDA(allow_smem(walk, wsmem));
+    RB_CUDA(allow_smem(compact, wsmem));
+    RB_CUDA(allow_smem(sequential, wsmem));
+  }
+  auto launch_pf = [&](const WalkArgs& args, uint64_t chunks, int mode) {
     const uint32_t g = mode == 2 ? 1 : grid_for(chunks * 32, 256, 3);  // one warp per chunk
-#define RB_PF(F, N)                                                                \
-    {                                                                              \
-      /* the kernel also has ~9 KB of static shared memory: opt in whenever the sum could pass 48 KB */ \
-      cudaError_t e__ = allow_smem(literal_scan<F, N>, wsmem, 48 * 1024); \
-      if (e__ != cudaSuccess) return e__;                                          \
-      literal_scan<F, N><<<g, 256, wsmem, st>>>(args, pf, mode);                   \
-      return cudaSuccess;                                                          \
-    }
-    if (pf_fast) switch (pf.n_bytes) { case 1: RB_PF(1, 1) case 2: RB_PF(1, 2) case 3: RB_PF(1, 3) default: RB_PF(1, 4) }
-    switch (pf.n_bytes) { case 1: RB_PF(0, 1) case 2: RB_PF(0, 2) case 3: RB_PF(0, 3) default: RB_PF(0, 4) }
-#undef RB_PF
+    pf_scan<<<g, 256, wsmem, st>>>(args, pf, mode);
   };
   auto launch_walk = [&](const WalkArgs& args, uint64_t work) {
-    if (use_pf) { (void)launch_pf(args, work, 1); return; }
-    const uint32_t g = grid_for(work, 256, 6);
-    if (wkind == 2) walk_chunks<2><<<g, 256, 0, st>>>(args);
-    else if (wkind == 1) walk_chunks<1><<<g, 256, wsmem, st>>>(args);
-    else walk_chunks<0><<<g, 256, wsmem, st>>>(args);
+    if (use_pf) launch_pf(args, work, 1);
+    else walk<<<grid_for(work, 256, 6), 256, wsmem, st>>>(args);
   };
   if (use_pf || cand) {
     if (use_pf) {
-      RB_CUDA(launch_pf(w, nc, 0));
+      launch_pf(w, nc, 0);
       RB_LAUNCH_CHECK("literal_scan");
     } else {
       if (int rc = cand_starts(d_text, n, io->own_lo, io->own_hi, !io->is_last)) return rc;
@@ -1185,10 +1156,8 @@ int Regex::find_all_shard_device(const uint8_t* d_text, uint64_t n, ShardIO* io,
       if (++dirty_rounds > tuning.max_stitch_rounds) {
         // chains that do not meet again: one sequential pass from the leftmost such chunk
         wd.seq_from = hc[3];
-        if (use_pf) (void)launch_pf(wd, 1, 2);
-        else if (wkind == 2) walk_sequential<2><<<1, 256, 0, st>>>(wd);
-        else if (wkind == 1) walk_sequential<1><<<1, 256, wsmem, st>>>(wd);
-        else walk_sequential<0><<<1, 256, wsmem, st>>>(wd);
+        if (use_pf) launch_pf(wd, 1, 2);
+        else sequential<<<1, 256, wsmem, st>>>(wd);
         RB_LAUNCH_CHECK("walk_sequential");
         stats.sequential_passes++;
         dirty_rounds = 0;
@@ -1198,23 +1167,15 @@ int Regex::find_all_shard_device(const uint8_t* d_text, uint64_t n, ShardIO* io,
       }
     }
   }
-  unsigned long long* grand = (unsigned long long*)(counters + 4);
-  scan_counts_local<<<(uint32_t)n_blocks, 1024, 0, st>>>(w.count, offset, block_sums, nc);
-  RB_LAUNCH_CHECK("scan_counts_local");
-  scan_block_sums<<<1, 1024, 0, st>>>(block_sums, n_blocks, grand);
-  RB_LAUNCH_CHECK("scan_block_sums");
-  scan_add_block_offsets<<<(uint32_t)n_blocks, 1024, 0, st>>>(offset, block_sums, nc);
-  RB_LAUNCH_CHECK("scan_add_block_offsets");
+  unsigned long long* grand;
+  if (int rc = prefix_sum(w.count, offset, nc, &grand)) return rc;
   if (w.cap > 0 && use_pf) {
     compact_staged<<<grid_for(nc, 256, 6), 256, 0, st>>>(w);
     RB_LAUNCH_CHECK("compact_staged");
-    RB_CUDA(launch_pf(w, nc, 3));  // chunks with more matches than staging slots: straight into the output
+    launch_pf(w, nc, 3);  // chunks with more matches than staging slots: straight into the output
     RB_LAUNCH_CHECK("literal_scan(overflow)");
   } else if (w.cap > 0) {
-    const uint32_t g = grid_for(nc, 256, 6);
-    if (wkind == 2) compact_spans<2><<<g, 256, 0, st>>>(w);
-    else if (wkind == 1) compact_spans<1><<<g, 256, wsmem, st>>>(w);
-    else compact_spans<0><<<g, 256, wsmem, st>>>(w);
+    compact<<<grid_for(nc, 256, 6), 256, wsmem, st>>>(w);
     RB_LAUNCH_CHECK("compact_spans");
   }
   uint64_t* h = (uint64_t*)pinned_;
@@ -1321,16 +1282,9 @@ int Regex::forward_range(const uint8_t* d_text, uint64_t n, uint64_t start, uint
   }
   if (fast_ok && seg % 64 == 0 && a.warm <= seg && n_full >= 34) {
     const uint64_t skip_lo = 1, skip_hi = 1 + (n_full - 1) / 32 * 32;
-    CUtensorMap tmap;
-    std::memset(&tmap, 0, sizeof tmap);
-    cuuint64_t dims[2] = {seg, skip_hi - skip_lo + 1};  // row 0 = segment skip_lo - 1 (warm-up source of the first warp)
-    cuuint64_t strides[1] = {seg};
-    cuuint32_t box[2] = {64, 32};
-    cuuint32_t estr[2] = {1, 1};
-    CUresult r = encode_tiled()(&tmap, CU_TENSOR_MAP_DATA_TYPE_UINT8, 2, (void*)(d_text + start + (skip_lo - 1) * (uint64_t)seg), dims, strides,
-                                box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                                CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r == CUDA_SUCCESS) {
+    CUtensorMap tmap{};
+    // row 0 = segment skip_lo - 1 (warm-up source of the first warp)
+    if (encode_segments(&tmap, d_text + start + (skip_lo - 1) * (uint64_t)seg, seg, skip_hi - skip_lo + 1)) {
       a.hot = fwd->hot;
       a.skip_lo = skip_lo;
       a.skip_hi = skip_hi;
@@ -1346,13 +1300,7 @@ int Regex::forward_range(const uint8_t* d_text, uint64_t n, uint64_t start, uint
   // step): a handful of 4 KiB segments walked by single threads, ~0.25 ms of pure latency (ncu
   // profiles/r02: 10 % issue, 3 % of the warps).  It runs beside the fast kernel on a second stream.
   if (fast_launched) {
-    if (!copy_stream_) {
-      cudaStream_t s1, s2;
-      RB_CUDA(cudaStreamCreateWithFlags(&s1, cudaStreamNonBlocking));
-      RB_CUDA(cudaStreamCreateWithFlags(&s2, cudaStreamNonBlocking));
-      copy_stream_ = s1;
-      back_stream_ = s2;
-    }
+    if (int rc = side_streams()) return rc;
     cudaStream_t side = (cudaStream_t)back_stream_;
     RB_CUDA(cudaStreamWaitEvent(side, (cudaEvent_t)fork_event_, 0));
     scan_fwd_reduce<<<grid_for(n_seg, tuning.block, tuning.blocks_per_sm), tuning.block, smem, side>>>(a);
@@ -1363,26 +1311,15 @@ int Regex::forward_range(const uint8_t* d_text, uint64_t n, uint64_t start, uint
     scan_fwd_reduce<<<grid_for(n_seg, tuning.block, tuning.blocks_per_sm), tuning.block, smem, st>>>(a);
     RB_LAUNCH_CHECK("scan_fwd_reduce");
   }
-  for (uint32_t round = 0;; round++) {
-    RB_CUDA(cudaMemsetAsync(counters, 0, 4, st));
-    verify_segments<<<grid_for(n_seg, 256, 8), 256, 0, st>>>(a.guess, a.fin, n_seg, 0, redo, counters);
-    RB_LAUNCH_CHECK("verify_segments");
-    RB_CUDA(cudaMemcpyAsync(pinned_, counters, 4, cudaMemcpyDeviceToHost, st));
-    RB_CUDA(cudaStreamSynchronize(st));
-    const uint32_t n_redo = *(uint32_t*)pinned_;
-    if (n_redo == 0) break;
-    stats.scan_redo_rounds++;
-    stats.scan_redo_segments += n_redo;
-    if (round == tuning.max_redo_rounds) {
-      if (int rc = solve_entries(&a, false)) return rc;
-      continue;
-    }
-    ScanArgs r = a;
-    r.redo_list = redo;
-    r.n_redo = counters;
+  ScanArgs r = a;
+  r.redo_list = redo;
+  r.n_redo = counters;
+  auto redo_launch = [&](uint32_t n_redo) -> int {
     scan_fwd_reduce<<<grid_for(n_redo, tuning.block, tuning.blocks_per_sm), tuning.block, smem, st>>>(r);
     RB_LAUNCH_CHECK("scan_fwd_reduce(redo)");
-  }
+    return 0;
+  };
+  if (int rc = settle_segments(a, false, redo_launch)) return rc;
   unsigned long long* result = (unsigned long long*)(counters + 4);
   uint64_t* h = (uint64_t*)pinned_ + 16;
   h[0] = kNone;
@@ -2548,6 +2485,16 @@ const uint8_t* Regex::upload_text(const uint8_t* text, uint64_t n, int* rc) {
   return d;
 }
 
+int Regex::side_streams() {
+  if (copy_stream_) return 0;
+  cudaStream_t s1, s2;
+  RB_CUDA(cudaStreamCreateWithFlags(&s1, cudaStreamNonBlocking));
+  RB_CUDA(cudaStreamCreateWithFlags(&s2, cudaStreamNonBlocking));
+  copy_stream_ = s1;
+  back_stream_ = s2;
+  return 0;
+}
+
 // Bytes per uploaded piece of a pipelined host find_all (RB200_PIPELINE_PIECE overrides; 0 = off).
 // Measured on 4 GiB of pinned host text: 43.8 GB/s upload-then-search, 51.7 GB/s pipelined
 // (the PCIe rate).  tests/test_gpu_parity.py::test_pipelined_host_find_all and
@@ -2572,13 +2519,7 @@ int Regex::find_all_host_pipelined(const uint8_t* text, uint64_t n, uint8_t* d, 
     RB_CUDA(cudaMemcpyAsync(d, text, n, cudaMemcpyHostToDevice, (cudaStream_t)stream_));
     return 1;
   }
-  if (!copy_stream_) {
-    cudaStream_t s1, s2;
-    RB_CUDA(cudaStreamCreateWithFlags(&s1, cudaStreamNonBlocking));
-    RB_CUDA(cudaStreamCreateWithFlags(&s2, cudaStreamNonBlocking));
-    copy_stream_ = s1;
-    back_stream_ = s2;
-  }
+  if (int rc = side_streams()) return rc;
   cudaStream_t up = (cudaStream_t)copy_stream_, back = (cudaStream_t)back_stream_;
   const uint64_t n_pieces = (n + piece - 1) / piece;
   std::vector<cudaEvent_t> arrived(n_pieces, nullptr);

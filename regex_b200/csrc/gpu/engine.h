@@ -5,6 +5,7 @@
 #pragma once
 #include <cstdint>
 #include <algorithm>
+#include <functional>
 #include <map>
 #include <memory>
 #include <mutex>
@@ -17,6 +18,7 @@
 namespace rbgpu {
 
 struct BatchArgs;  // launch.h
+struct ScanArgs;   // launch.h
 
 struct CompileOptions {
   uint32_t flags = 32;               // RURE_FLAG_* bits (rure.h:56-68); default = UNICODE
@@ -220,7 +222,14 @@ class Regex {
   ScanPlan plan_scan(const uint8_t* d_text, uint64_t base, uint64_t limit, bool fast_table);
   int scan_starts(const uint8_t* d_text, uint64_t n, uint64_t base, uint64_t limit, ShardIO* io, const ScanPlan& plan,
                   const void* fused_walk);
-  int solve_entries(const void* scan_args, bool reverse);
+  // Verify every segment's entry guess against its neighbour's exit (a.guess / a.fin, list in redo_) until none is
+  // wrong: redo(n) launches the scan over the n listed segments; after max_redo_rounds rounds solve_entries.
+  int settle_segments(const ScanArgs& a, bool reverse, const std::function<int(uint32_t)>& redo);
+  int solve_entries(const ScanArgs& a, bool reverse);
+  // State-map composition over the segments of g: K = the states below n_states that present_ marks (seeded by the
+  // caller), closed under the per-segment maps; leaves in exact_ the entry state of every segment, the first one
+  // in scan direction entered in the state at d_entry (device).
+  int compose_entries(const ScanArgs& g, bool reverse, const uint16_t* d_entry);
   int resolve_long_run(const uint8_t* d_text, uint64_t n, uint64_t s, bool text_continues, uint64_t* e_out);
   int all_spans_device(const uint8_t* d_text, uint64_t n, uint64_t** d_spans, uint64_t* m);
   int ensure_capture_program();
@@ -275,6 +284,7 @@ class Regex {
   int set_matches_batch_grouped(const uint8_t* d_text, const uint64_t* d_offsets, uint64_t n_rec, uint64_t* d_masks);
   const uint8_t* upload_text(const uint8_t* text, uint64_t n, int* rc);
   int find_all_host_pipelined(const uint8_t* text, uint64_t n, uint8_t* d, uint64_t* d_out, uint64_t* out, uint64_t cap, uint64_t* total);
+  int side_streams();  // creates copy_stream_ and back_stream_ on first use
 
   struct LazyUpload { const uint8_t* src; uint8_t* dst; uint64_t n, done; };  // host haystack uploaded wave by wave
   LazyUpload* lazy_ = nullptr;
@@ -297,7 +307,7 @@ class Regex {
   void* stream_ = nullptr;
   void* own_stream_ = nullptr;
   void* copy_stream_ = nullptr;  // host -> device pieces of a pipelined find_all
-  void* back_stream_ = nullptr;  // device -> host spans
+  void* back_stream_ = nullptr;  // device -> host spans of a pipelined find_all; the generic edge kernel of a forward scan
   void* ext_stream_ = nullptr;
   bool use_ext_stream_ = false;
   // scratch (grow-only)

@@ -3,6 +3,7 @@ automata whose state depends on far context, matches longer than many chunks, ch
 meet again, and the early exits of is_match / shortest_match / RegexSet::matches
 (src/dfa.rs:658-667, 675-682).  Results against the oracle on slices and against closed-form
 expectations at full size; the fix-up counters must stay small."""
+import random
 import re as pyre
 
 import numpy as np
@@ -53,6 +54,41 @@ def test_sticky_automaton_is_solved_by_state_map_composition():
     r2.set_tuning(seg=64, chunk=256)
     assert _spans(r2.find_all(small)) == O.OracleRegex(r"(?s)foo.*bar").find_iter(small)
     assert r2.last_stats()["map_passes"] > 0
+
+
+def test_state_map_composition_in_both_scan_directions():
+    """`(?s)foo.*bar` with 2400 bytes between the `foo` and the `bar`: on 64-byte segments the warm-up guess
+    is wrong for every segment between them, in both scan directions.  With no plain redo round allowed,
+    the entry states are composed from state maps at once: in the reverse start scan (find_all, whole and
+    in two shards) and in the forward scans (shortest_match, RegexSet::matches)."""
+    import torch
+    from test_gpu_parity import _run_gpu_shards
+    filler = xorshift_bytes(5, 2800, b"xyz \n")
+    text = filler[:200] + b"foo" + filler[200:2600] + b"bar" + filler[2600:]
+    d = torch.frombuffer(bytearray(text), dtype=torch.uint8).cuda()
+    pat = r"(?s)foo.*bar"
+    oracle = O.OracleRegex(pat)
+    exp = oracle.find_iter(text)
+    assert len(exp) == 1
+
+    def tuned(re_):
+        re_.set_tuning(seg=64)
+        re_.set_option("max_redo_rounds", 0)
+        return re_
+
+    r = tuned(R.BytesRegex(pat))
+    assert _spans(r.find_all(text)) == exp
+    assert r.last_stats()["map_passes"] > 0
+    assert r.shortest_match_device(d) == oracle.shortest_match_at(text)
+    assert r.last_stats()["map_passes"] > 0
+    pats = [pat, r"zzzq"]
+    s = tuned(R.BytesRegexSet(pats))
+    assert s.matches_device(d) == list(O.OracleRegex(pats).set_matches(text))
+    assert s.last_stats()["map_passes"] > 0
+    stats = {}
+    got = _run_gpu_shards(pat, text, d, 2, len(exp), halo=1 << 16, tuning={"seg": 64}, options={"max_redo_rounds": 0}, stats=stats)
+    assert got == exp
+    assert any(st["map_passes"] > 0 for st in stats.values()), stats
 
 
 def test_matches_longer_than_the_run_cap_against_python_re():
@@ -117,6 +153,30 @@ def test_chains_that_never_meet_fall_back_to_one_sequential_pass(chunk, n):
     r.set_option("max_stitch_rounds", 6)
     small = text[:100000]
     assert _spans(r.find_all(small)) == O.OracleRegex(r"(?s-u).{6,7}?").find_iter(small)
+
+
+def test_sequential_pass_with_a_generic_table_over_48_kib():
+    """The sequential pass stages the generic runner's table in shared memory as the chunk walks do: a tiling
+    pattern whose anchored table is over the 48 KiB a kernel gets without opting in."""
+    rng = random.Random(7)
+    alphabet = "abcdefghijklmnopqrstuvwxyz0123456789ABCD"
+    words = set()
+    while len(words) < 250:
+        words.add("".join(rng.choice(alphabet) for _ in range(6)))
+    pat = r"(?s-u).{7}|" + "|".join(sorted(words))
+    r = R.BytesRegex(pat)
+    table = r.dfa(R.DFA_FWD_ANCHORED_LF)["trans"]
+    assert 48 << 10 < table.nbytes <= 200 << 10, table.shape
+    r.force_generic(True)
+    r.set_tuning(chunk=256)
+    r.set_option("max_stitch_rounds", 0)
+    n = 200000
+    text = xorshift_bytes(3, n, b"abcdefgh\n")
+    got = r.find_all(text)
+    k = n // 7  # the 3 bytes left over are too few for a word
+    exp = np.stack([np.arange(k) * 7, np.arange(k) * 7 + 7], axis=1)
+    assert got.shape == exp.shape and (np.asarray(got, dtype=np.int64) == exp).all()
+    assert r.last_stats()["sequential_passes"] >= 1, r.last_stats()
 
 
 def test_forward_search_waves_and_early_exit():

@@ -522,8 +522,9 @@ def test_pipelined_host_find_all(monkeypatch):
 
 
 # ------------------------------------------- look-arounds at every kind of boundary ----
-def _run_gpu_shards(pat, text, d_text, world, exp_len, halo=256, tuning=None, options=None):
-    """Byte-range shards of `text` through one GPU (one thread per shard, in-process collectives)."""
+def _run_gpu_shards(pat, text, d_text, world, exp_len, halo=256, tuning=None, options=None, stats=None):
+    """Byte-range shards of `text` through one GPU (one thread per shard, in-process collectives).
+    `stats`: a dict that receives each rank's last_stats() once the boundary protocol is through."""
     import threading
     from regex_b200 import sharded
     comm = sharded.ThreadComm(world)
@@ -542,6 +543,8 @@ def _run_gpu_shards(pat, text, d_text, world, exp_len, halo=256, tuning=None, op
             eng = sharded.GpuShardEngine(re_, buf, cap=exp_len + 16)
             n_local, offset, total, _ = sharded.find_all_sharded(eng, geom, comm.view(rank), info["can_match_empty"], info["has_looks"])
             out[rank] = (offset, (eng.spans[:n_local] + geom.buf_lo).cpu().numpy(), total)
+            if stats is not None:
+                stats[rank] = re_.last_stats()
         except Exception as e:  # noqa: BLE001 -- surface instead of dead-locking the barrier
             errs.append(e)
             comm._barrier.abort()
