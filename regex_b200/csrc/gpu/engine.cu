@@ -89,6 +89,54 @@ struct Regex::DeviceDfa {
   }
 };
 
+// The scalars kernels count, flag or reduce into (one per object, allocated by init_device).  No two fields share
+// bytes; where one copy or memset covers several fields, an assert below keeps them together.
+struct DeviceScalars {
+  // settle_segments: [0] segments to redo.  Stitch (launch.h stitch_fast / stitch_resolve): [0] chunks to walk
+  // again, [1] changed decisions, [2] the general loop is needed, [3] smallest chunk index to walk again
+  uint32_t list[4];
+  unsigned long long long_req;   // stitch: smallest start of a run longer than kExactRunCap (kNone = none)
+  unsigned long long long_best;  // resolve_long_run: last match end + 1 in the window (0 = none)
+  uint32_t long_alive;           // resolve_long_run: the run is still alive at the window's end
+  uint32_t n_new;                // compose_entries: states closure_check added to K
+  uint32_t err_flag;             // walks: a match runs past the end of a shard's halo
+  uint32_t floor_flag;           // walks: a reverse-on-slice scan reaches the left end of the buffer
+  uint32_t first_deferred;       // stitch: entries_local's leftmost deferred chunk
+  uint16_t long_entry;           // resolve_long_run: the automaton's state at the run's start
+  uint8_t flag0;                 // start bitmaps: a match starts at position 0
+  unsigned long long task_counter;  // batch_refill: next task to hand out
+  unsigned long long cand_best;     // cand_shortest: earliest match end
+  unsigned long long fwd_result[1 + kMaxMaskWords];  // forward_range: first match end, OR of the pattern masks
+};
+
+// Pinned host side of the small copies (init_device).  A field staged for an async host-to-device copy is not
+// written again before the stream synchronises.
+struct HostScalars {
+  uint32_t list[4];              // a stitch round: DeviceScalars::list and long_req in one copy
+  unsigned long long long_req;
+  uint32_t n_redo;               // settle_segments
+  uint32_t err_flag, floor_flag; // find_all: DeviceScalars::err_flag and floor_flag in one copy
+  uint64_t n_matches;            // find_all
+  uint64_t exit[2];              // find_all: iterator state leaving the range (ChainKey, or out_p / out_lm of the last chunk)
+  uint64_t iter_total;           // iter_batch: matches of all records
+  uint64_t fwd_result[1 + kMaxMaskWords];  // forward_range: the initial result (staged), then the reduced one
+  uint16_t fwd_exit;             // forward_range: exit state
+  uint16_t rev_guess, rev_left;  // scan_starts, a shard: reverse-scan state assumed at own_hi, exact state at own_lo
+  uint16_t seed_state;           // scan_starts, a shard: the exact state at own_hi (staged) ...
+  uint32_t seed_seg, seed_count; // ... for one redo round of the top segment (staged)
+};
+
+// b directly follows a: one copy or memset covers both
+#define RB_FOLLOWS(S, a, b) static_assert(offsetof(S, b) == offsetof(S, a) + sizeof(S::a), #S ": " #b " must follow " #a)
+RB_FOLLOWS(DeviceScalars, list, long_req);
+RB_FOLLOWS(HostScalars, list, long_req);
+RB_FOLLOWS(DeviceScalars, long_best, long_alive);
+RB_FOLLOWS(DeviceScalars, err_flag, floor_flag);
+RB_FOLLOWS(HostScalars, err_flag, floor_flag);
+#undef RB_FOLLOWS
+static_assert(offsetof(DeviceScalars, first_deferred) == offsetof(DeviceScalars, list) + 12 * sizeof(uint32_t),
+              "stitch_resolve reads the leftmost deferred chunk as counters[12]");
+
 // ------------------------------------------------------------------ compile --
 Regex* Regex::compile(const std::vector<std::string>& patterns, const CompileOptions& opt, rb::Error* err) {
   return compile_impl(patterns, opt, err, nullptr, 0);
@@ -191,7 +239,8 @@ Regex* Regex::compile_impl(const std::vector<std::string>& patterns, const Compi
 
 Regex::~Regex() {
   for (auto*& d : dev_) { delete d; d = nullptr; }
-  if (pinned_) cudaFreeHost(pinned_);
+  if (h_scalars_) cudaFreeHost(h_scalars_);
+  if (d_scalars_) cudaFree(d_scalars_);
   for (void* e : timing_events_) if (e) cudaEventDestroy((cudaEvent_t)e);
   if (fork_event_) cudaEventDestroy((cudaEvent_t)fork_event_);
   if (join_event_) cudaEventDestroy((cudaEvent_t)join_event_);
@@ -265,7 +314,7 @@ int Regex::check(int e, const char* what) {
     if (rc__) return rc__;                              \
   } while (0)
 
-// Stream, pinned scalars and timing events of this object.  Every copy and kernel of the
+// Stream, device and pinned scalars and timing events of this object.  Every copy and kernel of the
 // library is issued on stream_ (or on the two pipeline streams, ordered by events).  The
 // library's own stream is a BLOCKING stream: it is ordered with the legacy default stream,
 // which is where a caller that never heard of streams (or torch's default stream) produced the
@@ -273,14 +322,15 @@ int Regex::check(int e, const char* what) {
 // `torch.zeros(...)` of the output buffer in the tests.  Callers on another stream pass it
 // with rure_b200_set_stream.
 int Regex::init_device() {
-  if (!pinned_) {
+  if (!h_scalars_) {
     int count = 0;
     if (cudaGetDeviceCount(&count) != cudaSuccess || count == 0)
       return fail("no CUDA device available: regex_b200 has no CPU matching path");
     cudaStream_t s;
     RB_CUDA(cudaStreamCreateWithFlags(&s, cudaStreamDefault));
     own_stream_ = s;
-    RB_CUDA(cudaMallocHost(&pinned_, 4096));
+    RB_CUDA(cudaMalloc(&d_scalars_, sizeof(DeviceScalars)));
+    RB_CUDA(cudaMallocHost(&h_scalars_, sizeof(HostScalars)));
     for (void*& e : timing_events_) {
       cudaEvent_t ev;
       RB_CUDA(cudaEventCreate(&ev));
@@ -521,11 +571,10 @@ int Regex::cand_starts(const uint8_t* d_text, uint64_t n, uint64_t base, uint64_
   CandArgs c;
   if (int rc = cand_args(&c)) return rc;
   uint64_t* bm = (uint64_t*)bitmap_.ensure(((n >> 6) + 2) * 8);
-  uint32_t* counters = (uint32_t*)counters_.ensure(128);
-  if (!bm || !counters) return fail("out of device memory (bitmap)");
+  if (!bm) return fail("out of device memory (bitmap)");
   const uint64_t words = std::max<uint64_t>(1, ((limit + 63) >> 6) - (base >> 6));
   cand_bitmap<<<grid_for(words, 256, 8), 256, 0, (cudaStream_t)stream_>>>(d_text, n, base, limit, text_continues ? 1 : 0, c, bm,
-                                                                        (uint8_t*)(counters + 24));
+                                                                        &d_scalars_->flag0);
   RB_LAUNCH_CHECK("cand_bitmap");
   return 0;
 }
@@ -544,9 +593,7 @@ int Regex::cand_shortest(const uint8_t* d_text, uint64_t n, uint64_t start, bool
     RB_CUDA(cudaMemcpyAsync(lazy_->dst + lazy_->done, lazy_->src + lazy_->done, lazy_->n - lazy_->done, cudaMemcpyHostToDevice, st));
     lazy_->done = lazy_->n;
   }
-  uint32_t* counters = (uint32_t*)counters_.ensure(128);
-  if (!counters) return fail("out of device memory (counters)");
-  unsigned long long* best = (unsigned long long*)(counters + 20);
+  unsigned long long* best = &d_scalars_->cand_best;
   RB_CUDA(cudaMemsetAsync(best, 0xFF, 8, st));
   const size_t smem = smem_for(fwd->view);
   RB_CUDA(allow_smem(rbgpu::cand_shortest, smem));  // (the kernel, not this member)
@@ -630,7 +677,6 @@ int Regex::resolve_long_run(const uint8_t* d_text, uint64_t n, uint64_t s, bool 
   g.n = n;
   g.base = s;
   g.seg = seg;
-  uint32_t* counters = (uint32_t*)counters_.ptr;
   // the start state at s: the look-behind flags come from the bytes next to s (pick_start_fwd)
   uint16_t start_state = fwd->view.start[32];
   if (!fwd->view.uniform_start) {
@@ -652,7 +698,7 @@ int Regex::resolve_long_run(const uint8_t* d_text, uint64_t n, uint64_t s, bool 
   // K: the states the run is in at segment boundaries, found as in solve_entries from the run's start state
   // (`(?s)foo.*bar`: 6 of 25 states); it only grows from one window to the next
   uint8_t* present = (uint8_t*)present_.ensure(65536);
-  uint16_t* d_first = (uint16_t*)(counters + 11);
+  uint16_t* d_first = &d_scalars_->long_entry;
   if (!present) return fail("out of device memory (long run)");
   RB_CUDA(cudaMemsetAsync(present, 0, 65536, st));
   {
@@ -669,9 +715,9 @@ int Regex::resolve_long_run(const uint8_t* d_text, uint64_t n, uint64_t s, bool 
     g.n_seg = std::max<uint64_t>(1, (end - s + seg - 1) / seg);
     if (int rc = compose_entries(g, false, d_first)) return rc;
     const uint16_t* exact = (const uint16_t*)exact_.ptr;
-    unsigned long long* best = (unsigned long long*)(counters + 8);
-    RB_CUDA(cudaMemsetAsync(best, 0, 12, st));  // best, then the alive flag at counters[10]
-    scan_last_match<<<grid_for(g.n_seg, 256, tuning.blocks_per_sm), 256, smem, st>>>(g, exact, best, counters + 10);
+    unsigned long long* best = &d_scalars_->long_best;
+    RB_CUDA(cudaMemsetAsync(best, 0, 12, st));  // long_best, then long_alive
+    scan_last_match<<<grid_for(g.n_seg, 256, tuning.blocks_per_sm), 256, smem, st>>>(g, exact, best, &d_scalars_->long_alive);
     RB_LAUNCH_CHECK("scan_last_match");
     uint32_t h[4] = {0, 0, 0, 0};
     RB_CUDA(d2h(h, best, 12));
@@ -682,7 +728,7 @@ int Regex::resolve_long_run(const uint8_t* d_text, uint64_t n, uint64_t s, bool 
       // the run meets the end of a shard's halo: the same verdict as the walk kernels give (err_flag), read
       // by the caller once the search is through
       const uint32_t one = 1;
-      RB_CUDA(cudaMemcpyAsync(counters + 28, &one, 4, cudaMemcpyHostToDevice, st));
+      RB_CUDA(cudaMemcpyAsync(&d_scalars_->err_flag, &one, 4, cudaMemcpyHostToDevice, st));
       RB_CUDA(cudaStreamSynchronize(st));
       *e_out = found ? found - 1 : n;
       return 0;
@@ -696,14 +742,14 @@ int Regex::resolve_long_run(const uint8_t* d_text, uint64_t n, uint64_t s, bool 
 // ------------------------------------------------- bounded fix-up of entry states --
 int Regex::settle_segments(const ScanArgs& a, bool reverse, const std::function<int(uint32_t)>& redo) {
   cudaStream_t st = (cudaStream_t)stream_;
-  uint32_t* counters = (uint32_t*)counters_.ptr;
+  uint32_t* d_redo = &d_scalars_->list[0];
   for (uint32_t round = 0;; round++) {
-    RB_CUDA(cudaMemsetAsync(counters, 0, 4, st));
-    verify_segments<<<grid_for(a.n_seg, 256, 8), 256, 0, st>>>(a.guess, a.fin, a.n_seg, reverse ? 1 : 0, (uint32_t*)redo_.ptr, counters);
+    RB_CUDA(cudaMemsetAsync(d_redo, 0, 4, st));
+    verify_segments<<<grid_for(a.n_seg, 256, 8), 256, 0, st>>>(a.guess, a.fin, a.n_seg, reverse ? 1 : 0, (uint32_t*)redo_.ptr, d_redo);
     RB_LAUNCH_CHECK("verify_segments");
-    RB_CUDA(cudaMemcpyAsync(pinned_, counters, 4, cudaMemcpyDeviceToHost, st));
+    RB_CUDA(cudaMemcpyAsync(&h_scalars_->n_redo, d_redo, 4, cudaMemcpyDeviceToHost, st));
     RB_CUDA(cudaStreamSynchronize(st));
-    const uint32_t n_redo = *(uint32_t*)pinned_;
+    const uint32_t n_redo = h_scalars_->n_redo;
     if (n_redo == 0) return 0;
     if (round == tuning.max_redo_rounds) {
       // wrong guesses keep cascading: solve every entry state at once, then one more redo round
@@ -750,7 +796,7 @@ int Regex::compose_entries(const ScanArgs& scan_args, bool reverse, const uint16
   const int dir = reverse ? 1 : 0;
   uint8_t* present = (uint8_t*)present_.ptr;
   uint16_t* d_kidx = (uint16_t*)kidx_.ensure(65536 * 2);
-  uint32_t* counters = (uint32_t*)counters_.ptr;
+  uint32_t* d_new = &d_scalars_->n_new;
   if (!d_kidx) return fail("out of device memory (state maps)");
   std::vector<uint8_t> h_present(65536);
   std::vector<uint16_t> K, kidx;
@@ -771,11 +817,11 @@ int Regex::compose_entries(const ScanArgs& scan_args, bool reverse, const uint16
     scan_map<<<grid_for(n_seg * k, 256, tuning.blocks_per_sm), 256, smem, st>>>(g, dir, d_states, k, maps);
     RB_LAUNCH_CHECK("scan_map");
     stats.map_passes += k;
-    RB_CUDA(cudaMemsetAsync(counters + 8, 0, 4, st));
-    closure_check<<<grid_for(n_seg * k, 256, 8), 256, 0, st>>>(maps, n_seg * k, d_kidx, present, counters + 8);
+    RB_CUDA(cudaMemsetAsync(d_new, 0, 4, st));
+    closure_check<<<grid_for(n_seg * k, 256, 8), 256, 0, st>>>(maps, n_seg * k, d_kidx, present, d_new);
     RB_LAUNCH_CHECK("closure_check");
     uint32_t n_new = 0;
-    RB_CUDA(d2h(&n_new, counters + 8, 4));  // also orders the host vectors above before they are rebuilt
+    RB_CUDA(d2h(&n_new, d_new, 4));  // also orders the host vectors above before they are rebuilt
     if (n_new == 0) break;
   }
   const uint32_t k = (uint32_t)K.size();
@@ -835,9 +881,8 @@ int Regex::scan_starts(const uint8_t* d_text, uint64_t n, uint64_t base, uint64_
   a.guess = (uint16_t*)guess_.ensure(n_seg * 2);
   a.fin = (uint16_t*)fin_.ensure((n_seg + 1) * 2);
   uint32_t* redo = (uint32_t*)redo_.ensure(n_seg * 4);
-  uint32_t* counters = (uint32_t*)counters_.ensure(128);
-  if (!a.bitmap || !a.guess || !a.fin || !redo || !counters) return fail("out of device memory (scan scratch)");
-  a.flag0 = (uint8_t*)(counters + 24);
+  if (!a.bitmap || !a.guess || !a.fin || !redo) return fail("out of device memory (scan scratch)");
+  a.flag0 = &d_scalars_->flag0;
   a.utf8_boundaries = utf8_mask;
   a.hot = rev->hot;
   size_t smem;
@@ -880,27 +925,26 @@ int Regex::scan_starts(const uint8_t* d_text, uint64_t n, uint64_t base, uint64_
   stats.scan_redo_rounds = stats.scan_redo_segments = stats.map_passes = 0;
   ScanArgs r = a;  // a redo round: only the listed segments, each entered with its neighbour's exit
   r.redo_list = redo;
-  r.n_redo = counters;
+  r.n_redo = &d_scalars_->list[0];
   auto redo_launch = [&](uint32_t n_redo) -> int {
     launch(r, n_redo);
     RB_LAUNCH_CHECK("scan_rev(redo)");
     return 0;
   };
   // A shard may be told the exact state at its top edge by its right neighbour.
-  uint16_t* h16 = (uint16_t*)pinned_ + 512;
+  HostScalars* h = h_scalars_;
   const bool shard = io && (!io->is_first || !io->is_last || io->rev_entry != kNoState || io->own_hi < n);
   if (shard) {
-    RB_CUDA(cudaMemcpyAsync(h16, a.guess + (n_seg - 1), 2, cudaMemcpyDeviceToHost, st));
+    RB_CUDA(cudaMemcpyAsync(&h->rev_guess, a.guess + (n_seg - 1), 2, cudaMemcpyDeviceToHost, st));
     RB_CUDA(cudaStreamSynchronize(st));
-    io->rev_guess = h16[0];
+    io->rev_guess = h->rev_guess;
     if (io->rev_entry != kNoState && io->rev_entry != io->rev_guess) {
-      h16[1] = (uint16_t)io->rev_entry;
-      uint32_t* h32 = (uint32_t*)pinned_ + 300;
-      h32[0] = (uint32_t)(n_seg - 1);
-      h32[1] = 1;
-      RB_CUDA(cudaMemcpyAsync(a.fin + n_seg, h16 + 1, 2, cudaMemcpyHostToDevice, st));
-      RB_CUDA(cudaMemcpyAsync(redo, h32, 4, cudaMemcpyHostToDevice, st));
-      RB_CUDA(cudaMemcpyAsync(counters, h32 + 1, 4, cudaMemcpyHostToDevice, st));
+      h->seed_state = (uint16_t)io->rev_entry;
+      h->seed_seg = (uint32_t)(n_seg - 1);
+      h->seed_count = 1;
+      RB_CUDA(cudaMemcpyAsync(a.fin + n_seg, &h->seed_state, 2, cudaMemcpyHostToDevice, st));
+      RB_CUDA(cudaMemcpyAsync(redo, &h->seed_seg, 4, cudaMemcpyHostToDevice, st));
+      RB_CUDA(cudaMemcpyAsync(&d_scalars_->list[0], &h->seed_count, 4, cudaMemcpyHostToDevice, st));
       stats.scan_redo_rounds++;
       stats.scan_redo_segments++;
       if (int rc = redo_launch(1)) return rc;
@@ -909,9 +953,9 @@ int Regex::scan_starts(const uint8_t* d_text, uint64_t n, uint64_t base, uint64_
   }
   if (int rc = settle_segments(a, true, redo_launch)) return rc;
   if (shard) {
-    RB_CUDA(cudaMemcpyAsync(h16, a.fin, 2, cudaMemcpyDeviceToHost, st));
+    RB_CUDA(cudaMemcpyAsync(&h->rev_left, a.fin, 2, cudaMemcpyDeviceToHost, st));
     RB_CUDA(cudaStreamSynchronize(st));
-    io->rev_left = h16[0];
+    io->rev_left = h->rev_left;
   }
   return 0;
 }
@@ -981,9 +1025,10 @@ int Regex::find_all_shard_device(const uint8_t* d_text, uint64_t n, ShardIO* io,
   if (rev) w.rev = rev->view;
   w.text = d_text;
   w.n = n;
-  if (!bitmap_.ensure(((n >> 6) + 2) * 8) || !counters_.ensure(128)) return fail("out of device memory (bitmap)");
+  if (!bitmap_.ensure(((n >> 6) + 2) * 8)) return fail("out of device memory (bitmap)");
   w.bitmap = (const uint64_t*)bitmap_.ptr;
-  w.flag0 = (const uint8_t*)((uint32_t*)counters_.ptr + 24);
+  DeviceScalars* ds = d_scalars_;
+  w.flag0 = &ds->flag0;
   w.base = io->own_lo;
   w.limit = io->own_hi;
   w.text_continues = !io->is_last;
@@ -1003,8 +1048,7 @@ int Regex::find_all_shard_device(const uint8_t* d_text, uint64_t n, ShardIO* io,
   w.meta = (uint32_t*)meta_.ensure(nc * 4);
   w.stage = (uint64_t*)stage_.ensure(nc * (uint64_t)w.stage_cap * 16);
   const uint64_t n_blocks = (nc + 1023) / 1024;
-  uint32_t* counters = (uint32_t*)counters_.ensure(128);
-  if (!w.in_p || !w.in_lm || !w.out_p || !w.out_lm || !w.count || !offset || !dirty_list || !w.first_cand || !w.skip || !w.meta || !w.stage || !counters)
+  if (!w.in_p || !w.in_lm || !w.out_p || !w.out_lm || !w.count || !offset || !dirty_list || !w.first_cand || !w.skip || !w.meta || !w.stage)
     return fail("out of device memory (walk scratch)");
   w.offset = offset;
   w.out = d_out;
@@ -1013,9 +1057,9 @@ int Regex::find_all_shard_device(const uint8_t* d_text, uint64_t n, ShardIO* io,
   w.emulate_slice = emulate;
   w.can_match_empty = can_match_empty;
   // entry states: chunk 0 starts the real chain at `start`; the rest speculate.
-  w.err_flag = counters + 28;
-  w.floor_flag = counters + 29;
-  // long anchored runs go to resolve_long_run (automata of up to 128 states); counters[6..7] = the request slot
+  w.err_flag = &ds->err_flag;
+  w.floor_flag = &ds->floor_flag;
+  // long anchored runs go to resolve_long_run (automata of up to 128 states), requested in long_req
   const bool can_resolve = fwd->view.n_states <= 128;
   uint64_t* long_tab = (uint64_t*)long_tab_.ensure(kMaxLongRuns * 16);
   if (!long_tab) return fail("out of device memory (long runs)");
@@ -1023,10 +1067,10 @@ int Regex::find_all_shard_device(const uint8_t* d_text, uint64_t n, ShardIO* io,
   w.exact_cap = can_resolve ? kExactRunCap : kNone;
   w.long_tab = long_tab;
   w.n_long = 0;
-  w.long_req = (unsigned long long*)(counters + 6);
+  w.long_req = &ds->long_req;
   RB_CUDA(cudaMemsetAsync(w.long_req, 0xFF, 8, st));
   w.clamp_p = io->chain_clamped ? io->chain_p : kNone;
-  RB_CUDA(cudaMemsetAsync(w.err_flag, 0, 8, st));
+  RB_CUDA(cudaMemsetAsync(w.err_flag, 0, 8, st));  // err_flag, floor_flag
   init_walk_entries<<<grid_for(nc, 256, 8), 256, 0, st>>>(w.in_p, w.in_lm, w.skip, nc, io->chain_p, io->chain_lm);
   RB_LAUNCH_CHECK("init_walk_entries");
   size_t wsmem = 0;
@@ -1094,14 +1138,15 @@ int Regex::find_all_shard_device(const uint8_t* d_text, uint64_t n, ShardIO* io,
   stats.stitch_rounds = stats.stitch_dirty_chunks = stats.sequential_passes = stats.long_runs = 0;
   const bool strict = emulate || can_match_empty;
   bool general = strict;
-  uint32_t* hc = (uint32_t*)pinned_ + 64;  // host copy of counters[0..3]
+  uint32_t* list = ds->list;
+  HostScalars* h = h_scalars_;
   if (!strict) {
-    RB_CUDA(cudaMemsetAsync(counters, 0, 16, st));
-    stitch_fast<<<grid_for(nc, 256, 8), 256, 0, st>>>(w, counters);
+    RB_CUDA(cudaMemsetAsync(list, 0, 16, st));
+    stitch_fast<<<grid_for(nc, 256, 8), 256, 0, st>>>(w, list);
     RB_LAUNCH_CHECK("stitch_fast");
-    RB_CUDA(cudaMemcpyAsync(hc, counters, 16, cudaMemcpyDeviceToHost, st));
+    RB_CUDA(cudaMemcpyAsync(h->list, list, 16, cudaMemcpyDeviceToHost, st));
     RB_CUDA(cudaStreamSynchronize(st));
-    general = hc[2] != 0;  // (a deferred chunk -- long run -- asks for the general loop too)
+    general = h->list[2] != 0;  // (a deferred chunk -- long run -- asks for the general loop too)
   }
   ChainKey* grand_key = nullptr;
   if (general) {
@@ -1111,22 +1156,22 @@ int Regex::find_all_shard_device(const uint8_t* d_text, uint64_t n, ShardIO* io,
     grand_key = btot + n_blocks;
     WalkArgs wd = w;
     wd.dirty_list = dirty_list;
-    wd.n_dirty = counters;
+    wd.n_dirty = list;
     uint32_t dirty_rounds = 0;
     for (;;) {
-      RB_CUDA(cudaMemsetAsync(counters + 12, 0xFF, 4, st));  // [12] leftmost deferred chunk
-      entries_local<<<(uint32_t)n_blocks, 1024, 0, st>>>(w, excl, btot, counters + 12);
+      RB_CUDA(cudaMemsetAsync(&ds->first_deferred, 0xFF, 4, st));
+      entries_local<<<(uint32_t)n_blocks, 1024, 0, st>>>(w, excl, btot, &ds->first_deferred);
       RB_LAUNCH_CHECK("entries_local");
       entries_blocks<<<1, 1024, 0, st>>>(btot, n_blocks, grand_key);
       RB_LAUNCH_CHECK("entries_blocks");
-      RB_CUDA(cudaMemsetAsync(counters, 0, 12, st));       // [0] chunks to walk again, [1] changed decisions
-      RB_CUDA(cudaMemsetAsync(counters + 3, 0xFF, 4, st));  // [3] smallest chunk index to walk again
-      stitch_resolve<<<grid_for(nc, 256, 8), 256, 0, st>>>(wd, excl, btot, counters);
+      RB_CUDA(cudaMemsetAsync(list, 0, 12, st));       // [0] chunks to walk again, [1] changed decisions
+      RB_CUDA(cudaMemsetAsync(list + 3, 0xFF, 4, st));  // [3] smallest chunk index to walk again
+      stitch_resolve<<<grid_for(nc, 256, 8), 256, 0, st>>>(wd, excl, btot, list);
       RB_LAUNCH_CHECK("stitch_resolve");
-      RB_CUDA(cudaMemcpyAsync(hc, counters, 32, cudaMemcpyDeviceToHost, st));
+      RB_CUDA(cudaMemcpyAsync(h->list, list, sizeof h->list + sizeof h->long_req, cudaMemcpyDeviceToHost, st));  // list, long_req
       RB_CUDA(cudaStreamSynchronize(st));
-      const uint32_t n_dirty = hc[0], n_changed = hc[1];
-      const uint64_t long_s = *(const uint64_t*)(hc + 6);
+      const uint32_t n_dirty = h->list[0], n_changed = h->list[1];
+      const uint64_t long_s = h->long_req;
       bool serve = long_s != kNone;
       if (serve) {
         // the request of a chunk that this round found covered by an earlier match is dropped
@@ -1155,7 +1200,7 @@ int Regex::find_all_shard_device(const uint8_t* d_text, uint64_t n, ShardIO* io,
       if (n_dirty == 0) continue;
       if (++dirty_rounds > tuning.max_stitch_rounds) {
         // chains that do not meet again: one sequential pass from the leftmost such chunk
-        wd.seq_from = hc[3];
+        wd.seq_from = h->list[3];
         if (use_pf) launch_pf(wd, 1, 2);
         else sequential<<<1, 256, wsmem, st>>>(wd);
         RB_LAUNCH_CHECK("walk_sequential");
@@ -1178,27 +1223,27 @@ int Regex::find_all_shard_device(const uint8_t* d_text, uint64_t n, ShardIO* io,
     compact<<<grid_for(nc, 256, 6), 256, wsmem, st>>>(w);
     RB_LAUNCH_CHECK("compact_spans");
   }
-  uint64_t* h = (uint64_t*)pinned_;
-  RB_CUDA(cudaMemcpyAsync(h, grand, 8, cudaMemcpyDeviceToHost, st));
+  RB_CUDA(cudaMemcpyAsync(&h->n_matches, grand, 8, cudaMemcpyDeviceToHost, st));
   if (grand_key) {  // exit state = the last contribution of the whole range
-    RB_CUDA(cudaMemcpyAsync(h + 1, grand_key, 16, cudaMemcpyDeviceToHost, st));
+    RB_CUDA(cudaMemcpyAsync(h->exit, grand_key, 16, cudaMemcpyDeviceToHost, st));
   } else {
-    RB_CUDA(cudaMemcpyAsync(h + 1, w.out_p + (nc - 1), 8, cudaMemcpyDeviceToHost, st));
-    RB_CUDA(cudaMemcpyAsync(h + 2, w.out_lm + (nc - 1), 8, cudaMemcpyDeviceToHost, st));
+    RB_CUDA(cudaMemcpyAsync(&h->exit[0], w.out_p + (nc - 1), 8, cudaMemcpyDeviceToHost, st));
+    RB_CUDA(cudaMemcpyAsync(&h->exit[1], w.out_lm + (nc - 1), 8, cudaMemcpyDeviceToHost, st));
   }
-  RB_CUDA(cudaMemcpyAsync(h + 3, w.err_flag, 8, cudaMemcpyDeviceToHost, st));
+  RB_CUDA(cudaMemcpyAsync(&h->err_flag, w.err_flag, 8, cudaMemcpyDeviceToHost, st));  // err_flag, floor_flag
   RB_CUDA(cudaEventRecord(ev[2], st));
   RB_CUDA(cudaStreamSynchronize(st));
-  io->n_matches = h[0];
+  io->n_matches = h->n_matches;
+  const uint64_t* x = h->exit;
   if (grand_key) {  // ChainKey: 0 = nothing in this range moved the iterator (speculative shard without candidates)
-    io->exit_p = h[1] == 0 ? kSpec : (h[1] == ~0ull ? kNone : h[1] - 1);
-    io->exit_lm = h[1] == 0 ? kNone : h[2];
+    io->exit_p = x[0] == 0 ? kSpec : (x[0] == ~0ull ? kNone : x[0] - 1);
+    io->exit_lm = x[0] == 0 ? kNone : x[1];
   } else {
-    io->exit_p = h[1];
-    io->exit_lm = h[2];
+    io->exit_p = x[0];
+    io->exit_lm = x[1];
   }
-  io->halo_overflow = ((uint32_t*)(h + 3))[0] != 0;
-  io->left_ctx_short = ((uint32_t*)(h + 3))[1] != 0;
+  io->halo_overflow = h->err_flag != 0;
+  io->left_ctx_short = h->floor_flag != 0;
   stats.fused = fused;
   stats.path = use_pf ? 3 : cand ? 4 : fused ? 2 : plan.fast ? 1 : 0;
   cudaEventElapsedTime(&stats.scan_ms, ev[0], ev[1]);
@@ -1266,8 +1311,7 @@ int Regex::forward_range(const uint8_t* d_text, uint64_t n, uint64_t start, uint
   a.guess = (uint16_t*)guess_.ensure(n_seg * 2);
   a.fin = (uint16_t*)fin_.ensure(n_seg * 2);
   uint32_t* redo = (uint32_t*)redo_.ensure(n_seg * 4);
-  uint32_t* counters = (uint32_t*)counters_.ensure(128);
-  if (!a.seg_first || (want_masks && !a.seg_mask) || !a.guess || !a.fin || !redo || !counters)
+  if (!a.seg_first || (want_masks && !a.seg_mask) || !a.guess || !a.fin || !redo)
     return fail("out of device memory (scan scratch)");
   RB_CUDA(allow_smem(scan_fwd_reduce, smem));
   // whole warps of full segments go to the fast kernel; segment 0, the ragged end and the EOF step stay generic
@@ -1313,25 +1357,25 @@ int Regex::forward_range(const uint8_t* d_text, uint64_t n, uint64_t start, uint
   }
   ScanArgs r = a;
   r.redo_list = redo;
-  r.n_redo = counters;
+  r.n_redo = &d_scalars_->list[0];
   auto redo_launch = [&](uint32_t n_redo) -> int {
     scan_fwd_reduce<<<grid_for(n_redo, tuning.block, tuning.blocks_per_sm), tuning.block, smem, st>>>(r);
     RB_LAUNCH_CHECK("scan_fwd_reduce(redo)");
     return 0;
   };
   if (int rc = settle_segments(a, false, redo_launch)) return rc;
-  unsigned long long* result = (unsigned long long*)(counters + 4);
-  uint64_t* h = (uint64_t*)pinned_ + 16;
+  unsigned long long* result = d_scalars_->fwd_result;
+  uint64_t* h = h_scalars_->fwd_result;
   h[0] = kNone;
   for (uint32_t w = 0; w < kMaxMaskWords; w++) h[1 + w] = 0;
   RB_CUDA(cudaMemcpyAsync(result, h, 8 * (1 + kMaxMaskWords), cudaMemcpyHostToDevice, st));
   reduce_segments<<<grid_for(n_seg, 256, 4), 256, 0, st>>>(a.seg_first, a.seg_mask, n_seg, mw, result);
   RB_LAUNCH_CHECK("reduce_segments");
   RB_CUDA(cudaMemcpyAsync(h, result, 8 * (1 + kMaxMaskWords), cudaMemcpyDeviceToHost, st));
-  RB_CUDA(cudaMemcpyAsync(h + 8, a.fin + (n_seg - 1), 2, cudaMemcpyDeviceToHost, st));
+  RB_CUDA(cudaMemcpyAsync(&h_scalars_->fwd_exit, a.fin + (n_seg - 1), 2, cudaMemcpyDeviceToHost, st));
   RB_CUDA(cudaStreamSynchronize(st));
   for (uint32_t w = 0; w < 1 + kMaxMaskWords; w++) result_host[w] = h[w];
-  *exit_state = *(uint16_t*)(h + 8);
+  *exit_state = h_scalars_->fwd_exit;
   return 0;
 }
 
@@ -1677,9 +1721,7 @@ int Regex::is_match_batch_device(const uint8_t* d_text, const uint64_t* d_offset
     a.task_recs = (uint32_t)std::min<uint64_t>(2048, per_task / 32 * 32);
     if (tuning.batch_refill >= 2) a.task_recs = std::max<uint32_t>(a.task_recs, 32);  // tests: whatever the size
     if (tuning.batch_refill && a.task_recs >= (tuning.batch_refill >= 2 ? 32u : 96u)) {
-      uint32_t* counters = (uint32_t*)counters_.ensure(128);
-      if (!counters) return fail("out of device memory (batch scratch)");
-      a.task_counter = (unsigned long long*)(counters + 16);
+      a.task_counter = &d_scalars_->task_counter;
       RB_CUDA(cudaMemsetAsync(a.task_counter, 0, 8, (cudaStream_t)stream_));
       // (8 KB of static shared memory for the result words on top of the table: opt in whenever the sum may pass 48 KB)
       RB_CUDA(allow_smem(batch_refill, smem, 48 * 1024));
@@ -1777,13 +1819,13 @@ int Regex::iter_batch(const uint8_t* d_text, const uint64_t* d_offsets, uint64_t
   // ---- exclusive scan over n_rec + 1 entries ----
   unsigned long long* grand;
   if (int rc = prefix_sum(d_match_offsets, d_match_offsets, n_rec + 1, &grand)) return rc;
-  uint64_t* h = (uint64_t*)pinned_;
+  uint64_t* h = &h_scalars_->iter_total;
   if (grow) {  // every span, into a buffer sized by the count
     RB_CUDA(cudaMemcpyAsync(h, grand, 8, cudaMemcpyDeviceToHost, st));
     RB_CUDA(cudaStreamSynchronize(st));
-    a.out_spans = (uint64_t*)grow->ensure(std::max<uint64_t>(h[0], 1) * 16);
+    a.out_spans = (uint64_t*)grow->ensure(std::max<uint64_t>(*h, 1) * 16);
     if (!a.out_spans) return fail("out of device memory (batch spans)");
-    a.cap = h[0];
+    a.cap = *h;
   }
   // ---- write ----
   if (a.cap > 0 && cand) {
@@ -1796,7 +1838,7 @@ int Regex::iter_batch(const uint8_t* d_text, const uint64_t* d_offsets, uint64_t
   }
   RB_CUDA(cudaMemcpyAsync(h, grand, 8, cudaMemcpyDeviceToHost, st));
   RB_CUDA(cudaStreamSynchronize(st));
-  *total = h[0];
+  *total = *h;
   return 0;
 }
 
@@ -2021,7 +2063,7 @@ int Regex::replace_sums(const uint8_t* d_text, uint64_t n, const uint64_t* spans
   const std::vector<uint8_t>& lits = rep_lits_;
   cudaStream_t st = (cudaStream_t)stream_;
   uint64_t* lens = (uint64_t*)lens_.ensure(std::max<uint64_t>(m, 1) * 8);
-  uint64_t* before = (uint64_t*)offset_.ensure(std::max<uint64_t>(m, 1) * 8);
+  uint64_t* before = (uint64_t*)lens_before_.ensure(std::max<uint64_t>(m, 1) * 8);
   uint8_t* d_lits = (uint8_t*)lits_.ensure(std::max<size_t>(lits.size(), 16));
   if (!lens || !before || !d_lits) return fail("out of device memory (replace scratch)");
   uint64_t* reps_before = (uint64_t*)reps_before_.ensure(std::max<uint64_t>(m, 1) * 8);
@@ -2341,9 +2383,9 @@ int Regex::replace_batch_device(const uint8_t* d_text, const uint64_t* d_offsets
     RB_LAUNCH_CHECK("batch_to_base");
   }
   if (int rc = replace_sums(d_text + first, last - first, spans, m, slots, out_len)) return rc;
-  batch_replace_offsets<<<grid_for(n_rec + 1, 256, 8), 256, 0, st>>>(d_offsets, moff, n_rec, (const uint64_t*)offset_.ptr,
-                                                                      (const uint64_t*)reps_before_.ptr, m, rep_totals_[0], rep_totals_[1],
-                                                                      d_out_offsets);
+  const ReplaceArgs& ra = *reinterpret_cast<const ReplaceArgs*>(rep_args_.data());
+  batch_replace_offsets<<<grid_for(n_rec + 1, 256, 8), 256, 0, st>>>(d_offsets, moff, n_rec, ra.lens_before, ra.reps_before, m, rep_totals_[0],
+                                                                      rep_totals_[1], d_out_offsets);
   RB_LAUNCH_CHECK("batch_replace_offsets");
   if (!d_out) {
     RB_CUDA(cudaStreamSynchronize(st));
@@ -2715,7 +2757,7 @@ int Regex::find_iter_batch_host(const uint8_t* text, const uint64_t* offsets, ui
   uint64_t* d_off;
   int rc = upload_batch(text, offsets, n_rec, &d, &d_off);
   if (rc) return rc;
-  uint64_t* d_moff = (uint64_t*)count_.ensure((n_rec + 1) * 8);
+  uint64_t* d_moff = (uint64_t*)bres_off_.ensure((n_rec + 1) * 8);
   if (!d_moff) return fail("out of device memory (batch)");
   if (!out) cap = 0;
   uint64_t* d_spans = cap ? (uint64_t*)out_.ensure(cap * 16) : nullptr;

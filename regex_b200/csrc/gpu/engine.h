@@ -17,8 +17,10 @@
 
 namespace rbgpu {
 
-struct BatchArgs;  // launch.h
-struct ScanArgs;   // launch.h
+struct BatchArgs;      // launch.h
+struct ScanArgs;       // launch.h
+struct DeviceScalars;  // engine.cu
+struct HostScalars;    // engine.cu
 
 struct CompileOptions {
   uint32_t flags = 32;               // RURE_FLAG_* bits (rure.h:56-68); default = UNICODE
@@ -310,11 +312,22 @@ class Regex {
   void* back_stream_ = nullptr;  // device -> host spans of a pipelined find_all; the generic edge kernel of a forward scan
   void* ext_stream_ = nullptr;
   bool use_ext_stream_ = false;
-  // scratch (grow-only)
-  DeviceBuf text_, bitmap_, guess_, fin_, redo_, counters_, seg_first_, seg_mask_;
-  DeviceBuf long_tab_;
+  DeviceScalars* d_scalars_ = nullptr;  // counters, flags and reductions of the kernels (device)
+  HostScalars* h_scalars_ = nullptr;    // pinned staging of the small copies to and from d_scalars_
+  // ---- device scratch (grow-only), grouped by the calls that own it ----
+  // whole-haystack scans (scan_starts, cand_starts, forward_range, settle_segments): start bitmap, segment entry
+  // guesses and exits, redo list, per-segment forward results
+  DeviceBuf bitmap_, guess_, fin_, redo_, seg_first_, seg_mask_;
+  // state-map composition (solve_entries, compose_entries, resolve_long_run)
+  DeviceBuf present_, kidx_, kstates_, maps_, comp_, bentry_, exact_;
+  // chunk walk and stitch (find_all_shard_device): chain entries and exits, match counts and offsets, dirty list,
+  // staged spans, stitch keys, resolved long runs
+  DeviceBuf in_p_, in_lm_, out_p_, out_lm_, count_, offset_, dirty_, first_cand_, skip_, meta_, stage_, excl_, btot_, long_tab_;
   static constexpr uint32_t kMaxLongRuns = 256;
-  DeviceBuf spans_all_, lens_, lits_, rep_out_, pieces_, reps_before_;
+  DeviceBuf block_sums_;  // prefix_sum (any caller)
+  // replace / split over one haystack: all spans, match lengths and the prefix sums of the match and replacement
+  // lengths, template literals
+  DeviceBuf spans_all_, lens_, lens_before_, reps_before_, lits_;
   uint64_t rep_totals_[2] = {0, 0};  // matched bytes, replacement bytes of the pending replace call
   std::vector<uint8_t> rep_args_, rep_lits_;  // launch.h ReplaceArgs image + literal bytes of the pending replace call
   int n_groups_ = 1;                      // capture groups incl. group 0
@@ -323,12 +336,14 @@ class Regex {
   DeviceBuf cap_insts_, cap_scratch_, cap_slots_, cap_span_;
   uint32_t cap_n_insts_ = 0, cap_start_ = 0;  // capture program on the device (0 = not uploaded yet)
   bool cap_anchored_ = false;
-  // batched replace / split / captures_iter (never shared with the whole-haystack calls, which the per-record
-  // captures_iter redo runs in between): match CSR and spans, kept CSR and spans, slots, divergence flags and list,
-  // and the host wrappers' results; the record offsets of every batched host wrapper (boffsets_)
+  // batched records (never shared with the whole-haystack calls, which the per-record captures_iter redo runs in
+  // between): match CSR and spans, kept CSR and spans, slots, divergence flags and list; the record offsets of
+  // every batched host wrapper (boffsets_) and the CSR and items of the find_iter / replace / split / captures_iter
+  // host wrappers (bres_off_, bres_)
   DeviceBuf bmoff_, bspans_, bkoff_, bkspans_, bslots_, bflags_, blist_, boffsets_, bres_off_, bres_;
-  DeviceBuf in_p_, in_lm_, out_p_, out_lm_, count_, offset_, dirty_, first_cand_, skip_, meta_, excl_, btot_, present_, kidx_, kstates_, maps_, comp_, bentry_, exact_, stage_, block_sums_, out_, bits_, masks_;
-  void* pinned_ = nullptr;  // small pinned staging area for counters / scalars
+  // host wrappers: the haystack, spans (also find_at_device's one span), split pieces, replace output, batched match
+  // bits and set masks
+  DeviceBuf text_, out_, pieces_, rep_out_, bits_, masks_;
   void* timing_events_[3] = {nullptr, nullptr, nullptr};
   void *fork_event_ = nullptr, *join_event_ = nullptr;  // forward scans: the generic edge kernel runs beside the fast one
   int pf_state_ = 0;               // 0 = not decided yet, 1 = prefilter applies, -1 = it does not
