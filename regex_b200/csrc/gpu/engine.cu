@@ -464,6 +464,8 @@ static uint32_t grid_for(uint64_t threads_needed, uint32_t block, uint32_t block
   return (uint32_t)std::max<uint64_t>(1, std::min(blocks, cap));
 }
 
+// The most dynamic shared memory a block can opt in to on sm_100 (allow_smem).
+static constexpr size_t kMaxDynamicSmem = 227 * 1024;
 static size_t fast_scan_smem(size_t table_bytes) {
   return table_bytes + 1024 + (1024 / 32) * (2 * 2048 + 64);  // kernels.cu kBoxStages, kRingBarBytes  // kernels.cu: tables, 512-aligned rings, mbarriers
 }
@@ -961,11 +963,14 @@ int Regex::scan_starts(const uint8_t* d_text, uint64_t n, uint64_t base, uint64_
 }
 
 // ------------------------------------------------------------------ find_all --
+// First bitmap bit of a search from `start` (bit i <-> position i + 1), rounded down to the 256-bit shard grain.
+static uint64_t shard_own_lo(uint64_t start) { return start ? (start - 1) & ~255ull : 0; }
+
 int Regex::find_all_device(const uint8_t* d_text, uint64_t n, uint64_t start, uint64_t* d_out, uint64_t cap, uint64_t* total) {
   *total = 0;
   if (start > n) return 0;  // re_trait.rs:198-200
   ShardIO io;
-  io.own_lo = start ? ((start - 1) & ~255ull) : 0;  // bit i <-> position i+1
+  io.own_lo = shard_own_lo(start);
   io.own_hi = n;
   io.chain_p = start;
   io.chain_lm = kNone;
@@ -974,15 +979,135 @@ int Regex::find_all_device(const uint8_t* d_text, uint64_t n, uint64_t start, ui
   return rc;
 }
 
-// Chain-walk kernels by runner kind (find_all_shard_device: 0 generic, 1 byte-indexed shared-memory table, 2 fixed
-// length), and the literal prefilter by [table runner][number of scanned bytes - 1].
+// The paths of a find_iter range, as stats.path reports them, and the chain walk's runners: the kernel tables below are
+// indexed by runner.
+enum WalkPath { kPathGeneric = 0, kPathFast = 1, kPathFused = 2, kPathPrefilter = 3, kPathCandidates = 4 };
+enum WalkRunner { kRunGeneric = 0, kRunTable = 1, kRunFixed = 2 };
 using WalkKernel = void (*)(WalkArgs);
 using PfKernel = void (*)(WalkArgs, PfArgs, int);
-static const WalkKernel kWalkChunks[3] = {walk_chunks<0>, walk_chunks<1>, walk_chunks<2>};
-static const WalkKernel kCompactSpans[3] = {compact_spans<0>, compact_spans<1>, compact_spans<2>};
-static const WalkKernel kWalkSequential[3] = {walk_sequential<0>, walk_sequential<1>, walk_sequential<2>};
-static const PfKernel kLiteralScan[2][4] = {{literal_scan<0, 1>, literal_scan<0, 2>, literal_scan<0, 3>, literal_scan<0, 4>},
-                                            {literal_scan<1, 1>, literal_scan<1, 2>, literal_scan<1, 3>, literal_scan<1, 4>}};
+
+struct Regex::WalkPlan {
+  ScanPlan scan;  // the reverse scan of the start bitmap (paths 0-2)
+  int path = kPathGeneric;
+  // byte-indexed table: uniform start state, 16-byte aligned text; fixed length: no haystack access, so every candidate
+  // must be a match start (not with candidate starts), and not as the prefilter's verifier
+  int runner = kRunGeneric;
+  bool fused = false;  // every lane of the fast scan kernel also walks its own segment (chunk == segment)
+  uint32_t chunk = 0;  // bitmap bits per chunk
+  size_t smem = 0;     // dynamic shared memory of the runner
+  PfArgs pf{};
+  WalkKernel walk = nullptr, compact = nullptr, sequential = nullptr;
+  PfKernel pf_scan = nullptr;  // the prefilter path, which launches it in place of the three above
+};
+
+Regex::WalkPlan Regex::plan_walk(const uint8_t* d_text, const ShardIO& io, const DeviceDfa* fwd, const DeviceDfa* revall) {
+  static const WalkKernel kWalkChunks[3] = {walk_chunks<0>, walk_chunks<1>, walk_chunks<2>};
+  static const WalkKernel kCompactSpans[3] = {compact_spans<0>, compact_spans<1>, compact_spans<2>};
+  static const WalkKernel kWalkSequential[3] = {walk_sequential<0>, walk_sequential<1>, walk_sequential<2>};
+  static const PfKernel kLiteralScan[2][4] = {{literal_scan<0, 1>, literal_scan<0, 2>, literal_scan<0, 3>, literal_scan<0, 4>},
+                                              {literal_scan<1, 1>, literal_scan<1, 2>, literal_scan<1, 3>, literal_scan<1, 4>}};  // [runner][bytes - 1]
+  WalkPlan p;
+  const bool cand = candidate_mode();
+  const bool aligned = ((uintptr_t)d_text & 15) == 0;
+  p.scan = plan_scan(d_text, io.own_lo, io.own_hi,
+                     !cand && hot_signed_ok(revall->hot) && fast_scan_smem(hot_bytes_signed(revall->hot)) <= kMaxDynamicSmem);
+  const bool table = fwd->hot.n != 0 && fwd->view.uniform_start && aligned && !tuning.force_generic;
+  // literal prefilter: no start bitmap at all -- literal_scan finds, verifies and chains the candidates
+  const bool pf = tuning.prefilter && !tuning.force_generic && aligned && plan_prefilter() &&
+                  (tuning.prefilter >= 2 || pf_freq_ <= kPrefilterAutoFreq);
+  const bool fixed = !pf && min_len == max_len && min_len > 0 && !has_looks && !tuning.force_generic && !cand;
+  p.runner = fixed ? kRunFixed : table ? kRunTable : kRunGeneric;
+  p.fused = !pf && !cand && p.scan.fast && p.runner != kRunGeneric && tuning.fuse && !io.reuse_scan &&
+            fast_scan_smem(hot_bytes_signed(revall->hot) + (p.runner == kRunTable ? hot_bytes(fwd->hot.n) : 0)) <= kMaxDynamicSmem;
+  p.path = pf ? kPathPrefilter : cand ? kPathCandidates : p.fused ? kPathFused : p.scan.fast ? kPathFast : kPathGeneric;
+  p.chunk = pf ? 8192 : p.fused ? p.scan.seg : std::max<uint32_t>(256, (tuning.chunk + 255) / 256 * 256);
+  p.smem = p.runner == kRunTable ? hot_bytes(fwd->hot.n) + 256 : p.runner == kRunGeneric ? smem_for(fwd->view) : 0;
+  p.walk = kWalkChunks[p.runner];
+  p.compact = kCompactSpans[p.runner];
+  p.sequential = kWalkSequential[p.runner];
+  if (pf) {
+    std::memcpy(&p.pf, pf_words_.data(), sizeof p.pf);
+    p.pf_scan = kLiteralScan[p.runner][p.pf.n_bytes - 1];
+  }
+  stats.path = p.path;
+  stats.fused = p.fused;
+  return p;
+}
+
+// ---- stitch: bring the speculative chunk walks into agreement with the sequential iterator (DESIGN.md §2) ----
+int Regex::stitch_chunks(WalkArgs* w, const std::function<int(const WalkArgs&, uint32_t)>& rewalk,
+                         const std::function<int(const WalkArgs&)>& sequential, ChainKey** grand_key) {
+  cudaStream_t st = (cudaStream_t)stream_;
+  const uint64_t nc = w->n_chunks, n_blocks = (nc + 1023) / 1024;
+  uint32_t* list = d_scalars_->list;
+  HostScalars* h = h_scalars_;
+  *grand_key = nullptr;
+  stats.stitch_rounds = stats.stitch_dirty_chunks = stats.sequential_passes = stats.long_runs = 0;
+  if (!has_looks && !can_match_empty) {
+    RB_CUDA(cudaMemsetAsync(list, 0, 16, st));
+    stitch_fast<<<grid_for(nc, 256, 8), 256, 0, st>>>(*w, list);
+    RB_LAUNCH_CHECK("stitch_fast");
+    RB_CUDA(cudaMemcpyAsync(h->list, list, 16, cudaMemcpyDeviceToHost, st));
+    RB_CUDA(cudaStreamSynchronize(st));
+    if (h->list[2] == 0) return 0;  // (a deferred chunk -- long run -- asks for the general loop too)
+  }
+  ChainKey* excl = (ChainKey*)excl_.ensure(nc * sizeof(ChainKey));
+  ChainKey* btot = (ChainKey*)btot_.ensure((n_blocks + 1) * sizeof(ChainKey));
+  if (!excl || !btot) return fail("out of device memory (stitch scratch)");
+  *grand_key = btot + n_blocks;
+  // *w over the dirty list, taken at each use so that it carries the long runs resolved so far
+  auto dirty = [&] { WalkArgs d = *w; d.dirty_list = (uint32_t*)dirty_.ptr; d.n_dirty = list; return d; };
+  for (uint32_t dirty_rounds = 0;;) {
+    RB_CUDA(cudaMemsetAsync(&d_scalars_->first_deferred, 0xFF, 4, st));
+    entries_local<<<(uint32_t)n_blocks, 1024, 0, st>>>(*w, excl, btot, &d_scalars_->first_deferred);
+    RB_LAUNCH_CHECK("entries_local");
+    entries_blocks<<<1, 1024, 0, st>>>(btot, n_blocks, *grand_key);
+    RB_LAUNCH_CHECK("entries_blocks");
+    RB_CUDA(cudaMemsetAsync(list, 0, 12, st));       // [0] chunks to walk again, [1] changed decisions
+    RB_CUDA(cudaMemsetAsync(list + 3, 0xFF, 4, st));  // [3] smallest chunk index to walk again
+    stitch_resolve<<<grid_for(nc, 256, 8), 256, 0, st>>>(dirty(), excl, btot, list);
+    RB_LAUNCH_CHECK("stitch_resolve");
+    RB_CUDA(cudaMemcpyAsync(h->list, list, sizeof h->list + sizeof h->long_req, cudaMemcpyDeviceToHost, st));  // list, long_req
+    RB_CUDA(cudaStreamSynchronize(st));
+    const uint32_t n_dirty = h->list[0], n_changed = h->list[1];
+    const uint64_t long_s = h->long_req;
+    bool serve = long_s != kNone;
+    if (serve) {
+      // the request of a chunk that this round found covered by an earlier match is dropped
+      uint32_t m = 0;
+      RB_CUDA(d2h(&m, w->meta + (long_s - w->base) / w->chunk, 4));
+      serve = (m >> 30) == kChunkDeferred;
+      if (!serve) RB_CUDA(cudaMemsetAsync(w->long_req, 0xFF, 8, st));
+    }
+    if (serve) {
+      // a chunk walked from its exact entry met a match longer than kExactRunCap: measure it in parallel,
+      // remember it, and let the stitch walk the deferred chunk again
+      if (w->n_long == kMaxLongRuns) return fail("more than 256 matches longer than 256 KiB in one search");
+      uint64_t e = kNone;
+      if (int rc = resolve_long_run(w->text, w->n, long_s, w->text_continues != 0, &e)) return rc;
+      const uint64_t pair[2] = {long_s, e};
+      RB_CUDA(cudaMemcpyAsync((uint64_t*)long_tab_.ptr + 2 * w->n_long, pair, 16, cudaMemcpyHostToDevice, st));
+      RB_CUDA(cudaMemsetAsync(w->long_req, 0xFF, 8, st));
+      RB_CUDA(cudaStreamSynchronize(st));
+      w->n_long++;
+      stats.long_runs++;
+    }
+    if (n_dirty == 0 && n_changed == 0 && !serve) return 0;
+    stats.stitch_rounds++;
+    stats.stitch_dirty_chunks += n_dirty;
+    if (n_dirty == 0) continue;
+    if (++dirty_rounds > tuning.max_stitch_rounds) {
+      // chains that do not meet again: one sequential pass from the leftmost such chunk
+      WalkArgs s = dirty();
+      s.seq_from = h->list[3];
+      if (int rc = sequential(s)) return rc;
+      stats.sequential_passes++;
+      dirty_rounds = 0;
+    } else if (int rc = rewalk(dirty(), n_dirty)) {
+      return rc;
+    }
+  }
+}
 
 int Regex::find_all_shard_device(const uint8_t* d_text, uint64_t n, ShardIO* io, uint64_t* d_out, uint64_t cap) {
   std::lock_guard<std::recursive_mutex> lock(mu_);
@@ -992,34 +1117,19 @@ int Regex::find_all_shard_device(const uint8_t* d_text, uint64_t n, ShardIO* io,
   if (is_set_) return fail("find requires exactly one pattern (RegexSet cannot be used with find, exec.rs:510-512)");
   if (io->own_hi > n || io->own_lo > io->own_hi || (io->own_lo & 255) || (!io->is_last && ((io->own_hi & 255) || io->own_hi == n)))
     return fail("bad shard geometry: own_lo/own_hi must be multiples of 256 inside the buffer (own_hi == n only for the last shard)");
-  DeviceDfa *fwd, *rev = nullptr;
+  DeviceDfa *fwd, *rev = nullptr, *revall = nullptr;
   if (int rc = ensure(kFwdAnchoredLF, &fwd)) return rc;
-  const bool emulate = has_looks;
-  if (emulate) if (int rc = ensure(kRevAnchoredLongest, &rev)) return rc;
+  if (has_looks) if (int rc = ensure(kRevAnchoredLongest, &rev)) return rc;
   // candidate-start mode: the start bitmap is a superset of the match starts (cand_bitmap), not the reverse scan's
-  const bool cand = candidate_mode();
-  DeviceDfa* revall = nullptr;
-  if (!cand) if (int rc = ensure(kRevUnanchoredAll, &revall)) return rc;
+  if (!candidate_mode()) if (int rc = ensure(kRevUnanchoredAll, &revall)) return rc;
   cudaStream_t st = (cudaStream_t)stream_;
   cudaEvent_t ev[3] = {(cudaEvent_t)timing_events_[0], (cudaEvent_t)timing_events_[1], (cudaEvent_t)timing_events_[2]};
   RB_CUDA(cudaEventRecord(ev[0], st));
-  const ScanPlan plan = plan_scan(d_text, io->own_lo, io->own_hi,
-                                   !cand && hot_signed_ok(revall->hot) && fast_scan_smem(hot_bytes_signed(revall->hot)) <= 227 * 1024);
-  // runner: 2 = fixed-length (no haystack access: every candidate must be a match start, so not with candidate
-  // starts), 1 = byte-indexed shared-memory table (uniform start state, 8-byte aligned text), 0 = generic
-  const bool wfixed = min_len == max_len && min_len > 0 && !emulate && !tuning.force_generic && !cand;
-  const bool wfast = !wfixed && fwd->hot.n != 0 && fwd->view.uniform_start && ((uintptr_t)d_text & 15) == 0 && !tuning.force_generic;
-  const int wkind = wfixed ? 2 : wfast ? 1 : 0;
-  // literal prefilter: no start bitmap at all -- literal_scan finds, verifies and chains the candidates
-  const bool use_pf = tuning.prefilter && !tuning.force_generic && ((uintptr_t)d_text & 15) == 0 && plan_prefilter() &&
-                      (tuning.prefilter >= 2 || pf_freq_ <= kPrefilterAutoFreq);
-  PfArgs pf{};
-  if (use_pf) std::memcpy(&pf, pf_words_.data(), sizeof pf);
-  const bool pf_fast = use_pf && fwd->hot.n != 0 && fwd->view.uniform_start;
-  // fused: every lane of the fast scan kernel also walks its own segment (chunk == segment)
-  const bool fused = !use_pf && !cand && plan.fast && wkind != 0 && tuning.fuse && !io->reuse_scan &&
-                     fast_scan_smem(hot_bytes_signed(revall->hot) + (wkind == 1 ? hot_bytes(fwd->hot.n) : 0)) <= 227 * 1024;
-
+  const WalkPlan plan = plan_walk(d_text, *io, fwd, revall);
+  const bool pf = plan.path == kPathPrefilter;
+  // literal_scan also has ~9 KB of static shared memory: opt in whenever the sum could pass 48 KB
+  if (pf) RB_CUDA(allow_smem(plan.pf_scan, plan.smem, 48 * 1024));
+  else for (WalkKernel k : {plan.walk, plan.compact, plan.sequential}) RB_CUDA(allow_smem(k, plan.smem));
   WalkArgs w{};
   w.fwd = fwd->view;
   if (rev) w.rev = rev->view;
@@ -1032,7 +1142,7 @@ int Regex::find_all_shard_device(const uint8_t* d_text, uint64_t n, ShardIO* io,
   w.base = io->own_lo;
   w.limit = io->own_hi;
   w.text_continues = !io->is_last;
-  w.chunk = use_pf ? 8192 : fused ? plan.seg : std::max<uint32_t>(256, (tuning.chunk + 255) / 256 * 256);
+  w.chunk = plan.chunk;
   w.stage_cap = std::max<uint32_t>(4, w.chunk / 64);
   w.n_chunks = std::max<uint64_t>(1, (w.limit - w.base + w.chunk - 1) / w.chunk);
   const uint64_t nc = w.n_chunks;
@@ -1042,191 +1152,86 @@ int Regex::find_all_shard_device(const uint8_t* d_text, uint64_t n, ShardIO* io,
   w.out_lm = (uint64_t*)out_lm_.ensure(nc * 8);
   w.count = (uint64_t*)count_.ensure(nc * 8);
   uint64_t* offset = (uint64_t*)offset_.ensure(nc * 8);
-  uint32_t* dirty_list = (uint32_t*)dirty_.ensure(nc * 4);
+  const void* dirty_list = dirty_.ensure(nc * 4);  // stitch_chunks
   w.first_cand = (uint64_t*)first_cand_.ensure(nc * 8);
   w.skip = (uint32_t*)skip_.ensure(nc * 4);
   w.meta = (uint32_t*)meta_.ensure(nc * 4);
   w.stage = (uint64_t*)stage_.ensure(nc * (uint64_t)w.stage_cap * 16);
-  const uint64_t n_blocks = (nc + 1023) / 1024;
   if (!w.in_p || !w.in_lm || !w.out_p || !w.out_lm || !w.count || !offset || !dirty_list || !w.first_cand || !w.skip || !w.meta || !w.stage)
     return fail("out of device memory (walk scratch)");
   w.offset = offset;
   w.out = d_out;
   w.cap = d_out ? cap : 0;
   w.utf8 = only_utf8;
-  w.emulate_slice = emulate;
+  w.emulate_slice = has_looks;
   w.can_match_empty = can_match_empty;
-  // entry states: chunk 0 starts the real chain at `start`; the rest speculate.
+  w.use_smem = plan.runner == kRunGeneric && plan.smem != 0;
+  if (plan.runner == kRunTable) w.fwd_hot = fwd->hot;
+  if (plan.runner == kRunFixed) w.fixed_len = min_len;
   w.err_flag = &ds->err_flag;
   w.floor_flag = &ds->floor_flag;
   // long anchored runs go to resolve_long_run (automata of up to 128 states), requested in long_req
-  const bool can_resolve = fwd->view.n_states <= 128;
-  uint64_t* long_tab = (uint64_t*)long_tab_.ensure(kMaxLongRuns * 16);
-  if (!long_tab) return fail("out of device memory (long runs)");
-  uint32_t n_long = 0;
-  w.exact_cap = can_resolve ? kExactRunCap : kNone;
-  w.long_tab = long_tab;
-  w.n_long = 0;
+  w.long_tab = (const uint64_t*)long_tab_.ensure(kMaxLongRuns * 16);
+  if (!w.long_tab) return fail("out of device memory (long runs)");
+  w.exact_cap = fwd->view.n_states <= 128 ? kExactRunCap : kNone;
   w.long_req = &ds->long_req;
   RB_CUDA(cudaMemsetAsync(w.long_req, 0xFF, 8, st));
   w.clamp_p = io->chain_clamped ? io->chain_p : kNone;
   RB_CUDA(cudaMemsetAsync(w.err_flag, 0, 8, st));  // err_flag, floor_flag
+  // entry states: chunk 0 starts the real chain at `start`; the rest speculate.
   init_walk_entries<<<grid_for(nc, 256, 8), 256, 0, st>>>(w.in_p, w.in_lm, w.skip, nc, io->chain_p, io->chain_lm);
   RB_LAUNCH_CHECK("init_walk_entries");
-  size_t wsmem = 0;
-  if (wfixed) {
-    w.fixed_len = min_len;
-  } else if (wfast) {
-    wsmem = hot_bytes(fwd->hot.n) + 256;
-    w.fwd_hot = fwd->hot;
-  } else {
-    wsmem = smem_for(fwd->view);
-    w.use_smem = wsmem != 0;
-  }
-  if (use_pf) {  // the prefilter's verifier: table runner (shared-memory hot table) or generic
-    w.fixed_len = 0;
-    if (pf_fast) {
-      wsmem = hot_bytes(fwd->hot.n) + 256;
-      w.fwd_hot = fwd->hot;
-    } else {
-      wsmem = smem_for(fwd->view);
-      w.use_smem = wsmem != 0;
-    }
-  }
-  const WalkKernel walk = kWalkChunks[wkind], compact = kCompactSpans[wkind], sequential = kWalkSequential[wkind];
-  const PfKernel pf_scan = use_pf ? kLiteralScan[pf_fast][pf.n_bytes - 1] : nullptr;
-  if (use_pf) {
-    // the kernel also has ~9 KB of static shared memory: opt in whenever the sum could pass 48 KB
-    RB_CUDA(allow_smem(pf_scan, wsmem, 48 * 1024));
-  } else {
-    RB_CUDA(allow_smem(walk, wsmem));
-    RB_CUDA(allow_smem(compact, wsmem));
-    RB_CUDA(allow_smem(sequential, wsmem));
-  }
-  auto launch_pf = [&](const WalkArgs& args, uint64_t chunks, int mode) {
-    const uint32_t g = mode == 2 ? 1 : grid_for(chunks * 32, 256, 3);  // one warp per chunk
-    pf_scan<<<g, 256, wsmem, st>>>(args, pf, mode);
+  auto launch_pf = [&](const WalkArgs& args, uint64_t chunks, int mode) {  // one warp per chunk
+    plan.pf_scan<<<mode == 2 ? 1 : grid_for(chunks * 32, 256, 3), 256, plan.smem, st>>>(args, plan.pf, mode);
   };
-  auto launch_walk = [&](const WalkArgs& args, uint64_t work) {
-    if (use_pf) launch_pf(args, work, 1);
-    else walk<<<grid_for(work, 256, 6), 256, wsmem, st>>>(args);
-  };
-  if (use_pf || cand) {
-    if (use_pf) {
+  if (plan.path < kPathPrefilter) {
+    if (int rc = scan_starts(d_text, n, io->own_lo, io->own_hi, io, plan.scan, plan.fused ? &w : nullptr)) return rc;
+  } else {
+    if (pf) {
       launch_pf(w, nc, 0);
       RB_LAUNCH_CHECK("literal_scan");
-    } else {
-      if (int rc = cand_starts(d_text, n, io->own_lo, io->own_hi, !io->is_last)) return rc;
+    } else if (int rc = cand_starts(d_text, n, io->own_lo, io->own_hi, !io->is_last)) {
+      return rc;
     }
     io->rev_guess = io->rev_entry != kNoState ? io->rev_entry : kPrefilterState;  // no reverse scan, nothing to guess
     io->rev_left = kPrefilterState;
     stats.scan_redo_rounds = stats.scan_redo_segments = stats.map_passes = 0;
-    RB_CUDA(cudaEventRecord(ev[1], st));
-    if (!use_pf) {
-      launch_walk(w, nc);
-      RB_LAUNCH_CHECK("walk_chunks");
-    }
-  } else {
-    if (int rc = scan_starts(d_text, n, io->own_lo, io->own_hi, io, plan, fused ? &w : nullptr)) return rc;
-    RB_CUDA(cudaEventRecord(ev[1], st));
-    if (!fused) {
-      launch_walk(w, nc);
-      RB_LAUNCH_CHECK("walk_chunks");
-    }
   }
-  // ---- stitch: bring the speculative chunk walks into agreement with the sequential iterator ----
-  stats.stitch_rounds = stats.stitch_dirty_chunks = stats.sequential_passes = stats.long_runs = 0;
-  const bool strict = emulate || can_match_empty;
-  bool general = strict;
-  uint32_t* list = ds->list;
-  HostScalars* h = h_scalars_;
-  if (!strict) {
-    RB_CUDA(cudaMemsetAsync(list, 0, 16, st));
-    stitch_fast<<<grid_for(nc, 256, 8), 256, 0, st>>>(w, list);
-    RB_LAUNCH_CHECK("stitch_fast");
-    RB_CUDA(cudaMemcpyAsync(h->list, list, 16, cudaMemcpyDeviceToHost, st));
-    RB_CUDA(cudaStreamSynchronize(st));
-    general = h->list[2] != 0;  // (a deferred chunk -- long run -- asks for the general loop too)
+  RB_CUDA(cudaEventRecord(ev[1], st));
+  if (!pf && !plan.fused) {
+    plan.walk<<<grid_for(nc, 256, 6), 256, plan.smem, st>>>(w);
+    RB_LAUNCH_CHECK("walk_chunks");
   }
-  ChainKey* grand_key = nullptr;
-  if (general) {
-    ChainKey* excl = (ChainKey*)excl_.ensure(nc * sizeof(ChainKey));
-    ChainKey* btot = (ChainKey*)btot_.ensure((n_blocks + 1) * sizeof(ChainKey));
-    if (!excl || !btot) return fail("out of device memory (stitch scratch)");
-    grand_key = btot + n_blocks;
-    WalkArgs wd = w;
-    wd.dirty_list = dirty_list;
-    wd.n_dirty = list;
-    uint32_t dirty_rounds = 0;
-    for (;;) {
-      RB_CUDA(cudaMemsetAsync(&ds->first_deferred, 0xFF, 4, st));
-      entries_local<<<(uint32_t)n_blocks, 1024, 0, st>>>(w, excl, btot, &ds->first_deferred);
-      RB_LAUNCH_CHECK("entries_local");
-      entries_blocks<<<1, 1024, 0, st>>>(btot, n_blocks, grand_key);
-      RB_LAUNCH_CHECK("entries_blocks");
-      RB_CUDA(cudaMemsetAsync(list, 0, 12, st));       // [0] chunks to walk again, [1] changed decisions
-      RB_CUDA(cudaMemsetAsync(list + 3, 0xFF, 4, st));  // [3] smallest chunk index to walk again
-      stitch_resolve<<<grid_for(nc, 256, 8), 256, 0, st>>>(wd, excl, btot, list);
-      RB_LAUNCH_CHECK("stitch_resolve");
-      RB_CUDA(cudaMemcpyAsync(h->list, list, sizeof h->list + sizeof h->long_req, cudaMemcpyDeviceToHost, st));  // list, long_req
-      RB_CUDA(cudaStreamSynchronize(st));
-      const uint32_t n_dirty = h->list[0], n_changed = h->list[1];
-      const uint64_t long_s = h->long_req;
-      bool serve = long_s != kNone;
-      if (serve) {
-        // the request of a chunk that this round found covered by an earlier match is dropped
-        uint32_t m = 0;
-        RB_CUDA(d2h(&m, w.meta + (long_s - w.base) / w.chunk, 4));
-        serve = (m >> 30) == kChunkDeferred;
-        if (!serve) RB_CUDA(cudaMemsetAsync(w.long_req, 0xFF, 8, st));
-      }
-      if (serve) {
-        // a chunk walked from its exact entry met a match longer than kExactRunCap: measure it in parallel,
-        // remember it, and let the stitch walk the deferred chunk again
-        if (n_long == kMaxLongRuns) return fail("more than 256 matches longer than 256 KiB in one search");
-        uint64_t e = kNone;
-        if (int rc = resolve_long_run(d_text, n, long_s, !io->is_last, &e)) return rc;
-        const uint64_t pair[2] = {long_s, e};
-        RB_CUDA(cudaMemcpyAsync(long_tab + 2 * n_long, pair, 16, cudaMemcpyHostToDevice, st));
-        RB_CUDA(cudaMemsetAsync(w.long_req, 0xFF, 8, st));
-        RB_CUDA(cudaStreamSynchronize(st));
-        n_long++;
-        w.n_long = wd.n_long = n_long;
-        stats.long_runs++;
-      }
-      if (n_dirty == 0 && n_changed == 0 && !serve) break;
-      stats.stitch_rounds++;
-      stats.stitch_dirty_chunks += n_dirty;
-      if (n_dirty == 0) continue;
-      if (++dirty_rounds > tuning.max_stitch_rounds) {
-        // chains that do not meet again: one sequential pass from the leftmost such chunk
-        wd.seq_from = h->list[3];
-        if (use_pf) launch_pf(wd, 1, 2);
-        else sequential<<<1, 256, wsmem, st>>>(wd);
-        RB_LAUNCH_CHECK("walk_sequential");
-        stats.sequential_passes++;
-        dirty_rounds = 0;
-      } else {
-        launch_walk(wd, n_dirty);
-        RB_LAUNCH_CHECK("walk_chunks(dirty)");
-      }
-    }
-  }
+  auto rewalk = [&](const WalkArgs& args, uint32_t n_dirty) {
+    if (pf) launch_pf(args, n_dirty, 1);
+    else plan.walk<<<grid_for(n_dirty, 256, 6), 256, plan.smem, st>>>(args);
+    RB_LAUNCH_CHECK("walk_chunks(dirty)");
+    return 0;
+  };
+  auto sequential = [&](const WalkArgs& args) {
+    if (pf) launch_pf(args, 1, 2);
+    else plan.sequential<<<1, 256, plan.smem, st>>>(args);
+    RB_LAUNCH_CHECK("walk_sequential");
+    return 0;
+  };
+  ChainKey* grand_key;
+  if (int rc = stitch_chunks(&w, rewalk, sequential, &grand_key)) return rc;
   unsigned long long* grand;
   if (int rc = prefix_sum(w.count, offset, nc, &grand)) return rc;
-  if (w.cap > 0 && use_pf) {
+  if (w.cap > 0 && pf) {
     compact_staged<<<grid_for(nc, 256, 6), 256, 0, st>>>(w);
     RB_LAUNCH_CHECK("compact_staged");
     launch_pf(w, nc, 3);  // chunks with more matches than staging slots: straight into the output
     RB_LAUNCH_CHECK("literal_scan(overflow)");
   } else if (w.cap > 0) {
-    compact<<<grid_for(nc, 256, 6), 256, wsmem, st>>>(w);
+    plan.compact<<<grid_for(nc, 256, 6), 256, plan.smem, st>>>(w);
     RB_LAUNCH_CHECK("compact_spans");
   }
+  HostScalars* h = h_scalars_;
   RB_CUDA(cudaMemcpyAsync(&h->n_matches, grand, 8, cudaMemcpyDeviceToHost, st));
   if (grand_key) {  // exit state = the last contribution of the whole range
     RB_CUDA(cudaMemcpyAsync(h->exit, grand_key, 16, cudaMemcpyDeviceToHost, st));
-  } else {
+  } else {  // the last chunk's exit
     RB_CUDA(cudaMemcpyAsync(&h->exit[0], w.out_p + (nc - 1), 8, cudaMemcpyDeviceToHost, st));
     RB_CUDA(cudaMemcpyAsync(&h->exit[1], w.out_lm + (nc - 1), 8, cudaMemcpyDeviceToHost, st));
   }
@@ -1234,18 +1239,12 @@ int Regex::find_all_shard_device(const uint8_t* d_text, uint64_t n, ShardIO* io,
   RB_CUDA(cudaEventRecord(ev[2], st));
   RB_CUDA(cudaStreamSynchronize(st));
   io->n_matches = h->n_matches;
+  // ChainKey: p + 1; 0 = nothing in this range moved the iterator (speculative shard without candidates), ~0 = the end
   const uint64_t* x = h->exit;
-  if (grand_key) {  // ChainKey: 0 = nothing in this range moved the iterator (speculative shard without candidates)
-    io->exit_p = x[0] == 0 ? kSpec : (x[0] == ~0ull ? kNone : x[0] - 1);
-    io->exit_lm = x[0] == 0 ? kNone : x[1];
-  } else {
-    io->exit_p = x[0];
-    io->exit_lm = x[1];
-  }
+  io->exit_p = !grand_key ? x[0] : x[0] == 0 ? kSpec : x[0] == kNone ? kNone : x[0] - 1;
+  io->exit_lm = grand_key && x[0] == 0 ? kNone : x[1];
   io->halo_overflow = h->err_flag != 0;
   io->left_ctx_short = h->floor_flag != 0;
-  stats.fused = fused;
-  stats.path = use_pf ? 3 : cand ? 4 : fused ? 2 : plan.fast ? 1 : 0;
   cudaEventElapsedTime(&stats.scan_ms, ev[0], ev[1]);
   cudaEventElapsedTime(&stats.walk_ms, ev[1], ev[2]);
   cudaEventElapsedTime(&stats.total_ms, ev[0], ev[2]);
@@ -1288,7 +1287,7 @@ int Regex::forward_range(const uint8_t* d_text, uint64_t n, uint64_t start, uint
   // patterns of a match by redoing that 64-byte group on the full table
   const bool fast_ok = (!want_masks || sparse_set_) && fwd->hot.n != 0 && !tuning.force_generic && tuning.tensor_tma && encode_tiled() &&
                        ((uintptr_t)d_text & 15) == 0 && (start & 63) == 0 &&
-                       fast_scan_smem(hot_bytes(fwd->hot.n)) <= 227 * 1024;
+                       fast_scan_smem(hot_bytes(fwd->hot.n)) <= kMaxDynamicSmem;
   const uint32_t seg = tuning.seg ? tuning.seg : (fast_ok ? 4096 : 1024);
   const uint64_t n_seg = (limit - start + seg - 1) / seg;
   if (n_seg >= 0xFFFFFFFFull) return fail("haystack too large for one scan (segment index overflow)");
@@ -2671,7 +2670,7 @@ int Regex::find_at_host(const uint8_t* text, uint64_t n, uint64_t start, bool* f
   cudaStream_t st = (cudaStream_t)stream_;
   const uint64_t buf_lo = start > 256 ? (start - 256) & ~255ull : 0;  // 256 bytes of left context for look-behind
   uint64_t resident = buf_lo;                                         // bytes [buf_lo, resident) are on the device
-  uint64_t own_lo = start ? ((start - 1) & ~255ull) : 0;              // bit i <-> position i + 1
+  uint64_t own_lo = shard_own_lo(start);
   uint64_t win = 64 << 10, halo = 64 << 10;
   uint64_t p = start, lm = kNone;
   for (;;) {

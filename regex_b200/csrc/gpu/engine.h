@@ -19,6 +19,8 @@ namespace rbgpu {
 
 struct BatchArgs;      // launch.h
 struct ScanArgs;       // launch.h
+struct WalkArgs;       // launch.h
+struct ChainKey;       // launch.h
 struct DeviceScalars;  // engine.cu
 struct HostScalars;    // engine.cu
 
@@ -222,6 +224,10 @@ class Regex {
   int check(int cuda_err, const char* what);
   struct ScanPlan { bool fast = false; uint32_t seg = 0, warm = 0; uint64_t n_seg = 0; };
   ScanPlan plan_scan(const uint8_t* d_text, uint64_t base, uint64_t limit, bool fast_table);
+  // find_all_shard_device's path for one range (engine.cu): the start bitmap's scan plan, the path stats.path reports,
+  // the chain walk's runner, chunk size, shared memory and kernels.  Also sets stats.path and stats.fused.
+  struct WalkPlan;
+  WalkPlan plan_walk(const uint8_t* d_text, const ShardIO& io, const DeviceDfa* fwd, const DeviceDfa* revall);
   int scan_starts(const uint8_t* d_text, uint64_t n, uint64_t base, uint64_t limit, ShardIO* io, const ScanPlan& plan,
                   const void* fused_walk);
   // Verify every segment's entry guess against its neighbour's exit (a.guess / a.fin, list in redo_) until none is
@@ -233,6 +239,13 @@ class Regex {
   // in scan direction entered in the state at d_entry (device).
   int compose_entries(const ScanArgs& g, bool reverse, const uint16_t* d_entry);
   int resolve_long_run(const uint8_t* d_text, uint64_t n, uint64_t s, bool text_continues, uint64_t* e_out);
+  // Bring the speculative chunk walks of *w into agreement with the sequential iterator (DESIGN.md §2): stitch_fast
+  // when no match can be empty or look around, then general rounds until nothing changes.  rewalk(args, n) walks the
+  // n chunks of args' dirty list again; after max_stitch_rounds rounds with re-walks, sequential(args) walks once from
+  // args.seq_from.  Long runs a round requests are measured (resolve_long_run) and added to w->long_tab.
+  // *grand_key: the general stitch's key of the whole range (device), null when it did not run.
+  int stitch_chunks(WalkArgs* w, const std::function<int(const WalkArgs&, uint32_t)>& rewalk,
+                    const std::function<int(const WalkArgs&)>& sequential, ChainKey** grand_key);
   int all_spans_device(const uint8_t* d_text, uint64_t n, uint64_t** d_spans, uint64_t* m);
   int ensure_capture_program();
   int launch_captures(const uint8_t* d_text, uint64_t n, const uint64_t* d_spans, uint64_t m, uint64_t* d_slots,
@@ -320,8 +333,8 @@ class Regex {
   DeviceBuf bitmap_, guess_, fin_, redo_, seg_first_, seg_mask_;
   // state-map composition (solve_entries, compose_entries, resolve_long_run)
   DeviceBuf present_, kidx_, kstates_, maps_, comp_, bentry_, exact_;
-  // chunk walk and stitch (find_all_shard_device): chain entries and exits, match counts and offsets, dirty list,
-  // staged spans, stitch keys, resolved long runs
+  // chunk walk and stitch (find_all_shard_device, stitch_chunks): chain entries and exits, match counts and offsets,
+  // dirty list, staged spans, stitch keys, resolved long runs
   DeviceBuf in_p_, in_lm_, out_p_, out_lm_, count_, offset_, dirty_, first_cand_, skip_, meta_, stage_, excl_, btot_, long_tab_;
   static constexpr uint32_t kMaxLongRuns = 256;
   DeviceBuf block_sums_;  // prefix_sum (any caller)
