@@ -13,6 +13,8 @@
  *   rure_b200_replace_batch   == rure_b200_replace(re, hay + off[i], off[i+1]-off[i], rep, ..., limit, ...) per record
  *   rure_b200_split_batch     == rure_b200_split(re, hay + off[i], off[i+1]-off[i], has_limit, limit, ...) per record
  *   rure_b200_captures_iter_batch == rure_b200_captures_all(re, hay + off[i], off[i+1]-off[i], ...) per record
+ *   rure_b200_stream_*        == rure_b200_find_all on the concatenation of every rure_b200_stream_write
+ *                                (spans as offsets into that concatenation; it need never exist in memory)
  * Functions return true on success; on failure rure_b200_last_error() (thread
  * local) describes what went wrong.  A missing GPU is a failure, never a
  * silent CPU fallback.
@@ -58,7 +60,9 @@ bool rure_b200_set_is_match(rure_set *set, const uint8_t *haystack, size_t lengt
 /* Host haystack.  Large haystacks (>= 128 MiB) are uploaded in 64 MiB pieces and each piece
  * is searched while later pieces are still in flight, spans travelling back meanwhile; the
  * result is identical to uploading first (environment RB200_PIPELINE_PIECE=<bytes> changes
- * the piece size, 0 turns the pipeline off).  Pinned host memory gives the full PCIe rate. */
+ * the piece size, 0 turns the pipeline off).  Pinned host memory gives the full PCIe rate.
+ * A haystack that, with its bitmap and spans, cannot be allocated on the device is searched
+ * through a stream window instead (see streams below; hold 256 MiB). */
 bool rure_b200_find_all(rure *re, const uint8_t *haystack, size_t length, rure_match *out,
                         size_t cap, size_t *n_total);
 bool rure_b200_count_all(rure *re, const uint8_t *haystack, size_t length, size_t *n_total);
@@ -227,15 +231,41 @@ bool rure_b200_shortest_match_shard_device(rure *re, const uint8_t *d_buffer, si
 bool rure_b200_set_matches_shard_device(rure_set *set, const uint8_t *d_buffer, size_t n_buffer,
                                         rure_b200_fwd_shard *io);
 
+/* ---- streams: find_iter over text fed in pieces --------------------------------
+ * For text that arrives in blocks (a file read with fread, a pipe, a log tail) or that is larger
+ * than device memory.  The stream keeps a bounded device window: 256 bytes of left context, the
+ * searched pieces whose spans are not final yet (at most four), and the bytes that arrived after
+ * them (about 5 * piece + hold + 16 MiB in all).  A piece's spans become final once the pieces
+ * after it have been searched and agree with it at their common edge (DESIGN.md section 8).
+ * rure_b200_stream_new: piece = bytes per searched piece, a multiple of 256 (0 = 64 MiB); hold =
+ * longest match always resolved (0 = piece) -- a longer match may fail the stream with "a match
+ * is longer than the stream window (... bytes)"; spans = 0 counts matches only.  NULL on failure.
+ * A rure compiled with rure_b200_compile_str may be streamed; a UTF-8 scalar may be split across
+ * writes.  rure_b200_stream_write copies `data` (any len, 0 too) and may block while pieces are
+ * searched; host memory from cudaMallocHost is uploaded without the extra copy.
+ * rure_b200_stream_finish ends the text and settles every remaining piece.
+ * rure_b200_stream_read pops up to cap final spans (offsets into the whole text), *n = popped.
+ * rure_b200_stream_count: final matches so far (read or not).  After a failure (see
+ * rure_b200_last_error) or after finish, writes fail.  Out of scope: forward searches (is_match,
+ * shortest_match, set matches), rure_find, replace, split and captures on such text. */
+typedef struct rure_b200_stream rure_b200_stream;
+rure_b200_stream *rure_b200_stream_new(rure *re, size_t piece, size_t hold, int spans);
+bool rure_b200_stream_write(rure_b200_stream *s, const uint8_t *data, size_t len);
+bool rure_b200_stream_finish(rure_b200_stream *s);
+bool rure_b200_stream_read(rure_b200_stream *s, rure_match *out, size_t cap, size_t *n);
+uint64_t rure_b200_stream_count(rure_b200_stream *s);
+void rure_b200_stream_free(rure_b200_stream *s);
+
 /* ---- threads ----------------------------------------------------------------
  * As in rure.h (regex-capi/include/rure.h:27-34) one compiled rure / rure_set may be used from
  * several threads at once.  The scalar entry points (rure_is_match, rure_find, rure_shortest_match,
  * rure_find_captures, rure_set_is_match, rure_set_matches and their rure_b200_* twins with an error
  * return) run concurrently: the engine keeps its device scratch per object, so a call that finds the
  * object busy runs on a clone compiled from the same source, kept with the handle.  The bulk,
- * device-pointer and shard entry points use the handle's primary engine and serialise; give every
- * thread (or shard) its own handle for those.  rure_b200_last_stats* and the options describe the
- * primary engine. */
+ * device-pointer, shard and stream entry points use the handle's primary engine and serialise
+ * (each stream call holds it while it searches); give every thread (or shard) its own handle for
+ * those.  One stream object must not be used from two threads at once.  rure_b200_last_stats* and
+ * the options describe the primary engine. */
 /* ---- diagnostics ----------------------------------------------------------- */
 const char *rure_b200_last_error(void);
 /* kernels launched by this library in this process (bench.py "gpu_launches") */
@@ -258,7 +288,10 @@ void rure_b200_set_last_stats_ex(rure_set *set, double *out, size_t n);
  * set matches (x16 per wave, 0 = one wave), "narrow_sets" 0/1, "max_stitch_rounds",
  * "max_redo_rounds", "batch_refill" 0/1 (batched is_match: lanes refill from a task of records), "prefilter" (0 never, 1 automatic: only for a single rare byte, 2 whenever the
  * pattern qualifies), "candidate_starts" 0/1 (tests: search from candidate starts with the anchored
- * automaton, as patterns over the DFA budget do, even when the unanchored automata fit).
+ * automaton, as patterns over the DFA budget do, even when the unanchored automata fit),
+ * "host_window" bytes (tests: rure_b200_find_all, rure_b200_count_all and rure_iter_next search
+ * host haystacks longer than this through a stream window of about this size; 0, the default,
+ * = only haystacks whose buffers cannot be allocated on the device).
  * Returns false for an unknown name.
  * Sets also take "set_group_patterns" k (tests): search in groups of at most k patterns even when
  * the product automaton fits, each group split further while its automaton is over the budget;

@@ -102,6 +102,12 @@ def _load():
         "rure_b200_find_all": (c_bool, [vp, u8p, sz, vp, sz, POINTER(sz)]),
         "rure_b200_count_all": (c_bool, [vp, u8p, sz, POINTER(sz)]),
         "rure_b200_set_matches_mask": (c_bool, [vp, u8p, sz, sz, POINTER(c_uint64)]),
+        "rure_b200_stream_new": (vp, [vp, sz, sz, c_int]),
+        "rure_b200_stream_write": (c_bool, [vp, u8p, sz]),
+        "rure_b200_stream_finish": (c_bool, [vp]),
+        "rure_b200_stream_read": (c_bool, [vp, vp, sz, POINTER(sz)]),
+        "rure_b200_stream_count": (c_uint64, [vp]),
+        "rure_b200_stream_free": (None, [vp]),
         "rure_b200_is_match_batch": (c_bool, [vp, u8p, vp, sz, vp]),
         "rure_b200_find_batch": (c_bool, [vp, u8p, vp, sz, vp, vp]),
         "rure_b200_set_matches_batch": (c_bool, [vp, u8p, vp, sz, vp]),
@@ -186,6 +192,59 @@ def _buf(data):
     if hasattr(data, "data_ptr"):  # pinned / CPU torch tensor
         return data.data_ptr(), data.numel() * data.element_size(), data
     raise TypeError(f"unsupported haystack type {type(data)!r}")
+
+
+class RegexStream:
+    """A find_iter stream (Regex.stream).  Usable as a context manager, which frees it on exit."""
+
+    def __init__(self, regex, piece=0, hold=0, spans=True):
+        self._re = regex  # keeps the compiled regex alive while the stream uses its engine
+        self._h = _lib.rure_b200_stream_new(regex._h, piece, hold, int(bool(spans)))
+        if not self._h:
+            raise Error(_last_error())
+        self._popped = 0
+
+    def write(self, data):
+        """Append bytes (bytes, bytearray, memoryview, uint8 numpy array or CPU tensor)."""
+        if isinstance(data, memoryview) and data.contiguous:
+            data = np.frombuffer(data, dtype=np.uint8)
+        p, n, keep = _buf(data)
+        if not _lib.rure_b200_stream_write(self._h, p, n):
+            raise Error(_last_error())
+
+    def finish(self):
+        """End of text: every remaining span becomes final."""
+        if not _lib.rure_b200_stream_finish(self._h):
+            raise Error(_last_error())
+
+    @property
+    def count(self):
+        """Final matches so far, read or not."""
+        return int(_lib.rure_b200_stream_count(self._h))
+
+    def read(self):
+        """The final spans not read yet, as a (k, 2) uint64 array of offsets into the whole text."""
+        k = self.count - self._popped
+        out = np.empty((max(k, 1), 2), dtype=np.uint64)
+        got = c_size_t()
+        _lib.rure_b200_stream_read(self._h, out.ctypes.data, k, byref(got))
+        self._popped += got.value
+        return out[: got.value]
+
+    def close(self):
+        if self._h:
+            _lib.rure_b200_stream_free(self._h)
+            self._h = None
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+    def __del__(self):
+        if _lib is not None:
+            self.close()
 
 
 class RegexBuilder:
@@ -391,6 +450,11 @@ class _Compiled:
         if not _lib.rure_b200_count_all(self._h, p, n, byref(total)):
             raise Error(_last_error())
         return total.value
+
+    def stream(self, piece=0, hold=0, spans=True):
+        """find_iter over text fed in pieces (include/rure_b200.h: streams): write() the text in any
+        blocks, finish(), and read() the spans, which equal find_all on the concatenation."""
+        return RegexStream(self, piece, hold, spans)
 
     def is_match_batch(self, text, offsets):
         """bool array, one per record text[offsets[i]:offsets[i+1]]."""

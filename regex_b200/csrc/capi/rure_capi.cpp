@@ -375,6 +375,35 @@ bool rure_b200_find_all(rure* re, const uint8_t* haystack, size_t length, rure_m
 bool rure_b200_count_all(rure* re, const uint8_t* haystack, size_t length, size_t* n_total) {
   return rure_b200_find_all(re, haystack, length, nullptr, 0, n_total);
 }
+
+// ------------------------------------------------------------------- streams --
+struct rure_b200_stream {
+  rbgpu::Stream* s;
+  ~rure_b200_stream() { delete s; }
+};
+static bool stream_ok(rure_b200_stream* s, int rc) {
+  if (rc == 0) return true;
+  g_last_error = s->s->error();
+  return false;
+}
+rure_b200_stream* rure_b200_stream_new(rure* re, size_t piece, size_t hold, int spans) {
+  std::string err;
+  rbgpu::Stream* s = rbgpu::Stream::create(re->re, piece, hold, spans != 0, 0, &err);
+  if (!s) {
+    g_last_error = err;
+    return nullptr;
+  }
+  return new rure_b200_stream{s};
+}
+bool rure_b200_stream_write(rure_b200_stream* s, const uint8_t* data, size_t len) { return stream_ok(s, s->s->write(data, len)); }
+bool rure_b200_stream_finish(rure_b200_stream* s) { return stream_ok(s, s->s->finish()); }
+bool rure_b200_stream_read(rure_b200_stream* s, rure_match* out, size_t cap, size_t* n) {
+  *n = s->s->read((uint64_t*)out, out ? cap : 0);
+  return true;
+}
+uint64_t rure_b200_stream_count(rure_b200_stream* s) { return s->s->count(); }
+void rure_b200_stream_free(rure_b200_stream* s) { delete s; }
+
 bool rure_b200_set_matches_mask(rure_set* s, const uint8_t* haystack, size_t length, size_t start, uint64_t* mask_words) {
   bool any;
   return ok(s->re, s->re->set_matches_host(haystack, length, start, &any, mask_words));
@@ -576,6 +605,7 @@ static bool set_option(Regex* r, const char* name, uint64_t value) {
   else if (k == "max_redo_rounds") t.max_redo_rounds = (uint32_t)value;
   else if (k == "prefilter") t.prefilter = (int)value;
   else if (k == "candidate_starts") t.candidate_starts = value != 0;
+  else if (k == "host_window") t.host_window = value;
   else { g_last_error = "unknown option: " + k; return false; }
   return true;
 }

@@ -933,9 +933,10 @@ int Regex::scan_starts(const uint8_t* d_text, uint64_t n, uint64_t base, uint64_
     RB_LAUNCH_CHECK("scan_rev(redo)");
     return 0;
   };
-  // A shard may be told the exact state at its top edge by its right neighbour.
+  // A shard may be told the exact state at its top edge by its right neighbour.  A range that starts inside the
+  // buffer reports its edge states too: a stream's last piece is checked against the piece before it.
   HostScalars* h = h_scalars_;
-  const bool shard = io && (!io->is_first || !io->is_last || io->rev_entry != kNoState || io->own_hi < n);
+  const bool shard = io && (!io->is_first || !io->is_last || io->rev_entry != kNoState || io->own_hi < n || io->own_lo > 0);
   if (shard) {
     RB_CUDA(cudaMemcpyAsync(&h->rev_guess, a.guess + (n_seg - 1), 2, cudaMemcpyDeviceToHost, st));
     RB_CUDA(cudaStreamSynchronize(st));
@@ -2624,6 +2625,8 @@ int Regex::find_all_host_pipelined(const uint8_t* text, uint64_t n, uint8_t* d, 
 int Regex::find_all_host(const uint8_t* text, uint64_t n, uint64_t start, uint64_t* out, uint64_t cap, uint64_t* total) {
   std::lock_guard<std::recursive_mutex> lock(mu_);
   int rc;
+  if ((rc = init_device())) return rc;
+  if (use_window(n, out ? cap : 0)) return find_all_window(text, n, start, out, cap, total);  // larger than the device
   if (start == 0 && n >= (8u << 20) && out && cap) {
     if ((rc = init_device())) return rc;
     uint8_t* dd = (uint8_t*)text_.ensure(n + 64);
@@ -2872,6 +2875,379 @@ int Regex::set_matches_batch_host(const uint8_t* text, const uint64_t* offsets, 
   if (!d_masks) return fail("out of device memory (batch)");
   if ((rc = set_matches_batch_device(d, d_off, n_rec, d_masks))) return rc;
   RB_CUDA(d2h(masks, d_masks, n_rec * 8 * mw));
+  return 0;
+}
+
+
+// ------------------------------------------------------------------- streams ----
+// A find_iter over text that arrives in pieces (DESIGN.md §8).  The stream's device window holds one contiguous
+// buffer: at least 256 bytes of left context, the searched pieces whose spans are not final yet (the pending pieces),
+// and every byte that arrived after them, which is the next piece and its halo.  Each search is one
+// find_all_shard_device call on that buffer.  A piece is final, and its spans leave, once a later piece reports at
+// its left edge the reverse-scan state its left neighbour assumed at its top; the pieces in between are made to
+// agree first (settle), each searched again from the exact state while it is still resident.
+static constexpr uint64_t kStreamPieceDefault = 64ull << 20;
+static constexpr uint64_t kStreamGranule = 8ull << 20;  // most bytes per upload (and per pinned staging buffer)
+
+Stream* Stream::create(Regex* re, uint64_t piece, uint64_t hold, bool spans, uint64_t start, std::string* err) {
+  std::lock_guard<std::recursive_mutex> lock(re->mu_);
+  std::unique_ptr<Stream> s(new Stream(re));
+  if (re->is_set_) {
+    *err = "find requires exactly one pattern (RegexSet cannot be used with find, exec.rs:510-512)";
+    return nullptr;
+  }
+  Regex::DeviceDfa* warm;  // picks the stream, creates the pinned scratch
+  if (re->init_device() || re->ensure(kFwdAnchoredLF, &warm) || re->side_streams()) {
+    *err = re->error_;
+    return nullptr;
+  }
+  s->piece_ = piece ? (piece + 255) & ~255ull : kStreamPieceDefault;
+  s->hold_ = hold ? (hold + 255) & ~255ull : s->piece_;
+  s->halo_ = std::min<uint64_t>(64 << 10, s->hold_);
+  s->granule_ = std::min(kStreamGranule, std::max<uint64_t>(256, s->piece_ / 2));
+  // left context + the pending pieces + the next piece + its longest halo + the uploads in flight
+  s->cap_ = 4096 + (kMaxPending + 1) * s->piece_ + s->hold_ + 2 * s->granule_;
+  s->spans_ = spans;
+  s->base_ = s->end_ = buf_lo(start);
+  s->next_lo_ = shard_own_lo(start);
+  s->chain_p_ = start;
+  s->chain_lm_ = kNone;
+  if (!s->win_.ensure(s->cap_ + 64)) {
+    *err = "out of device memory (stream window of " + std::to_string(s->cap_) + " bytes)";
+    return nullptr;
+  }
+  for (int k = 0; k < 2; k++) {
+    cudaEvent_t ev;
+    if (cudaMallocHost(&s->staging_[k], s->granule_) != cudaSuccess || cudaEventCreateWithFlags(&ev, cudaEventDisableTiming) != cudaSuccess) {
+      *err = "out of pinned host memory (stream staging)";
+      return nullptr;
+    }
+    s->staging_ev_[k] = ev;
+  }
+  cudaEvent_t ev;
+  if (cudaEventCreateWithFlags(&ev, cudaEventDisableTiming) != cudaSuccess) {
+    *err = "cannot create a CUDA event";
+    return nullptr;
+  }
+  s->moved_ev_ = ev;
+  return s.release();
+}
+
+Stream::~Stream() {
+  std::lock_guard<std::recursive_mutex> lock(re_->mu_);
+  if (re_->copy_stream_) cudaStreamSynchronize((cudaStream_t)re_->copy_stream_);
+  if (re_->stream_) cudaStreamSynchronize((cudaStream_t)re_->stream_);
+  for (int k = 0; k < 2; k++) {
+    if (staging_[k]) cudaFreeHost(staging_[k]);
+    if (staging_ev_[k]) cudaEventDestroy((cudaEvent_t)staging_ev_[k]);
+  }
+  for (auto& u : uploads_) cudaEventDestroy((cudaEvent_t)u.second);
+  for (void* e : free_events_) cudaEventDestroy((cudaEvent_t)e);
+  if (moved_ev_) cudaEventDestroy((cudaEvent_t)moved_ev_);
+}
+
+int Stream::fail(const std::string& msg) {
+  error_ = msg;
+  failed_ = true;
+  return -1;
+}
+int Stream::cuda(int e, const char* what) {
+  if (e == cudaSuccess) return 0;
+  return fail(std::string("CUDA error in ") + what + ": " + cudaGetErrorString((cudaError_t)e));
+}
+#define RB_STREAM_CUDA(call)                            \
+  do {                                                  \
+    int rc__ = cuda((int)(call), #call);                \
+    if (rc__) return rc__;                              \
+  } while (0)
+
+int Stream::write(const uint8_t* data, uint64_t len) {
+  std::lock_guard<std::recursive_mutex> lock(re_->mu_);
+  if (failed_) return -1;
+  if (finished_) return fail("write after finish: the stream's text has ended");
+  if (re_->init_device()) return fail(re_->error_);
+  cudaPointerAttributes attr;
+  const bool pinned = len && cudaPointerGetAttributes(&attr, data) == cudaSuccess && attr.type == cudaMemoryTypeHost;
+  cudaGetLastError();  // a pageable pointer is not an error
+  bool progressed;
+  while (len && !done_) {
+    const uint64_t want = std::min(len, granule_);
+    if (cap_ - (end_ - base_) < want) {
+      do {
+        if (int rc = step(&progressed)) return rc;
+      } while (progressed);
+      if (int rc = make_room(want)) return rc;
+    }
+    const uint64_t k = std::min(want, cap_ - (end_ - base_));
+    if (int rc = upload(data, k, pinned)) return rc;
+    data += k;
+    len -= k;
+  }
+  do {
+    if (int rc = step(&progressed)) return rc;
+  } while (progressed);
+  // the caller may reuse its buffer once write returns: uploads straight from it must have landed
+  if (pinned) RB_STREAM_CUDA(cudaStreamSynchronize((cudaStream_t)re_->copy_stream_));
+  return 0;
+}
+
+int Stream::finish() {
+  std::lock_guard<std::recursive_mutex> lock(re_->mu_);
+  if (failed_) return -1;
+  if (finished_) return 0;
+  if (re_->init_device()) return fail(re_->error_);
+  finished_ = true;
+  while (!done_) {
+    bool progressed;
+    if (int rc = step(&progressed)) return rc;
+    if (!progressed) return fail("internal error: the stream cannot settle its last piece");
+  }
+  RB_STREAM_CUDA(cudaStreamSynchronize((cudaStream_t)re_->stream_));  // spans copied to the sink
+  return 0;
+}
+
+uint64_t Stream::read(uint64_t* out, uint64_t cap) {
+  const uint64_t k = std::min(cap, (queue_.size() - queue_head_) / 2);
+  if (k) std::memcpy(out, queue_.data() + queue_head_, k * 16);
+  queue_head_ += 2 * k;
+  if (queue_head_ == queue_.size()) {
+    queue_.clear();
+    queue_head_ = 0;
+  } else if (queue_head_ > queue_.size() / 2) {
+    queue_.erase(queue_.begin(), queue_.begin() + queue_head_);
+    queue_head_ = 0;
+  }
+  return k;
+}
+
+int Stream::upload(const uint8_t* data, uint64_t len, bool pinned) {
+  cudaStream_t up = (cudaStream_t)re_->copy_stream_;
+  const uint8_t* src = data;
+  int k = next_staging_;
+  if (!pinned) {  // through pinned staging: the copy engine reads one buffer while the other is filled
+    next_staging_ ^= 1;
+    RB_STREAM_CUDA(cudaEventSynchronize((cudaEvent_t)staging_ev_[k]));
+    std::memcpy(staging_[k], data, len);
+    src = staging_[k];
+  }
+  RB_STREAM_CUDA(cudaMemcpyAsync((uint8_t*)win_.ptr + (end_ - base_), src, len, cudaMemcpyHostToDevice, up));
+  if (!pinned) RB_STREAM_CUDA(cudaEventRecord((cudaEvent_t)staging_ev_[k], up));
+  cudaEvent_t ev;
+  if (!free_events_.empty()) {
+    ev = (cudaEvent_t)free_events_.back();
+    free_events_.pop_back();
+  } else {
+    RB_STREAM_CUDA(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
+  }
+  end_ += len;
+  uploads_.push_back({end_, ev});
+  RB_STREAM_CUDA(cudaEventRecord(ev, up));
+  return 0;
+}
+
+int Stream::wait_uploads(uint64_t upto) {
+  size_t i = 0;
+  while (i < uploads_.size() && uploads_[i].first < upto) i++;
+  if (i == uploads_.size()) {
+    if (i == 0) return 0;
+    i--;
+  }
+  // uploads are ordered on the copy stream: waiting for the one that ends at or after upto covers those before it
+  RB_STREAM_CUDA(cudaStreamWaitEvent((cudaStream_t)re_->stream_, (cudaEvent_t)uploads_[i].second, 0));
+  for (size_t j = 0; j < i; j++) free_events_.push_back(uploads_[j].second);
+  uploads_.erase(uploads_.begin(), uploads_.begin() + i);
+  return 0;
+}
+
+// Drop the bytes no search reads again (left of the pending piece's 256 bytes of context) by moving the rest to the
+// front of the window.  The move runs on the engine's stream after every upload, in steps of at most the distance
+// moved so that no copy overlaps itself; uploads into the freed room wait for it.
+int Stream::make_room(uint64_t want) {
+  const uint64_t keep = n_pend_ ? pend_[0].lo : next_lo_;
+  const uint64_t nb = std::max(base_, keep >= 256 ? keep - 256 : 0);
+  if (cap_ - (end_ - nb) < want) return fail("internal error: the stream window is full");
+  if (nb == base_) return 0;
+  cudaStream_t st = (cudaStream_t)re_->stream_;
+  uint8_t* w = (uint8_t*)win_.ptr;
+  const uint64_t len = end_ - nb, off = nb - base_;
+  if (int rc = wait_uploads(end_)) return rc;
+  for (uint64_t d = 0; d < len; d += off)
+    RB_STREAM_CUDA(cudaMemcpyAsync(w + d, w + off + d, std::min(off, len - d), cudaMemcpyDeviceToDevice, st));
+  RB_STREAM_CUDA(cudaEventRecord((cudaEvent_t)moved_ev_, st));
+  RB_STREAM_CUDA(cudaStreamWaitEvent((cudaStream_t)re_->copy_stream_, (cudaEvent_t)moved_ev_, 0));
+  base_ = nb;
+  return 0;
+}
+
+// One find_all_shard_device call over the window for piece p (p->lo, hi, entry_*, buf in).  Returns 1 when a match
+// runs past the bytes that have arrived: the halo has grown, search again once they are there.
+int Stream::search(Piece* p, uint32_t rev_entry) {
+  const uint64_t n_end = finished_ ? end_ : std::min(end_, p->hi + halo_);
+  if (int rc = wait_uploads(n_end)) return rc;
+  ShardIO io;
+  io.own_lo = p->lo - base_;
+  io.own_hi = p->hi - base_;
+  io.is_first = base_ == 0;
+  io.is_last = finished_ && n_end == end_;
+  io.rev_entry = rev_entry;
+  if (p->entry_p < base_) {  // the iterator stands left of the window: enter at its first byte (sharded.py)
+    io.chain_p = 0;
+    io.chain_lm = kNone;
+    io.chain_clamped = true;
+  } else {
+    io.chain_p = p->entry_p - base_;
+    io.chain_lm = p->entry_lm == kNone || p->entry_lm < base_ ? kNone : p->entry_lm - base_;
+  }
+  p->has_spans = spans_ && !(sink_ && emitted_ >= sink_cap_);
+  DeviceBuf& buf = dspan_[p->buf];
+  if (p->has_spans && !buf.ensure(std::max<uint64_t>(4096, piece_ / 32) * 16)) return fail("out of device memory (stream spans)");
+  for (;;) {
+    uint64_t* d_out = p->has_spans ? (uint64_t*)buf.ptr : nullptr;
+    const uint64_t cap = p->has_spans ? buf.cap / 16 : 0;
+    if (re_->find_all_shard_device((const uint8_t*)win_.ptr, n_end - base_, &io, d_out, cap)) {
+      if (io.halo_overflow && !io.is_last) {
+        if (n_end - p->hi >= hold_)
+          return fail("a match is longer than the stream window (" + std::to_string(hold_) + " bytes): enlarge hold");
+        halo_ = std::min(hold_, (n_end - p->hi) * 8);
+        return 1;
+      }
+      if (io.left_ctx_short)
+        return fail("a look-around pattern needs text left of the stream window (" + std::to_string(p->lo - base_) +
+                    " bytes of left context): the iterator stands further back than the window keeps");
+      return fail(re_->error_);
+    }
+    if (!p->has_spans || io.n_matches <= cap) break;
+    // more spans than the buffer holds: grow it and search the piece again
+    if (!buf.ensure(io.n_matches * 20)) return fail("out of device memory (stream spans)");
+  }
+  if (p->has_spans && io.n_matches) {
+    cudaStream_t st = (cudaStream_t)re_->stream_;
+    add_to_words<<<grid_for(2 * io.n_matches, 256, 4), 256, 0, st>>>((uint64_t*)buf.ptr, 2 * io.n_matches, base_);
+    g_launches++;
+    RB_STREAM_CUDA(cudaGetLastError());
+  }
+  auto to_stream = [&](uint64_t v) { return v == kNone || v == kSpec ? v : v + base_; };
+  p->n = io.n_matches;
+  p->rev_guess = io.rev_guess;
+  p->rev_left = io.rev_left;
+  p->exit_p = to_stream(io.exit_p);
+  p->exit_lm = to_stream(io.exit_lm);
+  return 0;
+}
+
+int Stream::step(bool* progressed) {
+  *progressed = false;
+  if (done_) return 0;
+  Piece p;
+  p.lo = next_lo_;
+  p.hi = next_lo_ + piece_;
+  if (finished_) p.hi = std::min(p.hi, end_);
+  else if (end_ < p.hi + halo_) return 0;  // its bytes and halo have not all arrived
+  const bool last = finished_ && p.hi == end_;
+  p.entry_p = chain_p_;
+  p.entry_lm = chain_lm_;
+  bool used[kMaxPending + 2] = {};
+  for (int k = 0; k < n_pend_; k++) used[pend_[k].buf] = true;
+  while (used[p.buf]) p.buf++;
+  *progressed = true;
+  if (int rc = search(&p, kNoState)) return rc < 0 ? rc : 0;
+  pend_[n_pend_++] = p;
+  next_lo_ = p.hi;
+  chain_p_ = p.exit_p;
+  chain_lm_ = p.exit_lm;
+  const bool ended = last || chain_p_ == kNone;  // the text or the iteration ended (a failed slice emulation)
+  // A wrong rev_left of p (p's own top guess was wrong) looks the same as a wrong guess of the piece before it, so a
+  // mismatch waits for later pieces while the window holds them; a match is taken as the exact state.
+  if (n_pend_ == 1 || (!ended && n_pend_ <= kMaxPending && pend_[n_pend_ - 2].rev_guess != p.rev_left)) {
+    if (ended) return finish_pending();
+    return 0;
+  }
+  if (int rc = settle()) return rc;
+  if (ended) return finish_pending();
+  // every piece but p is final
+  for (int k = 0; k + 1 < n_pend_; k++)
+    if (int rc = emit(pend_[k])) return rc;
+  emitted_guess_ = pend_[n_pend_ - 2].rev_guess;
+  emitted_any_ = true;
+  pend_[0] = pend_[n_pend_ - 1];
+  n_pend_ = 1;
+  return 0;
+}
+
+int Stream::finish_pending() {
+  for (int k = 0; k < n_pend_; k++)
+    if (int rc = emit(pend_[k])) return rc;
+  n_pend_ = 0;
+  done_ = true;
+  return 0;
+}
+
+// Taking the newest pending piece's rev_left as exact, make every edge between pending pieces agree: right to left,
+// a piece whose top guess differs from its right neighbour's rev_left is searched again from that state (which may
+// change its own rev_left), then, left to right, every piece whose entering iterator state changed is searched again.
+int Stream::settle() {
+  const std::string too_long = "a match is longer than the stream window (" + std::to_string(hold_) + " bytes)";
+  int first = n_pend_;
+  for (int k = n_pend_ - 2; k >= 0; k--) {
+    if (pend_[k].rev_guess == pend_[k + 1].rev_left) continue;
+    if (int rc = search(&pend_[k], pend_[k + 1].rev_left)) return rc < 0 ? rc : fail(too_long);
+    first = k;
+  }
+  // The emitted piece before the pending ones was checked against the first pending piece's rev_left at the time;
+  // spans that left cannot be taken back.  This is the only wrong guess not caught while both pieces of its edge are
+  // still resident.
+  if (first == 0 && emitted_any_ && pend_[0].rev_left != emitted_guess_)
+    return fail("the reverse scan's state at a piece edge changed after the piece left the stream; use larger pieces");
+  for (int k = std::max(first, 0) + 1; k < n_pend_; k++) {
+    Piece& q = pend_[k];
+    if (q.entry_p == pend_[k - 1].exit_p && q.entry_lm == pend_[k - 1].exit_lm) continue;
+    q.entry_p = pend_[k - 1].exit_p;
+    q.entry_lm = pend_[k - 1].exit_lm;
+    if (int rc = search(&q, k + 1 < n_pend_ ? pend_[k + 1].rev_left : kNoState)) return rc < 0 ? rc : fail(too_long);
+  }
+  const Piece& p = pend_[n_pend_ - 1];
+  chain_p_ = p.exit_p;
+  chain_lm_ = p.exit_lm;
+  return 0;
+}
+
+int Stream::emit(const Piece& p) {
+  cudaStream_t st = (cudaStream_t)re_->stream_;
+  const uint64_t* src = (const uint64_t*)dspan_[p.buf].ptr;
+  if (p.has_spans && p.n && sink_) {
+    const uint64_t k = std::min(p.n, sink_cap_ > emitted_ ? sink_cap_ - emitted_ : 0);
+    if (k) RB_STREAM_CUDA(cudaMemcpyAsync(sink_ + 2 * emitted_, src, k * 16, cudaMemcpyDeviceToHost, st));
+  } else if (p.has_spans && p.n) {
+    const size_t old = queue_.size();
+    queue_.resize(old + 2 * p.n);
+    RB_STREAM_CUDA(cudaMemcpyAsync(queue_.data() + old, src, p.n * 16, cudaMemcpyDeviceToHost, st));
+    RB_STREAM_CUDA(cudaStreamSynchronize(st));
+  }
+  emitted_ += p.n;
+  return 0;
+}
+#undef RB_STREAM_CUDA
+
+bool Regex::use_window(uint64_t n, uint64_t cap) {
+  if (tuning.host_window) return n > tuning.host_window;
+  // The buffers the whole-haystack paths take anyway: the haystack, its start bitmap and the spans.
+  if (text_.ensure(n + 64) && bitmap_.ensure(((n >> 6) + 2) * 8) && (cap == 0 || out_.ensure(cap * 16))) return false;
+  cudaGetLastError();  // the failed allocation is not an error of a later call
+  return true;
+}
+
+int Regex::find_all_window(const uint8_t* text, uint64_t n, uint64_t start, uint64_t* out, uint64_t cap, uint64_t* total) {
+  *total = 0;
+  if (start > n) return 0;  // re_trait.rs:198-200
+  const uint64_t w = tuning.host_window;
+  const uint64_t piece = w ? std::max<uint64_t>(256, w / 8 / 256 * 256) : kStreamPieceDefault;
+  std::string err;
+  std::unique_ptr<Stream> s(Stream::create(this, piece, w ? piece : 4 * kStreamPieceDefault, out && cap, start, &err));
+  if (!s) return fail(err);
+  s->sink(out, cap);
+  const uint64_t lo = Stream::buf_lo(start);
+  if (s->write(text + lo, n - lo) || s->finish()) return fail(s->error());
+  *total = s->count();
   return 0;
 }
 

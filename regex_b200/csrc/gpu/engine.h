@@ -52,6 +52,8 @@ struct Tuning {
   uint32_t max_stitch_rounds = 16;  // re-walk rounds before the stitch falls back to one sequential pass
   uint32_t max_redo_rounds = 3;     // scan redo rounds before segment entry states are solved by state-map composition
   bool candidate_starts = false;    // tests: search from candidate starts (as over-budget patterns do) even when the unanchored automata fit
+  uint64_t host_window = 0;         // find_all_host: device window in bytes (pieces of an eighth of it) for haystacks larger than it;
+                                    // 0 = automatic (a window only when the haystack, its bitmap and the spans cannot be allocated)
 };
 
 struct Stats {  // filled by the last single-haystack call (diagnostics, bench roofline)
@@ -92,6 +94,8 @@ class DeviceBuf {
   void* ptr = nullptr;
   size_t cap = 0;
 };
+
+class Stream;
 
 class Regex {
  public:
@@ -215,6 +219,7 @@ class Regex {
   bool candidate_mode() const { return !is_set_ && (unanchored_too_big_ || tuning.candidate_starts); }
 
  private:
+  friend class Stream;
   Regex() = default;
   struct DeviceDfa;
   int init_device();
@@ -298,6 +303,9 @@ class Regex {
                   rb::Error* err);
   int set_matches_batch_grouped(const uint8_t* d_text, const uint64_t* d_offsets, uint64_t n_rec, uint64_t* d_masks);
   const uint8_t* upload_text(const uint8_t* text, uint64_t n, int* rc);
+  // find_all_host through a bounded device window (Stream) for haystacks that do not fit the device
+  bool use_window(uint64_t n, uint64_t cap);
+  int find_all_window(const uint8_t* text, uint64_t n, uint64_t start, uint64_t* out, uint64_t cap, uint64_t* total);
   int find_all_host_pipelined(const uint8_t* text, uint64_t n, uint8_t* d, uint64_t* d_out, uint64_t* out, uint64_t cap, uint64_t* total);
   int side_streams();  // creates copy_stream_ and back_stream_ on first use
 
@@ -362,6 +370,69 @@ class Regex {
   int pf_state_ = 0;               // 0 = not decided yet, 1 = prefilter applies, -1 = it does not
   uint32_t pf_freq_ = 0;           // estimated frequency of the scanned bytes, parts per 65536
   std::vector<uint32_t> pf_words_; // PfArgs image (engine.cu)
+};
+
+// find_iter over text that arrives in pieces, through a bounded device window (DESIGN.md §8): the concatenation of
+// every write is the haystack, and the spans read back are find_all_host on that concatenation, as stream offsets.
+// The stream owns its window, upload staging and span buffers; each call locks the engine it searches with.
+class Stream {
+ public:
+  // piece: bytes per searched piece (0 = 64 MiB); hold: longest match always resolved (0 = the piece size);
+  // spans false: count only.  start: the iteration begins there (the first byte written is at
+  // buf_lo(start), at most 256 bytes before it).  Null on failure (*err says why).
+  static Stream* create(Regex* re, uint64_t piece, uint64_t hold, bool spans, uint64_t start, std::string* err);
+  static uint64_t buf_lo(uint64_t start) { return start > 256 ? (start - 256) & ~255ull : 0; }
+  ~Stream();
+  int write(const uint8_t* data, uint64_t len);  // copies; may search pieces before it returns
+  int finish();                                  // end of text: settles every remaining piece
+  uint64_t read(uint64_t* out, uint64_t cap);    // pops up to cap final spans
+  uint64_t count() const { return emitted_; }   // final matches so far
+  const std::string& error() const { return error_; }
+  // find_all_host's bounded window: spans go straight to out (the first cap of them) instead of the read queue
+  void sink(uint64_t* out, uint64_t cap) { sink_ = out; sink_cap_ = cap; }
+
+ private:
+  struct Piece {  // one searched piece (stream offsets)
+    uint64_t lo = 0, hi = 0, entry_p = 0, entry_lm = 0, exit_p = 0, exit_lm = 0, n = 0;
+    uint32_t rev_guess = 0, rev_left = 0;
+    int buf = 0;             // which span buffer holds its spans
+    bool has_spans = false;  // searched with a span buffer (else counted only)
+  };
+  explicit Stream(Regex* re) : re_(re) {}
+  int fail(const std::string& msg);
+  int cuda(int e, const char* what);
+  int upload(const uint8_t* data, uint64_t len, bool pinned);
+  int wait_uploads(uint64_t upto);  // the engine's stream waits until stream bytes [.., upto) have arrived
+  int make_room(uint64_t want);
+  int search(Piece* p, uint32_t rev_entry);  // p->lo/hi/entry in, the rest out
+  int step(bool* progressed);                // searches and settles the next piece when its bytes are there
+  int settle();          // makes the edges between pending pieces agree (engine.cu)
+  int finish_pending();  // emits every pending piece: nothing follows
+  int emit(const Piece& p);
+  Regex* re_;
+  std::string error_;
+  uint64_t piece_ = 0, hold_ = 0, granule_ = 0, cap_ = 0, halo_ = 0;  // cap_: window bytes
+  bool spans_ = true, finished_ = false, done_ = false, failed_ = false;
+  DeviceBuf win_;             // device window: stream bytes [base_, end_) at win_.ptr
+  uint64_t base_ = 0, end_ = 0;
+  uint64_t next_lo_ = 0, chain_p_ = 0, chain_lm_ = 0;  // next piece to search, iterator state entering it
+  static constexpr int kMaxPending = 4;  // pieces kept waiting for a reverse-scan edge to agree
+  Piece pend_[kMaxPending + 1];          // searched, not final yet, left to right
+  int n_pend_ = 0;
+  bool emitted_any_ = false;
+  uint32_t emitted_guess_ = 0;           // rev_guess of the last emitted piece
+  DeviceBuf dspan_[kMaxPending + 2];     // spans of the pending pieces and of the one being searched (stream offsets)
+  uint8_t* staging_[2] = {nullptr, nullptr};  // pinned, double-buffered
+  void* staging_ev_[2] = {nullptr, nullptr};
+  int next_staging_ = 0;
+  std::vector<std::pair<uint64_t, void*>> uploads_;  // (stream end offset, event) of uploads not yet waited for
+  std::vector<void*> free_events_;
+  void* moved_ev_ = nullptr;  // the last window move (uploads into the freed room wait for it)
+  uint64_t emitted_ = 0;
+  std::vector<uint64_t> queue_;  // final spans not read yet, from queue_head_
+  uint64_t queue_head_ = 0;
+  uint64_t* sink_ = nullptr;
+  uint64_t sink_cap_ = 0;
 };
 
 uint64_t kernel_launches();  // total kernels launched by this library in this process

@@ -2195,6 +2195,9 @@ __global__ void span_lengths(const uint64_t* spans, uint64_t n_matches, uint64_t
   for (uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x; i < n_matches; i += (uint64_t)gridDim.x * blockDim.x)
     lens[i] = spans[2 * i + 1] - spans[2 * i];
 }
+__global__ void add_to_words(uint64_t* words, uint64_t n, uint64_t add) {
+  for (uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x; i < n; i += (uint64_t)gridDim.x * blockDim.x) words[i] += add;
+}
 // span of group g of match i (kNone start = the group did not take part: expands to nothing)
 __device__ __forceinline__ void rep_group(const ReplaceArgs& a, uint64_t i, uint32_t g, uint64_t* s, uint64_t* e) {
   if (g == 0 || !a.slots) { *s = a.spans[2 * i]; *e = a.spans[2 * i + 1]; return; }

@@ -138,6 +138,8 @@ struct ReplaceArgs {
 };
 __global__ void replace_lengths(ReplaceArgs a, uint64_t* rep_lens);
 __global__ void span_lengths(const uint64_t* spans, uint64_t n_matches, uint64_t* lens);
+// words[i] += add (window-relative spans of a stream -> stream offsets)
+__global__ void add_to_words(uint64_t* words, uint64_t n, uint64_t add);
 __global__ void replace_gaps(ReplaceArgs a, uint64_t matched_total, uint64_t replaced_total);
 __global__ void replace_matches(ReplaceArgs a);
 // pieces[i] = text between match i-1 and match i; limit as splitn (0 = none)
