@@ -15,6 +15,9 @@
  *   rure_b200_captures_iter_batch == rure_b200_captures_all(re, hay + off[i], off[i+1]-off[i], ...) per record
  *   rure_b200_stream_*        == rure_b200_find_all on the concatenation of every rure_b200_stream_write
  *                                (spans as offsets into that concatenation; it need never exist in memory)
+ *   rure_b200_match_stream_*  == rure_b200_shortest_match / rure_b200_is_match (rure) and
+ *                                rure_b200_set_is_match / rure_b200_set_matches_mask (rure_set) on the
+ *                                concatenation of every rure_b200_match_stream_write
  * Functions return true on success; on failure rure_b200_last_error() (thread
  * local) describes what went wrong.  A missing GPU is a failure, never a
  * silent CPU fallback.
@@ -62,7 +65,11 @@ bool rure_b200_set_is_match(rure_set *set, const uint8_t *haystack, size_t lengt
  * result is identical to uploading first (environment RB200_PIPELINE_PIECE=<bytes> changes
  * the piece size, 0 turns the pipeline off).  Pinned host memory gives the full PCIe rate.
  * A haystack that, with its bitmap and spans, cannot be allocated on the device is searched
- * through a stream window instead (see streams below; hold 256 MiB). */
+ * through a stream window instead (see streams below; hold 256 MiB).  The same holds for the
+ * forward searches (rure_is_match, rure_shortest_match, rure_set_is_match, rure_set_matches,
+ * rure_b200_set_matches_mask and their rure_b200_* twins) through a match stream window: a
+ * haystack the device cannot hold is fed piece by piece and the transfer stops at the piece that
+ * decides the answer. */
 bool rure_b200_find_all(rure *re, const uint8_t *haystack, size_t length, rure_match *out,
                         size_t cap, size_t *n_total);
 bool rure_b200_count_all(rure *re, const uint8_t *haystack, size_t length, size_t *n_total);
@@ -246,8 +253,8 @@ bool rure_b200_set_matches_shard_device(rure_set *set, const uint8_t *d_buffer, 
  * rure_b200_stream_finish ends the text and settles every remaining piece.
  * rure_b200_stream_read pops up to cap final spans (offsets into the whole text), *n = popped.
  * rure_b200_stream_count: final matches so far (read or not).  After a failure (see
- * rure_b200_last_error) or after finish, writes fail.  Out of scope: forward searches (is_match,
- * shortest_match, set matches), rure_find, replace, split and captures on such text. */
+ * rure_b200_last_error) or after finish, writes fail.  Forward searches have match streams
+ * (below).  Out of scope: rure_find, replace, split and captures on such text. */
 typedef struct rure_b200_stream rure_b200_stream;
 rure_b200_stream *rure_b200_stream_new(rure *re, size_t piece, size_t hold, int spans);
 bool rure_b200_stream_write(rure_b200_stream *s, const uint8_t *data, size_t len);
@@ -255,6 +262,37 @@ bool rure_b200_stream_finish(rure_b200_stream *s);
 bool rure_b200_stream_read(rure_b200_stream *s, rure_match *out, size_t cap, size_t *n);
 uint64_t rure_b200_stream_count(rure_b200_stream *s);
 void rure_b200_stream_free(rure_b200_stream *s);
+
+/* ---- match streams: is_match, shortest_match and RegexSet matches over text fed in pieces ----
+ * The forward automaton's state flows left to right, so each piece is entered in the exact exit
+ * state of the piece before it and nothing is ever searched twice.  The window holds 256 bytes of
+ * left context, the piece being searched and the bytes after it (about 2 * piece + hold + 16 MiB).
+ * rure_b200_match_stream_new / rure_b200_set_match_stream_new: piece and hold as for
+ * rure_b200_stream_new; hold only matters for patterns searched from candidate starts (over the
+ * DFA budget), whose matches may run past a piece: a match longer than hold fails the stream with
+ * "a match is longer than the stream window (... bytes)".  masks != 0: the set stream reports which
+ * patterns match (rure_b200_set_matches_mask); masks == 0: only whether any does
+ * (rure_b200_set_is_match).  NULL on failure.
+ * The stream is decided once nothing written later can change its answer: a match was found (a
+ * rure, or a set without masks), every pattern matched (a set with masks), no automaton can match
+ * any more (e.g. `^foo` on text that starts otherwise), or finish ran.  Writes after that return
+ * true without uploading or searching anything, so a reader may stop feeding as soon as
+ * state.decided is set.  Writes after finish, and every call after a failure, fail.  Failures and
+ * the thread rules are those of rure_b200_stream_*. */
+typedef struct rure_b200_match_stream rure_b200_match_stream;
+typedef struct rure_b200_match_state {
+  int32_t decided;    /* nothing written later can change found / end / the mask (always set after finish) */
+  int32_t found;      /* a match ends in the text searched so far; never reverts */
+  uint64_t end;       /* least match end so far (stream offset); final once decided */
+  uint64_t searched;  /* stream bytes searched so far; stops growing once decided */
+} rure_b200_match_state;
+rure_b200_match_stream *rure_b200_match_stream_new(rure *re, size_t piece, size_t hold);
+rure_b200_match_stream *rure_b200_set_match_stream_new(rure_set *set, size_t piece, size_t hold, int masks);
+bool rure_b200_match_stream_write(rure_b200_match_stream *s, const uint8_t *data, size_t len);
+bool rure_b200_match_stream_finish(rure_b200_match_stream *s);
+/* mask_words: (rure_set_len + 63) / 64 words for a set stream created with masks != 0, else may be NULL */
+bool rure_b200_match_stream_state(rure_b200_match_stream *s, rure_b200_match_state *out, uint64_t *mask_words);
+void rure_b200_match_stream_free(rure_b200_match_stream *s);
 
 /* ---- threads ----------------------------------------------------------------
  * As in rure.h (regex-capi/include/rure.h:27-34) one compiled rure / rure_set may be used from
@@ -289,9 +327,10 @@ void rure_b200_set_last_stats_ex(rure_set *set, double *out, size_t n);
  * "max_redo_rounds", "batch_refill" 0/1 (batched is_match: lanes refill from a task of records), "prefilter" (0 never, 1 automatic: only for a single rare byte, 2 whenever the
  * pattern qualifies), "candidate_starts" 0/1 (tests: search from candidate starts with the anchored
  * automaton, as patterns over the DFA budget do, even when the unanchored automata fit),
- * "host_window" bytes (tests: rure_b200_find_all, rure_b200_count_all and rure_iter_next search
- * host haystacks longer than this through a stream window of about this size; 0, the default,
- * = only haystacks whose buffers cannot be allocated on the device).
+ * "host_window" bytes (tests: rure_b200_find_all, rure_b200_count_all, rure_iter_next and the
+ * forward searches -- is_match, shortest_match, set is_match and set matches -- search host
+ * haystacks longer than this through a stream window of about this size; 0, the default, = only
+ * haystacks whose buffers cannot be allocated on the device).
  * Returns false for an unknown name.
  * Sets also take "set_group_patterns" k (tests): search in groups of at most k patterns even when
  * the product automaton fits, each group split further while its automaton is over the budget;

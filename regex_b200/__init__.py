@@ -42,6 +42,10 @@ class _Shard(ctypes.Structure):  # include/rure_b200.h: rure_b200_shard
                 ("n_matches", c_uint64), ("halo_overflow", c_uint32), ("chain_clamped", c_uint32)]
 
 
+class _MatchState(ctypes.Structure):  # include/rure_b200.h: rure_b200_match_state
+    _fields_ = [("decided", ctypes.c_int32), ("found", ctypes.c_int32), ("end", c_uint64), ("searched", c_uint64)]
+
+
 class _FwdShard(ctypes.Structure):  # include/rure_b200.h: rure_b200_fwd_shard
     _fields_ = [("own_lo", c_uint64), ("own_hi", c_uint64), ("is_first", ctypes.c_int32), ("is_last", ctypes.c_int32),
                 ("entry_state", c_uint32), ("entry_used", c_uint32), ("exit_state", c_uint32), ("found", c_uint32),
@@ -108,6 +112,12 @@ def _load():
         "rure_b200_stream_read": (c_bool, [vp, vp, sz, POINTER(sz)]),
         "rure_b200_stream_count": (c_uint64, [vp]),
         "rure_b200_stream_free": (None, [vp]),
+        "rure_b200_match_stream_new": (vp, [vp, sz, sz]),
+        "rure_b200_set_match_stream_new": (vp, [vp, sz, sz, c_int]),
+        "rure_b200_match_stream_write": (c_bool, [vp, u8p, sz]),
+        "rure_b200_match_stream_finish": (c_bool, [vp]),
+        "rure_b200_match_stream_state": (c_bool, [vp, POINTER(_MatchState), vp]),
+        "rure_b200_match_stream_free": (None, [vp]),
         "rure_b200_is_match_batch": (c_bool, [vp, u8p, vp, sz, vp]),
         "rure_b200_find_batch": (c_bool, [vp, u8p, vp, sz, vp, vp]),
         "rure_b200_set_matches_batch": (c_bool, [vp, u8p, vp, sz, vp]),
@@ -234,6 +244,91 @@ class RegexStream:
     def close(self):
         if self._h:
             _lib.rure_b200_stream_free(self._h)
+            self._h = None
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+    def __del__(self):
+        if _lib is not None:
+            self.close()
+
+
+class MatchStream:
+    """is_match / shortest_match (Regex.match_stream) or RegexSet is_match / matches (RegexSet.match_stream) over
+    text written in pieces.  Usable as a context manager, which frees it on exit."""
+
+    def __init__(self, owner, piece=0, hold=0, n_patterns=None, masks=False):
+        self._owner = owner  # keeps the compiled regex or set alive while the stream uses its engine
+        if n_patterns is None:
+            self._h = _lib.rure_b200_match_stream_new(owner._h, piece, hold)
+            self._mw = 0
+        else:
+            self._h = _lib.rure_b200_set_match_stream_new(owner._h, piece, hold, int(bool(masks)))
+            self._mw = max(1, (n_patterns + 63) // 64) if masks else 0
+        if not self._h:
+            raise Error(_last_error())
+        self._n = n_patterns
+
+    def write(self, data):
+        """Append bytes (as RegexStream.write).  Once decided, writes return at once without searching."""
+        if isinstance(data, memoryview) and data.contiguous:
+            data = np.frombuffer(data, dtype=np.uint8)
+        p, n, keep = _buf(data)
+        if not _lib.rure_b200_match_stream_write(self._h, p, n):
+            raise Error(_last_error())
+
+    def finish(self):
+        """End of text: the answer becomes final."""
+        if not _lib.rure_b200_match_stream_finish(self._h):
+            raise Error(_last_error())
+
+    def _state(self):
+        st = _MatchState()
+        words = (c_uint64 * max(1, self._mw))()
+        if not _lib.rure_b200_match_stream_state(self._h, byref(st), words if self._mw else None):
+            raise Error(_last_error())
+        return st, list(words)[: self._mw]
+
+    @property
+    def decided(self):
+        """Nothing written later can change the answer (always true after finish)."""
+        return bool(self._state()[0].decided)
+
+    @property
+    def found(self):
+        return bool(self._state()[0].found)
+
+    @property
+    def end(self):
+        """Least match end so far (offset into the whole text), None when there is none."""
+        st = self._state()[0]
+        return int(st.end) if st.found else None
+
+    @property
+    def searched(self):
+        """Bytes of the text searched so far; stops growing once decided."""
+        return int(self._state()[0].searched)
+
+    @property
+    def mask(self):
+        """Pattern mask words of a set stream created with masks=True."""
+        if not self._mw:
+            raise Error("this stream was created without masks")
+        return self._state()[1]
+
+    @property
+    def matches(self):
+        """Indices of the patterns that match in the text so far (a set stream created with masks=True)."""
+        words = self.mask
+        return [i for i in range(self._n) if (words[i // 64] >> (i % 64)) & 1]
+
+    def close(self):
+        if self._h:
+            _lib.rure_b200_match_stream_free(self._h)
             self._h = None
 
     def __enter__(self):
@@ -455,6 +550,11 @@ class _Compiled:
         """find_iter over text fed in pieces (include/rure_b200.h: streams): write() the text in any
         blocks, finish(), and read() the spans, which equal find_all on the concatenation."""
         return RegexStream(self, piece, hold, spans)
+
+    def match_stream(self, piece=0, hold=0):
+        """is_match / shortest_match over text fed in pieces (include/rure_b200.h: match streams): write() the text
+        in any blocks; `decided`, `found` and `end` equal shortest_match on the concatenation once decided."""
+        return MatchStream(self, piece, hold)
 
     def is_match_batch(self, text, offsets):
         """bool array, one per record text[offsets[i]:offsets[i+1]]."""
@@ -806,6 +906,11 @@ class _SetBase:
         p, n, keep = _buf(text)
         words = self.matches_mask(text, start)  # rure_b200_set_matches_mask reports failures; rure_set_matches aborts
         return [i for i in range(len(self)) if (words[i // 64] >> (i % 64)) & 1]
+
+    def match_stream(self, piece=0, hold=0, masks=True):
+        """is_match / matches over text fed in pieces (include/rure_b200.h: match streams); masks=False answers
+        only whether any pattern matches."""
+        return MatchStream(self, piece, hold, len(self), masks)
 
     def matches_mask(self, text, start=0):
         p, n, keep = _buf(text)

@@ -404,6 +404,48 @@ bool rure_b200_stream_read(rure_b200_stream* s, rure_match* out, size_t cap, siz
 uint64_t rure_b200_stream_count(rure_b200_stream* s) { return s->s->count(); }
 void rure_b200_stream_free(rure_b200_stream* s) { delete s; }
 
+struct rure_b200_match_stream {
+  rbgpu::MatchStream* s;
+  size_t mask_words;  // 0: no masks
+  ~rure_b200_match_stream() { delete s; }
+};
+static rure_b200_match_stream* match_stream_new(Regex* re, size_t piece, size_t hold, bool masks) {
+  std::string err;
+  rbgpu::MatchStream* s = rbgpu::MatchStream::create(re, piece, hold, masks, 0, &err);
+  if (!s) {
+    g_last_error = err;
+    return nullptr;
+  }
+  return new rure_b200_match_stream{s, masks ? (re->n_patterns() + 63) / 64 : 0};
+}
+static bool match_stream_ok(rure_b200_match_stream* s, int rc) {
+  if (rc == 0) return true;
+  g_last_error = s->s->error();
+  return false;
+}
+rure_b200_match_stream* rure_b200_match_stream_new(rure* re, size_t piece, size_t hold) { return match_stream_new(re->re, piece, hold, false); }
+rure_b200_match_stream* rure_b200_set_match_stream_new(rure_set* set, size_t piece, size_t hold, int masks) {
+  return match_stream_new(set->re, piece, hold, masks != 0);
+}
+bool rure_b200_match_stream_write(rure_b200_match_stream* s, const uint8_t* data, size_t len) {
+  return match_stream_ok(s, s->s->write(data, len));
+}
+bool rure_b200_match_stream_finish(rure_b200_match_stream* s) { return match_stream_ok(s, s->s->finish()); }
+bool rure_b200_match_stream_state(rure_b200_match_stream* s, rure_b200_match_state* out, uint64_t* mask_words) {
+  if (!s->s->error().empty()) {
+    g_last_error = s->s->error();
+    return false;
+  }
+  out->decided = s->s->decided();
+  out->found = s->s->found();
+  out->end = out->found && s->s->end() != ~0ull ? s->s->end() : 0;
+  out->searched = s->s->searched();
+  if (mask_words)
+    for (size_t w = 0; w < s->mask_words; w++) mask_words[w] = s->s->mask()[w];
+  return true;
+}
+void rure_b200_match_stream_free(rure_b200_match_stream* s) { delete s; }
+
 bool rure_b200_set_matches_mask(rure_set* s, const uint8_t* haystack, size_t length, size_t start, uint64_t* mask_words) {
   bool any;
   return ok(s->re, s->re->set_matches_host(haystack, length, start, &any, mask_words));

@@ -106,6 +106,7 @@ struct DeviceScalars {
   uint8_t flag0;                 // start bitmaps: a match starts at position 0
   unsigned long long task_counter;  // batch_refill: next task to hand out
   unsigned long long cand_best;     // cand_shortest: earliest match end
+  uint32_t cand_overflow;           // cand_shortest in a stream's window: a run reached the window's end undecided
   unsigned long long fwd_result[1 + kMaxMaskWords];  // forward_range: first match end, OR of the pattern masks
 };
 
@@ -585,11 +586,8 @@ int Regex::cand_starts(const uint8_t* d_text, uint64_t n, uint64_t base, uint64_
 // enters from s, in the waves of forward_reduce (64 MiB, x16 each); a wave is the last one once the best end lies
 // at or before the next wave's first candidate.
 int Regex::cand_shortest(const uint8_t* d_text, uint64_t n, uint64_t start, bool* found, uint64_t* end) {
-  DeviceDfa* fwd;
+  DeviceDfa* fwd;  // picks the stream, creates the scalars
   if (int rc = ensure(kFwdAnchoredLF, &fwd)) return rc;
-  CandArgs c;
-  if (int rc = cand_args(&c)) return rc;
-  c.utf8_boundaries = 0;  // the earliest end: an empty match inside a UTF-8 sequence never ends before one at `start`
   cudaStream_t st = (cudaStream_t)stream_;
   if (lazy_ && lazy_->done < lazy_->n) {  // host haystack: an anchored run may read to its end
     RB_CUDA(cudaMemcpyAsync(lazy_->dst + lazy_->done, lazy_->src + lazy_->done, lazy_->n - lazy_->done, cudaMemcpyHostToDevice, st));
@@ -597,9 +595,6 @@ int Regex::cand_shortest(const uint8_t* d_text, uint64_t n, uint64_t start, bool
   }
   unsigned long long* best = &d_scalars_->cand_best;
   RB_CUDA(cudaMemsetAsync(best, 0xFF, 8, st));
-  const size_t smem = smem_for(fwd->view);
-  RB_CUDA(allow_smem(rbgpu::cand_shortest, smem));  // (the kernel, not this member)
-  const uint32_t seg = 1024;
   uint64_t wave = tuning.wave0 ? (tuning.wave0 + 4095) / 4096 * 4096 : 0;
   uint64_t lo = start, b = kNone;
   const uint64_t hi = n + 1;  // candidate positions [start, n]
@@ -607,9 +602,7 @@ int Regex::cand_shortest(const uint8_t* d_text, uint64_t n, uint64_t start, bool
   for (;;) {
     uint64_t limit = hi;
     if (wave && hi - lo > 2 * wave) limit = lo + wave;
-    const uint64_t n_seg = (limit - lo + seg - 1) / seg;
-    rbgpu::cand_shortest<<<grid_for(n_seg, 256, tuning.blocks_per_sm), 256, smem, st>>>(fwd->view, smem != 0, c, d_text, n, lo, limit, seg, best);
-    RB_LAUNCH_CHECK("cand_shortest");
+    if (int rc = cand_shortest_range(d_text, n, lo, limit, false, best, nullptr)) return rc;
     stats.waves++;
     RB_CUDA(d2h(&b, best, 8));
     if (limit == hi || (b != kNone && b <= limit)) break;
@@ -617,6 +610,23 @@ int Regex::cand_shortest(const uint8_t* d_text, uint64_t n, uint64_t start, bool
     wave *= 16;
   }
   if (b != kNone) { *found = true; *end = b; }
+  return 0;
+}
+
+int Regex::cand_shortest_range(const uint8_t* d_text, uint64_t n, uint64_t lo, uint64_t hi, bool text_continues, unsigned long long* best,
+                               uint32_t* overflow) {
+  DeviceDfa* fwd;
+  if (int rc = ensure(kFwdAnchoredLF, &fwd)) return rc;
+  CandArgs c;
+  if (int rc = cand_args(&c)) return rc;
+  c.utf8_boundaries = 0;  // the earliest end: an empty match inside a UTF-8 sequence never ends before one at `start`
+  const size_t smem = smem_for(fwd->view);
+  RB_CUDA(allow_smem(rbgpu::cand_shortest, smem));  // (the kernel, not this member)
+  const uint32_t seg = 1024;
+  const uint64_t n_seg = (hi - lo + seg - 1) / seg;
+  rbgpu::cand_shortest<<<grid_for(n_seg, 256, tuning.blocks_per_sm), 256, smem, (cudaStream_t)stream_>>>(
+      fwd->view, smem != 0, c, d_text, n, lo, hi, seg, best, text_continues ? 1 : 0, overflow);
+  RB_LAUNCH_CHECK("cand_shortest");
   return 0;
 }
 
@@ -1401,19 +1411,10 @@ int Regex::forward_reduce(const uint8_t* d_text, uint64_t n, uint64_t start, boo
   if (int rc = init_device()) return rc;
   // The automata of this search: the product automaton, or one per pattern group.  Every wave runs each group that
   // is still open over the same positions; each group carries its own state into the next wave.
-  std::vector<Regex*> tabs{this};
-  std::vector<uint32_t> firsts{0};
-  if (!groups_.empty()) {
-    if (entry != kNoEntry || end != ~0ull) return fail("a RegexSet searched in pattern groups cannot be searched in shards");
-    tabs.clear();
-    for (auto& g : groups_) {
-      g->tuning = tuning;
-      g->sparse_set_ = sparse_set_;
-      g->set_stream(stream_);
-      tabs.push_back(g.get());
-    }
-    firsts = group_first_;
-  }
+  if (!groups_.empty() && (entry != kNoEntry || end != ~0ull)) return fail("a RegexSet searched in pattern groups cannot be searched in shards");
+  std::vector<Regex*> tabs;
+  std::vector<uint32_t> firsts;
+  forward_tabs(&tabs, &firsts);
   const uint32_t n_tab = (uint32_t)tabs.size();
   std::vector<uint32_t> entries(n_tab, entry);
   std::vector<char> done(n_tab, 0);
@@ -1437,24 +1438,8 @@ int Regex::forward_reduce(const uint8_t* d_text, uint64_t n, uint64_t start, boo
     }
     std::copy(result_host + 1, result_host + 1 + rw, before.begin());
     bool live = false;
-    for (uint32_t g = 0; g < n_tab; g++) {
-      if (done[g]) continue;
-      uint64_t r[1 + kMaxMaskWords];
-      uint32_t exit_state = 0;
-      if (int rc = tabs[g]->forward_range(d_text, n, lo, limit, entries[g], want_masks, r, &exit_state))
-        return tabs[g] == this ? rc : fail(tabs[g]->last_error());
-      result_host[0] = std::min(result_host[0], r[0]);
-      // group-local mask bit j is pattern firsts[g] + j
-      const uint32_t w0 = firsts[g] / 64, sh = firsts[g] % 64;
-      for (uint32_t w = 0; w < kMaxMaskWords && w0 + w < rw; w++) {
-        result_host[1 + w0 + w] |= r[1 + w] << sh;
-        if (sh && w0 + w + 1 < rw) result_host[2 + w0 + w] |= r[1 + w] >> (64 - sh);
-      }
-      entries[g] = exit_state;
-      if (exit_out) *exit_out = exit_state;
-      if (exit_state == 0) done[g] = 1;  // dead state: an anchored search that can no longer match
-      live = live || !done[g];
-    }
+    if (int rc = forward_step(tabs, firsts, d_text, n, lo, limit, want_masks, &entries, &done, result_host, &live)) return rc;
+    if (exit_out) *exit_out = entries[0];  // (shards have one automaton)
     stats.waves++;
     bool fresh = false;
     for (uint32_t w = 0; w < rw; w++) fresh = fresh || (result_host[1 + w] & ~before[w]);
@@ -1482,18 +1467,62 @@ int Regex::forward_reduce(const uint8_t* d_text, uint64_t n, uint64_t start, boo
           if ((sr[1 + j / 64] >> (j % 64)) & 1) result_host[1 + open[j] / 64] |= 1ull << (open[j] % 64);
         break;
       }
-      // a group whose patterns have all matched needs no further waves
-      for (uint32_t g = 0; g < n_tab && n_tab > 1; g++) {
-        const uint32_t hi = g + 1 < n_tab ? firsts[g + 1] : n_pat;
-        bool all = true;
-        for (uint32_t i = firsts[g]; i < hi && all; i++) all = (result_host[1 + i / 64] >> (i % 64)) & 1;
-        if (all) done[g] = 1;
-      }
+      retire_matched(firsts, result_host, &done);
     }
     lo = limit;
     wave *= 16;
   }
   return 0;
+}
+
+void Regex::forward_tabs(std::vector<Regex*>* tabs, std::vector<uint32_t>* firsts) {
+  tabs->assign(1, this);
+  firsts->assign(1, 0);
+  if (groups_.empty()) return;
+  tabs->clear();
+  for (auto& g : groups_) {
+    g->tuning = tuning;
+    g->sparse_set_ = sparse_set_;
+    g->set_stream(stream_);
+    tabs->push_back(g.get());
+  }
+  *firsts = group_first_;
+}
+
+int Regex::forward_step(const std::vector<Regex*>& tabs, const std::vector<uint32_t>& firsts, const uint8_t* d_text, uint64_t n, uint64_t lo,
+                        uint64_t limit, bool want_masks, std::vector<uint32_t>* entries, std::vector<char>* done, uint64_t* result_host,
+                        bool* live) {
+  const uint32_t rw = result_words() - 1;
+  *live = false;
+  for (uint32_t g = 0; g < tabs.size(); g++) {
+    if ((*done)[g]) continue;
+    uint64_t r[1 + kMaxMaskWords];
+    uint32_t exit_state = 0;
+    if (int rc = tabs[g]->forward_range(d_text, n, lo, limit, (*entries)[g], want_masks, r, &exit_state))
+      return tabs[g] == this ? rc : fail(tabs[g]->last_error());
+    result_host[0] = std::min(result_host[0], r[0]);
+    // group-local mask bit j is pattern firsts[g] + j
+    const uint32_t w0 = firsts[g] / 64, sh = firsts[g] % 64;
+    for (uint32_t w = 0; w < kMaxMaskWords && w0 + w < rw; w++) {
+      result_host[1 + w0 + w] |= r[1 + w] << sh;
+      if (sh && w0 + w + 1 < rw) result_host[2 + w0 + w] |= r[1 + w] >> (64 - sh);
+    }
+    (*entries)[g] = exit_state;
+    if (exit_state == 0) (*done)[g] = 1;  // dead state: an anchored search that can no longer match
+    *live = *live || !(*done)[g];
+  }
+  return 0;
+}
+
+// a group whose patterns have all matched needs no further search
+void Regex::retire_matched(const std::vector<uint32_t>& firsts, const uint64_t* result_host, std::vector<char>* done) const {
+  const uint32_t n_tab = (uint32_t)firsts.size(), n_pat = (uint32_t)patterns_.size();
+  for (uint32_t g = 0; g < n_tab && n_tab > 1; g++) {
+    const uint32_t hi = g + 1 < n_tab ? firsts[g + 1] : n_pat;
+    bool all = true;
+    for (uint32_t i = firsts[g]; i < hi && all; i++) all = (result_host[1 + i / 64] >> (i % 64)) & 1;
+    if (all) (*done)[g] = 1;
+  }
 }
 
 // ------------------------------------------------------------ pattern groups --
@@ -2720,6 +2749,7 @@ int Regex::shortest_match_host(const uint8_t* text, uint64_t n, uint64_t start, 
   std::lock_guard<std::recursive_mutex> lock(mu_);
   *found = false;
   if (int rc = init_device()) return rc;
+  if (use_match_window(n)) return match_window(text, n, start, false, found, end, nullptr);  // larger than the device
   uint8_t* d = (uint8_t*)text_.ensure(n + 64);
   if (!d) return fail("out of device memory (haystack)");
   LazyUpload up{text, d, n, start > 256 ? (start - 256) & ~255ull : 0};
@@ -2732,6 +2762,10 @@ int Regex::set_matches_host(const uint8_t* text, uint64_t n, uint64_t start, boo
   std::lock_guard<std::recursive_mutex> lock(mu_);
   *any = false;
   if (int rc = init_device()) return rc;
+  if (use_match_window(n)) {  // larger than the device
+    for (uint32_t w = 0; w < (patterns_.size() + 63) / 64; w++) masks[w] = 0;
+    return match_window(text, n, start, true, any, nullptr, masks);
+  }
   uint8_t* d = (uint8_t*)text_.ensure(n + 64);
   if (!d) return fail("out of device memory (haystack)");
   LazyUpload up{text, d, n, start > 256 ? (start - 256) & ~255ull : 0};
@@ -2889,51 +2923,9 @@ int Regex::set_matches_batch_host(const uint8_t* text, const uint64_t* offsets, 
 static constexpr uint64_t kStreamPieceDefault = 64ull << 20;
 static constexpr uint64_t kStreamGranule = 8ull << 20;  // most bytes per upload (and per pinned staging buffer)
 
-Stream* Stream::create(Regex* re, uint64_t piece, uint64_t hold, bool spans, uint64_t start, std::string* err) {
-  std::lock_guard<std::recursive_mutex> lock(re->mu_);
-  std::unique_ptr<Stream> s(new Stream(re));
-  if (re->is_set_) {
-    *err = "find requires exactly one pattern (RegexSet cannot be used with find, exec.rs:510-512)";
-    return nullptr;
-  }
-  Regex::DeviceDfa* warm;  // picks the stream, creates the pinned scratch
-  if (re->init_device() || re->ensure(kFwdAnchoredLF, &warm) || re->side_streams()) {
-    *err = re->error_;
-    return nullptr;
-  }
-  s->piece_ = piece ? (piece + 255) & ~255ull : kStreamPieceDefault;
-  s->hold_ = hold ? (hold + 255) & ~255ull : s->piece_;
-  s->halo_ = std::min<uint64_t>(64 << 10, s->hold_);
-  s->granule_ = std::min(kStreamGranule, std::max<uint64_t>(256, s->piece_ / 2));
-  // left context + the pending pieces + the next piece + its longest halo + the uploads in flight
-  s->cap_ = 4096 + (kMaxPending + 1) * s->piece_ + s->hold_ + 2 * s->granule_;
-  s->spans_ = spans;
-  s->base_ = s->end_ = buf_lo(start);
-  s->next_lo_ = shard_own_lo(start);
-  s->chain_p_ = start;
-  s->chain_lm_ = kNone;
-  if (!s->win_.ensure(s->cap_ + 64)) {
-    *err = "out of device memory (stream window of " + std::to_string(s->cap_) + " bytes)";
-    return nullptr;
-  }
-  for (int k = 0; k < 2; k++) {
-    cudaEvent_t ev;
-    if (cudaMallocHost(&s->staging_[k], s->granule_) != cudaSuccess || cudaEventCreateWithFlags(&ev, cudaEventDisableTiming) != cudaSuccess) {
-      *err = "out of pinned host memory (stream staging)";
-      return nullptr;
-    }
-    s->staging_ev_[k] = ev;
-  }
-  cudaEvent_t ev;
-  if (cudaEventCreateWithFlags(&ev, cudaEventDisableTiming) != cudaSuccess) {
-    *err = "cannot create a CUDA event";
-    return nullptr;
-  }
-  s->moved_ev_ = ev;
-  return s.release();
-}
-
-Stream::~Stream() {
+// ---- the window both streams share ----
+StreamWindow::~StreamWindow() {
+  if (!re_) return;
   std::lock_guard<std::recursive_mutex> lock(re_->mu_);
   if (re_->copy_stream_) cudaStreamSynchronize((cudaStream_t)re_->copy_stream_);
   if (re_->stream_) cudaStreamSynchronize((cudaStream_t)re_->stream_);
@@ -2945,6 +2937,142 @@ Stream::~Stream() {
   for (void* e : free_events_) cudaEventDestroy((cudaEvent_t)e);
   if (moved_ev_) cudaEventDestroy((cudaEvent_t)moved_ev_);
 }
+
+int StreamWindow::init(Regex* re, uint64_t cap, uint64_t granule, uint64_t base, std::string* err) {
+  re_ = re;
+  cap_ = cap;
+  granule_ = granule;
+  base_ = end_ = base;
+  if (re->side_streams()) {
+    *err = re->error_;
+    return -1;
+  }
+  if (!buf_.ensure(cap_ + 64)) {
+    *err = "out of device memory (stream window of " + std::to_string(cap_) + " bytes)";
+    return -1;
+  }
+  for (int k = 0; k < 2; k++) {
+    cudaEvent_t ev;
+    if (cudaMallocHost(&staging_[k], granule_) != cudaSuccess || cudaEventCreateWithFlags(&ev, cudaEventDisableTiming) != cudaSuccess) {
+      *err = "out of pinned host memory (stream staging)";
+      return -1;
+    }
+    staging_ev_[k] = ev;
+  }
+  cudaEvent_t ev;
+  if (cudaEventCreateWithFlags(&ev, cudaEventDisableTiming) != cudaSuccess) {
+    *err = "cannot create a CUDA event";
+    return -1;
+  }
+  moved_ev_ = ev;
+  return 0;
+}
+
+bool StreamWindow::pinned(const uint8_t* data, uint64_t len) {
+  cudaPointerAttributes attr;
+  const bool p = len && cudaPointerGetAttributes(&attr, data) == cudaSuccess && attr.type == cudaMemoryTypeHost;
+  cudaGetLastError();  // a pageable pointer is not an error
+  return p;
+}
+
+#define RB_WINDOW_CUDA(call)                                                                      \
+  do {                                                                                            \
+    const cudaError_t e__ = (call);                                                               \
+    if (e__ != cudaSuccess) {                                                                     \
+      *err = std::string("CUDA error in ") + #call + ": " + cudaGetErrorString(e__);              \
+      return -1;                                                                                  \
+    }                                                                                             \
+  } while (0)
+
+int StreamWindow::upload(const uint8_t* data, uint64_t len, bool pinned, std::string* err) {
+  cudaStream_t up = (cudaStream_t)re_->copy_stream_;
+  const uint8_t* src = data;
+  int k = next_staging_;
+  if (!pinned) {  // through pinned staging: the copy engine reads one buffer while the other is filled
+    next_staging_ ^= 1;
+    RB_WINDOW_CUDA(cudaEventSynchronize((cudaEvent_t)staging_ev_[k]));
+    std::memcpy(staging_[k], data, len);
+    src = staging_[k];
+  }
+  RB_WINDOW_CUDA(cudaMemcpyAsync((uint8_t*)buf_.ptr + (end_ - base_), src, len, cudaMemcpyHostToDevice, up));
+  if (!pinned) RB_WINDOW_CUDA(cudaEventRecord((cudaEvent_t)staging_ev_[k], up));
+  cudaEvent_t ev;
+  if (!free_events_.empty()) {
+    ev = (cudaEvent_t)free_events_.back();
+    free_events_.pop_back();
+  } else {
+    RB_WINDOW_CUDA(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
+  }
+  end_ += len;
+  uploads_.push_back({end_, ev});
+  RB_WINDOW_CUDA(cudaEventRecord(ev, up));
+  return 0;
+}
+
+int StreamWindow::wait_uploads(uint64_t upto, std::string* err) {
+  size_t i = 0;
+  while (i < uploads_.size() && uploads_[i].first < upto) i++;
+  if (i == uploads_.size()) {
+    if (i == 0) return 0;
+    i--;
+  }
+  // uploads are ordered on the copy stream: waiting for the one that ends at or after upto covers those before it
+  RB_WINDOW_CUDA(cudaStreamWaitEvent((cudaStream_t)re_->stream_, (cudaEvent_t)uploads_[i].second, 0));
+  for (size_t j = 0; j < i; j++) free_events_.push_back(uploads_[j].second);
+  uploads_.erase(uploads_.begin(), uploads_.begin() + i);
+  return 0;
+}
+
+// The move runs on the engine's stream after every upload, in steps of at most the distance moved so that no copy
+// overlaps itself; uploads into the freed room wait for it.
+int StreamWindow::make_room(uint64_t keep_from, uint64_t want, std::string* err) {
+  const uint64_t nb = std::max<uint64_t>(base_, keep_from >= 256 ? (keep_from - 256) & ~255ull : 0);
+  if (cap_ - (end_ - nb) < want) {
+    *err = "internal error: the stream window is full";
+    return -1;
+  }
+  if (nb == base_) return 0;
+  cudaStream_t st = (cudaStream_t)re_->stream_;
+  uint8_t* w = (uint8_t*)buf_.ptr;
+  const uint64_t len = end_ - nb, off = nb - base_;
+  if (int rc = wait_uploads(end_, err)) return rc;
+  for (uint64_t d = 0; d < len; d += off)
+    RB_WINDOW_CUDA(cudaMemcpyAsync(w + d, w + off + d, std::min(off, len - d), cudaMemcpyDeviceToDevice, st));
+  RB_WINDOW_CUDA(cudaEventRecord((cudaEvent_t)moved_ev_, st));
+  RB_WINDOW_CUDA(cudaStreamWaitEvent((cudaStream_t)re_->copy_stream_, (cudaEvent_t)moved_ev_, 0));
+  base_ = nb;
+  return 0;
+}
+#undef RB_WINDOW_CUDA
+
+// ---- find_iter streams ----
+Stream* Stream::create(Regex* re, uint64_t piece, uint64_t hold, bool spans, uint64_t start, std::string* err) {
+  std::lock_guard<std::recursive_mutex> lock(re->mu_);
+  std::unique_ptr<Stream> s(new Stream(re));
+  if (re->is_set_) {
+    *err = "find requires exactly one pattern (RegexSet cannot be used with find, exec.rs:510-512)";
+    return nullptr;
+  }
+  Regex::DeviceDfa* warm;  // picks the stream, creates the pinned scratch
+  if (re->init_device() || re->ensure(kFwdAnchoredLF, &warm)) {
+    *err = re->error_;
+    return nullptr;
+  }
+  s->piece_ = piece ? (piece + 255) & ~255ull : kStreamPieceDefault;
+  s->hold_ = hold ? (hold + 255) & ~255ull : s->piece_;
+  s->halo_ = std::min<uint64_t>(64 << 10, s->hold_);
+  s->granule_ = std::min(kStreamGranule, std::max<uint64_t>(256, s->piece_ / 2));
+  // left context + the pending pieces + the next piece + its longest halo + the uploads in flight
+  const uint64_t cap = 4096 + (kMaxPending + 1) * s->piece_ + s->hold_ + 2 * s->granule_;
+  s->spans_ = spans;
+  s->next_lo_ = shard_own_lo(start);
+  s->chain_p_ = start;
+  s->chain_lm_ = kNone;
+  if (s->win_.init(re, cap, s->granule_, buf_lo(start), err)) return nullptr;
+  return s.release();
+}
+
+Stream::~Stream() = default;
 
 int Stream::fail(const std::string& msg) {
   error_ = msg;
@@ -2966,20 +3094,18 @@ int Stream::write(const uint8_t* data, uint64_t len) {
   if (failed_) return -1;
   if (finished_) return fail("write after finish: the stream's text has ended");
   if (re_->init_device()) return fail(re_->error_);
-  cudaPointerAttributes attr;
-  const bool pinned = len && cudaPointerGetAttributes(&attr, data) == cudaSuccess && attr.type == cudaMemoryTypeHost;
-  cudaGetLastError();  // a pageable pointer is not an error
+  const bool pinned = StreamWindow::pinned(data, len);
   bool progressed;
   while (len && !done_) {
     const uint64_t want = std::min(len, granule_);
-    if (cap_ - (end_ - base_) < want) {
+    if (win_.room() < want) {
       do {
         if (int rc = step(&progressed)) return rc;
       } while (progressed);
-      if (int rc = make_room(want)) return rc;
+      if (win_.make_room(n_pend_ ? pend_[0].lo : next_lo_, want, &error_)) return fail(error_);
     }
-    const uint64_t k = std::min(want, cap_ - (end_ - base_));
-    if (int rc = upload(data, k, pinned)) return rc;
+    const uint64_t k = std::min(want, win_.room());
+    if (win_.upload(data, k, pinned, &error_)) return fail(error_);
     data += k;
     len -= k;
   }
@@ -3020,83 +3146,25 @@ uint64_t Stream::read(uint64_t* out, uint64_t cap) {
   return k;
 }
 
-int Stream::upload(const uint8_t* data, uint64_t len, bool pinned) {
-  cudaStream_t up = (cudaStream_t)re_->copy_stream_;
-  const uint8_t* src = data;
-  int k = next_staging_;
-  if (!pinned) {  // through pinned staging: the copy engine reads one buffer while the other is filled
-    next_staging_ ^= 1;
-    RB_STREAM_CUDA(cudaEventSynchronize((cudaEvent_t)staging_ev_[k]));
-    std::memcpy(staging_[k], data, len);
-    src = staging_[k];
-  }
-  RB_STREAM_CUDA(cudaMemcpyAsync((uint8_t*)win_.ptr + (end_ - base_), src, len, cudaMemcpyHostToDevice, up));
-  if (!pinned) RB_STREAM_CUDA(cudaEventRecord((cudaEvent_t)staging_ev_[k], up));
-  cudaEvent_t ev;
-  if (!free_events_.empty()) {
-    ev = (cudaEvent_t)free_events_.back();
-    free_events_.pop_back();
-  } else {
-    RB_STREAM_CUDA(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
-  }
-  end_ += len;
-  uploads_.push_back({end_, ev});
-  RB_STREAM_CUDA(cudaEventRecord(ev, up));
-  return 0;
-}
-
-int Stream::wait_uploads(uint64_t upto) {
-  size_t i = 0;
-  while (i < uploads_.size() && uploads_[i].first < upto) i++;
-  if (i == uploads_.size()) {
-    if (i == 0) return 0;
-    i--;
-  }
-  // uploads are ordered on the copy stream: waiting for the one that ends at or after upto covers those before it
-  RB_STREAM_CUDA(cudaStreamWaitEvent((cudaStream_t)re_->stream_, (cudaEvent_t)uploads_[i].second, 0));
-  for (size_t j = 0; j < i; j++) free_events_.push_back(uploads_[j].second);
-  uploads_.erase(uploads_.begin(), uploads_.begin() + i);
-  return 0;
-}
-
-// Drop the bytes no search reads again (left of the pending piece's 256 bytes of context) by moving the rest to the
-// front of the window.  The move runs on the engine's stream after every upload, in steps of at most the distance
-// moved so that no copy overlaps itself; uploads into the freed room wait for it.
-int Stream::make_room(uint64_t want) {
-  const uint64_t keep = n_pend_ ? pend_[0].lo : next_lo_;
-  const uint64_t nb = std::max(base_, keep >= 256 ? keep - 256 : 0);
-  if (cap_ - (end_ - nb) < want) return fail("internal error: the stream window is full");
-  if (nb == base_) return 0;
-  cudaStream_t st = (cudaStream_t)re_->stream_;
-  uint8_t* w = (uint8_t*)win_.ptr;
-  const uint64_t len = end_ - nb, off = nb - base_;
-  if (int rc = wait_uploads(end_)) return rc;
-  for (uint64_t d = 0; d < len; d += off)
-    RB_STREAM_CUDA(cudaMemcpyAsync(w + d, w + off + d, std::min(off, len - d), cudaMemcpyDeviceToDevice, st));
-  RB_STREAM_CUDA(cudaEventRecord((cudaEvent_t)moved_ev_, st));
-  RB_STREAM_CUDA(cudaStreamWaitEvent((cudaStream_t)re_->copy_stream_, (cudaEvent_t)moved_ev_, 0));
-  base_ = nb;
-  return 0;
-}
-
 // One find_all_shard_device call over the window for piece p (p->lo, hi, entry_*, buf in).  Returns 1 when a match
 // runs past the bytes that have arrived: the halo has grown, search again once they are there.
 int Stream::search(Piece* p, uint32_t rev_entry) {
-  const uint64_t n_end = finished_ ? end_ : std::min(end_, p->hi + halo_);
-  if (int rc = wait_uploads(n_end)) return rc;
+  const uint64_t base = win_.base(), end = win_.end();
+  const uint64_t n_end = finished_ ? end : std::min(end, p->hi + halo_);
+  if (win_.wait_uploads(n_end, &error_)) return fail(error_);
   ShardIO io;
-  io.own_lo = p->lo - base_;
-  io.own_hi = p->hi - base_;
-  io.is_first = base_ == 0;
-  io.is_last = finished_ && n_end == end_;
+  io.own_lo = p->lo - base;
+  io.own_hi = p->hi - base;
+  io.is_first = base == 0;
+  io.is_last = finished_ && n_end == end;
   io.rev_entry = rev_entry;
-  if (p->entry_p < base_) {  // the iterator stands left of the window: enter at its first byte (sharded.py)
+  if (p->entry_p < base) {  // the iterator stands left of the window: enter at its first byte (sharded.py)
     io.chain_p = 0;
     io.chain_lm = kNone;
     io.chain_clamped = true;
   } else {
-    io.chain_p = p->entry_p - base_;
-    io.chain_lm = p->entry_lm == kNone || p->entry_lm < base_ ? kNone : p->entry_lm - base_;
+    io.chain_p = p->entry_p - base;
+    io.chain_lm = p->entry_lm == kNone || p->entry_lm < base ? kNone : p->entry_lm - base;
   }
   p->has_spans = spans_ && !(sink_ && emitted_ >= sink_cap_);
   DeviceBuf& buf = dspan_[p->buf];
@@ -3104,7 +3172,7 @@ int Stream::search(Piece* p, uint32_t rev_entry) {
   for (;;) {
     uint64_t* d_out = p->has_spans ? (uint64_t*)buf.ptr : nullptr;
     const uint64_t cap = p->has_spans ? buf.cap / 16 : 0;
-    if (re_->find_all_shard_device((const uint8_t*)win_.ptr, n_end - base_, &io, d_out, cap)) {
+    if (re_->find_all_shard_device(win_.ptr(), n_end - base, &io, d_out, cap)) {
       if (io.halo_overflow && !io.is_last) {
         if (n_end - p->hi >= hold_)
           return fail("a match is longer than the stream window (" + std::to_string(hold_) + " bytes): enlarge hold");
@@ -3112,7 +3180,7 @@ int Stream::search(Piece* p, uint32_t rev_entry) {
         return 1;
       }
       if (io.left_ctx_short)
-        return fail("a look-around pattern needs text left of the stream window (" + std::to_string(p->lo - base_) +
+        return fail("a look-around pattern needs text left of the stream window (" + std::to_string(p->lo - base) +
                     " bytes of left context): the iterator stands further back than the window keeps");
       return fail(re_->error_);
     }
@@ -3122,11 +3190,11 @@ int Stream::search(Piece* p, uint32_t rev_entry) {
   }
   if (p->has_spans && io.n_matches) {
     cudaStream_t st = (cudaStream_t)re_->stream_;
-    add_to_words<<<grid_for(2 * io.n_matches, 256, 4), 256, 0, st>>>((uint64_t*)buf.ptr, 2 * io.n_matches, base_);
+    add_to_words<<<grid_for(2 * io.n_matches, 256, 4), 256, 0, st>>>((uint64_t*)buf.ptr, 2 * io.n_matches, base);
     g_launches++;
     RB_STREAM_CUDA(cudaGetLastError());
   }
-  auto to_stream = [&](uint64_t v) { return v == kNone || v == kSpec ? v : v + base_; };
+  auto to_stream = [&](uint64_t v) { return v == kNone || v == kSpec ? v : v + base; };
   p->n = io.n_matches;
   p->rev_guess = io.rev_guess;
   p->rev_left = io.rev_left;
@@ -3141,9 +3209,10 @@ int Stream::step(bool* progressed) {
   Piece p;
   p.lo = next_lo_;
   p.hi = next_lo_ + piece_;
-  if (finished_) p.hi = std::min(p.hi, end_);
-  else if (end_ < p.hi + halo_) return 0;  // its bytes and halo have not all arrived
-  const bool last = finished_ && p.hi == end_;
+  const uint64_t end = win_.end();
+  if (finished_) p.hi = std::min(p.hi, end);
+  else if (end < p.hi + halo_) return 0;  // its bytes and halo have not all arrived
+  const bool last = finished_ && p.hi == end;
   p.entry_p = chain_p_;
   p.entry_lm = chain_lm_;
   bool used[kMaxPending + 2] = {};
@@ -3227,6 +3296,193 @@ int Stream::emit(const Piece& p) {
   return 0;
 }
 #undef RB_STREAM_CUDA
+
+// ---- forward streams: is_match / shortest_match / RegexSet matches ----
+// Each piece is one forward_step (DFA) or one cand_shortest launch (candidate starts) on the window.  Pieces after the
+// first begin on multiples of 256; a DFA piece is searched once it and the 64 bytes after it have arrived (what
+// forward_reduce's lazy upload brings), a candidate-start piece once look_ bytes after it have.
+MatchStream* MatchStream::create(Regex* re, uint64_t piece, uint64_t hold, bool want_masks, uint64_t start, std::string* err) {
+  std::lock_guard<std::recursive_mutex> lock(re->mu_);
+  std::unique_ptr<MatchStream> s(new MatchStream(re));
+  if (re->init_device()) {
+    *err = re->error_;
+    return nullptr;
+  }
+  s->piece_ = piece ? (piece + 255) & ~255ull : kStreamPieceDefault;
+  s->hold_ = hold ? (hold + 255) & ~255ull : s->piece_;
+  s->look_ = std::min<uint64_t>(64 << 10, s->hold_);
+  s->want_masks_ = want_masks && re->is_set_;
+  s->cand_ = re->candidate_mode();
+  s->next_lo_ = start;
+  s->res_.assign(re->result_words(), 0);
+  s->res_[0] = kNone;
+  if (!s->cand_) {
+    re->forward_tabs(&s->tabs_, &s->firsts_);
+    s->entries_.assign(s->tabs_.size(), kNoEntry);
+    s->done_.assign(s->tabs_.size(), 0);
+  }
+  s->decided_ = re->patterns_.empty();  // an empty set matches nothing
+  const uint64_t granule = std::min(kStreamGranule, std::max<uint64_t>(256, s->piece_ / 2));
+  // left context + the piece + the bytes after it (the look-ahead, at most hold) + the uploads in flight
+  const uint64_t cap = 4096 + s->piece_ + s->hold_ + 2 * granule;
+  if (s->win_.init(re, cap, granule, Stream::buf_lo(start), err)) return nullptr;
+  return s.release();
+}
+
+MatchStream::~MatchStream() = default;
+
+int MatchStream::fail(const std::string& msg) {
+  error_ = msg;
+  failed_ = true;
+  return -1;
+}
+
+bool MatchStream::found() const {
+  bool any = res_[0] != kNone;
+  for (size_t w = 1; w < res_.size(); w++) any = any || res_[w];
+  return any;
+}
+
+int MatchStream::write(const uint8_t* data, uint64_t len) {
+  std::lock_guard<std::recursive_mutex> lock(re_->mu_);
+  if (failed_) return -1;
+  if (finished_) return fail("write after finish: the stream's text has ended");
+  if (decided_) return 0;
+  if (re_->init_device()) return fail(re_->error_);
+  const bool pinned = StreamWindow::pinned(data, len);
+  bool progressed;
+  while (len && !decided_) {
+    const uint64_t want = std::min(len, win_.granule());
+    if (win_.room() < want) {
+      do {
+        if (int rc = step(&progressed)) return rc;
+      } while (progressed);
+      if (decided_) break;
+      if (win_.make_room(next_lo_, want, &error_)) return fail(error_);
+    }
+    const uint64_t k = std::min(want, win_.room());
+    if (win_.upload(data, k, pinned, &error_)) return fail(error_);
+    data += k;
+    len -= k;
+  }
+  do {
+    if (int rc = step(&progressed)) return rc;
+  } while (progressed);
+  // the caller may reuse its buffer once write returns: uploads straight from it must have landed
+  if (pinned && cudaStreamSynchronize((cudaStream_t)re_->copy_stream_) != cudaSuccess) return fail("CUDA error in the stream upload");
+  return 0;
+}
+
+int MatchStream::finish() {
+  std::lock_guard<std::recursive_mutex> lock(re_->mu_);
+  if (failed_) return -1;
+  if (finished_) return 0;
+  if (re_->init_device()) return fail(re_->error_);
+  finished_ = true;
+  while (!decided_) {
+    bool progressed;
+    if (int rc = step(&progressed)) return rc;
+    if (!progressed) return fail("internal error: the stream cannot search its last piece");
+  }
+  if (cudaStreamSynchronize((cudaStream_t)re_->stream_) != cudaSuccess) return fail("CUDA error at the end of the stream");
+  return 0;
+}
+
+int MatchStream::step(bool* progressed) {
+  *progressed = false;
+  if (decided_) return 0;
+  const uint64_t end = win_.end();
+  uint64_t hi = (next_lo_ & ~255ull) + piece_;
+  if (finished_) hi = std::min(hi, end);
+  else if (end < hi + (cand_ ? look_ : 64)) return 0;  // its bytes and the look-ahead have not all arrived
+  const bool last = finished_ && hi == end;
+  *progressed = true;
+  bool advanced = true;
+  if (int rc = cand_ ? search_cand(hi, last, &advanced) : search_dfa(hi, last)) return rc;
+  if (!advanced) return 0;  // the look-ahead grew: search the piece again once its bytes are there
+  next_lo_ = hi;
+  re_->stats.waves = ++pieces_;
+  decided_ = decided_ || last;
+  return 0;
+}
+
+int MatchStream::search_dfa(uint64_t hi, bool last) {
+  const uint64_t base = win_.base();
+  const uint64_t n_end = finished_ ? win_.end() : hi + 64;
+  if (win_.wait_uploads(n_end, &error_)) return fail(error_);
+  const uint64_t n = n_end - base;
+  std::vector<uint64_t> r(res_.size(), 0);
+  r[0] = kNone;
+  bool live;
+  if (re_->forward_step(tabs_, firsts_, win_.ptr(), n, next_lo_ - base, last ? n + 1 : hi - base, want_masks_, &entries_, &done_, r.data(), &live))
+    return fail(re_->error_);
+  if (r[0] != kNone) res_[0] = std::min(res_[0], r[0] + base);
+  for (size_t w = 1; w < r.size(); w++) res_[w] |= r[w];
+  re_->stats.groups = (uint32_t)tabs_.size();
+  if (want_masks_) {  // every pattern has matched, or no automaton is open (dead, or all its patterns matched)
+    re_->retire_matched(firsts_, res_.data(), &done_);
+    bool all = true;
+    for (size_t i = 0; i < re_->patterns_.size() && all; i++) all = (res_[1 + i / 64] >> (i % 64)) & 1;
+    decided_ = all || std::find(done_.begin(), done_.end(), 0) == done_.end();
+  } else {  // a first match end: no later piece has an earlier one
+    decided_ = !live || res_[0] != kNone;
+  }
+  return 0;
+}
+
+int MatchStream::search_cand(uint64_t hi, bool last, bool* advanced) {
+  const uint64_t base = win_.base();
+  const uint64_t n_end = finished_ ? win_.end() : hi + look_;
+  if (win_.wait_uploads(n_end, &error_)) return fail(error_);
+  const uint64_t n = n_end - base;
+  cudaStream_t st = (cudaStream_t)re_->stream_;
+  unsigned long long* best = &re_->d_scalars_->cand_best;
+  uint32_t* overflow = &re_->d_scalars_->cand_overflow;
+  // a bound found in an earlier piece past its end: candidates in [next_lo_, bound) may still end before it
+  const uint64_t seed = res_[0] == kNone ? kNone : res_[0] - base;
+  if (cudaMemcpyAsync(best, &seed, 8, cudaMemcpyHostToDevice, st) != cudaSuccess || cudaMemsetAsync(overflow, 0, 4, st) != cudaSuccess)
+    return fail("CUDA error in the stream's candidate search");
+  if (re_->cand_shortest_range(win_.ptr(), n, next_lo_ - base, last ? n + 1 : hi - base, !finished_, best, overflow)) return fail(re_->error_);
+  uint64_t b = kNone;
+  uint32_t o = 0;
+  if (re_->d2h(&b, best, 8) || re_->d2h(&o, overflow, 4)) return fail("CUDA error in the stream's candidate search");
+  if (o && b == kNone) {
+    // a run reached the end of the window undecided: read further past the piece, up to hold bytes
+    if (look_ >= hold_) return fail("a match is longer than the stream window (" + std::to_string(hold_) + " bytes): enlarge hold");
+    look_ = std::min(hold_, look_ * 8);
+    *advanced = false;
+    return 0;
+  }
+  if (b != kNone) res_[0] = b + base;
+  decided_ = res_[0] != kNone && res_[0] <= hi;  // every later candidate, and so its end, lies at or after hi
+  return 0;
+}
+
+bool Regex::use_match_window(uint64_t n) {
+  if (tuning.host_window) return n > tuning.host_window;
+  if (text_.ensure(n + 64)) return false;  // the buffer the resident path takes anyway
+  cudaGetLastError();  // the failed allocation is not an error of a later call
+  return true;
+}
+
+// shortest_match_host / set_matches_host through a MatchStream: the text goes up piece by piece and stops at the
+// piece that decides the answer.
+int Regex::match_window(const uint8_t* text, uint64_t n, uint64_t start, bool want_masks, bool* found, uint64_t* end, uint64_t* masks) {
+  *found = false;
+  if (start > n) return 0;
+  const uint64_t w = tuning.host_window;
+  const uint64_t piece = w ? std::max<uint64_t>(256, w / 8 / 256 * 256) : kStreamPieceDefault;
+  std::string err;
+  std::unique_ptr<MatchStream> s(MatchStream::create(this, piece, w ? piece : 4 * kStreamPieceDefault, want_masks, start, &err));
+  if (!s) return fail(err);
+  const uint64_t lo = Stream::buf_lo(start);
+  if (s->write(text + lo, n - lo) || s->finish()) return fail(s->error());
+  *found = s->found();
+  if (*found && end) *end = s->end();
+  if (masks)
+    for (uint32_t i = 0; i < (patterns_.size() + 63) / 64; i++) masks[i] = s->mask()[i];
+  return 0;
+}
 
 bool Regex::use_window(uint64_t n, uint64_t cap) {
   if (tuning.host_window) return n > tuning.host_window;

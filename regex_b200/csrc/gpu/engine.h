@@ -52,8 +52,9 @@ struct Tuning {
   uint32_t max_stitch_rounds = 16;  // re-walk rounds before the stitch falls back to one sequential pass
   uint32_t max_redo_rounds = 3;     // scan redo rounds before segment entry states are solved by state-map composition
   bool candidate_starts = false;    // tests: search from candidate starts (as over-budget patterns do) even when the unanchored automata fit
-  uint64_t host_window = 0;         // find_all_host: device window in bytes (pieces of an eighth of it) for haystacks larger than it;
-                                    // 0 = automatic (a window only when the haystack, its bitmap and the spans cannot be allocated)
+  uint64_t host_window = 0;         // find_all_host, shortest_match_host, set_matches_host: device window in bytes (pieces of an
+                                    // eighth of it) for haystacks larger than it; 0 = automatic (a window only when the haystack,
+                                    // and for find_all its bitmap and the spans, cannot be allocated)
 };
 
 struct Stats {  // filled by the last single-haystack call (diagnostics, bench roofline)
@@ -96,6 +97,8 @@ class DeviceBuf {
 };
 
 class Stream;
+class StreamWindow;
+class MatchStream;
 
 class Regex {
  public:
@@ -220,6 +223,8 @@ class Regex {
 
  private:
   friend class Stream;
+  friend class StreamWindow;
+  friend class MatchStream;
   Regex() = default;
   struct DeviceDfa;
   int init_device();
@@ -282,6 +287,11 @@ class Regex {
   // start bitmap (scan_rev format) of the candidates at positions (base, limit], plus position 0 when base == 0
   int cand_starts(const uint8_t* d_text, uint64_t n, uint64_t base, uint64_t limit, bool text_continues);
   int cand_shortest(const uint8_t* d_text, uint64_t n, uint64_t start, bool* found, uint64_t* end);
+  // one cand_shortest launch over the candidates [lo, hi) with *best (device) as the bound; text_continues: the
+  // buffer ends before the text does, and a run that reaches n undecided sets *overflow (device) instead of taking
+  // the end-of-text step
+  int cand_shortest_range(const uint8_t* d_text, uint64_t n, uint64_t lo, uint64_t hi, bool text_continues, unsigned long long* best,
+                          uint32_t* overflow);
   // batched records from candidate starts: mode 0 is_match, 1 find, 2 / 3 find_iter count / write pass
   int cand_batch(int mode, const uint8_t* d_text, const uint64_t* d_offsets, uint64_t n_rec, uint32_t* d_bits, uint64_t* d_spans,
                  uint64_t* d_match_offsets, uint64_t cap);
@@ -292,6 +302,17 @@ class Regex {
                      uint32_t entry = 0xFFFFFFFFu, uint32_t* exit_out = nullptr);
   int forward_range(const uint8_t* d_text, uint64_t n, uint64_t start, uint64_t limit, uint32_t entry, bool want_masks,
                     uint64_t* result_host, uint32_t* exit_state);
+  // The automata of a forward search: this object (the product automaton), or one per pattern group, with the first
+  // pattern of each.
+  void forward_tabs(std::vector<Regex*>* tabs, std::vector<uint32_t>* firsts);
+  // Positions [lo, limit) for every automaton g of tabs not done[g], entered in entries[g]: entries[g] becomes its
+  // exit state, done[g] is set on the dead state 0, result_host (result_words()) takes the least first end and the
+  // OR of the masks (group-local bit j is pattern firsts[g] + j).  *live: some automaton is still open.
+  int forward_step(const std::vector<Regex*>& tabs, const std::vector<uint32_t>& firsts, const uint8_t* d_text, uint64_t n, uint64_t lo,
+                   uint64_t limit, bool want_masks, std::vector<uint32_t>* entries, std::vector<char>* done, uint64_t* result_host,
+                   bool* live);
+  // marks done every group all of whose patterns are set in result_host's mask
+  void retire_matched(const std::vector<uint32_t>& firsts, const uint64_t* result_host, std::vector<char>* done) const;
   int subset(const std::vector<uint32_t>& members, Regex** out);
   // Pattern groups: plan contiguous ranges of at most `chunk` patterns whose kind-2 automata fit the budget
   // (ranges over budget are halved); `plan` non-null compiles those ranges as given.
@@ -306,6 +327,10 @@ class Regex {
   // find_all_host through a bounded device window (Stream) for haystacks that do not fit the device
   bool use_window(uint64_t n, uint64_t cap);
   int find_all_window(const uint8_t* text, uint64_t n, uint64_t start, uint64_t* out, uint64_t cap, uint64_t* total);
+  // shortest_match_host / set_matches_host through a bounded device window (MatchStream) for haystacks that do not
+  // fit the device (or are longer than tuning.host_window)
+  bool use_match_window(uint64_t n);
+  int match_window(const uint8_t* text, uint64_t n, uint64_t start, bool want_masks, bool* found, uint64_t* end, uint64_t* masks);
   int find_all_host_pipelined(const uint8_t* text, uint64_t n, uint8_t* d, uint64_t* d_out, uint64_t* out, uint64_t cap, uint64_t* total);
   int side_streams();  // creates copy_stream_ and back_stream_ on first use
 
@@ -372,6 +397,38 @@ class Regex {
   std::vector<uint32_t> pf_words_; // PfArgs image (engine.cu)
 };
 
+// The device window of a stream (DESIGN.md §8): stream bytes [base(), end()) at ptr(), one contiguous buffer of cap
+// bytes.  Host bytes go up on the engine's copy stream, straight from pinned memory or through two pinned staging
+// buffers filled alternately; each upload records an event, and a search waits only for the uploads it reads.
+class StreamWindow {
+ public:
+  ~StreamWindow();
+  // cap: window bytes; granule: most bytes per upload; base: stream offset of the first byte written (256-aligned)
+  int init(Regex* re, uint64_t cap, uint64_t granule, uint64_t base, std::string* err);
+  const uint8_t* ptr() const { return (const uint8_t*)buf_.ptr; }
+  uint64_t base() const { return base_; }
+  uint64_t end() const { return end_; }
+  uint64_t room() const { return cap_ - (end_ - base_); }
+  uint64_t granule() const { return granule_; }
+  static bool pinned(const uint8_t* data, uint64_t len);
+  int upload(const uint8_t* data, uint64_t len, bool pinned, std::string* err);
+  int wait_uploads(uint64_t upto, std::string* err);  // the engine's stream waits until stream bytes [.., upto) have arrived
+  // Drop the bytes left of keep_from's 256 bytes of context (rounded down to 256) by moving the rest to the front;
+  // fails when want bytes still do not fit.
+  int make_room(uint64_t keep_from, uint64_t want, std::string* err);
+
+ private:
+  Regex* re_ = nullptr;
+  DeviceBuf buf_;
+  uint64_t cap_ = 0, granule_ = 0, base_ = 0, end_ = 0;
+  uint8_t* staging_[2] = {nullptr, nullptr};  // pinned, double-buffered
+  void* staging_ev_[2] = {nullptr, nullptr};
+  int next_staging_ = 0;
+  std::vector<std::pair<uint64_t, void*>> uploads_;  // (stream end offset, event) of uploads not yet waited for
+  std::vector<void*> free_events_;
+  void* moved_ev_ = nullptr;  // the last window move (uploads into the freed room wait for it)
+};
+
 // find_iter over text that arrives in pieces, through a bounded device window (DESIGN.md §8): the concatenation of
 // every write is the haystack, and the spans read back are find_all_host on that concatenation, as stream offsets.
 // The stream owns its window, upload staging and span buffers; each call locks the engine it searches with.
@@ -401,9 +458,6 @@ class Stream {
   explicit Stream(Regex* re) : re_(re) {}
   int fail(const std::string& msg);
   int cuda(int e, const char* what);
-  int upload(const uint8_t* data, uint64_t len, bool pinned);
-  int wait_uploads(uint64_t upto);  // the engine's stream waits until stream bytes [.., upto) have arrived
-  int make_room(uint64_t want);
   int search(Piece* p, uint32_t rev_entry);  // p->lo/hi/entry in, the rest out
   int step(bool* progressed);                // searches and settles the next piece when its bytes are there
   int settle();          // makes the edges between pending pieces agree (engine.cu)
@@ -411,10 +465,9 @@ class Stream {
   int emit(const Piece& p);
   Regex* re_;
   std::string error_;
-  uint64_t piece_ = 0, hold_ = 0, granule_ = 0, cap_ = 0, halo_ = 0;  // cap_: window bytes
+  uint64_t piece_ = 0, hold_ = 0, granule_ = 0, halo_ = 0;
   bool spans_ = true, finished_ = false, done_ = false, failed_ = false;
-  DeviceBuf win_;             // device window: stream bytes [base_, end_) at win_.ptr
-  uint64_t base_ = 0, end_ = 0;
+  StreamWindow win_;
   uint64_t next_lo_ = 0, chain_p_ = 0, chain_lm_ = 0;  // next piece to search, iterator state entering it
   static constexpr int kMaxPending = 4;  // pieces kept waiting for a reverse-scan edge to agree
   Piece pend_[kMaxPending + 1];          // searched, not final yet, left to right
@@ -422,17 +475,52 @@ class Stream {
   bool emitted_any_ = false;
   uint32_t emitted_guess_ = 0;           // rev_guess of the last emitted piece
   DeviceBuf dspan_[kMaxPending + 2];     // spans of the pending pieces and of the one being searched (stream offsets)
-  uint8_t* staging_[2] = {nullptr, nullptr};  // pinned, double-buffered
-  void* staging_ev_[2] = {nullptr, nullptr};
-  int next_staging_ = 0;
-  std::vector<std::pair<uint64_t, void*>> uploads_;  // (stream end offset, event) of uploads not yet waited for
-  std::vector<void*> free_events_;
-  void* moved_ev_ = nullptr;  // the last window move (uploads into the freed room wait for it)
   uint64_t emitted_ = 0;
   std::vector<uint64_t> queue_;  // final spans not read yet, from queue_head_
   uint64_t queue_head_ = 0;
   uint64_t* sink_ = nullptr;
   uint64_t sink_cap_ = 0;
+};
+
+// is_match / shortest_match (a Regex) and RegexSet is_match / matches (a set) over text that arrives in pieces,
+// through a bounded device window (DESIGN.md §8): the answers are those of shortest_match_host / set_matches_host on
+// the concatenation of every write.  The automaton state flows left to right, so each piece is entered in the exact
+// exit state of the piece before it; only the last piece after finish takes the end-of-text step.
+class MatchStream {
+ public:
+  // piece, hold: as Stream (hold only bounds the look-ahead of candidate-start patterns); want_masks: a set reports
+  // which patterns match.  start: the search begins there (the first byte written is at Stream::buf_lo(start)).
+  static MatchStream* create(Regex* re, uint64_t piece, uint64_t hold, bool want_masks, uint64_t start, std::string* err);
+  ~MatchStream();
+  int write(const uint8_t* data, uint64_t len);  // copies; does nothing once decided
+  int finish();
+  // decided: nothing written later changes found, end or the mask; end: least match end (stream offset), kNone when
+  // none; searched: stream offset up to which positions have been searched; mask: result_words() - 1 words
+  bool decided() const { return decided_; }
+  bool found() const;
+  uint64_t end() const { return res_[0]; }
+  uint64_t searched() const { return next_lo_; }
+  const uint64_t* mask() const { return res_.data() + 1; }
+  const std::string& error() const { return error_; }
+
+ private:
+  explicit MatchStream(Regex* re) : re_(re) {}
+  int fail(const std::string& msg);
+  int step(bool* progressed);  // searches the next piece when its bytes are there
+  int search_dfa(uint64_t hi, bool last);
+  int search_cand(uint64_t hi, bool last, bool* wait);
+  void decide();
+  Regex* re_;
+  std::string error_;
+  uint64_t piece_ = 0, hold_ = 0, look_ = 0;  // look_: bytes past a piece a candidate-start search reads (grows x8)
+  bool want_masks_ = false, cand_ = false, finished_ = false, decided_ = false, failed_ = false;
+  StreamWindow win_;
+  uint64_t next_lo_ = 0;              // next position to search (stream offset)
+  uint64_t pieces_ = 0;               // pieces searched (stats.waves)
+  std::vector<Regex*> tabs_;          // the automata (product, or one per pattern group)
+  std::vector<uint32_t> firsts_, entries_;
+  std::vector<char> done_;
+  std::vector<uint64_t> res_;         // least first end, then the OR of the masks
 };
 
 uint64_t kernel_launches();  // total kernels launched by this library in this process

@@ -489,10 +489,13 @@ __device__ __forceinline__ uint64_t anchored_end(const DfaView& d, const Table& 
 
 // First position at which the automaton, started at s with the flags there, enters a match state (the
 // shortest_match_at end, exec.rs:382-468); kNone when it dies first or reaches `bound`.
+// halo_err: non-null when the text continues past n (a stream's window): a run that reaches n undecided sets it and
+// returns kNone instead of taking the end-of-text step.
 __device__ __forceinline__ uint64_t earliest_end(const DfaView& d, const Table& T, const uint8_t* text, uint64_t n, uint64_t s,
-                                                 uint64_t bound = kNone) {
+                                                 uint64_t bound = kNone, uint32_t* halo_err = nullptr) {
   uint32_t st = pick_start_fwd(d, text, n, s);
   for (uint64_t q = s; st != 0 && q < bound; q++) {
+    if (q >= n && halo_err) { *halo_err = 1; return kNone; }
     st = q < n ? T.step(st, __ldg(text + q)) : T.step_eof(st);
     if (st >= d.match_lo) return q;
     if (q >= n) break;
@@ -3132,7 +3135,7 @@ __global__ void cand_bitmap(const uint8_t* text, uint64_t n, uint64_t base, uint
 // each of its candidates s below the best end known so far and stops at the first match state (before the
 // first Match nothing is cut, so that is the earliest end of any match from s).
 __global__ void cand_shortest(DfaView fwd, int use_smem, CandArgs c, const uint8_t* text, uint64_t n, uint64_t lo, uint64_t hi,
-                              uint32_t seg, unsigned long long* best) {
+                              uint32_t seg, unsigned long long* best, int text_continues, uint32_t* overflow) {
   __shared__ uint8_t cm[256];
   for (uint32_t i = threadIdx.x; i < 256; i += blockDim.x) cm[i] = c.mask[i];
   __syncthreads();
@@ -3144,7 +3147,7 @@ __global__ void cand_shortest(DfaView fwd, int use_smem, CandArgs c, const uint8
     for (uint64_t s = s_lo; s < s_hi && s < b; s++) {
       if ((s & 255) == 0) b = min(b, (uint64_t)*(volatile unsigned long long*)best);
       if (!cand_at(cm, c.depth, text, n, s)) continue;
-      const uint64_t e = earliest_end(fwd, T, text, n, s, b);
+      const uint64_t e = earliest_end(fwd, T, text, n, s, b, text_continues ? overflow : nullptr);
       if (e != kNone) {
         b = e;
         atomicMin(best, (unsigned long long)e);

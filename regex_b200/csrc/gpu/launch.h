@@ -110,9 +110,10 @@ struct CandArgs {
 __global__ void cand_bitmap(const uint8_t* text, uint64_t n, uint64_t base, uint64_t limit, int text_continues, CandArgs c,
                             uint64_t* bitmap, uint8_t* flag0);
 // *best = min(*best, the first position where the anchored automaton, started at a candidate s in [lo, hi), enters a
-// match state); one lane per seg positions
+// match state); one lane per seg positions.  text_continues: the text goes on after n (a stream's window); a run that
+// reaches n undecided sets *overflow.
 __global__ void cand_shortest(DfaView fwd, int use_smem, CandArgs c, const uint8_t* text, uint64_t n, uint64_t lo, uint64_t hi,
-                              uint32_t seg, unsigned long long* best);
+                              uint32_t seg, unsigned long long* best, int text_continues, uint32_t* overflow);
 
 // ---- bulk operations over the span list (src/re_bytes.rs:316-360 split, :476-535 replacen) ----
 // The replacement of one match is a sequence of parts: literal bytes, or the text of a capture
